@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (B200, CUDA library)
     python bench.py --impl reference --steps K --warmup W    # CPU arm (C port of the reference's algorithm)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write what the timed steps computed to DIR/*.npy
 
 Workload (config.workload): BASELINE.json configs[3], the slalom cylinder field.  The 16384 x 16384 grid with
 100k agents is row-decomposed into bands of 2048 rows; one band (16384 x 2048 nodes, 12.5k agents, T = 2 s
@@ -234,6 +235,50 @@ def smooth_density(nx, rows, row0):
     return 0.5 * (1.0 + np.sin(2 * np.pi * x / 97.0)[None, :] * np.cos(2 * np.pi * y / 61.0)[:, None])
 
 
+DUMP_FIELD_BYTES, DUMP_AGENT_BYTES = 48 << 20, 8 << 20   # --dump-outputs: at most 56 MB of float64 in all
+
+
+def field_sample(opt):
+    """--dump-outputs: what a caller of compute_optimal_velocity reads after the solve, vx_opt / vy_opt (nt-1, Ny-2, Nx-2),
+    at the same fixed, seeded sample of nodes in every slice (the full field of the bench room is ~27 GB per component),
+    and the solve's step counts"""
+    import torch
+    n_sl = opt.nt_opt - 1
+    per = max(1, DUMP_FIELD_BYTES // (16 * max(n_sl, 1)))
+    rng = np.random.RandomState(20240)
+    ii = torch.from_numpy(rng.randint(0, opt.Ny - 2, per)).cuda()
+    jj = torch.from_numpy(rng.randint(0, opt.Nx - 2, per)).cuda()
+    vx = torch.empty((n_sl, per), dtype=torch.float64, device="cuda")
+    vy = torch.empty_like(vx)
+    for s in range(n_sl):   # slice s of vx_opt, as optimals.choose_optimal_velocity reads it
+        if opt.d_vx is not None:
+            sx, sy = opt.d_vx[s], opt.d_vy[s]
+        else:
+            sx, sy = opt._ctx.hjb_vels(opt.d_phi[opt.nt_opt - 1 - s], opt._prm)
+        vx[s], vy[s] = sx[ii, jj], sy[ii, jj]
+    st = opt.last_stats
+    return {"hjb_vx_opt_sample": vx.cpu().numpy(), "hjb_vy_opt_sample": vy.cpu().numpy(),
+            "hjb_nfev_accepted_rejected": np.array([st["nfev"], st["n_accepted"], st["n_rejected"]], dtype=np.float64)}
+
+
+def agent_sample(simu):
+    """--dump-outputs: the agents' state after simulation.advance() -- x, y, vx, vy, time, status and the step at which each
+    agent left (-1: still inside) -- all agents, or a fixed, seeded sample of them if that would exceed DUMP_AGENT_BYTES"""
+    idx = np.arange(simu.N)
+    if simu.N * 7 * 8 > DUMP_AGENT_BYTES:
+        idx = np.sort(np.random.RandomState(20241).choice(simu.N, DUMP_AGENT_BYTES // (7 * 8), replace=False))
+    now = simu._h_now[idx]
+    return {"gcfm_x": now[:, 0], "gcfm_y": now[:, 1], "gcfm_vx": now[:, 2], "gcfm_vy": now[:, 3],
+            "gcfm_time": simu._h_timev[idx], "gcfm_status": simu._h_status[idx].astype(np.float64),
+            "gcfm_exit_step": simu._exit_step[idx].astype(np.float64)}
+
+
+def write_dump(out_dir, arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def parity_block(world, rank, note):
     """untimed multi-GPU parity, through the same code path the timed region used (peer-memory step kernel):
     (1) HJB: a reduced room (2048 x 256 N nodes, smooth random density > 0, a wall straddling every band edge) solved by
@@ -388,6 +433,7 @@ def run_slalom(args, world, rank, local_rank):
     ms_max, step_ms_max = allmax([ev0.elapsed_time(ev1), cls_ms[0]])
     value = nfev_total * cells / (ms_max * 1e-3) / 1e9
     note(f"device-resident: {value:.2f} Gcu/s, {ms_max / K:.1f} ms/solve")
+    dump = field_sample(opt) if args.dump_outputs else None   # the field of the last timed solve, before e2e overwrites it
 
     # ---- end to end: host m -> H2D, solve, D2H of a scalar checksum of the t = 0 field slice ----------
     def checksum():
@@ -448,6 +494,10 @@ def run_slalom(args, world, rank, local_rank):
             pairs += simu._ctx.gcfm_last_pairs()
     barrier()
     g_wall, g_dev = allmax([time.perf_counter() - g0, dev_ms * 1e-3])
+    if dump is not None:
+        dump.update(agent_sample(simu))
+        write_dump(args.dump_outputs, dump)
+        note(f"outputs written to {args.dump_outputs}: {sorted(dump)}")
     pair_tflops = pairs * FP64_INST_PER_PAIR * 2.0 / g_dev / 1e12   # FMA-equivalent flops of the FP64-pipe instructions
     gcfm = {"metric": "gcfm_agent_steps_per_s", "value": agent_steps / g_dev, "unit": "agent-steps/s",
             "e2e_value": agent_steps / g_wall, "agents": simu.N, "steps": args.gcfm_steps,
@@ -558,7 +608,13 @@ def main():
     ap.add_argument("--field", default=os.environ.get("OC_FIELD", "phi"), choices=["phi", "velocity"],
                     help="field storage: phi samples (API default; sampler differentiates) or vx/vy slices")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed as DIR/<name>.npy (float64, <= 56 MB): a fixed, "
+                         "seeded sample of vx_opt / vy_opt of the last timed HJB solve, its step counts, and the agents' "
+                         "state after the timed GCFM steps (slalom workload on one GPU)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "slalom" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs supports the slalom workload of the CUDA library on one GPU")
     if args.impl == "reference":
         if args.T is None:
             args.T = T_DEFAULT
