@@ -155,6 +155,7 @@ int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, const oc_hjb
  * d_V[b], d_m[b] (d_m or entries nullable), d_phi[b] (nt,Ny,Nx), d_vx[b], d_vy[b] (nt-1,Ny-2,Nx-2): arrays of
  * n_rooms device pointers held in HOST memory; d_phi or (d_vx and d_vy) may be NULL.  stats: n_rooms entries.
  * prm->fused, forced_h and profile are ignored (always the stage-fused kernel, free-running controller).
+ * Without d_phi a step attempt may emit at most 6 t_eval samples (OC_ERR_ARG otherwise: pass d_phi for a dense t_eval).
  * Returns OC_ERR_STEP_TOO_SMALL if any room's integration stopped early (its stats.status == -1). */
 /* Chunk height (prm->chunk_rows) that balances halo recomputation against wave quantisation for `copies` rooms solved
  * side by side; the default of a single solve is oc_hjb_plan_chunk_rows(ctx, 1). */
@@ -172,7 +173,8 @@ int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const *d_V, const
  *  - virtual (cfg.n_virtual > 1, no communicator needed): one process emulates n_virtual bands on one GPU with
  *    device copies as the halo exchange; arrays are FULL-grid shaped as for oc_hjb_solve.  Used by the tests to
  *    show that the decomposition does not change a bit of the result (with prm.chunk_rows fixed).
- * Only the stage-fused path exists here (prm.fused is ignored).  Bands are equal and multiples of 16 rows. */
+ * Only the stage-fused path exists here (prm.fused is ignored).  Bands are equal and multiples of 16 rows.  Without
+ * d_phi an accepted step may emit at most 6 t_eval samples (OC_ERR_ARG otherwise). */
 typedef struct {
     int n_virtual;   /* > 1: virtual bands in one process; otherwise the communicator of oc_dist_init is used */
     int own0, own1;  /* distributed mode: global rows [own0, own1) of this rank (= rank*rows .. (rank+1)*rows) */

@@ -587,11 +587,15 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
             }
             const int n_emit = t_eval_i - ia_lo;
             const bool want_out = d_phi || (d_vx && d_vy);
-            fused_attempt = use_fused && (!want_out || n_emit <= fused::NE_MAX);
+            // more than NE_MAX samples: with a phi output the step is launched again for the remaining samples (as the
+            // batched and row-band solves do, so their results stay bit-identical); the NE_MAX scratch slices of a
+            // velocity-only solve cannot hold them, that attempt takes the stage-wise path
+            fused_attempt = use_fused && (!want_out || d_phi || n_emit <= fused::NE_MAX);
             double se;
             if (fused_attempt) {
-                // one launch: 6 RHS evaluations, y_new, f_new, error partial sums and the (speculative) dense
-                // output samples; a rejected attempt's samples are overwritten by the step that finally covers them
+                // one launch per NE_MAX samples: 6 RHS evaluations, y_new, f_new, error partial sums and the
+                // (speculative) dense output samples; a rejected attempt's samples are overwritten by the step that
+                // finally covers them.  A repeated launch recomputes identical y_new / f_new / error sums.
                 fused::Args fa{};
                 fa.y = s.y; fa.k1 = s.K[0]; fa.coef = s.coef; fa.ynew = s.ynew; fa.k7 = s.K[6]; fa.partial = s.partial;
                 fa.ha21 = h * RK_A[1][0];
@@ -604,9 +608,10 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
                 fa.A = s.diff_over_dxdy; fa.rtol = rtol; fa.atol = atol;
                 fa.Ny = s.Ny; fa.Nx = s.Nx; fa.RC = s.fused_rc;
                 fa.row_base = 0; fa.own0 = 0; fa.own1 = s.Ny; fa.phi_row_base = 0;
-                int ne = 0;
-                if (want_out) {
-                    for (int ia = t_eval_i - 1; ia >= ia_lo; ia--, ne++) {
+                int ia = want_out ? t_eval_i - 1 : ia_lo - 1;
+                do {
+                    int ne = 0;
+                    for (; ia >= ia_lo && ne < fused::NE_MAX; ia--, ne++) {
                         const int kd = nt - 1 - ia;
                         const double x = (t_eval[kd] - t) / h;  // RkDenseOutput: (t - t_old)/h
                         double pw[4] = {x, x * x, x * x * x, x * x * x * x};
@@ -617,9 +622,11 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
                         }
                         fa.phi[ne] = d_phi ? d_phi + (size_t)kd * n : phi_scratch + (size_t)ne * n;
                     }
-                }
-                if (final_in_kernel) final_reduce_args(ctx, 0, fa);
-                if ((rc = s.launch_fused(ne, fa))) return rc;
+                    // every launch finishes its own reduction (one ticket round, one sequence number); the same stream
+                    // orders them, the host waits for the last one's
+                    if (final_in_kernel) final_reduce_args(ctx, 0, fa);
+                    if ((rc = s.launch_fused(ne, fa))) return rc;
+                } while (ia >= ia_lo);
                 stats->nfev += 6;
                 if (final_in_kernel) {
                     if ((rc = wait_final(ctx, 0, fa.seq, s.st, &se))) return rc;
@@ -753,9 +760,9 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
 // ---------------------------------------------------------------------------------------------------
 // Batched solve for ensembles of independent rooms on one grid shape (BASELINE configs[4], SURVEY 8e).
 // Every room keeps its own RK45 controller (t, h, accept/reject, t_eval cursor: the reference integrates each
-// room separately, optimals.py:193-196) and its own CUDA stream; a room's step attempt is ONE launch of the
-// stage-fused kernel followed by the fixed-order reduction, exactly the launches oc_hjb_solve issues, so every
-// room's result is bit-identical to solving it alone (with the same prm->chunk_rows).  The host serves the rooms
+// room separately, optimals.py:193-196) and its own CUDA stream; a room's step attempt is one launch of the
+// stage-fused kernel per 6 samples followed by the fixed-order reduction, exactly the launches oc_hjb_solve issues, so
+// every room's result is bit-identical to solving it alone (with the same prm->chunk_rows).  The host serves the rooms
 // round-robin: while it reads room b's error norm and enqueues b's next attempt, the other rooms' kernels keep
 // the GPU busy -- small grids (512^2: ~10 us of device work per attempt) are launch-latency bound one at a time.
 namespace {
@@ -945,6 +952,14 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         // the samples this attempt emits if accepted, NE_MAX per launch; with more than NE_MAX samples inside one
         // step (only when h >> dt) the step is simply launched again for the remaining samples: the re-launch
         // recomputes identical y_new / f_new / error sums
+        if (!d_phi && r.t_eval_i - r.ia_lo > fused::NE_MAX) {
+            oc::set_error("batched solve without a phi output supports at most %d samples per step", fused::NE_MAX);
+            return OC_ERR_ARG;
+        }
+        // an attempt waits in an NE bucket only when ALL its samples fit one launch.  The launches of a longer attempt
+        // share the room's ticket counter and result slot, so they must not overlap: they go out in order on the
+        // room's own stream (the sequence OC_BATCH_PER_ROOM gives every attempt).
+        const bool to_bucket = batched && r.t_eval_i - r.ia_lo <= fused::NE_MAX;
         int ia = r.t_eval_i - 1;
         do {
             int ne = 0;
@@ -961,17 +976,13 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
                 fa.phi[ne] = d_phi ? r.phi + (size_t)kd * n : r.phi + (size_t)((r.t_eval_i - 1 - ia) % fused::NE_MAX) * n;
             }
             if (final_in_kernel) { final_reduce_args(ctx, (int)(&r - rooms.data()), fa); r.wait_seq = fa.seq; }
-            if (batched && ia < r.ia_lo) {  // all samples fit one launch (the rule): wait in the NE bucket
+            if (to_bucket) {
                 r.fa = fa;
                 buckets[ne].push_back(&r);
                 break;
             }
             int rc = s.launch_fused(ne, fa);
             if (rc) return rc;
-            if (!d_phi && ia >= r.ia_lo) {
-                oc::set_error("batched solve without a phi output supports at most %d samples per step", fused::NE_MAX);
-                return OC_ERR_ARG;
-            }
         } while (ia >= r.ia_lo);
         r.st.nfev += 6;
         if (!final_in_kernel) {
@@ -1095,11 +1106,22 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         if (!rc) rc = flush();  // one batched launch per NE class for everything that became ready in this sweep
         if (progressed) { idle = 0; continue; }
         if ((++idle & 0x3ffff) == 0) {  // nothing became ready for a long time: make sure no launch has failed
+            bool all_idle = true;
             for (int q = 0; q < n_streams && !rc; q++) {
                 cudaError_t e = cudaStreamQuery(ctx->batch_streams[q]);
-                if (e != cudaSuccess && e != cudaErrorNotReady) {
+                if (e == cudaErrorNotReady) all_idle = false;
+                else if (e != cudaSuccess) {
                     oc::set_error("batched HJB solve: %s", cudaGetErrorString(e));
                     cudaGetLastError();
+                    rc = OC_ERR_CUDA;
+                }
+            }
+            // every stream has drained, so every launched attempt has published its error sum (ocfinal::wait): a room
+            // still waiting after one more look never gets one -- an error instead of a host that spins for ever
+            for (int b = 0; b < n_rooms && !rc && all_idle && final_in_kernel; b++) {
+                BatchRoom &r = rooms[b];
+                if (r.phase == BatchRoom::STEP && !final_ready(ctx, b, r.wait_seq, &r.step_sum)) {
+                    oc::set_error("batched HJB solve: room %d: fused RK45 step did not deliver its error sum", b);
                     rc = OC_ERR_CUDA;
                 }
             }
