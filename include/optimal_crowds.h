@@ -305,10 +305,13 @@ int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, doub
  * (blockIdx.y = member) instead of 7 launches per member, and the members' per-step randomness drawn in C from their own
  * legacy MT19937 states (mt_key[m]: 624 words; mt_pos, has_gauss, cached_gauss: arrays of n = get_state()[2:5]; all
  * advanced in place) exactly as oc_rng_step_draw / the reference would.  Every member keeps its own context (workspace,
- * grid); all on one device.  Arrays are indexed by member: ctxs, prms, Ns, the SoA state pointers, keys / n_keys,
- * n_active (agents inside at step start) and simu_step.  sweep_ctas: CTAs of the sweep per member (0 = 8).
+ * grid); all on one device.  Members may differ in grid, crowd size, target sets, field storage (velocity or phi slices)
+ * and displacement margin.  Arrays are indexed by member: ctxs, prms, Ns, the SoA state pointers, keys / n_keys,
+ * n_active (agents inside at step start) and simu_step.  sweep_ctas: CTAs of the sweep per member (0 = 8).  The
+ * launch-wide knobs (gcfm_split, gcfm_overlap, gcfm_ws_pair) are read from ctxs[0].
  * _finish waits, returns every member's exit log (exit_log[m]: capacity Ns[m]) and status rc_out[m] (OC_OK or
- * OC_ERR_SAMPLER_RANGE as oc_gcfm_step); members whose fast attempt was void are redone on the exact slow path.
+ * OC_ERR_SAMPLER_RANGE as oc_gcfm_step); a member whose fast attempt was void is redone alone, after the batch, with
+ * the single-step kernels on its own context's settings (margin, knobs, gcfm_sweep_ctas), as oc_gcfm_step would.
  * Results are bit-identical to stepping every member with oc_gcfm_step. */
 int oc_gcfm_step_multi_launch(int n, oc_ctx *const *ctxs, const oc_gcfm_params *const *prms, const int *Ns,
                               double *const *x, double *const *y, double *const *vx, double *const *vy,

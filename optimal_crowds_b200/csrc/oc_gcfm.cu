@@ -1907,6 +1907,12 @@ extern "C" int oc_gcfm_step_multi_launch(int n, oc_ctx *const *ctxs, const oc_gc
         off[m + 1] = off[m] + (((size_t)Ns[m] * sizeof(int) + 7) / 8) * 8 + (size_t)2 * n_active[m] * sizeof(double);
         max_N = std::max(max_N, Ns[m]);
     }
+    // a void member attempt is redone in oc_gcfm_step_multi_finish with the single-step kernels: their shared-memory
+    // limits and the member's resident grids must be set even if this context never took a single step
+    for (int m = 0; m < n; m++) {
+        int rc = gcfm_device_setup(ctxs[m]);
+        if (rc) return rc;
+    }
     const size_t arena = off[n] + 64, rec_bytes = sizeof(GcfmMember) * (size_t)n;
     if (c0->multi_bytes < arena + rec_bytes) {
         if (c0->multi_pinned) cudaFreeHost(c0->multi_pinned);
