@@ -22,9 +22,9 @@ struct oc_ctx {
     double *hjb_scratch = nullptr;  // phi slices of the fused step when only velocities are stored
     size_t hjb_scratch_bytes = 0;
     double *hjb_partial = nullptr;  // per-tile error partial sums
-    size_t hjb_partial_n = 0;
+    size_t hjb_partial_bytes = 0;
     double *h_pinned = nullptr;  // pinned host scratch (row-group sums, flags)
-    size_t h_pinned_n = 0;
+    size_t h_pinned_bytes = 0;
     // GCFM workspace
     void *gcfm_ws = nullptr;
     size_t gcfm_ws_bytes = 0;
@@ -86,7 +86,7 @@ struct oc_ctx {
     double *batch_ws = nullptr;
     size_t batch_ws_bytes = 0;
     double *batch_pinned = nullptr;
-    size_t batch_pinned_n = 0;
+    size_t batch_pinned_bytes = 0;
     std::vector<cudaStream_t> batch_streams;
     std::vector<cudaEvent_t> batch_events;
 };
@@ -108,6 +108,26 @@ inline void count_launch(int n = 1) { g_launches.fetch_add(n, std::memory_order_
             return OC_ERR_CUDA;                                                                \
         }                                                                                      \
     } while (0)
+
+// Grows a reusable device buffer (or, with `pinned`, page-locked host buffer) to at least `need` bytes.  The old
+// buffer is released and forgotten before the new allocation, so after a failed one no freed buffer stays on record.
+template <typename T>
+inline int oc_ensure_buffer(T *&buf, size_t &bytes, size_t need, bool pinned, const char *what) {
+    if (bytes >= need) return OC_OK;
+    if (pinned) cudaFreeHost(buf);
+    else cudaFree(buf);
+    buf = nullptr;
+    bytes = 0;
+    void *p = nullptr;
+    if ((pinned ? cudaMallocHost(&p, need) : cudaMalloc(&p, need)) != cudaSuccess) {
+        cudaGetLastError();
+        oc::set_error("cannot allocate %zu bytes of %s", need, what);
+        return OC_ERR_NOMEM;
+    }
+    buf = (T *)p;
+    bytes = need;
+    return OC_OK;
+}
 
 #define OC_ARG(cond, msg)                  \
     do {                                   \

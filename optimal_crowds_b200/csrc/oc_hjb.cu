@@ -1,6 +1,8 @@
 // oc_hjb.cu -- HJB solve on sm_100a: RHS stencil (K1), RK45 stage kernels with the stage combination
-// fused into the stencil load (K2, stage-wise formulation), dense output + velocity epilogue (K3) and
-// the host-side replica of scipy's RK45 controller.
+// fused into the stencil load (K2, stage-wise formulation), dense output + velocity epilogue (K3), and the host
+// drivers of the single-room and batched solves.  Both drivers (and the row-band solve, oc_hjb_dist.cu) step
+// scipy's RK45 controller rk45::Controller (oc_rk45.h) and fill the fused step's per-attempt constants with
+// fused::set_attempt (oc_hjb_fused.cuh).
 //
 // Reference: optimals.py:124-206 (compute_optimal_velocity) + scipy 1.18.1 solve_ivp/RK45
 // (rk.py:14-71,85-180,538-565,715-737; common.py:63-134; ivp.py:604-621,659-728; base.py:179-210).
@@ -22,11 +24,6 @@
 #include "oc_vels.h"
 
 namespace {
-
-#define RK_A rk45::A
-#define RK_B rk45::B
-#define RK_E rk45::E
-#define RK_P rk45::P
 
 constexpr int TX = 128, TY = 16, NTHREADS = 256;  // stage tile
 constexpr int SW = TX + 2;                        // smem row pitch (doubles)
@@ -368,36 +365,18 @@ struct Solver {
 };
 
 int ensure_ws(oc_ctx *ctx, size_t n, int nbx, int nby) {
-    size_t need = 10 * n * sizeof(double);
-    if (ctx->hjb_ws_bytes < need) {
-        if (ctx->hjb_ws) cudaFree(ctx->hjb_ws);
-        ctx->hjb_ws = nullptr;
-        ctx->hjb_ws_bytes = 0;
-        if (cudaMalloc(&ctx->hjb_ws, need) != cudaSuccess) {
-            cudaGetLastError();
-            oc::set_error("cannot allocate %zu bytes of HJB workspace", need);
-            return OC_ERR_NOMEM;
-        }
-        ctx->hjb_ws_bytes = need;
-    }
+    int rc = oc_ensure_buffer(ctx->hjb_ws, ctx->hjb_ws_bytes, 10 * n * sizeof(double), false, "HJB workspace");
+    if (rc) return rc;
     // large enough for the stage tiles and for any fused-step plan (>= 32-row chunks, 240-column tiles)
     size_t np = (size_t)2 * nbx * nby + nby + 64;
     {
         size_t fgx = (size_t)(nbx * TX + fused::VX - 1) / fused::VX + 1, fgy = (size_t)(nby * TY + 15) / 16 + 1;
         np = std::max(np, 2 * fgx * fgy + fgy + 64);
     }
-    if (ctx->hjb_partial_n < np) {
-        if (ctx->hjb_partial) cudaFree(ctx->hjb_partial);
-        OC_CUDA(cudaMalloc(&ctx->hjb_partial, np * sizeof(double)));
-        ctx->hjb_partial_n = np;
-    }
+    if ((rc = oc_ensure_buffer(ctx->hjb_partial, ctx->hjb_partial_bytes, np * sizeof(double), false, "HJB partial sums")))
+        return rc;
     size_t hp = (size_t)std::max(nby, (nby * TY + 15) / 16 + 1) + 16;
-    if (ctx->h_pinned_n < hp) {
-        if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-        OC_CUDA(cudaMallocHost(&ctx->h_pinned, hp * sizeof(double)));
-        ctx->h_pinned_n = hp;
-    }
-    return OC_OK;
+    return oc_ensure_buffer(ctx->h_pinned, ctx->h_pinned_bytes, hp * sizeof(double), true, "pinned host scratch");
 }
 
 int ensure_final_reduce(oc_ctx *ctx, int slots) { return ocfinal::ensure(ctx, slots); }
@@ -479,14 +458,11 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
     const double sqrt_n = std::sqrt((double)n);
     memset(stats, 0, sizeof(*stats));
     s.profile = prm->profile != 0;
-    int ntr = 0;
     OC_CUDA(cudaEventRecord(ctx->ev0, s.st));
 
     prep_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s.st>>>(d_V, d_m, prm->g, 1.0 / (prm->mu * s2), n, s.coef, s.y);
     s.launches++;
-    const double t_bound = 0.0;
-    const double direction = (t_bound != T) ? (t_bound > T ? 1.0 : -1.0) : 1.0;
-    double t = T;
+    rk45::Controller ctl(T, t_eval, nt);
     // rk.py:94: f = fun(t0, y0)
     {
         Comb c{};
@@ -495,35 +471,25 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
         stats->nfev++;
     }
     // common.py:109-134 select_initial_step
-    double h_abs;
-    {
-        double interval = std::fabs(t_bound - T);
-        if (interval == 0.0) h_abs = 0.0;
-        else {
-            dim3 grid(s.nbx, s.nby);
-            init_norm_kernel<<<grid, NTHREADS, 0, s.st>>>(s.y, s.K[0], nullptr, rtol, atol, s.Ny, s.Nx, s.partial, 0);
-            s.launches++;
-            double s0, s1, sq2;
-            if ((rc = s.reduce_to_host(0, &s0))) return rc;
-            if ((rc = s.reduce_to_host((size_t)s.nbx * s.nby, &s1))) return rc;
-            double d0 = std::sqrt(s0) / sqrt_n, d1 = std::sqrt(s1) / sqrt_n;
-            double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-            h0 = std::min(h0, interval);
-            Comb c{};
-            c.y = s.y; c.k[0] = s.K[0]; c.a[0] = 1.0; c.h = h0 * direction;  // y1 = y0 + h0*direction*f0
-            s.stage(1, c, s.K[1]);
-            stats->nfev++;
-            init_norm_kernel<<<grid, NTHREADS, 0, s.st>>>(s.y, s.K[0], s.K[1], rtol, atol, s.Ny, s.Nx, s.partial, 1);
-            s.launches++;
-            if ((rc = s.reduce_to_host(0, &sq2))) return rc;
-            double d2 = std::sqrt(sq2) / sqrt_n / h0;
-            double h1;
-            if (d1 <= 1e-15 && d2 <= 1e-15) h1 = std::max(1e-6, h0 * 1e-3);
-            else h1 = std::pow(0.01 / std::max(d1, d2), 1.0 / 5.0);
-            h_abs = std::min(std::min(100 * h0, h1), interval);
-        }
+    if (ctl.needs_initial_step()) {
+        dim3 grid(s.nbx, s.nby);
+        init_norm_kernel<<<grid, NTHREADS, 0, s.st>>>(s.y, s.K[0], nullptr, rtol, atol, s.Ny, s.Nx, s.partial, 0);
+        s.launches++;
+        double s0, s1, sq2;
+        if ((rc = s.reduce_to_host(0, &s0))) return rc;
+        if ((rc = s.reduce_to_host((size_t)s.nbx * s.nby, &s1))) return rc;
+        const double d1 = std::sqrt(s1) / sqrt_n;
+        const double h0 = ctl.initial_h0(std::sqrt(s0) / sqrt_n, d1);
+        Comb c{};
+        c.y = s.y; c.k[0] = s.K[0]; c.a[0] = 1.0; c.h = h0 * ctl.direction;  // y1 = y0 + h0*direction*f0
+        s.stage(1, c, s.K[1]);
+        stats->nfev++;
+        init_norm_kernel<<<grid, NTHREADS, 0, s.st>>>(s.y, s.K[0], s.K[1], rtol, atol, s.Ny, s.Nx, s.partial, 1);
+        s.launches++;
+        if ((rc = s.reduce_to_host(0, &sq2))) return rc;
+        ctl.set_initial_step(h0, d1, std::sqrt(sq2) / sqrt_n / h0);
     }
-    stats->h0 = h_abs;
+    stats->h0 = ctl.h_abs;
 
     // stage-fused path (prm->fused): needs room for NE_MAX phi slices when only velocities are requested
     // the fused kernel mirrors up to 6 rows / 8 columns across the boundary: tiny grids take the stage-wise path
@@ -534,63 +500,29 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
         cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, ctx->device);
         s.fused_plan(n_sm, prm->chunk_rows);
         size_t np_need = (size_t)2 * s.fused_gx * s.fused_gy + s.fused_gy;
-        if (ctx->hjb_partial_n < np_need || ctx->h_pinned_n < (size_t)s.fused_gy + 16) {
+        if (ctx->hjb_partial_bytes < np_need * sizeof(double) || ctx->h_pinned_bytes < ((size_t)s.fused_gy + 16) * sizeof(double)) {
             oc::set_error("internal: fused partial buffers too small");
             return OC_ERR_ARG;
         }
         if (!d_phi && d_vx && d_vy) {
             size_t need = (size_t)fused::NE_MAX * n * sizeof(double);
-            if (ctx->hjb_scratch_bytes < need) {
-                if (ctx->hjb_scratch) cudaFree(ctx->hjb_scratch);
-                ctx->hjb_scratch = nullptr; ctx->hjb_scratch_bytes = 0;
-                if (cudaMalloc(&ctx->hjb_scratch, need) != cudaSuccess) {
-                    cudaGetLastError();
-                    oc::set_error("cannot allocate %zu bytes of phi scratch", need);
-                    return OC_ERR_NOMEM;
-                }
-                ctx->hjb_scratch_bytes = need;
-            }
+            if ((rc = oc_ensure_buffer(ctx->hjb_scratch, ctx->hjb_scratch_bytes, need, false, "phi scratch"))) return rc;
             phi_scratch = ctx->hjb_scratch;
         }
     }
-    int t_eval_i = nt;  // ivp.py:617-621
-    int n_out = 0, status = 1;
-    const double error_exponent = -1.0 / 5.0;
     const size_t n_int = (size_t)(s.Ny - 2) * (s.Nx - 2);
     const bool final_in_kernel = use_fused && s.fused_gy <= fused::MAX_FINAL_ROWS;
     if (final_in_kernel && (rc = ensure_final_reduce(ctx, 1))) return rc;
+    const bool want_out = d_phi || (d_vx && d_vy);
 
-    while (status == 1) {
-        if (t == t_bound) { status = 0; break; }  // base.py:193-198
-        double min_step = 10 * std::fabs(std::nextafter(t, direction * INFINITY) - t);
-        if (h_abs < min_step) h_abs = min_step;
-        bool accepted = false, rejected = false;
-        double h = 0, t_new = 0;
-        while (!accepted) {
-            if (h_abs < min_step) { status = -1; break; }
-            h = h_abs * direction;
-            if (prm->forced_h && ntr < prm->n_forced_h) h = prm->forced_h[ntr];  // teacher-forced (tests)
-            t_new = t + h;
-            if (direction * (t_new - t_bound) > 0) t_new = t_bound;
-            h = t_new - t;
-            h_abs = std::fabs(h);
-            // t_eval samples this attempt would emit if accepted (ivp.py:715-728): ascending indices
-            // [ia_lo, t_eval_i) with t_eval >= t_new
-            int ia_lo;
-            {
-                int lo = 0, hi = nt;
-                while (lo < hi) {
-                    int mid = (lo + hi) / 2;
-                    if (t_eval[nt - 1 - mid] < t_new) lo = mid + 1; else hi = mid;
-                }
-                ia_lo = std::min(lo, t_eval_i);
-            }
-            const int n_emit = t_eval_i - ia_lo;
-            const bool want_out = d_phi || (d_vx && d_vy);
+    while (ctl.begin_step()) {
+        bool accepted = false;
+        while (!accepted && ctl.propose(prm->forced_h, prm->n_forced_h)) {  // forced_h: teacher-forced (tests)
+            const double h = ctl.h;
             // more than NE_MAX samples: with a phi output the step is launched again for the remaining samples (as the
             // batched and row-band solves do, so their results stay bit-identical); the NE_MAX scratch slices of a
             // velocity-only solve cannot hold them, that attempt takes the stage-wise path
-            fused_attempt = use_fused && (!want_out || d_phi || n_emit <= fused::NE_MAX);
+            fused_attempt = use_fused && (!want_out || d_phi || ctl.n_emit() <= fused::NE_MAX);
             double se;
             if (fused_attempt) {
                 // one launch per NE_MAX samples: 6 RHS evaluations, y_new, f_new, error partial sums and the
@@ -598,35 +530,20 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
                 // finally covers them.  A repeated launch recomputes identical y_new / f_new / error sums.
                 fused::Args fa{};
                 fa.y = s.y; fa.k1 = s.K[0]; fa.coef = s.coef; fa.ynew = s.ynew; fa.k7 = s.K[6]; fa.partial = s.partial;
-                fa.ha21 = h * RK_A[1][0];
-                for (int j = 0; j < 2; j++) fa.ha3[j] = h * RK_A[2][j];
-                for (int j = 0; j < 3; j++) fa.ha4[j] = h * RK_A[3][j];
-                for (int j = 0; j < 4; j++) fa.ha5[j] = h * RK_A[4][j];
-                for (int j = 0; j < 5; j++) fa.ha6[j] = h * RK_A[5][j];
-                for (int j = 0; j < 6; j++) fa.hb[j] = h * RK_B[j];
-                for (int j = 0; j < 7; j++) fa.he[j] = h * RK_E[j];
                 fa.A = s.diff_over_dxdy; fa.rtol = rtol; fa.atol = atol;
                 fa.Ny = s.Ny; fa.Nx = s.Nx; fa.RC = s.fused_rc;
                 fa.row_base = 0; fa.own0 = 0; fa.own1 = s.Ny; fa.phi_row_base = 0;
-                int ia = want_out ? t_eval_i - 1 : ia_lo - 1;
+                const int n_emit = want_out ? ctl.n_emit() : 0;
+                int e0 = 0;
                 do {
-                    int ne = 0;
-                    for (; ia >= ia_lo && ne < fused::NE_MAX; ia--, ne++) {
-                        const int kd = nt - 1 - ia;
-                        const double x = (t_eval[kd] - t) / h;  // RkDenseOutput: (t - t_old)/h
-                        double pw[4] = {x, x * x, x * x * x, x * x * x * x};
-                        for (int j = 0; j < 7; j++) {
-                            double acc = 0.0;
-                            for (int q = 0; q < 4; q++) acc += RK_P[j][q] * pw[q];
-                            fa.w[ne][j] = h * acc;
-                        }
-                        fa.phi[ne] = d_phi ? d_phi + (size_t)kd * n : phi_scratch + (size_t)ne * n;
-                    }
+                    const int ne = std::min(n_emit - e0, fused::NE_MAX);
+                    fused::set_attempt(fa, ctl, e0, ne, d_phi, phi_scratch, n);
                     // every launch finishes its own reduction (one ticket round, one sequence number); the same stream
                     // orders them, the host waits for the last one's
                     if (final_in_kernel) final_reduce_args(ctx, 0, fa);
                     if ((rc = s.launch_fused(ne, fa))) return rc;
-                } while (ia >= ia_lo);
+                    e0 += ne;
+                } while (e0 < n_emit);
                 stats->nfev += 6;
                 if (final_in_kernel) {
                     if ((rc = wait_final(ctx, 0, fa.seq, s.st, &se))) return rc;
@@ -636,7 +553,7 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
             for (int sgi = 1; sgi < 6; sgi++) {
                 Comb c{};
                 c.y = s.y; c.h = h;
-                for (int j = 0; j < sgi; j++) { c.k[j] = s.K[j]; c.a[j] = RK_A[sgi][j]; }
+                for (int j = 0; j < sgi; j++) { c.k[j] = s.K[j]; c.a[j] = rk45::A[sgi][j]; }
                 s.stage(sgi, c, s.K[sgi]);
             }
             {
@@ -645,50 +562,29 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
                 c.y = s.y; c.h = h;
                 int m = 0;
                 for (int j = 0; j < 6; j++)
-                    if (j != 1) { c.k[m] = s.K[j]; c.a[m] = RK_B[j]; m++; }
+                    if (j != 1) { c.k[m] = s.K[j]; c.a[m] = rk45::B[j]; m++; }
                 ErrArgs ea{};
                 for (int j = 0; j < 6; j++) ea.k[j] = s.K[j];
-                for (int j = 0; j < 7; j++) ea.e[j] = RK_E[j];
+                for (int j = 0; j < 7; j++) ea.e[j] = rk45::E[j];
                 ea.h = h; ea.rtol = rtol; ea.atol = atol;
                 s.launch_stage<5, 1>(c, s.K[6], s.ynew, ea);
             }
             stats->nfev += 6;
             if ((rc = s.reduce_to_host(0, &se))) return rc;
             }
-            double error_norm = std::sqrt(se) / sqrt_n;  // rk.py:147, common.py:63-65
+            const double error_norm = std::sqrt(se) / sqrt_n;  // rk.py:147, common.py:63-65
+            const int ntr = ctl.attempts();
             if (trace_h && ntr < trace_cap) { trace_h[ntr] = h; trace_err[ntr] = error_norm; }
-            ntr++;
-            if (error_norm < 1) {  // rk.py:149-161
-                double factor = (error_norm == 0) ? 10.0 : std::min(10.0, 0.9 * std::pow(error_norm, error_exponent));
-                if (rejected) factor = std::min(1.0, factor);
-                h_abs *= factor;
-                accepted = true;
-                stats->n_accepted++;
-            } else {  // rk.py:162-165
-                h_abs *= std::max(0.2, 0.9 * std::pow(error_norm, error_exponent));
-                rejected = true;
-                stats->n_rejected++;
-            }
+            accepted = ctl.judge(error_norm);
         }
-        if (status == -1) break;
-        const double t_old = t;
-        if (direction * (t_new - t_bound) >= 0) status = 0;  // base.py:205-208
+        if (!accepted) break;  // step too small
 
-        // ivp.py:715-728, direction < 0: first ascending index with t_eval_asc >= t_new
-        int lo = 0, hi = nt;
-        while (lo < hi) {
-            int mid = (lo + hi) / 2;
-            if (t_eval[nt - 1 - mid] < t_new) lo = mid + 1; else hi = mid;
-        }
-        const int t_eval_i_new = lo;
         if (fused_attempt) {
             // samples were written by the step kernel; only the gradient-to-velocity conversion is left
-            int ne = 0;
-            for (int ia = t_eval_i - 1; ia >= t_eval_i_new; ia--, ne++) {
-                const int kd = nt - 1 - ia;
-                n_out++;
+            for (int e = 0; e < ctl.n_emit(); e++) {
+                const int kd = ctl.sample_column(e);
                 if (d_vx && d_vy && kd >= 1) {
-                    const double *ph = d_phi ? d_phi + (size_t)kd * n : phi_scratch + (size_t)ne * n;
+                    const double *ph = fused::sample_slice(ctl, e, d_phi, phi_scratch, n);
                     const int sl = nt - 1 - kd;
                     dim3 grid((s.Nx - 2 + 63) / 64, (s.Ny - 2 + 3) / 4);
                     s.begin(1, 8.0 * (double)n * 3);
@@ -698,43 +594,39 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
                     s.launches++;
                 }
             }
-            t_eval_i = t_eval_i_new;
-        } else if (t_eval_i_new < t_eval_i) {
-            const double hh = t_new - t_old;
-            int ia = t_eval_i - 1;
-            while (ia >= t_eval_i_new) {
+        } else {
+            int e = 0;
+            while (e < ctl.n_emit()) {
                 DenseArgs a{};
                 a.yold = s.y;
-                for (int j = 0; j < 7; j++) { a.k[j] = s.K[j]; for (int p = 0; p < 4; p++) a.P[j][p] = RK_P[j][p]; }
-                a.h = hh; a.mu = prm->mu; a.lim = prm->lim; a.inv_two_dx = 1.0 / (2 * ctx->dx); a.inv_two_dy = 1.0 / (2 * ctx->dy);
-                int e = 0;
+                for (int j = 0; j < 7; j++) { a.k[j] = s.K[j]; for (int p = 0; p < 4; p++) a.P[j][p] = rk45::P[j][p]; }
+                a.h = ctl.h; a.mu = prm->mu; a.lim = prm->lim; a.inv_two_dx = 1.0 / (2 * ctx->dx); a.inv_two_dy = 1.0 / (2 * ctx->dy);
+                int m = 0;
                 bool any = false;
-                for (; e < DMAX && ia >= t_eval_i_new; ia--) {
-                    int kd = nt - 1 - ia;  // column of sol.y
-                    a.x[e] = (t_eval[kd] - t_old) / hh;
-                    a.phi[e] = d_phi ? d_phi + (size_t)kd * n : nullptr;
+                for (; m < DMAX && e < ctl.n_emit(); e++) {
+                    int kd = ctl.sample_column(e);  // column of sol.y
+                    a.x[m] = ctl.sample_x(e);
+                    a.phi[m] = d_phi ? d_phi + (size_t)kd * n : nullptr;
                     int sl = nt - 1 - kd;  // vx_opt slice (optimals.py:200-204); column 0 (phi_T) has none
                     bool has_v = d_vx && d_vy && kd >= 1;
-                    a.vx[e] = has_v ? d_vx + (size_t)sl * n_int : nullptr;
-                    a.vy[e] = has_v ? d_vy + (size_t)sl * n_int : nullptr;
-                    if (a.phi[e] || a.vx[e]) { any = true; e++; }
-                    n_out++;
+                    a.vx[m] = has_v ? d_vx + (size_t)sl * n_int : nullptr;
+                    a.vy[m] = has_v ? d_vy + (size_t)sl * n_int : nullptr;
+                    if (a.phi[m] || a.vx[m]) { any = true; m++; }
                 }
-                a.n_emit = e;
+                a.n_emit = m;
                 if (any) {
                     dim3 grid((s.Nx + DTX - 1) / DTX, (s.Ny + DTY - 1) / DTY);
                     double words = 7.0;  // y_old + K[0], K[2..6]
-                    for (int q = 0; q < e; q++) words += (a.phi[q] ? 1.0 : 0.0) + (a.vx[q] ? 2.0 : 0.0);
+                    for (int q = 0; q < m; q++) words += (a.phi[q] ? 1.0 : 0.0) + (a.vx[q] ? 2.0 : 0.0);
                     s.begin(1, 8.0 * (double)n * words);
                     hjb_dense_kernel<<<grid, NTHREADS, 0, s.st>>>(a, s.Ny, s.Nx);
                     s.end();
                     s.launches++;
                 }
             }
-            t_eval_i = t_eval_i_new;
         }
         // accept (rk.py:167-174): y <- y_new, f <- f_new (FSAL: pointer swaps)
-        t = t_new;
+        ctl.accept();
         std::swap(s.y, s.ynew);
         std::swap(s.K[0], s.K[6]);
     }
@@ -745,13 +637,12 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
     OC_CUDA(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     stats->gpu_ms = ms;
     s.collect(stats);
-    stats->status = status;
-    stats->n_out = n_out;
+    ctl.report(stats);
     stats->launches = s.launches;
     oc::count_launch(s.launches);
-    if (trace_n) *trace_n = ntr;
-    if (status == -1) {
-        oc::set_error("RK45: required step size is less than spacing between numbers (t=%g)", t);
+    if (trace_n) *trace_n = ctl.attempts();
+    if (ctl.status == -1) {
+        oc::set_error("RK45: required step size is less than spacing between numbers (t=%g)", ctl.t);
         return OC_ERR_STEP_TOO_SMALL;
     }
     return OC_OK;
@@ -771,15 +662,13 @@ struct BatchRoom {
     Solver s;
     enum Phase { START, INIT0, INIT1, STEP, DONE } phase = START;
     const double *V = nullptr, *m = nullptr;
-    double *phi = nullptr, *vx = nullptr, *vy = nullptr;
+    double *phi = nullptr, *scratch = nullptr, *vx = nullptr, *vy = nullptr;  // scratch: NE_MAX slices, without phi
     double *rs_d = nullptr, *rs_h = nullptr;  // row-group sums (device / pinned host), 3 regions of `rs_stride`
     int rs_stride = 0;
     cudaEvent_t ev = nullptr;
     unsigned long long wait_seq = 0;     // sequence number of the step attempt in flight (in-kernel final reduction)
-    // controller state (rk.py:111-176, base.py:179-210, ivp.py:659-728)
-    double t = 0, h_abs = 0, h = 0, t_new = 0, min_step = 0, h0 = 0, d1 = 0;
-    bool rejected = false;
-    int status = 1, t_eval_i = 0, n_out = 0, ia_lo = 0;
+    rk45::Controller ctl;
+    double h0 = 0, d1 = 0;               // select_initial_step between its two norm reductions
     double step_sum = 0.0;               // error sum delivered by the last CTA of the attempt
     fused::Args fa{};                    // the attempt waiting in a bucket for its batched launch
     oc_hjb_stats st{};
@@ -811,24 +700,11 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
     const size_t np = ((std::max((size_t)2 * nbx * nby, (size_t)fgx * fgy) + 8) + 1) & ~(size_t)1;
     const int rs_stride = ((std::max(nby, fgy) + 8) + 1) & ~1;
     const size_t per_room = (5 + (need_scratch ? fused::NE_MAX : 0)) * n + np + 3 * (size_t)rs_stride;
-    const size_t need = per_room * n_rooms * sizeof(double);
-    if (ctx->batch_ws_bytes < need) {
-        if (ctx->batch_ws) cudaFree(ctx->batch_ws);
-        ctx->batch_ws = nullptr; ctx->batch_ws_bytes = 0;
-        if (cudaMalloc(&ctx->batch_ws, need) != cudaSuccess) {
-            cudaGetLastError();
-            oc::set_error("cannot allocate %zu bytes of batched HJB workspace (%d rooms)", need, n_rooms);
-            return OC_ERR_NOMEM;
-        }
-        ctx->batch_ws_bytes = need;
-    }
-    const size_t pin_need = (size_t)3 * rs_stride * n_rooms;
-    if (ctx->batch_pinned_n < pin_need) {
-        if (ctx->batch_pinned) cudaFreeHost(ctx->batch_pinned);
-        ctx->batch_pinned = nullptr; ctx->batch_pinned_n = 0;
-        OC_CUDA(cudaMallocHost(&ctx->batch_pinned, pin_need * sizeof(double)));
-        ctx->batch_pinned_n = pin_need;
-    }
+    int rc = oc_ensure_buffer(ctx->batch_ws, ctx->batch_ws_bytes, per_room * n_rooms * sizeof(double), false,
+                              "batched HJB workspace");
+    if (rc) return rc;
+    const size_t pin_need = (size_t)3 * rs_stride * n_rooms * sizeof(double);
+    if ((rc = oc_ensure_buffer(ctx->batch_pinned, ctx->batch_pinned_bytes, pin_need, true, "batched HJB host sums"))) return rc;
     constexpr int MAX_STREAMS = 32;
     const int n_streams = std::min(n_rooms, MAX_STREAMS);
     while ((int)ctx->batch_streams.size() < n_streams) {
@@ -849,14 +725,9 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
 
     const double s2 = prm->sigma * prm->sigma;
     const double rtol = prm->rtol, atol = prm->atol, sqrt_n = std::sqrt((double)n);
-    const double t_bound = 0.0, direction = (t_bound != T) ? (t_bound > T ? 1.0 : -1.0) : 1.0;
-    const double error_exponent = -1.0 / 5.0;
     const bool want_v = d_vx && d_vy;
     const bool final_in_kernel = fgy <= fused::MAX_FINAL_ROWS;
-    if (final_in_kernel) {
-        int frc = ensure_final_reduce(ctx, n_rooms);
-        if (frc) return frc;
-    }
+    if (final_in_kernel && (rc = ensure_final_reduce(ctx, n_rooms))) return rc;
     std::vector<BatchRoom> rooms(n_rooms);
     for (int b = 0; b < n_rooms; b++) {
         BatchRoom &r = rooms[b];
@@ -866,7 +737,6 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         s.ctx = ctx; s.st = ctx->batch_streams[b % n_streams]; s.Ny = Ny; s.Nx = Nx; s.n = n; s.nbx = nbx; s.nby = nby;
         s.coef = ws; s.y = ws + n; s.ynew = ws + 2 * n; s.K[0] = ws + 3 * n; s.K[6] = ws + 4 * n;
         s.K[1] = s.K[6];  // f(y0 + h0 f0) of select_initial_step lives in the (still unused) f_new array
-        double *scratch = need_scratch ? ws + 5 * n : nullptr;
         s.partial = ws + (5 + (need_scratch ? fused::NE_MAX : 0)) * n;
         r.rs_d = s.partial + np;
         r.rs_h = ctx->batch_pinned + (size_t)3 * rs_stride * b;
@@ -874,10 +744,11 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         s.diff_over_dxdy = (-0.5 * s2) / (ctx->dx * ctx->dy);
         s.fused_gx = fgx; s.fused_rc = frc; s.fused_gy = fgy;
         r.V = d_V[b]; r.m = d_m ? d_m[b] : nullptr;
-        r.phi = d_phi ? d_phi[b] : scratch;
+        r.phi = d_phi ? d_phi[b] : nullptr;
+        r.scratch = need_scratch ? ws + 5 * n : nullptr;
         r.vx = want_v ? d_vx[b] : nullptr; r.vy = want_v ? d_vy[b] : nullptr;
         r.ev = ctx->batch_events[b];
-        r.t = T; r.t_eval_i = nt;
+        r.ctl = rk45::Controller(T, t_eval, nt);
     }
     // room-local helpers ------------------------------------------------------------------------------
     auto reduce_async = [&](BatchRoom &r, size_t off, int gx, int gy, int slot) {
@@ -891,14 +762,6 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         const double *p = r.rs_h + (size_t)slot * r.rs_stride;
         for (int i = 0; i < gy; i++) s += p[i];  // fixed global order
         return s;
-    };
-    auto lower_index = [&](double t_new) {  // ivp.py:715-728, direction < 0: first ascending index with t_eval >= t_new
-        int lo = 0, hi = nt;
-        while (lo < hi) {
-            int mid = (lo + hi) / 2;
-            if (t_eval[nt - 1 - mid] < t_new) lo = mid + 1; else hi = mid;
-        }
-        return lo;
     };
     // Batched launches: the step attempts that become ready during one polling sweep are grouped by their number of
     // dense-output samples NE and launched together, up to fused::BATCH_MAX rooms per launch (blockIdx.z = room), instead
@@ -927,54 +790,32 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         }
         return OC_OK;
     };
-    // enqueue one step attempt of room r (fused kernel + reduction); returns false when the room has finished
+    // enqueue one step attempt of room r (fused kernel + reduction); the room is DONE when its step became too small
     auto attempt = [&](BatchRoom &r) -> int {
-        if (r.h_abs < r.min_step) { r.status = -1; r.phase = BatchRoom::DONE; return OC_OK; }
-        double h = r.h_abs * direction;
-        double t_new = r.t + h;
-        if (direction * (t_new - t_bound) > 0) t_new = t_bound;
-        h = t_new - r.t;
-        r.h = h; r.t_new = t_new; r.h_abs = std::fabs(h);
-        r.ia_lo = std::min(lower_index(t_new), r.t_eval_i);
+        rk45::Controller &c = r.ctl;
+        if (!c.propose()) { r.phase = BatchRoom::DONE; return OC_OK; }
         fused::Args fa{};
         Solver &s = r.s;
         fa.y = s.y; fa.k1 = s.K[0]; fa.coef = s.coef; fa.ynew = s.ynew; fa.k7 = s.K[6]; fa.partial = s.partial;
-        fa.ha21 = h * RK_A[1][0];
-        for (int j = 0; j < 2; j++) fa.ha3[j] = h * RK_A[2][j];
-        for (int j = 0; j < 3; j++) fa.ha4[j] = h * RK_A[3][j];
-        for (int j = 0; j < 4; j++) fa.ha5[j] = h * RK_A[4][j];
-        for (int j = 0; j < 5; j++) fa.ha6[j] = h * RK_A[5][j];
-        for (int j = 0; j < 6; j++) fa.hb[j] = h * RK_B[j];
-        for (int j = 0; j < 7; j++) fa.he[j] = h * RK_E[j];
         fa.A = s.diff_over_dxdy; fa.rtol = rtol; fa.atol = atol;
         fa.Ny = Ny; fa.Nx = Nx; fa.RC = frc;
         fa.row_base = 0; fa.own0 = 0; fa.own1 = Ny; fa.phi_row_base = 0;
         // the samples this attempt emits if accepted, NE_MAX per launch; with more than NE_MAX samples inside one
         // step (only when h >> dt) the step is simply launched again for the remaining samples: the re-launch
         // recomputes identical y_new / f_new / error sums
-        if (!d_phi && r.t_eval_i - r.ia_lo > fused::NE_MAX) {
+        if (!d_phi && c.n_emit() > fused::NE_MAX) {
             oc::set_error("batched solve without a phi output supports at most %d samples per step", fused::NE_MAX);
             return OC_ERR_ARG;
         }
         // an attempt waits in an NE bucket only when ALL its samples fit one launch.  The launches of a longer attempt
         // share the room's ticket counter and result slot, so they must not overlap: they go out in order on the
         // room's own stream (the sequence OC_BATCH_PER_ROOM gives every attempt).
-        const bool to_bucket = batched && r.t_eval_i - r.ia_lo <= fused::NE_MAX;
-        int ia = r.t_eval_i - 1;
+        const bool to_bucket = batched && c.n_emit() <= fused::NE_MAX;
+        int e0 = 0;
         do {
-            int ne = 0;
-            for (; ia >= r.ia_lo && ne < fused::NE_MAX; ia--, ne++) {
-                const int kd = nt - 1 - ia;
-                const double x = (t_eval[kd] - r.t) / h;  // RkDenseOutput: (t - t_old)/h
-                const double pw[4] = {x, x * x, x * x * x, x * x * x * x};
-                for (int j = 0; j < 7; j++) {
-                    double acc = 0.0;
-                    for (int q = 0; q < 4; q++) acc += RK_P[j][q] * pw[q];
-                    fa.w[ne][j] = h * acc;
-                }
-                // without a phi output the samples go to the room's scratch slices (velocities are derived on accept)
-                fa.phi[ne] = d_phi ? r.phi + (size_t)kd * n : r.phi + (size_t)((r.t_eval_i - 1 - ia) % fused::NE_MAX) * n;
-            }
+            const int ne = std::min(c.n_emit() - e0, fused::NE_MAX);
+            // without a phi output the samples go to the room's scratch slices (velocities are derived on accept)
+            fused::set_attempt(fa, c, e0, ne, r.phi, r.scratch, n);
             if (final_in_kernel) { final_reduce_args(ctx, (int)(&r - rooms.data()), fa); r.wait_seq = fa.seq; }
             if (to_bucket) {
                 r.fa = fa;
@@ -983,7 +824,8 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
             }
             int rc = s.launch_fused(ne, fa);
             if (rc) return rc;
-        } while (ia >= r.ia_lo);
+            e0 += ne;
+        } while (e0 < c.n_emit());
         r.st.nfev += 6;
         if (!final_in_kernel) {
             reduce_async(r, 0, fgx, fgy, 0);
@@ -993,10 +835,7 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         return OC_OK;
     };
     auto start_step = [&](BatchRoom &r) -> int {  // base.py:179-210 step(): one call of _step_impl
-        if (r.t == t_bound) { r.status = 0; r.phase = BatchRoom::DONE; return OC_OK; }
-        r.min_step = 10 * std::fabs(std::nextafter(r.t, direction * INFINITY) - r.t);
-        if (r.h_abs < r.min_step) r.h_abs = r.min_step;
-        r.rejected = false;
+        if (!r.ctl.begin_step()) { r.phase = BatchRoom::DONE; return OC_OK; }
         return attempt(r);
     };
     auto advance = [&](BatchRoom &r) -> int {
@@ -1009,7 +848,7 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
             c.y = s.y;
             s.stage(0, c, s.K[0]);  // rk.py:94
             r.st.nfev++;
-            if (std::fabs(t_bound - T) == 0.0) { r.h_abs = 0.0; r.st.h0 = 0.0; return start_step(r); }
+            if (!r.ctl.needs_initial_step()) { r.st.h0 = 0.0; return start_step(r); }
             init_norm_kernel<<<dim3(nbx, nby), NTHREADS, 0, s.st>>>(s.y, s.K[0], nullptr, rtol, atol, Ny, Nx, s.partial, 0);
             s.launches++;
             reduce_async(r, 0, nbx, nby, 0);
@@ -1019,12 +858,10 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
             return OC_OK;
         }
         case BatchRoom::INIT0: {  // common.py:109-127
-            const double d0 = std::sqrt(host_sum(r, nby, 0)) / sqrt_n, d1 = std::sqrt(host_sum(r, nby, 1)) / sqrt_n;
-            double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-            h0 = std::min(h0, std::fabs(t_bound - T));
-            r.h0 = h0; r.d1 = d1;
+            r.d1 = std::sqrt(host_sum(r, nby, 1)) / sqrt_n;
+            r.h0 = r.ctl.initial_h0(std::sqrt(host_sum(r, nby, 0)) / sqrt_n, r.d1);
             Comb c{};
-            c.y = s.y; c.k[0] = s.K[0]; c.a[0] = 1.0; c.h = h0 * direction;
+            c.y = s.y; c.k[0] = s.K[0]; c.a[0] = 1.0; c.h = r.h0 * r.ctl.direction;
             s.stage(1, c, s.K[1]);
             r.st.nfev++;
             init_norm_kernel<<<dim3(nbx, nby), NTHREADS, 0, s.st>>>(s.y, s.K[0], s.K[1], rtol, atol, Ny, Nx, s.partial, 1);
@@ -1035,32 +872,18 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
             return OC_OK;
         }
         case BatchRoom::INIT1: {  // common.py:127-134
-            const double d2 = std::sqrt(host_sum(r, nby, 2)) / sqrt_n / r.h0;
-            double h1;
-            if (r.d1 <= 1e-15 && d2 <= 1e-15) h1 = std::max(1e-6, r.h0 * 1e-3);
-            else h1 = std::pow(0.01 / std::max(r.d1, d2), 1.0 / 5.0);
-            r.h_abs = std::min(std::min(100 * r.h0, h1), std::fabs(t_bound - T));
-            r.st.h0 = r.h_abs;
+            r.ctl.set_initial_step(r.h0, r.d1, std::sqrt(host_sum(r, nby, 2)) / sqrt_n / r.h0);
+            r.st.h0 = r.ctl.h_abs;
             return start_step(r);
         }
         case BatchRoom::STEP: {  // rk.py:146-165
             const double error_norm = std::sqrt(final_in_kernel ? r.step_sum : host_sum(r, fgy, 0)) / sqrt_n;
-            if (!(error_norm < 1)) {
-                r.h_abs *= std::max(0.2, 0.9 * std::pow(error_norm, error_exponent));
-                r.rejected = true;
-                r.st.n_rejected++;
-                return attempt(r);
-            }
-            double factor = (error_norm == 0) ? 10.0 : std::min(10.0, 0.9 * std::pow(error_norm, error_exponent));
-            if (r.rejected) factor = std::min(1.0, factor);
-            r.h_abs *= factor;
-            r.st.n_accepted++;
-            const int t_eval_i_new = lower_index(r.t_new);
-            for (int ia = r.t_eval_i - 1; ia >= t_eval_i_new; ia--) {
-                const int kd = nt - 1 - ia;
-                r.n_out++;
+            rk45::Controller &c = r.ctl;
+            if (!c.judge(error_norm)) return attempt(r);
+            for (int e = 0; e < c.n_emit(); e++) {
+                const int kd = c.sample_column(e);
                 if (want_v && kd >= 1) {  // slice s = vels(sol.y[:, nt-1-s]) (optimals.py:200-204)
-                    const double *ph = d_phi ? r.phi + (size_t)kd * n : r.phi + (size_t)((r.t_eval_i - 1 - ia) % fused::NE_MAX) * n;
+                    const double *ph = fused::sample_slice(c, e, r.phi, r.scratch, n);
                     const int sl = nt - 1 - kd;
                     dim3 grid((Nx - 2 + 63) / 64, (Ny - 2 + 3) / 4);
                     vels_kernel<<<grid, NTHREADS, 0, s.st>>>(ph, Ny, Nx, prm->mu, prm->lim, 1.0 / (2 * ctx->dx), 1.0 / (2 * ctx->dy),
@@ -1068,18 +891,15 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
                     s.launches++;
                 }
             }
-            r.t_eval_i = t_eval_i_new;
-            const bool finished = direction * (r.t_new - t_bound) >= 0;  // base.py:205-208
-            r.t = r.t_new;
+            c.accept();
             std::swap(s.y, s.ynew);
             std::swap(s.K[0], s.K[6]);
-            if (finished) { r.status = 0; r.phase = BatchRoom::DONE; return OC_OK; }
             return start_step(r);
         }
         default: return OC_OK;
         }
     };
-    int rc = OC_OK, live = n_rooms;
+    int live = n_rooms;
     for (int b = 0; b < n_rooms && !rc; b++) {
         rc = advance(rooms[b]);
         if (rooms[b].phase == BatchRoom::DONE) live--;
@@ -1141,14 +961,15 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
     int bad = -1, total_launches = 0;
     for (int b = 0; b < n_rooms; b++) {
         BatchRoom &r = rooms[b];
-        r.st.status = r.status; r.st.n_out = r.n_out; r.st.launches = r.s.launches; r.st.gpu_ms = ms;
+        r.ctl.report(&r.st);
+        r.st.launches = r.s.launches; r.st.gpu_ms = ms;
         total_launches += r.s.launches;
         stats[b] = r.st;
-        if (r.status == -1 && bad < 0) bad = b;
+        if (r.ctl.status == -1 && bad < 0) bad = b;
     }
     oc::count_launch(total_launches);
     if (bad >= 0) {
-        oc::set_error("RK45: required step size is less than spacing between numbers (room %d, t=%g)", bad, rooms[bad].t);
+        oc::set_error("RK45: required step size is less than spacing between numbers (room %d, t=%g)", bad, rooms[bad].ctl.t);
         return OC_ERR_STEP_TOO_SMALL;
     }
     return OC_OK;

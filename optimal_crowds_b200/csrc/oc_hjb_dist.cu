@@ -362,22 +362,9 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
     const size_t per_band = 5 * n_store + n_partial + ((want_v && !d_phi) ? (size_t)fused::NE_MAX * (band_rows + 2) * Nx : 0);
     const int seg = (std::max(gy_f, gy_t) + 1) & ~1;  // row sums per band
     const size_t need = (per_band * nb_local + (size_t)2 * seg * nbands + 64) * sizeof(double);
-    if (ctx->dist_ws_bytes < need) {
-        if (ctx->dist_ws) cudaFree(ctx->dist_ws);
-        ctx->dist_ws = nullptr; ctx->dist_ws_bytes = 0;
-        if (cudaMalloc(&ctx->dist_ws, need) != cudaSuccess) {
-            cudaGetLastError();
-            oc::set_error("cannot allocate %zu bytes of banded HJB workspace", need);
-            return OC_ERR_NOMEM;
-        }
-        ctx->dist_ws_bytes = need;
-    }
-    const size_t pin_need = (size_t)seg * nbands + 16;
-    if (ctx->h_pinned_n < pin_need) {
-        if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-        OC_CUDA(cudaMallocHost(&ctx->h_pinned, pin_need * sizeof(double)));
-        ctx->h_pinned_n = pin_need;
-    }
+    if ((rc0 = oc_ensure_buffer(ctx->dist_ws, ctx->dist_ws_bytes, need, false, "banded HJB workspace"))) return rc0;
+    const size_t pin_need = ((size_t)seg * nbands + 16) * sizeof(double);
+    if ((rc0 = oc_ensure_buffer(ctx->h_pinned, ctx->h_pinned_bytes, pin_need, true, "pinned host scratch"))) return rc0;
     double *wsp = (double *)ctx->dist_ws;
     double *rowsum_loc = wsp; wsp += (size_t)seg * nbands;   // this process's band sums (virtual: all bands)
     double *rowsum_all = wsp; wsp += (size_t)seg * nbands;   // gathered over all ranks
@@ -410,7 +397,7 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
     }
 
     memset(stats, 0, sizeof(*stats));
-    int launches = 0, ntr = 0;
+    int launches = 0;
     const double s2 = prm->sigma * prm->sigma;
     const double A = (-0.5 * s2) / (ctx->dx * ctx->dy);
     const double rtol = prm->rtol, atol = prm->atol, sqrt_n = std::sqrt((double)n_glob);
@@ -502,8 +489,7 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
     }
     if ((rc = exchange({&Band::coef}, 0, nullptr))) return rc;
 
-    const double t_bound = 0.0, direction = (t_bound != T) ? (t_bound > T ? 1.0 : -1.0) : 1.0;
-    double t = T;
+    rk45::Controller ctl(T, t_eval, nt);
     dim3 grid_t(gx_t, gy_t);
     const size_t nb_t = (size_t)gx_t * gy_t;
     // rk.py:94 f0 = fun(t0, y0) and the d0, d1 norms of select_initial_step (common.py:109-118)
@@ -513,32 +499,22 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
     }
     stats->nfev++;
     if ((rc = exchange({&Band::f}, 0, nullptr))) return rc;
-    double h_abs;
-    {
-        const double interval = std::fabs(t_bound - T);
-        if (interval == 0.0) h_abs = 0.0;
-        else {
-            double s0, s1, sq2;
-            if ((rc = reduce(0, gx_t, gy_t, &s0))) return rc;
-            if ((rc = reduce(nb_t, gx_t, gy_t, &s1))) return rc;
-            const double d0 = std::sqrt(s0) / sqrt_n, d1 = std::sqrt(s1) / sqrt_n;
-            double h0 = (d0 < 1e-5 || d1 < 1e-5) ? 1e-6 : 0.01 * d0 / d1;
-            h0 = std::min(h0, interval);
-            for (Band &b : bands) {  // f1 = fun(t0 + h0*dir, y0 + h0*dir*f0) into ynew (scratch)
-                rhs_band_kernel<<<grid_t, NT, 0, st>>>(b.y, b.f, h0 * direction, b.coef, b.ynew, b.v, A, rtol, atol,
-                                                      b.partial, 1);
-                launches++;
-            }
-            stats->nfev++;
-            if ((rc = reduce(0, gx_t, gy_t, &sq2))) return rc;
-            const double d2 = std::sqrt(sq2) / sqrt_n / h0;
-            double h1;
-            if (d1 <= 1e-15 && d2 <= 1e-15) h1 = std::max(1e-6, h0 * 1e-3);
-            else h1 = std::pow(0.01 / std::max(d1, d2), 1.0 / 5.0);
-            h_abs = std::min(std::min(100 * h0, h1), interval);
+    if (ctl.needs_initial_step()) {
+        double s0, s1, sq2;
+        if ((rc = reduce(0, gx_t, gy_t, &s0))) return rc;
+        if ((rc = reduce(nb_t, gx_t, gy_t, &s1))) return rc;
+        const double d1 = std::sqrt(s1) / sqrt_n;
+        const double h0 = ctl.initial_h0(std::sqrt(s0) / sqrt_n, d1);
+        for (Band &b : bands) {  // f1 = fun(t0 + h0*dir, y0 + h0*dir*f0) into ynew (scratch)
+            rhs_band_kernel<<<grid_t, NT, 0, st>>>(b.y, b.f, h0 * ctl.direction, b.coef, b.ynew, b.v, A, rtol, atol,
+                                                  b.partial, 1);
+            launches++;
         }
+        stats->nfev++;
+        if ((rc = reduce(0, gx_t, gy_t, &sq2))) return rc;
+        ctl.set_initial_step(h0, d1, std::sqrt(sq2) / sqrt_n / h0);
     }
-    stats->h0 = h_abs;
+    stats->h0 = ctl.h_abs;
 
     fused::MapCache maps;  // TMA descriptors of the band arrays
     auto launch_fused = [&](int ne, fused::Args &fa, dim3 grid) -> int {
@@ -552,38 +528,16 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
         return (double *)ctx->p2p_peer[q] + (mine - (const double *)ctx->p2p_buf);
     };
 
-    int t_eval_i = nt, n_out = 0, status = 1;
     unsigned long long p2p_wait_seq = 0;
-    const double error_exponent = -1.0 / 5.0;
     cudaEvent_t pe0 = nullptr, pe1 = nullptr;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof;  // one pair per attempt, read after the final synchronisation
     double step_ms = 0.0;
     int step_launches = 0;
 
-    while (status == 1) {
-        if (t == t_bound) { status = 0; break; }
-        const double min_step = 10 * std::fabs(std::nextafter(t, direction * INFINITY) - t);
-        if (h_abs < min_step) h_abs = min_step;
-        bool accepted = false, rejected = false;
-        double h = 0, t_new = 0;
-        int ia_lo = 0;
-        while (!accepted) {
-            if (h_abs < min_step) { status = -1; break; }
-            h = h_abs * direction;
-            if (prm->forced_h && ntr < prm->n_forced_h) h = prm->forced_h[ntr];
-            t_new = t + h;
-            if (direction * (t_new - t_bound) > 0) t_new = t_bound;
-            h = t_new - t;
-            h_abs = std::fabs(h);
-            {
-                int lo = 0, hi = nt;
-                while (lo < hi) {
-                    int mid = (lo + hi) / 2;
-                    if (t_eval[nt - 1 - mid] < t_new) lo = mid + 1; else hi = mid;
-                }
-                ia_lo = std::min(lo, t_eval_i);
-            }
-            const int n_emit = want_out ? t_eval_i - ia_lo : 0;
+    while (ctl.begin_step()) {
+        bool accepted = false;
+        while (!accepted && ctl.propose(prm->forced_h, prm->n_forced_h)) {
+            const int n_emit = want_out ? ctl.n_emit() : 0;
             // samples beyond NE_MAX per launch: repeat the (identical) step for the next batch
             int done = 0;
             do {
@@ -593,29 +547,10 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
                     fused::Args fa{};
                     fa.y = b.y; fa.k1 = b.f; fa.coef = b.coef; fa.ynew = b.ynew; fa.k7 = b.fnew;
                     fa.partial = b.partial + 2 * nb_t;
-                    fa.ha21 = h * rk45::A[1][0];
-                    for (int j = 0; j < 2; j++) fa.ha3[j] = h * rk45::A[2][j];
-                    for (int j = 0; j < 3; j++) fa.ha4[j] = h * rk45::A[3][j];
-                    for (int j = 0; j < 4; j++) fa.ha5[j] = h * rk45::A[4][j];
-                    for (int j = 0; j < 5; j++) fa.ha6[j] = h * rk45::A[5][j];
-                    for (int j = 0; j < 6; j++) fa.hb[j] = h * rk45::B[j];
-                    for (int j = 0; j < 7; j++) fa.he[j] = h * rk45::E[j];
                     fa.A = A; fa.rtol = rtol; fa.atol = atol;
                     fa.Ny = Ny; fa.Nx = Nx; fa.RC = rc_rows;
                     fa.row_base = b.v.row_base; fa.own0 = b.v.own0; fa.own1 = b.v.own1; fa.phi_row_base = b.phi_row_base;
-                    for (int e = 0; e < ne; e++) {
-                        const int ia = t_eval_i - 1 - (done + e);
-                        const int kd = nt - 1 - ia;
-                        const double x = (t_eval[kd] - t) / h;
-                        const double pw[4] = {x, x * x, x * x * x, x * x * x * x};
-                        for (int j = 0; j < 7; j++) {
-                            double acc = 0.0;
-                            for (int qq = 0; qq < 4; qq++) acc += rk45::P[j][qq] * pw[qq];
-                            fa.w[e][j] = h * acc;
-                        }
-                        fa.phi[e] = d_phi ? d_phi + (size_t)kd * b.phi_slice
-                                          : b.scratch + (size_t)((done + e) % fused::NE_MAX) * b.phi_slice;
-                    }
+                    fused::set_attempt(fa, ctl, done, ne, d_phi, b.scratch, b.phi_slice);
                     if (use_p2p) {
                         // sequence numbers of this mode carry bit 62, so a value left in the result slot by a
                         // single-GPU solve on the same context (its own counter) can never look like an answer
@@ -653,24 +588,13 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
             } else if ((rc = reduce(2 * nb_t, gx_f, gy_f, &se, true))) return rc;
             if (prm->profile) step_launches += nb_local;
             const double error_norm = std::sqrt(se) / sqrt_n;
-            if (trace_h && ntr < trace_cap) { trace_h[ntr] = h; trace_err[ntr] = error_norm; }
-            ntr++;
-            if (error_norm < 1) {
-                double factor = (error_norm == 0) ? 10.0 : std::min(10.0, 0.9 * std::pow(error_norm, error_exponent));
-                if (rejected) factor = std::min(1.0, factor);
-                h_abs *= factor;
-                accepted = true;
-                stats->n_accepted++;
-            } else {
-                h_abs *= std::max(0.2, 0.9 * std::pow(error_norm, error_exponent));
-                rejected = true;
-                stats->n_rejected++;
-            }
+            const int ntr = ctl.attempts();
+            if (trace_h && ntr < trace_cap) { trace_h[ntr] = ctl.h; trace_err[ntr] = error_norm; }
+            accepted = ctl.judge(error_norm);
         }
-        if (status == -1) break;
-        if (direction * (t_new - t_bound) >= 0) status = 0;
+        if (!accepted) break;  // step too small
         // ---- accepted: velocities of the emitted samples, halo exchange of the new state
-        const int n_emit = t_eval_i - ia_lo;
+        const int n_emit = ctl.n_emit();
         if (want_v && !d_phi && n_emit > fused::NE_MAX) {
             oc::set_error("banded solve: more than %d samples in one step need d_phi storage", fused::NE_MAX);
             return OC_ERR_ARG;
@@ -678,10 +602,8 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
         std::vector<double *> phis;
         if (want_v)
             for (int e = 0; e < n_emit; e++) {
-                const int kd = nt - 1 - (t_eval_i - 1 - e);
-                if (kd < 1) continue;
-                for (Band &b : bands)
-                    phis.push_back(d_phi ? d_phi + (size_t)kd * b.phi_slice : b.scratch + (size_t)e * b.phi_slice);
+                if (ctl.sample_column(e) < 1) continue;
+                for (Band &b : bands) phis.push_back(fused::sample_slice(ctl, e, d_phi, b.scratch, b.phi_slice));
             }
         for (Band &b : bands) { std::swap(b.y, b.ynew); std::swap(b.f, b.fnew); }  // FSAL (rk.py:167-174)
         // the halo rows of the new y, f travelled with the error sums; only the halo rows of the emitted phi slices are
@@ -689,13 +611,13 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
         if (dist && want_v && !phis.empty() && (rc = exchange({}, (int)phis.size(), phis.data()))) return rc;
         if (dist && !want_v && xhi && d_phi && !defer_phi_halo) {
             std::vector<double *> hp;
-            for (int e = 0; e < n_emit; e++) hp.push_back(d_phi + (size_t)(nt - 1 - (t_eval_i - 1 - e)) * bands[0].phi_slice);
+            for (int e = 0; e < n_emit; e++) hp.push_back(fused::sample_slice(ctl, e, d_phi, nullptr, bands[0].phi_slice));
             if (!hp.empty() && (rc = exchange({}, (int)hp.size(), hp.data()))) return rc;
         }
         if (want_v) {
             size_t pi = 0;
             for (int e = 0; e < n_emit; e++) {
-                const int kd = nt - 1 - (t_eval_i - 1 - e);
+                const int kd = ctl.sample_column(e);
                 if (kd < 1) continue;
                 const int sl = nt - 1 - kd;
                 for (Band &b : bands) {
@@ -708,26 +630,16 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
                 }
             }
         }
-        n_out += n_emit;
-        t_eval_i = ia_lo;
-        t = t_new;
+        ctl.accept();
     }
-    if (defer_phi_halo && status == 0 && nranks > 1) {
+    if (defer_phi_halo && ctl.status == 0 && nranks > 1) {
         // all nt samples are final now: one packed exchange of their halo rows (see phi_halo_rows_kernel)
         Band &b = bands[0];
         const int up = 1 + xhi;                       // rows I send up / receive from below
         const size_t n_up = (size_t)nt * up * Nx, n_dn = (size_t)nt * Nx;
         const size_t need = 2 * (n_up + n_dn) * sizeof(double);
-        if (ctx->dist_halo_bytes < need) {
-            if (ctx->dist_halo) cudaFree(ctx->dist_halo);
-            ctx->dist_halo = nullptr; ctx->dist_halo_bytes = 0;
-            if (cudaMalloc(&ctx->dist_halo, need) != cudaSuccess) {
-                cudaGetLastError();
-                oc::set_error("cannot allocate %zu bytes for the phi halo exchange", need);
-                return OC_ERR_NOMEM;
-            }
-            ctx->dist_halo_bytes = need;
-        }
+        if ((rc = oc_ensure_buffer(ctx->dist_halo, ctx->dist_halo_bytes, need, false, "phi halo exchange staging")))
+            return rc;
         double *s_up = (double *)ctx->dist_halo, *s_dn = s_up + n_up, *r_up = s_dn + n_dn, *r_dn = r_up + n_dn;
         const int blocks = 592;
         if (rank > 0) phi_halo_rows_kernel<<<blocks, 256, 0, st>>>(d_phi, b.phi_slice, nt, Nx, 1, up, s_up, 1);
@@ -758,16 +670,15 @@ extern "C" int oc_hjb_solve_band(oc_ctx *ctx, const oc_band_cfg *cfg, const doub
     }
     cudaGetLastError();
     stats->gpu_ms = ms;
-    stats->status = status;
-    stats->n_out = n_out;
+    ctl.report(stats);
     stats->launches = launches;
     stats->cls_launches[0] = step_launches;
     stats->cls_ms[0] = step_ms;
     stats->cls_bytes[0] = 0;  // filled by the caller from nfev (40 B/cell/attempt + 8 B/cell/sample)
     oc::count_launch(launches);
-    if (trace_n) *trace_n = ntr;
-    if (status == -1) {
-        oc::set_error("RK45: required step size is less than spacing between numbers (t=%g)", t);
+    if (trace_n) *trace_n = ctl.attempts();
+    if (ctl.status == -1) {
+        oc::set_error("RK45: required step size is less than spacing between numbers (t=%g)", ctl.t);
         return OC_ERR_STEP_TOO_SMALL;
     }
     return OC_OK;

@@ -36,6 +36,8 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "oc_rk45.h"
+
 namespace fused {
 
 #ifndef OC_BX
@@ -133,6 +135,35 @@ struct alignas(64) Args {
     double *peer_inbox[P2P_MAX_RANKS];  // inbox of rank q as seen from this GPU; [my_rank] is the local one
 };
 constexpr int MAX_FINAL_ROWS = 2 * 6 * (BX + 2) - 8;  // chunk-row sums are staged in the (then idle) exchange buffer
+
+// Where sample e of the controller's current attempt goes: column kd of `phi` (slices of `slice` elements), or, when
+// only velocities are stored (phi == NULL), scratch slot e % NE_MAX.
+inline double *sample_slice(const rk45::Controller &c, int e, double *phi, double *scratch, size_t slice) {
+    return phi ? phi + (size_t)c.sample_column(e) * slice : scratch + (size_t)(e % NE_MAX) * slice;
+}
+// The per-attempt constants of one launch for the controller's current attempt: the tableau times h, and for samples
+// [e0, e0 + ne) the dense-output weights (RkDenseOutput, rk.py:723-737) and destination slices.  The caller sets the
+// arrays, geometry, tickets and peer pointers.
+inline void set_attempt(Args &a, const rk45::Controller &c, int e0, int ne, double *phi, double *scratch, size_t slice) {
+    const double h = c.h;
+    a.ha21 = h * rk45::A[1][0];
+    for (int j = 0; j < 2; j++) a.ha3[j] = h * rk45::A[2][j];
+    for (int j = 0; j < 3; j++) a.ha4[j] = h * rk45::A[3][j];
+    for (int j = 0; j < 4; j++) a.ha5[j] = h * rk45::A[4][j];
+    for (int j = 0; j < 5; j++) a.ha6[j] = h * rk45::A[5][j];
+    for (int j = 0; j < 6; j++) a.hb[j] = h * rk45::B[j];
+    for (int j = 0; j < 7; j++) a.he[j] = h * rk45::E[j];
+    for (int i = 0; i < ne; i++) {
+        const double x = c.sample_x(e0 + i);
+        const double pw[4] = {x, x * x, x * x * x, x * x * x * x};
+        for (int j = 0; j < 7; j++) {
+            double acc = 0.0;
+            for (int q = 0; q < 4; q++) acc += rk45::P[j][q] * pw[q];
+            a.w[i][j] = h * acc;
+        }
+        a.phi[i] = sample_slice(c, e0 + i, phi, scratch, slice);
+    }
+}
 
 // ---- per-thread cp.async (LDGSTS) staging: the BULK = false variant
 // predicated forms: the unrolled row body has no divergent region (a branch around the loads / stores makes ptxas save
