@@ -224,8 +224,11 @@ typedef struct {
     double dx, dy, room_length, room_height;
     int Ny, Nx;
     /* Distributed step (one room on several GPUs, SURVEY.md section 8e): the agents are replicated on every rank; a
-     * rank evaluates the field sample and the wall force only for the agents whose sampled node row lies in
-     * [own0, own1) -- its band of the row-decomposed field -- the per-agent terms are merged bit-exactly over the
+     * rank evaluates the field sample and the wall force only for the agents it owns: those whose first sampled node
+     * row i0 + 1 lies in [own0, own1), its band of the row-decomposed field.  i0 is the sampler's own row index after
+     * numpy's wrap of a negative index (an agent at y < 0 reads the last rows, so the last band owns it), and the
+     * band's phi slices hold every row the sampler then reads.  A row index out of range even after the wrap is
+     * clamped into [0, Ny-1], so every agent has exactly one owner.  The per-agent terms are merged bit-exactly over the
      * communicator of oc_dist_init, and every rank then runs the identical sequential sweep (a room's sweep is one
      * dependency chain).  own0 = own1 = 0: single-GPU step, everything local. */
     int own0, own1;

@@ -100,14 +100,18 @@ __device__ __forceinline__ double py_floordiv(double vx, double wx) {
     return copysign(0.0, vx / wx);
 }
 
-// node row whose band "owns" an agent in a row-decomposed run: the first of the (up to) two rows the sampler reads
-// (i0 + 1 in node indexing), clamped into the grid so that every position -- also one the sampler refuses -- has
-// exactly one owner.  The sampler then reads node rows i0 .. i0+3, i.e. owner-1 .. owner+2.
-__device__ __forceinline__ int sampler_owner_row(const oc_gcfm_params &p, double y) {
-    long long i0 = (y < p.room_height - p.dy) ? (long long)py_floordiv(y, p.dy) : (long long)(p.Ny - 3);
-    if (!(y == y)) i0 = 0;
-    i0 = i0 < -1 ? -1 : (i0 > p.Ny - 2 ? p.Ny - 2 : i0);
-    return (int)i0 + 1;
+// optimals.py:234-248, one axis of the sampler's index rule, for the sampler and for the owner of an agent in a
+// row-decomposed run alike: the (up to) two indices k0, k1 into the interior field (n - 2 nodes along the axis) with the
+// top clamp, CPython's floor division and numpy's wrap of a negative index (an agent at c < 0, where k1 == k0).  The
+// result can still be out of range (the reference raises IndexError): the caller checks it.
+__device__ __forceinline__ void sampler_axis(double c, double extent, double step, int n, long long &k0, long long &k1) {
+    if (c < extent - step) {
+        k0 = (long long)py_floordiv(c, step);
+        k1 = (c > step) ? k0 + 1 : k0;
+    } else {
+        k0 = k1 = n - 3;
+    }
+    if (k0 < 0) { k0 += n - 2; k1 = k0; }  // silently, no exception (App. C #7)
 }
 
 // optimals.py:212-250 -- returns 1 if the reference would raise IndexError (negative indices wrap like numpy's)
@@ -117,22 +121,9 @@ __device__ int choose_velocity(const oc_gcfm_params &p, const KeyDev &k, double 
     oy = 0.0;
     if (t >= k.nt_opt - 1) return 0;
     long long j0, j1, i0, i1;
-    if (x < p.room_length - p.dx) {
-        j0 = (long long)py_floordiv(x, p.dx);
-        j1 = (x > p.dx) ? j0 + 1 : j0;
-    } else {
-        j0 = j1 = p.Nx - 3;
-    }
-    if (y < p.room_height - p.dy) {
-        i0 = (long long)py_floordiv(y, p.dy);
-        i1 = (y > p.dy) ? i0 + 1 : i0;
-    } else {
-        i0 = i1 = p.Ny - 3;
-    }
+    sampler_axis(x, p.room_length, p.dx, p.Nx, j0, j1);
+    sampler_axis(y, p.room_height, p.dy, p.Ny, i0, i1);
     const int W = p.Nx - 2, H = p.Ny - 2;
-    // numpy wraps negative indices: an agent at x < 0 (then j1 == j0) reads column W + j0, silently (App. C #7)
-    if (j0 < 0) { j0 += W; j1 = j0; }
-    if (i0 < 0) { i0 += H; i1 = i0; }
     if (j0 < 0 || j1 >= W || i0 < 0 || i1 >= H || t < 0) return 1;
     double ax, ay, bx, by;
     if (k.vx) {
@@ -576,8 +567,14 @@ __device__ __forceinline__ void noise_index_body(int N, const Ws &w) {
 __device__ __forceinline__ bool agent_owned(const oc_gcfm_params &p, int key, double yi) {
     // key-sharded run: the rank that solved this agent's target set evaluates it
     if (p.key_mod > 0 && key % p.key_mod != p.key_rem) return false;
-    if (p.own1 > p.own0) {  // row-decomposed run: the rank whose band holds the sampled rows
-        const int orow = sampler_owner_row(p, yi);
+    if (p.own1 > p.own0) {
+        // row-decomposed run: the rank whose band holds node row i0 + 1 of the sampler's (wrapped) row indices; its phi
+        // slices hold node rows own0 - 1 .. own1 + 1, i.e. every row the sampler reads (i0 .. i1 + 2).  A row index the
+        // sampler refuses is clamped into the grid: the sampler raises the range flag before it reads anything, so any
+        // single owner will do
+        long long i0, i1;
+        sampler_axis(yi, p.room_height, p.dy, p.Ny, i0, i1);
+        const long long orow = i0 + 1 < 0 ? 0 : (i0 + 1 > p.Ny - 1 ? p.Ny - 1 : i0 + 1);
         if (orow < p.own0 || orow >= p.own1) return false;
     }
     return true;

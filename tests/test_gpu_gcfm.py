@@ -305,10 +305,9 @@ def test_step_with_nobody_inside_and_single_agent(cfg):
 
 
 def test_row_band_field_storage_and_ownership_change_no_bit(cfg):
-    """distributed-step building blocks on one GPU: (a) phi slices stored as a row band (phi_row0 / phi_rows, here
-    one band that covers the grid plus the halo rows) sample exactly like full-grid slices; (b) with an ownership
-    range the agents outside it get all-zero terms, the owned ones the same bits as the single-GPU step, so the
-    bit-wise maximum over bands (what oc_gcfm_step does over NCCL) reassembles the single-GPU step."""
+    """one band that owns every row: phi slices stored as a row band (phi_row0 = -1, phi_rows = Ny + 3: the grid plus
+    one halo row below and two above) and an ownership range [0, Ny) give the single-GPU step's bits over whole runs.
+    Bands smaller than the grid, and key shards, are checked in test_gpu_gcfm_band.py."""
     import torch
     from optimal_crowds_b200 import _lib
     L, H, N, steps = 12.0, 9.0, 120, 6
