@@ -146,7 +146,7 @@ int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, const oc_hjb
                  const double *t_eval, int nt, double *d_phi, double *d_vx, double *d_vy, oc_hjb_stats *stats,
                  double *trace_h, double *trace_err, int trace_cap, int *trace_n, void *stream);
 
-/* ------------------------------------------------------------------ batched HJB solve (ensembles)
+/* ------------------------------------------------------------------ batched HJB solves (ensembles)
  * n_rooms independent solves on the context's grid shape (BASELINE configs[4]: ensembles of rooms / seeds, one
  * batch per GPU; the reference would call optimals.compute_optimal_velocity once per room, optimals.py:124-206).
  * Every room keeps its own RK45 controller state and runs on its own CUDA stream, so the rooms' kernels overlap
@@ -160,9 +160,31 @@ int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, const oc_hjb
 /* Chunk height (prm->chunk_rows) that balances halo recomputation against wave quantisation for `copies` rooms solved
  * side by side; the default of a single solve is oc_hjb_plan_chunk_rows(ctx, 1). */
 int oc_hjb_plan_chunk_rows(oc_ctx *ctx, int copies);
+/* All rooms with the model parameters of prm and the one horizon (T, t_eval, nt): oc_hjb_solve_multi with n_rooms
+ * identical oc_hjb_room entries. */
 int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const *d_V, const double *const *d_m,
                        const oc_hjb_params *prm, double T, const double *t_eval, int nt, double *const *d_phi,
                        double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats, void *stream);
+
+/* What one room of oc_hjb_solve_multi does not share with the others: its model parameters (sigma, mu, g of its
+ * config.json, optimals.py:66-70) and its horizon.  d_phi[b] holds rooms[b].nt slices, d_vx[b] / d_vy[b] nt-1. */
+typedef struct {
+    double sigma, mu, g;        /* config.json hjb_params of this room */
+    double T;                   /* t_span = (T, 0) */
+    const double *t_eval;       /* host, nt decreasing values: np.linspace(T, 0, nt) (optimals.py:194) */
+    int nt;
+    int pad_;
+} oc_hjb_room;
+/* The batched solve with per-room model parameters and horizons (ensembles whose members have their own
+ * configuration).  Each room's result is bit-identical to oc_hjb_solve of that room alone with prm's sigma, mu, g
+ * replaced by the room's and the room's (T, t_eval, nt).  Shared by all rooms: prm->rtol, atol, lim and chunk_rows (the
+ * launch grid); prm->sigma, mu and g are not read.  Step attempts of rooms with different nt still share the batched
+ * launches, which are grouped by the number of samples per launch.  Without d_phi the limit of 6 t_eval samples per
+ * attempt applies to every room.  OC_ERR_ARG if rooms is NULL, a room's t_eval is NULL or its nt < 1, sigma or mu is not
+ * a finite positive number, or g is not finite.  Everything else as oc_hjb_solve_batch. */
+int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const *d_V, const double *const *d_m,
+                       const oc_hjb_room *rooms, const oc_hjb_params *prm, double *const *d_phi, double *const *d_vx,
+                       double *const *d_vy, oc_hjb_stats *stats, void *stream);
 
 /* ------------------------------------------------------------------ row-decomposed HJB solve (multi-GPU)
  * The grid of the context is split into bands of rows (SURVEY.md section 8e).  Two modes:

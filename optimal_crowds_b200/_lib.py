@@ -58,6 +58,11 @@ class HjbStats(C.Structure):
         return d
 
 
+class HjbRoom(C.Structure):
+    _fields_ = [("sigma", C.c_double), ("mu", C.c_double), ("g", C.c_double), ("T", C.c_double), ("t_eval", dp),
+                ("nt", C.c_int), ("pad_", C.c_int)]
+
+
 class BandCfg(C.Structure):
     _fields_ = [("n_virtual", C.c_int), ("own0", C.c_int), ("own1", C.c_int), ("phi_extra_hi", C.c_int)]
 
@@ -82,7 +87,7 @@ _lib = None
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
            "oc_hjb_solve", "oc_hjb_rhs", "oc_hjb_vels", "oc_wall_tiles_bytes", "oc_wall_tiles", "oc_gcfm_step",
            "oc_wall_force", "oc_pair_force", "oc_density", "oc_gcfm_last_ms", "oc_dist_unique_id", "oc_dist_init",
-           "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_gcfm_step_launch",
+           "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_gcfm_step_launch",
            "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run"]
 
 
@@ -137,6 +142,8 @@ def load():
     vpp = C.POINTER(C.c_void_p)
     lib.oc_hjb_solve_batch.argtypes = [C.c_void_p, C.c_int, vpp, vpp, C.POINTER(HjbParams), C.c_double, dp, C.c_int,
                                        vpp, vpp, vpp, C.POINTER(HjbStats), C.c_void_p]
+    lib.oc_hjb_solve_multi.argtypes = [C.c_void_p, C.c_int, vpp, vpp, C.POINTER(HjbRoom), C.POINTER(HjbParams), vpp, vpp,
+                                       vpp, C.POINTER(HjbStats), C.c_void_p]
     lib.oc_upload.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]
     lib.oc_dist_unique_id.argtypes = [C.c_void_p]
     lib.oc_dist_init.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
@@ -185,6 +192,25 @@ def _dev(t):
 def _stream():
     import torch
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+def _ptrs(ts, B):
+    """host array of B device pointers of CUDA tensors (None entries: NULL), or NULL for ts None"""
+    if ts is None:
+        return None
+    arr = (C.c_void_p * B)()
+    for q, t in enumerate(ts):
+        if t is not None:
+            assert t.is_cuda and t.is_contiguous()
+            arr[q] = t.data_ptr()
+    return arr
+
+
+def _batch_results(rc, st, out_phi, out_vx, out_vy):
+    check(rc, allow=(OC_ERR_STEP_TOO_SMALL,))
+    return [{"stats": st[q].asdict(), "phi": out_phi[q] if out_phi is not None else None,
+             "vx": out_vx[q] if out_vx is not None else None, "vy": out_vy[q] if out_vx is not None else None,
+             "rc": rc if st[q].status == -1 else 0} for q in range(len(st))]
 
 
 def grid_shape(room_length, room_height, grid_step):
@@ -360,28 +386,40 @@ class Context:
         (phi slices (nt,Ny,Nx) are allocated when no output is given).  Returns a list of per-room dicts."""
         B = len(Vs)
         t_eval = np.linspace(T, 0, nt)
-        if out_phi is None and not (want_vel or out_vx is not None):
-            out_phi = [self.empty(nt, self.Ny, self.Nx) for _ in range(B)]
-        if want_vel and out_vx is None:
-            out_vx = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for _ in range(B)]
-            out_vy = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for _ in range(B)]
-
-        def ptrs(ts):
-            if ts is None:
-                return None
-            arr = (C.c_void_p * B)()
-            for q, t in enumerate(ts):
-                if t is not None:
-                    assert t.is_cuda and t.is_contiguous()
-                    arr[q] = t.data_ptr()
-            return arr
+        out_phi, out_vx, out_vy = self._batch_outputs([nt] * B, out_phi, out_vx, out_vy, want_vel)
         st = (HjbStats * B)()
-        rc = load().oc_hjb_solve_batch(self.h, B, ptrs(Vs), ptrs(ms), C.byref(prm), float(T), _hp(t_eval), int(nt),
-                                       ptrs(out_phi), ptrs(out_vx), ptrs(out_vy), st, _stream())
-        check(rc, allow=(OC_ERR_STEP_TOO_SMALL,))
-        return [{"stats": st[q].asdict(), "phi": out_phi[q] if out_phi is not None else None,
-                 "vx": out_vx[q] if out_vx is not None else None, "vy": out_vy[q] if out_vx is not None else None,
-                 "rc": rc if st[q].status == -1 else 0} for q in range(B)]
+        rc = load().oc_hjb_solve_batch(self.h, B, _ptrs(Vs, B), _ptrs(ms, B), C.byref(prm), float(T), _hp(t_eval),
+                                       int(nt), _ptrs(out_phi, B), _ptrs(out_vx, B), _ptrs(out_vy, B), st, _stream())
+        return _batch_results(rc, st, out_phi, out_vx, out_vy)
+
+    def hjb_solve_multi(self, Vs, ms, rooms, prm: HjbParams, out_phi=None, out_vx=None, out_vy=None, want_vel=False):
+        """hjb_solve_batch with per-room model parameters and horizons (oc_hjb_solve_multi).  rooms: one
+        dict(sigma, mu, g, T, nt) per room, t_eval = np.linspace(T, 0, nt) as optimals.py:194 builds it; prm gives the
+        shared rtol, atol, lim and chunk_rows (its sigma, mu and g are not used).  Outputs as hjb_solve_batch, sized by
+        each room's nt."""
+        B = len(Vs)
+        if len(rooms) != B:
+            raise ValueError("one rooms entry per room expected")
+        nts = [int(r["nt"]) for r in rooms]
+        t_evals = [np.linspace(r["T"], 0, nt) for r, nt in zip(rooms, nts)]   # alive until the call returns
+        spec = (HjbRoom * B)()
+        for q, (r, te) in enumerate(zip(rooms, t_evals)):
+            spec[q] = HjbRoom(float(r["sigma"]), float(r["mu"]), float(r["g"]), float(r["T"]),
+                              _hp(te) if len(te) else None, nts[q], 0)
+        out_phi, out_vx, out_vy = self._batch_outputs(nts, out_phi, out_vx, out_vy, want_vel)
+        st = (HjbStats * B)()
+        rc = load().oc_hjb_solve_multi(self.h, B, _ptrs(Vs, B), _ptrs(ms, B), spec, C.byref(prm), _ptrs(out_phi, B),
+                                       _ptrs(out_vx, B), _ptrs(out_vy, B), st, _stream())
+        return _batch_results(rc, st, out_phi, out_vx, out_vy)
+
+    def _batch_outputs(self, nts, out_phi, out_vx, out_vy, want_vel):
+        """the outputs of a batched solve: phi slices (nt,Ny,Nx) per room when no output is given"""
+        if out_phi is None and not (want_vel or out_vx is not None):
+            out_phi = [self.empty(nt, self.Ny, self.Nx) for nt in nts]
+        if want_vel and out_vx is None:
+            out_vx = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for nt in nts]
+            out_vy = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for nt in nts]
+        return out_phi, out_vx, out_vy
 
     def plan_chunk_rows(self, copies=1):
         """chunk height the fused solver picks for `copies` rooms of this grid side by side (oc_hjb_plan_chunk_rows)"""

@@ -656,6 +656,9 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
 // every room's result is bit-identical to solving it alone (with the same prm->chunk_rows).  The host serves the rooms
 // round-robin: while it reads room b's error norm and enqueues b's next attempt, the other rooms' kernels keep
 // the GPU busy -- small grids (512^2: ~10 us of device work per attempt) are launch-latency bound one at a time.
+// oc_hjb_solve_multi is the one implementation: every room brings its own sigma, mu, g (prep_kernel's coefficients, the
+// diffusion constant of the step kernel, vels_kernel's mu -- all kernel arguments already) and its own horizon (its
+// controller); oc_hjb_solve_batch gives every room the same ones.
 namespace {
 
 struct BatchRoom {
@@ -667,7 +670,8 @@ struct BatchRoom {
     int rs_stride = 0;
     cudaEvent_t ev = nullptr;
     unsigned long long wait_seq = 0;     // sequence number of the step attempt in flight (in-kernel final reduction)
-    rk45::Controller ctl;
+    rk45::Controller ctl;                // the room's horizon: T, t_eval, nt
+    double g = 0, inv_mu_s2 = 0, mu = 0; // prep_kernel's coefficients, vels_kernel's mu (s.diff_over_dxdy: its sigma)
     double h0 = 0, d1 = 0;               // select_initial_step between its two norm reductions
     double step_sum = 0.0;               // error sum delivered by the last CTA of the attempt
     fused::Args fa{};                    // the attempt waiting in a bucket for its batched launch
@@ -680,8 +684,23 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
                                   const oc_hjb_params *prm, double T, const double *t_eval, int nt,
                                   double *const *d_phi, double *const *d_vx, double *const *d_vy,
                                   oc_hjb_stats *stats, void *stream) {
+    OC_ARG(prm && n_rooms >= 1, "NULL argument");
+    std::vector<oc_hjb_room> same(n_rooms, oc_hjb_room{prm->sigma, prm->mu, prm->g, T, t_eval, nt, 0});
+    return oc_hjb_solve_multi(ctx, n_rooms, d_V, d_m, same.data(), prm, d_phi, d_vx, d_vy, stats, stream);
+}
+
+extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const *d_V, const double *const *d_m,
+                                  const oc_hjb_room *spec, const oc_hjb_params *prm, double *const *d_phi,
+                                  double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats, void *stream) {
     OC_ARG(ctx && d_V && prm && stats && n_rooms >= 1, "NULL argument");
-    OC_ARG(nt >= 1 && t_eval, "t_eval required");
+    OC_ARG(spec, "rooms (per-room parameters and horizons) required");
+    for (int b = 0; b < n_rooms; b++) {
+        const oc_hjb_room &p = spec[b];
+        OC_ARG(p.nt >= 1 && p.t_eval, "t_eval required");
+        OC_ARG(std::isfinite(p.sigma) && p.sigma > 0, "sigma must be a finite positive number");
+        OC_ARG(std::isfinite(p.mu) && p.mu > 0, "mu must be a finite positive number");
+        OC_ARG(std::isfinite(p.g), "g must be finite");
+    }
     OC_ARG(d_phi || (d_vx && d_vy), "an output (d_phi or d_vx,d_vy) is required");
     const int Ny = ctx->Ny, Nx = ctx->Nx;
     OC_ARG(Ny > fused::HY + 1 && Nx > fused::HX + 1, "grid too small for the stage-fused kernel");
@@ -723,7 +742,6 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
     OC_CUDA(cudaEventRecord(ev_in, main_st));
     for (int q = 0; q < n_streams; q++) OC_CUDA(cudaStreamWaitEvent(ctx->batch_streams[q], ev_in, 0));
 
-    const double s2 = prm->sigma * prm->sigma;
     const double rtol = prm->rtol, atol = prm->atol, sqrt_n = std::sqrt((double)n);
     const bool want_v = d_vx && d_vy;
     const bool final_in_kernel = fgy <= fused::MAX_FINAL_ROWS;
@@ -741,14 +759,16 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         r.rs_d = s.partial + np;
         r.rs_h = ctx->batch_pinned + (size_t)3 * rs_stride * b;
         r.rs_stride = rs_stride;
+        const double s2 = spec[b].sigma * spec[b].sigma;   // the expressions of oc_hjb_solve, with the room's values
         s.diff_over_dxdy = (-0.5 * s2) / (ctx->dx * ctx->dy);
+        r.g = spec[b].g; r.inv_mu_s2 = 1.0 / (spec[b].mu * s2); r.mu = spec[b].mu;
         s.fused_gx = fgx; s.fused_rc = frc; s.fused_gy = fgy;
         r.V = d_V[b]; r.m = d_m ? d_m[b] : nullptr;
         r.phi = d_phi ? d_phi[b] : nullptr;
         r.scratch = need_scratch ? ws + 5 * n : nullptr;
         r.vx = want_v ? d_vx[b] : nullptr; r.vy = want_v ? d_vy[b] : nullptr;
         r.ev = ctx->batch_events[b];
-        r.ctl = rk45::Controller(T, t_eval, nt);
+        r.ctl = rk45::Controller(spec[b].T, spec[b].t_eval, spec[b].nt);
     }
     // room-local helpers ------------------------------------------------------------------------------
     auto reduce_async = [&](BatchRoom &r, size_t off, int gx, int gy, int slot) {
@@ -842,7 +862,7 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
         Solver &s = r.s;
         switch (r.phase) {
         case BatchRoom::START: {
-            prep_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s.st>>>(r.V, r.m, prm->g, 1.0 / (prm->mu * s2), n, s.coef, s.y);
+            prep_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s.st>>>(r.V, r.m, r.g, r.inv_mu_s2, n, s.coef, s.y);
             s.launches++;
             Comb c{};
             c.y = s.y;
@@ -884,9 +904,9 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
                 const int kd = c.sample_column(e);
                 if (want_v && kd >= 1) {  // slice s = vels(sol.y[:, nt-1-s]) (optimals.py:200-204)
                     const double *ph = fused::sample_slice(c, e, r.phi, r.scratch, n);
-                    const int sl = nt - 1 - kd;
+                    const int sl = c.nt - 1 - kd;
                     dim3 grid((Nx - 2 + 63) / 64, (Ny - 2 + 3) / 4);
-                    vels_kernel<<<grid, NTHREADS, 0, s.st>>>(ph, Ny, Nx, prm->mu, prm->lim, 1.0 / (2 * ctx->dx), 1.0 / (2 * ctx->dy),
+                    vels_kernel<<<grid, NTHREADS, 0, s.st>>>(ph, Ny, Nx, r.mu, prm->lim, 1.0 / (2 * ctx->dx), 1.0 / (2 * ctx->dy),
                                                              r.vx + (size_t)sl * n_int, r.vy + (size_t)sl * n_int);
                     s.launches++;
                 }

@@ -7,13 +7,17 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
   * every member is an ordinary ``simulations.simulation`` whose randomness comes from its own
     ``np.random.RandomState(seed)`` -- the very stream ``np.random.seed(seed)`` gives the reference, so member i
     reproduces the stand-alone run with that seed bit for bit (tests/test_gpu_ensemble.py);
-  * the HJB fields of all members of a wave are solved by ONE ``oc_hjb_solve_batch`` call: one RK45 controller and
+  * the HJB fields of all members of a wave are solved by ONE ``oc_hjb_solve_multi`` call: one RK45 controller and
     one CUDA stream per member, the members' step kernels overlapping on the GPU;
   * the GCFM steps of the members advance in lock-step: every member's sweep is launched on its own stream
     (``oc_gcfm_step_launch``) before any is finished (``oc_gcfm_step_finish``), so the host's per-step work (RNG
     draws, exit bookkeeping) of one member overlaps the other members' kernels;
   * members are processed in waves sized to the GPU's memory (a 512^2 room with T = 20 s holds 2.1 GB of field
-    samples), and only the per-member results are kept.
+    samples), and only the per-member results are kept;
+  * ``configs``: every member may bring its own overrides of config.json (model parameters, ``dt``, re-solve
+    frequency, ...; one grid step for all).  Its HJB solves then run with its own sigma, mu, g and horizon inside the
+    same batched call (``oc_hjb_solve_multi``), its re-solves happen at its own steps, and it still equals the
+    stand-alone ``simulation(..., config=...)`` run bit for bit (tests/test_gpu_ensemble_params.py).
 """
 from __future__ import annotations
 
@@ -23,7 +27,7 @@ import io
 
 import numpy as np
 
-from . import _lib, simulations
+from . import _lib, optimals, simulations
 
 
 def shard(n_members: int, rank: int, world: int):
@@ -50,10 +54,25 @@ def _ctx_key(room_length, room_height, step):
     return (torch.cuda.current_device(), float(room_length), float(room_height), float(step))
 
 
-def plan_waves(members, bytes_per_member: int, budget_bytes: int, max_wave: int = 256):
-    """split the member list into waves that fit `budget_bytes` of device memory"""
-    per = max(1, min(max_wave, budget_bytes // max(bytes_per_member, 1)))
-    return [members[i:i + per] for i in range(0, len(members), per)]
+def plan_waves(members, bytes_per_member, budget_bytes: int, max_wave: int = 256):
+    """split the member list, in order, into waves that fit `budget_bytes` of device memory and hold at most `max_wave`
+    members; a member that does not fit on its own gets a wave of its own.  bytes_per_member: one count for all
+    members, or one count per member"""
+    if isinstance(bytes_per_member, (int, np.integer)):
+        bytes_per_member = [bytes_per_member] * len(members)
+    if len(bytes_per_member) != len(members):
+        raise ValueError("one byte count per member expected")
+    waves, cur, used = [], [], 0
+    for m, b in zip(members, bytes_per_member):
+        b = max(int(b), 1)
+        if cur and (len(cur) == max_wave or used + b > budget_bytes):
+            waves.append(cur)
+            cur, used = [], 0
+        cur.append(m)
+        used += b
+    if cur:
+        waves.append(cur)
+    return waves
 
 
 def gather_results(local: dict, group=None) -> dict:
@@ -75,10 +94,13 @@ class ensemble:
     ``evac_time`` (simulation time when the run stopped), ``steps``, ``inside`` (agents left inside: 0 = evacuation
     complete), ``exit_order`` (agent ids in exit order), ``exit_step`` (per agent, -1 = still inside),
     ``times`` (per-agent clocks, as evac_times() returns them), ``final`` (N,4: x, y, vx, vy) and ``hjb`` (solver
-    statistics per target set)."""
+    statistics per target set) and ``config`` (the member's effective configuration).
+
+    ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
+    ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``."""
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
-                 memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True):
+                 memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None):
         # chunk_rows: 0 = every room chunked as if it were alone (members are then bit-identical to stand-alone runs with
         # default settings, whatever the wave size); n > 0 = fixed; "wave" = planned for the wave size (fastest)
         self.chunk_plan_for_wave = chunk_rows == "wave"
@@ -91,6 +113,17 @@ class ensemble:
             self.rooms = list(rooms)
         else:
             self.rooms = [rooms] * len(self.seeds)
+        # the members' configurations, merged and checked before anything touches a GPU
+        base = optimals._load_config()
+        if configs is None:
+            self.overrides = [None] * len(self.seeds)
+        else:
+            self.overrides = list(configs)
+            if len(self.overrides) != len(self.seeds):
+                raise ValueError("one configuration per seed expected")
+        self.configs = [optimals._merge_config(base, o) if o is not None else base for o in self.overrides]
+        if len({c["grid_step"] for c in self.configs}) > 1:
+            raise ValueError("ensemble members must share grid_step (one grid for the batched solves)")
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -110,12 +143,13 @@ class ensemble:
         # a finished member's library context (device workspace, page-locked buffers, streams) serves the next member
         # of the same room size: a wave of 128 members otherwise pays 128 x (cudaMalloc + cudaMallocHost + frees) per pass
         room = simulations._load_room(self.rooms[idx])
-        step = simulations._load_config()["grid_step"]
+        step = self.configs[idx]["grid_step"]
         free = _CTX_POOL.get(_ctx_key(room["room_length"], room["room_height"], step))
         ctx = free.pop() if free else None
         return simulations.simulation(self.rooms[idx], self.T, recompute=self.recompute, record=self.record,
                                       field_storage=self.field_storage, fused=1, lookahead=False,
-                                      rng=np.random.RandomState(self.seeds[idx]), chunk_rows=self.chunk_rows, _ctx=ctx)
+                                      rng=np.random.RandomState(self.seeds[idx]), chunk_rows=self.chunk_rows,
+                                      config=self.overrides[idx], _ctx=ctx)
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -148,23 +182,26 @@ class ensemble:
         return ctx
 
     def _solve_wave(self, sims):
-        """simulation._solve_all for every member of the wave in one batched call per target set"""
+        """simulation._solve_all for the given members in one batched call per target set, each member with its own
+        sigma, mu, g, horizon and density"""
         import torch
         first = sims[0]
         sctx = self._solver_ctx(first)
-        d_ms = None
-        if first.simu_step > 0:
-            d_ms = [s._density_device(s.sigma_convolution) for s in sims]
+        # simulations.py:424-425: density * (simu_step > 0), per member
+        d_ms = [s._density_device(s.sigma_convolution) if s.simu_step > 0 else None for s in sims]
+        if all(m is None for m in d_ms):
+            d_ms = None
+        nts = [round((self.T - s.time) / s.dt) for s in sims]                  # optimals.py:140
+        if min(nts) < 1:
+            raise ValueError("Values in `t_eval` are not within `t_span`.")
         cells = 0
         for k, key in enumerate(first.targets):
             opts = [list(s.targets.values())[k] for s in sims]
-            nt = round((self.T - first.time) / first.dt)                    # optimals.py:140
-            if nt < 1:
-                raise ValueError("Values in `t_eval` are not within `t_span`.")
-            for o in opts:
+            for o, nt in zip(opts, nts):
                 if nt - 1 > o._n_slices:
                     raise IndexError("re-solve asks for more slices than the field was allocated for")
-            prm = opts[0]._prm
+            rooms = [dict(sigma=o.sigma, mu=o.mu, g=o.g, T=self.T, nt=nt) for o, nt in zip(opts, nts)]
+            prm = opts[0]._prm   # (rtol, atol, lim, chunk_rows: the same for every member)
             if self.chunk_plan_for_wave:
                 # chunk height planned for the whole wave (a 512^2 room alone would be cut into 16-row chunks to fill the
                 # GPU; 64 rooms side by side fill it with 64-row chunks and recompute far fewer halo rows).  The chunking
@@ -175,12 +212,14 @@ class ensemble:
             vel = self.field_storage == "velocity"
             import time as _t
             _t0 = _t.perf_counter()
-            res = sctx.hjb_solve_batch([o.d_V for o in opts], d_ms, prm, self.T, nt,
-                                             out_phi=None if vel else [o.d_phi for o in opts],
-                                             out_vx=[o.d_vx for o in opts] if vel else None,
-                                             out_vy=[o.d_vy for o in opts] if vel else None)
+            res = sctx.hjb_solve_multi([o.d_V for o in opts], d_ms, rooms, prm,
+                                       out_phi=None if vel else [o.d_phi for o in opts],
+                                       out_vx=[o.d_vx for o in opts] if vel else None,
+                                       out_vy=[o.d_vy for o in opts] if vel else None)
             self.stats["hjb_call_ms"] = self.stats.get("hjb_call_ms", 0.0) + (_t.perf_counter() - _t0) * 1e3
-            for o, r, s in zip(opts, res, sims):
+            self.stats["hjb_calls"] = self.stats.get("hjb_calls", 0) + 1
+            self.stats["hjb_call_rooms"] = self.stats.get("hjb_call_rooms", 0) + len(opts)
+            for o, r, s, nt in zip(opts, res, sims, nts):
                 o.t, o.nt_opt, o.last_stats = s.time, nt, r["stats"]
                 o._h_vx = o._h_vy = None
                 if r["stats"]["status"] == -1:
@@ -222,15 +261,17 @@ class ensemble:
             batch = _lib.GcfmBatch([dict(ctx=s._ctx, prm=s._gcfm_prm, state=s._state, vdes=s._d_vdes, key_id=s._d_key,
                                          keys=s._keys(), rng=s._np_random) for s in sims], sweep_ctas=ctas_b)
         while live:
-            first = sims[live[0]]
-            rebind = False
-            if self.recompute and first.simu_step % first.recompute_step == 0 and first.simu_step > 0:
-                self.stats["cell_updates"] += self._solve_wave([sims[q] for q in live])
-                rebind = True
+            # simulations.py:421: the members due for a re-solve at their own step (their own dt and recompute
+            # frequency), solved together; the others keep their fields
+            due = [q for q in live if self.recompute and sims[q].simu_step % sims[q].recompute_step == 0
+                   and sims[q].simu_step > 0]
+            rebind = bool(due)
+            if due:
+                self.stats["cell_updates"] += self._solve_wave([sims[q] for q in due])
             tl0 = time.perf_counter()
             if batch is not None:
                 if rebind:
-                    for q in live:
+                    for q in due:
                         batch.members[q]["keys"] = sims[q]._keys()
                 for q in live:
                     s = sims[q]
@@ -265,7 +306,7 @@ class ensemble:
             self.results[i] = dict(seed=self.seeds[i], evac_time=s.time, steps=s.simu_step, inside=int(s.inside), N=s.N,
                                    exit_order=np.array(s._exit_order, dtype=np.int64), exit_step=s._exit_step.copy(),
                                    times=np.array(s._h_timev, dtype=float), final=np.array(s._h_now, dtype=float),
-                                   hjb={k: o.last_stats for k, o in s.targets.items()})
+                                   hjb={k: o.last_stats for k, o in s.targets.items()}, config=self.configs[i])
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3
@@ -297,10 +338,11 @@ class ensemble:
         if not self.mine:
             return gather_results({}) if gather else {}
         probe = simulations._load_room(self.rooms[self.mine[0]])
-        cfg = simulations._load_config()
-        Ny, Nx = _lib.grid_shape(probe["room_length"], probe["room_height"], cfg["grid_step"])
+        cfgs = [self.configs[i] for i in self.mine]
+        Ny, Nx = _lib.grid_shape(probe["room_length"], probe["room_height"], cfgs[0]["grid_step"])
         n_keys = len({' or '.join(b[5:]) for b in probe["initial_boxes"].values()})
-        per = field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage)
+        # (a member's field samples: round(T/dt) slices of its own dt)
+        per = [field_bytes_per_member(Ny, Nx, self.T, c["dt"], n_keys, self.field_storage) for c in cfgs]
         budget = self.memory_budget
         if budget is None:
             free, _total = torch.cuda.mem_get_info()

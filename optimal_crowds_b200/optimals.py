@@ -31,6 +31,23 @@ def _load_config():
     raise FileNotFoundError("config.json")
 
 
+def _merge_config(base, overrides):
+    """``base`` (a loaded config.json) with ``overrides`` applied: a new dict, ``base`` is left as it is.  Nested dicts
+    (``hjb_params``) are merged key by key.  A key that ``base`` does not have raises KeyError: a misspelt parameter
+    must not run the default silently."""
+    merged = dict(base)
+    for k, v in (overrides or {}).items():
+        if k not in base:
+            raise KeyError(f"unknown configuration key {k!r} (config.json has {sorted(base)})")
+        if isinstance(base[k], dict):
+            if not isinstance(v, dict):
+                raise TypeError(f"configuration key {k!r} takes a dict of overrides")
+            merged[k] = _merge_config(base[k], v)
+        else:
+            merged[k] = v
+    return merged
+
+
 def _load_room(room):
     if isinstance(room, dict):
         return room

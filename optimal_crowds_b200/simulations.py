@@ -21,7 +21,7 @@ import os
 import numpy as np
 
 from . import _crowd, _lib, _rng, optimals, pedestrians
-from .optimals import _load_config, _load_room
+from .optimals import _load_config, _load_room, _merge_config
 
 warnings.filterwarnings("ignore")  # simulations.py:15
 
@@ -127,7 +127,7 @@ class simulation:
     TRACK_CHUNK = 64  # steps per block of the device-resident trajectory record
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
-                 rng=None, chunk_rows=0, band=False, shard_keys=False, _ctx=None):
+                 rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -139,11 +139,15 @@ class simulation:
         in its band, and runs the (replicated, deterministic) sweep; every rank must use the same seed),
         ``shard_keys`` (True: the target sets -- one HJB field each, simulations.py:113-121 -- are dealt round-robin to the
         ranks of torch.distributed: a rank solves and stores only its keys' fields and evaluates the field samples / wall
-        forces of the agents heading for them; merge and sweep as for ``band``)."""
+        forces of the agents heading for them; merge and sweep as for ``band``), ``config`` (a dict of overrides of
+        config.json, e.g. ``{"dt": 0.01, "hjb_params": {"g": -0.01}}``: nested ``hjb_params`` are merged key by key, a
+        key config.json does not have raises KeyError; ``_config`` is the effective configuration)."""
         import torch
         self._np_random = rng if rng is not None else np.random
         self.recompute = recompute
         var_config = _load_config()       # simulations.py:42
+        if config is not None:
+            var_config = _merge_config(var_config, config)
         var_room = _load_room(room)       # simulations.py:47
         self._config, self._room = var_config, var_room
         self.room_length = var_room['room_length']
