@@ -166,25 +166,43 @@ int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const *d_V, const
                        const oc_hjb_params *prm, double T, const double *t_eval, int nt, double *const *d_phi,
                        double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats, void *stream);
 
-/* What one room of oc_hjb_solve_multi does not share with the others: its model parameters (sigma, mu, g of its
- * config.json, optimals.py:66-70) and its horizon.  d_phi[b] holds rooms[b].nt slices, d_vx[b] / d_vy[b] nt-1. */
+/* What one room of oc_hjb_solve_multi / oc_hjb_solve_grids does not share with the others: its model parameters (sigma,
+ * mu, g of its config.json, optimals.py:66-70), its horizon and its chunking.  d_phi[b] holds rooms[b].nt slices,
+ * d_vx[b] / d_vy[b] nt-1. */
 typedef struct {
     double sigma, mu, g;        /* config.json hjb_params of this room */
     double T;                   /* t_span = (T, 0) */
     const double *t_eval;       /* host, nt decreasing values: np.linspace(T, 0, nt) (optimals.py:194) */
     int nt;
-    int pad_;
+    int chunk_rows;             /* rows per CTA chunk of this room's fused step (>= 0): 0 = prm->chunk_rows, and when that
+                                   is 0 too, the plan a stand-alone oc_hjb_solve of the room's grid makes.  The room's
+                                   result is bit-identical to oc_hjb_solve with prm->chunk_rows set to the value used */
 } oc_hjb_room;
 /* The batched solve with per-room model parameters and horizons (ensembles whose members have their own
  * configuration).  Each room's result is bit-identical to oc_hjb_solve of that room alone with prm's sigma, mu, g
- * replaced by the room's and the room's (T, t_eval, nt).  Shared by all rooms: prm->rtol, atol, lim and chunk_rows (the
- * launch grid); prm->sigma, mu and g are not read.  Step attempts of rooms with different nt still share the batched
+ * replaced by the room's and the room's (T, t_eval, nt).  Shared by all rooms: prm->rtol, atol, lim and, for rooms whose
+ * own chunk_rows is 0, prm->chunk_rows; prm->sigma, mu and g are not read.  Step attempts of rooms with different nt still share the batched
  * launches, which are grouped by the number of samples per launch.  Without d_phi the limit of 6 t_eval samples per
  * attempt applies to every room.  OC_ERR_ARG if rooms is NULL, a room's t_eval is NULL or its nt < 1, sigma or mu is not
- * a finite positive number, or g is not finite.  Everything else as oc_hjb_solve_batch. */
+ * a finite positive number, or g is not finite.  A negative prm->chunk_rows means the grid's own plan, as in oc_hjb_solve.
+ * Everything else as oc_hjb_solve_batch. */
 int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const *d_V, const double *const *d_m,
                        const oc_hjb_room *rooms, const oc_hjb_params *prm, double *const *d_phi, double *const *d_vx,
                        double *const *d_vy, oc_hjb_stats *stats, void *stream);
+/* The batched solve over rooms of different grids (ensembles of different room layouts): room b is solved on the grid
+ * of the context grids[b] -- its Ny, Nx, dx, dy -- and is bit-identical to oc_hjb_solve(grids[b], ...) with the room's
+ * sigma, mu, g, horizon and chunk_rows.  d_V[b], d_m[b] and the outputs are shaped by that grid: (Ny,Nx), d_phi[b]
+ * (nt,Ny,Nx), d_vx[b] / d_vy[b] (nt-1,Ny-2,Nx-2).  `ctx` owns everything the call uses (workspace, streams, events,
+ * page-locked sums, final-reduction slots); the grid contexts are only read.  Step attempts of rooms of every shape share
+ * the batched launches (one flattened grid of all their CTAs, up to 24 rooms per launch).  A negative chunk_rows is an
+ * error here (the room's or prm's; oc_hjb_solve_multi keeps treating a negative prm->chunk_rows as 0).  oc_hjb_solve_multi is this
+ * call with grids[b] = ctx.  OC_ERR_ARG, besides the cases of oc_hjb_solve_multi, if grids or an entry is NULL, a grid
+ * lives on another device than ctx, a grid is too small for the stage-fused kernel (Ny <= 7 or Nx <= 9), or a
+ * chunk_rows (the room's or prm's) is negative. */
+int oc_hjb_solve_grids(oc_ctx *ctx, int n_rooms, oc_ctx *const *grids, const double *const *d_V,
+                       const double *const *d_m, const oc_hjb_room *rooms, const oc_hjb_params *prm,
+                       double *const *d_phi, double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats,
+                       void *stream);
 
 /* ------------------------------------------------------------------ row-decomposed HJB solve (multi-GPU)
  * The grid of the context is split into bands of rows (SURVEY.md section 8e).  Two modes:

@@ -60,7 +60,7 @@ class HjbStats(C.Structure):
 
 class HjbRoom(C.Structure):
     _fields_ = [("sigma", C.c_double), ("mu", C.c_double), ("g", C.c_double), ("T", C.c_double), ("t_eval", dp),
-                ("nt", C.c_int), ("pad_", C.c_int)]
+                ("nt", C.c_int), ("chunk_rows", C.c_int)]
 
 
 class BandCfg(C.Structure):
@@ -87,7 +87,7 @@ _lib = None
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
            "oc_hjb_solve", "oc_hjb_rhs", "oc_hjb_vels", "oc_wall_tiles_bytes", "oc_wall_tiles", "oc_gcfm_step",
            "oc_wall_force", "oc_pair_force", "oc_density", "oc_gcfm_last_ms", "oc_dist_unique_id", "oc_dist_init",
-           "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_gcfm_step_launch",
+           "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_hjb_solve_grids", "oc_gcfm_step_launch",
            "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run"]
 
 
@@ -144,6 +144,8 @@ def load():
                                        vpp, vpp, vpp, C.POINTER(HjbStats), C.c_void_p]
     lib.oc_hjb_solve_multi.argtypes = [C.c_void_p, C.c_int, vpp, vpp, C.POINTER(HjbRoom), C.POINTER(HjbParams), vpp, vpp,
                                        vpp, C.POINTER(HjbStats), C.c_void_p]
+    lib.oc_hjb_solve_grids.argtypes = [C.c_void_p, C.c_int, vpp, vpp, vpp, C.POINTER(HjbRoom), C.POINTER(HjbParams), vpp,
+                                       vpp, vpp, C.POINTER(HjbStats), C.c_void_p]
     lib.oc_upload.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]
     lib.oc_dist_unique_id.argtypes = [C.c_void_p]
     lib.oc_dist_init.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int]
@@ -211,6 +213,19 @@ def _batch_results(rc, st, out_phi, out_vx, out_vy):
     return [{"stats": st[q].asdict(), "phi": out_phi[q] if out_phi is not None else None,
              "vx": out_vx[q] if out_vx is not None else None, "vy": out_vy[q] if out_vx is not None else None,
              "rc": rc if st[q].status == -1 else 0} for q in range(len(st))]
+
+
+def _room_spec(rooms, B):
+    """oc_hjb_room entries of dict(sigma, mu, g, T, nt[, chunk_rows]) rooms, t_eval = np.linspace(T, 0, nt) as
+    optimals.py:194 builds it; returns the array and the t_eval arrays it points to (alive until the call returns)"""
+    if len(rooms) != B:
+        raise ValueError("one rooms entry per room expected")
+    t_evals = [np.linspace(r["T"], 0, int(r["nt"])) for r in rooms]
+    spec = (HjbRoom * B)()
+    for q, (r, te) in enumerate(zip(rooms, t_evals)):
+        spec[q] = HjbRoom(float(r["sigma"]), float(r["mu"]), float(r["g"]), float(r["T"]),
+                          _hp(te) if len(te) else None, int(r["nt"]), int(r.get("chunk_rows", 0)))
+    return spec, t_evals
 
 
 def grid_shape(room_length, room_height, grid_step):
@@ -386,7 +401,7 @@ class Context:
         (phi slices (nt,Ny,Nx) are allocated when no output is given).  Returns a list of per-room dicts."""
         B = len(Vs)
         t_eval = np.linspace(T, 0, nt)
-        out_phi, out_vx, out_vy = self._batch_outputs([nt] * B, out_phi, out_vx, out_vy, want_vel)
+        out_phi, out_vx, out_vy = self._batch_outputs([self] * B, [nt] * B, out_phi, out_vx, out_vy, want_vel)
         st = (HjbStats * B)()
         rc = load().oc_hjb_solve_batch(self.h, B, _ptrs(Vs, B), _ptrs(ms, B), C.byref(prm), float(T), _hp(t_eval),
                                        int(nt), _ptrs(out_phi, B), _ptrs(out_vx, B), _ptrs(out_vy, B), st, _stream())
@@ -398,27 +413,40 @@ class Context:
         shared rtol, atol, lim and chunk_rows (its sigma, mu and g are not used).  Outputs as hjb_solve_batch, sized by
         each room's nt."""
         B = len(Vs)
-        if len(rooms) != B:
-            raise ValueError("one rooms entry per room expected")
-        nts = [int(r["nt"]) for r in rooms]
-        t_evals = [np.linspace(r["T"], 0, nt) for r, nt in zip(rooms, nts)]   # alive until the call returns
-        spec = (HjbRoom * B)()
-        for q, (r, te) in enumerate(zip(rooms, t_evals)):
-            spec[q] = HjbRoom(float(r["sigma"]), float(r["mu"]), float(r["g"]), float(r["T"]),
-                              _hp(te) if len(te) else None, nts[q], 0)
-        out_phi, out_vx, out_vy = self._batch_outputs(nts, out_phi, out_vx, out_vy, want_vel)
+        spec, keep = _room_spec(rooms, B)
+        out_phi, out_vx, out_vy = self._batch_outputs([self] * B, [int(r["nt"]) for r in rooms], out_phi, out_vx, out_vy,
+                                                      want_vel)
         st = (HjbStats * B)()
         rc = load().oc_hjb_solve_multi(self.h, B, _ptrs(Vs, B), _ptrs(ms, B), spec, C.byref(prm), _ptrs(out_phi, B),
                                        _ptrs(out_vx, B), _ptrs(out_vy, B), st, _stream())
         return _batch_results(rc, st, out_phi, out_vx, out_vy)
 
-    def _batch_outputs(self, nts, out_phi, out_vx, out_vy, want_vel):
-        """the outputs of a batched solve: phi slices (nt,Ny,Nx) per room when no output is given"""
+    def hjb_solve_grids(self, grids, Vs, ms, rooms, prm: HjbParams, out_phi=None, out_vx=None, out_vy=None,
+                        want_vel=False):
+        """hjb_solve_multi over rooms of different grids (oc_hjb_solve_grids): room q is solved on the grid of the
+        Context grids[q] (its shape and spacing); this context only lends the workspace, streams and result slots.
+        rooms: dict(sigma, mu, g, T, nt) and optionally chunk_rows (0 = prm.chunk_rows, then the room's own plan).
+        Outputs as hjb_solve_multi, each sized by its room's grid and nt."""
+        B = len(Vs)
+        if len(grids) != B:
+            raise ValueError("one grid per room expected")
+        spec, keep = _room_spec(rooms, B)
+        out_phi, out_vx, out_vy = self._batch_outputs(grids, [int(r["nt"]) for r in rooms], out_phi, out_vx, out_vy,
+                                                      want_vel)
+        st = (HjbStats * B)()
+        hs = (C.c_void_p * B)(*[g.h.value for g in grids])
+        rc = load().oc_hjb_solve_grids(self.h, B, hs, _ptrs(Vs, B), _ptrs(ms, B), spec, C.byref(prm), _ptrs(out_phi, B),
+                                       _ptrs(out_vx, B), _ptrs(out_vy, B), st, _stream())
+        return _batch_results(rc, st, out_phi, out_vx, out_vy)
+
+    @staticmethod
+    def _batch_outputs(grids, nts, out_phi, out_vx, out_vy, want_vel):
+        """the outputs of a batched solve: phi slices (nt,Ny,Nx) of each room's grid when no output is given"""
         if out_phi is None and not (want_vel or out_vx is not None):
-            out_phi = [self.empty(nt, self.Ny, self.Nx) for nt in nts]
+            out_phi = [g.empty(nt, g.Ny, g.Nx) for g, nt in zip(grids, nts)]
         if want_vel and out_vx is None:
-            out_vx = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for nt in nts]
-            out_vy = [self.empty(max(nt - 1, 0), self.Ny - 2, self.Nx - 2) for nt in nts]
+            out_vx = [g.empty(max(nt - 1, 0), g.Ny - 2, g.Nx - 2) for g, nt in zip(grids, nts)]
+            out_vy = [g.empty(max(nt - 1, 0), g.Ny - 2, g.Nx - 2) for g, nt in zip(grids, nts)]
         return out_phi, out_vx, out_vy
 
     def plan_chunk_rows(self, copies=1):

@@ -649,16 +649,17 @@ extern "C" int oc_hjb_solve(oc_ctx *ctx, const double *d_V, const double *d_m, c
 }
 
 // ---------------------------------------------------------------------------------------------------
-// Batched solve for ensembles of independent rooms on one grid shape (BASELINE configs[4], SURVEY 8e).
+// Batched solve for ensembles of independent rooms (BASELINE configs[4], SURVEY 8e).
 // Every room keeps its own RK45 controller (t, h, accept/reject, t_eval cursor: the reference integrates each
 // room separately, optimals.py:193-196) and its own CUDA stream; a room's step attempt is one launch of the
 // stage-fused kernel per 6 samples followed by the fixed-order reduction, exactly the launches oc_hjb_solve issues, so
-// every room's result is bit-identical to solving it alone (with the same prm->chunk_rows).  The host serves the rooms
+// every room's result is bit-identical to solving it alone (with the same chunk_rows).  The host serves the rooms
 // round-robin: while it reads room b's error norm and enqueues b's next attempt, the other rooms' kernels keep
 // the GPU busy -- small grids (512^2: ~10 us of device work per attempt) are launch-latency bound one at a time.
-// oc_hjb_solve_multi is the one implementation: every room brings its own sigma, mu, g (prep_kernel's coefficients, the
-// diffusion constant of the step kernel, vels_kernel's mu -- all kernel arguments already) and its own horizon (its
-// controller); oc_hjb_solve_batch gives every room the same ones.
+// oc_hjb_solve_grids is the one implementation: every room brings its own grid (shape and spacing: every size, tile
+// grid, workspace offset and norm below is the room's), its own sigma, mu, g (prep_kernel's coefficients, the diffusion
+// constant of the step kernel, vels_kernel's mu -- all kernel arguments already) and its own horizon (its controller);
+// oc_hjb_solve_multi gives every room the context's grid, oc_hjb_solve_batch also the same parameters.
 namespace {
 
 struct BatchRoom {
@@ -668,6 +669,9 @@ struct BatchRoom {
     double *phi = nullptr, *scratch = nullptr, *vx = nullptr, *vy = nullptr;  // scratch: NE_MAX slices, without phi
     double *rs_d = nullptr, *rs_h = nullptr;  // row-group sums (device / pinned host), 3 regions of `rs_stride`
     int rs_stride = 0;
+    size_t n_int = 0;                    // interior cells: one vx / vy slice
+    double sqrt_n = 0, dx = 0, dy = 0;   // the room's grid
+    bool final_in_kernel = false;        // its fused step finishes the error sum in the launch (fused_gy small enough)
     cudaEvent_t ev = nullptr;
     unsigned long long wait_seq = 0;     // sequence number of the step attempt in flight (in-kernel final reduction)
     rk45::Controller ctl;                // the room's horizon: T, t_eval, nt
@@ -692,38 +696,72 @@ extern "C" int oc_hjb_solve_batch(oc_ctx *ctx, int n_rooms, const double *const 
 extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const *d_V, const double *const *d_m,
                                   const oc_hjb_room *spec, const oc_hjb_params *prm, double *const *d_phi,
                                   double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats, void *stream) {
+    OC_ARG(ctx && prm && n_rooms >= 1, "NULL argument");
+    std::vector<oc_ctx *> grids(n_rooms, ctx);
+    oc_hjb_params p = *prm;
+    if (p.chunk_rows < 0) p.chunk_rows = 0;  // as oc_hjb_solve: a negative chunk_rows means the grid's own plan
+    return oc_hjb_solve_grids(ctx, n_rooms, grids.data(), d_V, d_m, spec, &p, d_phi, d_vx, d_vy, stats, stream);
+}
+
+extern "C" int oc_hjb_solve_grids(oc_ctx *ctx, int n_rooms, oc_ctx *const *grids, const double *const *d_V,
+                                  const double *const *d_m, const oc_hjb_room *spec, const oc_hjb_params *prm,
+                                  double *const *d_phi, double *const *d_vx, double *const *d_vy, oc_hjb_stats *stats,
+                                  void *stream) {
     OC_ARG(ctx && d_V && prm && stats && n_rooms >= 1, "NULL argument");
+    OC_ARG(grids, "grids (one context per room) required");
     OC_ARG(spec, "rooms (per-room parameters and horizons) required");
+    OC_ARG(prm->chunk_rows >= 0, "chunk_rows must not be negative");
     for (int b = 0; b < n_rooms; b++) {
         const oc_hjb_room &p = spec[b];
         OC_ARG(p.nt >= 1 && p.t_eval, "t_eval required");
         OC_ARG(std::isfinite(p.sigma) && p.sigma > 0, "sigma must be a finite positive number");
         OC_ARG(std::isfinite(p.mu) && p.mu > 0, "mu must be a finite positive number");
         OC_ARG(std::isfinite(p.g), "g must be finite");
+        OC_ARG(p.chunk_rows >= 0, "a room's chunk_rows must not be negative");
+        OC_ARG(grids[b], "NULL grid");
+        OC_ARG(grids[b]->device == ctx->device, "a room's grid lives on another device than ctx");
+        OC_ARG(grids[b]->Ny > fused::HY + 1 && grids[b]->Nx > fused::HX + 1, "grid too small for the stage-fused kernel");
     }
     OC_ARG(d_phi || (d_vx && d_vy), "an output (d_phi or d_vx,d_vy) is required");
-    const int Ny = ctx->Ny, Nx = ctx->Nx;
-    OC_ARG(Ny > fused::HY + 1 && Nx > fused::HX + 1, "grid too small for the stage-fused kernel");
     OC_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t main_st = (cudaStream_t)stream;
-    const size_t n = (size_t)Ny * Nx, n_int = (size_t)(Ny - 2) * (Nx - 2);
-    const int nbx = (Nx + TX - 1) / TX, nby = (Ny + TY - 1) / TY;
     int n_sm = 148;
     cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, ctx->device);
-    const int fgx = (Nx + fused::VX - 1) / fused::VX;
-    const int frc = prm->chunk_rows > 0 ? prm->chunk_rows : fused::plan_chunk_rows(Nx, Ny, n_sm, 1, 0);
-    const int fgy = (Ny + frc - 1) / frc;
-    // per room: coef, y, y_new, f, f_new (+ NE_MAX phi slices when only velocities are kept) ; partial sums
+    // per room: coef, y, y_new, f, f_new (+ NE_MAX phi slices when only velocities are kept) ; partial sums ; row sums
     const bool need_scratch = !d_phi;
-    // (even numbers of doubles: every room's arrays stay 16-byte aligned for the TMA descriptors)
-    const size_t np = ((std::max((size_t)2 * nbx * nby, (size_t)fgx * fgy) + 8) + 1) & ~(size_t)1;
-    const int rs_stride = ((std::max(nby, fgy) + 8) + 1) & ~1;
-    const size_t per_room = (5 + (need_scratch ? fused::NE_MAX : 0)) * n + np + 3 * (size_t)rs_stride;
-    int rc = oc_ensure_buffer(ctx->batch_ws, ctx->batch_ws_bytes, per_room * n_rooms * sizeof(double), false,
+    const bool want_v = d_vx && d_vy;
+    std::vector<BatchRoom> rooms(n_rooms);
+    std::vector<size_t> ws_off(n_rooms + 1, 0);
+    std::vector<size_t> pin_off(n_rooms + 1, 0), np_room(n_rooms);
+    bool any_final = false;
+    for (int b = 0; b < n_rooms; b++) {
+        const oc_ctx *gr = grids[b];
+        BatchRoom &r = rooms[b];
+        Solver &s = r.s;
+        // the expressions of oc_hjb_solve, with the room's grid
+        s.Ny = gr->Ny; s.Nx = gr->Nx;
+        s.n = (size_t)s.Ny * s.Nx;
+        r.n_int = (size_t)(s.Ny - 2) * (s.Nx - 2);
+        s.nbx = (s.Nx + TX - 1) / TX; s.nby = (s.Ny + TY - 1) / TY;
+        const int rc_rows = spec[b].chunk_rows > 0 ? spec[b].chunk_rows : prm->chunk_rows;
+        s.fused_plan(n_sm, rc_rows);
+        r.dx = gr->dx; r.dy = gr->dy;
+        r.sqrt_n = std::sqrt((double)s.n);
+        r.final_in_kernel = s.fused_gy <= fused::MAX_FINAL_ROWS;
+        any_final = any_final || r.final_in_kernel;
+        // (even numbers of doubles: every room's arrays stay 16-byte aligned for the TMA descriptors)
+        const size_t np = np_room[b] = ((std::max((size_t)2 * s.nbx * s.nby, (size_t)s.fused_gx * s.fused_gy) + 8) + 1) & ~(size_t)1;
+        r.rs_stride = ((std::max(s.nby, s.fused_gy) + 8) + 1) & ~1;
+        const size_t per_room = (5 + (need_scratch ? fused::NE_MAX : 0)) * s.n + np + 3 * (size_t)r.rs_stride;
+        ws_off[b + 1] = ws_off[b] + ((per_room + 1) & ~(size_t)1);
+        pin_off[b + 1] = pin_off[b] + 3 * (size_t)r.rs_stride;
+    }
+    int rc = oc_ensure_buffer(ctx->batch_ws, ctx->batch_ws_bytes, ws_off[n_rooms] * sizeof(double), false,
                               "batched HJB workspace");
     if (rc) return rc;
-    const size_t pin_need = (size_t)3 * rs_stride * n_rooms * sizeof(double);
-    if ((rc = oc_ensure_buffer(ctx->batch_pinned, ctx->batch_pinned_bytes, pin_need, true, "batched HJB host sums"))) return rc;
+    if ((rc = oc_ensure_buffer(ctx->batch_pinned, ctx->batch_pinned_bytes, pin_off[n_rooms] * sizeof(double), true,
+                               "batched HJB host sums")))
+        return rc;
     constexpr int MAX_STREAMS = 32;
     const int n_streams = std::min(n_rooms, MAX_STREAMS);
     while ((int)ctx->batch_streams.size() < n_streams) {
@@ -742,27 +780,23 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
     OC_CUDA(cudaEventRecord(ev_in, main_st));
     for (int q = 0; q < n_streams; q++) OC_CUDA(cudaStreamWaitEvent(ctx->batch_streams[q], ev_in, 0));
 
-    const double rtol = prm->rtol, atol = prm->atol, sqrt_n = std::sqrt((double)n);
-    const bool want_v = d_vx && d_vy;
-    const bool final_in_kernel = fgy <= fused::MAX_FINAL_ROWS;
-    if (final_in_kernel && (rc = ensure_final_reduce(ctx, n_rooms))) return rc;
-    std::vector<BatchRoom> rooms(n_rooms);
+    const double rtol = prm->rtol, atol = prm->atol;
+    if (any_final && (rc = ensure_final_reduce(ctx, n_rooms))) return rc;
     for (int b = 0; b < n_rooms; b++) {
         BatchRoom &r = rooms[b];
         OC_ARG(d_V[b] && (!d_phi || d_phi[b]) && (!want_v || (d_vx[b] && d_vy[b])), "NULL room pointer");
-        double *ws = ctx->batch_ws + per_room * b;
+        double *ws = ctx->batch_ws + ws_off[b];
         Solver &s = r.s;
-        s.ctx = ctx; s.st = ctx->batch_streams[b % n_streams]; s.Ny = Ny; s.Nx = Nx; s.n = n; s.nbx = nbx; s.nby = nby;
+        const size_t n = s.n;
+        s.ctx = ctx; s.st = ctx->batch_streams[b % n_streams];
         s.coef = ws; s.y = ws + n; s.ynew = ws + 2 * n; s.K[0] = ws + 3 * n; s.K[6] = ws + 4 * n;
         s.K[1] = s.K[6];  // f(y0 + h0 f0) of select_initial_step lives in the (still unused) f_new array
         s.partial = ws + (5 + (need_scratch ? fused::NE_MAX : 0)) * n;
-        r.rs_d = s.partial + np;
-        r.rs_h = ctx->batch_pinned + (size_t)3 * rs_stride * b;
-        r.rs_stride = rs_stride;
+        r.rs_d = s.partial + np_room[b];
+        r.rs_h = ctx->batch_pinned + pin_off[b];
         const double s2 = spec[b].sigma * spec[b].sigma;   // the expressions of oc_hjb_solve, with the room's values
-        s.diff_over_dxdy = (-0.5 * s2) / (ctx->dx * ctx->dy);
+        s.diff_over_dxdy = (-0.5 * s2) / (r.dx * r.dy);
         r.g = spec[b].g; r.inv_mu_s2 = 1.0 / (spec[b].mu * s2); r.mu = spec[b].mu;
-        s.fused_gx = fgx; s.fused_rc = frc; s.fused_gy = fgy;
         r.V = d_V[b]; r.m = d_m ? d_m[b] : nullptr;
         r.phi = d_phi ? d_phi[b] : nullptr;
         r.scratch = need_scratch ? ws + 5 * n : nullptr;
@@ -784,29 +818,34 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
         return s;
     };
     // Batched launches: the step attempts that become ready during one polling sweep are grouped by their number of
-    // dense-output samples NE and launched together, up to fused::BATCH_MAX rooms per launch (blockIdx.z = room), instead
-    // of one launch per room: 512^2 rooms need ~10 us of device work per attempt, less than a launch round trip.  Only
-    // with phi output (velocity-only storage converts scratch slices on the room's own stream) and with the in-kernel
-    // final reduction; a room's arithmetic is unchanged (same kernel body, same chunking, same reduction order).
-    const bool batched = d_phi != nullptr && final_in_kernel && !getenv("OC_BATCH_PER_ROOM");
-    std::vector<BatchRoom *> buckets[fused::NE_MAX + 1];
+    // dense-output samples NE and their staging variant (TMA for even Nx, LDGSTS otherwise) and launched together, up to
+    // fused::BATCH_MAX rooms of any grid shapes per launch (a flattened grid of all their CTAs; fewer when the launch's
+    // CTA-to-room table cannot describe them, see fused::set_batch_table), instead of one launch per
+    // room: 512^2 rooms need ~10 us of device work per attempt, less than a launch round trip.  Only with phi output
+    // (velocity-only storage converts scratch slices on the room's own stream) and for rooms with the in-kernel final
+    // reduction; a room's arithmetic is unchanged (same kernel body, same chunking, same reduction order).
+    const bool batched = d_phi != nullptr && !getenv("OC_BATCH_PER_ROOM");
+    std::vector<BatchRoom *> buckets[fused::NE_MAX + 1][2];
     std::vector<fused::BatchArgs> host_ba(1);
     int bucket_launches = 0;
     auto flush = [&]() -> int {
         for (int ne = 0; ne <= fused::NE_MAX; ne++) {
-            auto &bk = buckets[ne];
-            for (size_t off = 0; off < bk.size(); off += fused::BATCH_MAX) {
-                const int nb = (int)std::min<size_t>(fused::BATCH_MAX, bk.size() - off);
-                for (int q = 0; q < nb; q++) {
-                    BatchRoom &r = *bk[off + q];
-                    fused::set_tensor_maps(r.fa, Ny, &r.s.maps);
-                    host_ba[0].a[q] = r.fa;
+            for (int bulk = 0; bulk < 2; bulk++) {
+                auto &bk = buckets[ne][bulk];
+                for (size_t off = 0; off < bk.size();) {
+                    int nb = (int)std::min<size_t>(fused::BATCH_MAX, bk.size() - off);
+                    int ngx[fused::BATCH_MAX], ngy[fused::BATCH_MAX];
+                    for (int q = 0; q < nb; q++) { ngx[q] = bk[off + q]->s.fused_gx; ngy[q] = bk[off + q]->s.fused_gy; }
+                    int ctas;
+                    while ((ctas = fused::set_batch_table(host_ba[0], nb, ngx, ngy)) == 0) nb--;
+                    for (int q = 0; q < nb; q++) host_ba[0].a[q] = bk[off + q]->fa;
+                    cudaStream_t st = ctx->batch_streams[(bucket_launches++) % n_streams];
+                    OC_CUDA(fused::launch_batch(ne, bulk != 0, host_ba[0], ctas, st));
+                    rooms[0].s.launches++;
+                    off += nb;
                 }
-                cudaStream_t st = ctx->batch_streams[(bucket_launches++) % n_streams];
-                OC_CUDA(fused::launch_batch(ne, host_ba[0], nb, dim3(fgx, fgy), st));
-                rooms[0].s.launches++;
+                bk.clear();
             }
-            bk.clear();
         }
         return OC_OK;
     };
@@ -818,8 +857,8 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
         Solver &s = r.s;
         fa.y = s.y; fa.k1 = s.K[0]; fa.coef = s.coef; fa.ynew = s.ynew; fa.k7 = s.K[6]; fa.partial = s.partial;
         fa.A = s.diff_over_dxdy; fa.rtol = rtol; fa.atol = atol;
-        fa.Ny = Ny; fa.Nx = Nx; fa.RC = frc;
-        fa.row_base = 0; fa.own0 = 0; fa.own1 = Ny; fa.phi_row_base = 0;
+        fa.Ny = s.Ny; fa.Nx = s.Nx; fa.RC = s.fused_rc;
+        fa.row_base = 0; fa.own0 = 0; fa.own1 = s.Ny; fa.phi_row_base = 0;
         // the samples this attempt emits if accepted, NE_MAX per launch; with more than NE_MAX samples inside one
         // step (only when h >> dt) the step is simply launched again for the remaining samples: the re-launch
         // recomputes identical y_new / f_new / error sums
@@ -827,19 +866,20 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
             oc::set_error("batched solve without a phi output supports at most %d samples per step", fused::NE_MAX);
             return OC_ERR_ARG;
         }
-        // an attempt waits in an NE bucket only when ALL its samples fit one launch.  The launches of a longer attempt
+        // an attempt waits in a bucket only when ALL its samples fit one launch.  The launches of a longer attempt
         // share the room's ticket counter and result slot, so they must not overlap: they go out in order on the
         // room's own stream (the sequence OC_BATCH_PER_ROOM gives every attempt).
-        const bool to_bucket = batched && c.n_emit() <= fused::NE_MAX;
+        const bool to_bucket = batched && r.final_in_kernel && c.n_emit() <= fused::NE_MAX;
         int e0 = 0;
         do {
             const int ne = std::min(c.n_emit() - e0, fused::NE_MAX);
             // without a phi output the samples go to the room's scratch slices (velocities are derived on accept)
-            fused::set_attempt(fa, c, e0, ne, r.phi, r.scratch, n);
-            if (final_in_kernel) { final_reduce_args(ctx, (int)(&r - rooms.data()), fa); r.wait_seq = fa.seq; }
+            fused::set_attempt(fa, c, e0, ne, r.phi, r.scratch, s.n);
+            if (r.final_in_kernel) { final_reduce_args(ctx, (int)(&r - rooms.data()), fa); r.wait_seq = fa.seq; }
             if (to_bucket) {
+                fused::set_tensor_maps(fa, s.Ny, &s.maps);
                 r.fa = fa;
-                buckets[ne].push_back(&r);
+                buckets[ne][fused::bulk_ok(fa) ? 1 : 0].push_back(&r);
                 break;
             }
             int rc = s.launch_fused(ne, fa);
@@ -847,8 +887,8 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
             e0 += ne;
         } while (e0 < c.n_emit());
         r.st.nfev += 6;
-        if (!final_in_kernel) {
-            reduce_async(r, 0, fgx, fgy, 0);
+        if (!r.final_in_kernel) {
+            reduce_async(r, 0, s.fused_gx, s.fused_gy, 0);
             cudaEventRecord(r.ev, s.st);
         }
         r.phase = BatchRoom::STEP;
@@ -860,6 +900,8 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
     };
     auto advance = [&](BatchRoom &r) -> int {
         Solver &s = r.s;
+        const size_t n = s.n;
+        const int Ny = s.Ny, Nx = s.Nx, nbx = s.nbx, nby = s.nby;
         switch (r.phase) {
         case BatchRoom::START: {
             prep_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s.st>>>(r.V, r.m, r.g, r.inv_mu_s2, n, s.coef, s.y);
@@ -878,8 +920,8 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
             return OC_OK;
         }
         case BatchRoom::INIT0: {  // common.py:109-127
-            r.d1 = std::sqrt(host_sum(r, nby, 1)) / sqrt_n;
-            r.h0 = r.ctl.initial_h0(std::sqrt(host_sum(r, nby, 0)) / sqrt_n, r.d1);
+            r.d1 = std::sqrt(host_sum(r, nby, 1)) / r.sqrt_n;
+            r.h0 = r.ctl.initial_h0(std::sqrt(host_sum(r, nby, 0)) / r.sqrt_n, r.d1);
             Comb c{};
             c.y = s.y; c.k[0] = s.K[0]; c.a[0] = 1.0; c.h = r.h0 * r.ctl.direction;
             s.stage(1, c, s.K[1]);
@@ -892,12 +934,12 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
             return OC_OK;
         }
         case BatchRoom::INIT1: {  // common.py:127-134
-            r.ctl.set_initial_step(r.h0, r.d1, std::sqrt(host_sum(r, nby, 2)) / sqrt_n / r.h0);
+            r.ctl.set_initial_step(r.h0, r.d1, std::sqrt(host_sum(r, nby, 2)) / r.sqrt_n / r.h0);
             r.st.h0 = r.ctl.h_abs;
             return start_step(r);
         }
         case BatchRoom::STEP: {  // rk.py:146-165
-            const double error_norm = std::sqrt(final_in_kernel ? r.step_sum : host_sum(r, fgy, 0)) / sqrt_n;
+            const double error_norm = std::sqrt(r.final_in_kernel ? r.step_sum : host_sum(r, s.fused_gy, 0)) / r.sqrt_n;
             rk45::Controller &c = r.ctl;
             if (!c.judge(error_norm)) return attempt(r);
             for (int e = 0; e < c.n_emit(); e++) {
@@ -906,8 +948,8 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
                     const double *ph = fused::sample_slice(c, e, r.phi, r.scratch, n);
                     const int sl = c.nt - 1 - kd;
                     dim3 grid((Nx - 2 + 63) / 64, (Ny - 2 + 3) / 4);
-                    vels_kernel<<<grid, NTHREADS, 0, s.st>>>(ph, Ny, Nx, r.mu, prm->lim, 1.0 / (2 * ctx->dx), 1.0 / (2 * ctx->dy),
-                                                             r.vx + (size_t)sl * n_int, r.vy + (size_t)sl * n_int);
+                    vels_kernel<<<grid, NTHREADS, 0, s.st>>>(ph, Ny, Nx, r.mu, prm->lim, 1.0 / (2 * r.dx), 1.0 / (2 * r.dy),
+                                                             r.vx + (size_t)sl * r.n_int, r.vy + (size_t)sl * r.n_int);
                     s.launches++;
                 }
             }
@@ -931,7 +973,7 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
         for (int b = 0; b < n_rooms && !rc; b++) {
             BatchRoom &r = rooms[b];
             if (r.phase == BatchRoom::DONE) continue;
-            if (final_in_kernel && r.phase == BatchRoom::STEP) {
+            if (r.final_in_kernel && r.phase == BatchRoom::STEP) {
                 // the attempt's last CTA publishes the error sum in mapped host memory: no event, no copy
                 if (!final_ready(ctx, b, r.wait_seq, &r.step_sum)) continue;
             } else {
@@ -958,9 +1000,9 @@ extern "C" int oc_hjb_solve_multi(oc_ctx *ctx, int n_rooms, const double *const 
             }
             // every stream has drained, so every launched attempt has published its error sum (ocfinal::wait): a room
             // still waiting after one more look never gets one -- an error instead of a host that spins for ever
-            for (int b = 0; b < n_rooms && !rc && all_idle && final_in_kernel; b++) {
+            for (int b = 0; b < n_rooms && !rc && all_idle; b++) {
                 BatchRoom &r = rooms[b];
-                if (r.phase == BatchRoom::STEP && !final_ready(ctx, b, r.wait_seq, &r.step_sum)) {
+                if (r.final_in_kernel && r.phase == BatchRoom::STEP && !final_ready(ctx, b, r.wait_seq, &r.step_sum)) {
                     oc::set_error("batched HJB solve: room %d: fused RK45 step did not deliver its error sum", b);
                     rc = OC_ERR_CUDA;
                 }

@@ -33,6 +33,8 @@
 #include <cuda.h>  // CUtensorMap (types only: the encoder is fetched through cudaGetDriverEntryPoint)
 #include <cuda_runtime.h>
 
+#include <algorithm>
+#include <climits>
 #include <cstddef>
 #include <cstdint>
 
@@ -264,22 +266,26 @@ struct __align__(128) Smem {
     double cst[(1 + NE_MAX) * 6];  // h*E and the dense-output weights (made opaque to the compiler, see below)
     double red[BX / 32];
     unsigned long long full[NG];   // one mbarrier per tile buffer (TMA)
+    unsigned tile[4];              // bx, by, ngx, ngy of the batched kernel (hjb_fused_body<..., STASH = true>)
 };
 static_assert(sizeof(double2) * 2 * 3 * (BX + 2) >= sizeof(double) * MAX_FINAL_ROWS, "final reduction staging");
 
 __device__ __forceinline__ int mirror(int i, int n) { return i < 0 ? -i : (i >= n ? 2 * (n - 1) - i : i); }
 
-template <int NE, bool P2P, bool BULK>
-__device__ __forceinline__ void hjb_fused_body(const Args &a) {
+// (bx, by): this CTA's tile column and chunk row; (ngx, ngy): the tile grid of its room.  STASH: keep the four in shared
+// memory across the row loop (the batched kernel derives them from its launch table: they cannot be re-read from special
+// registers as blockIdx / gridDim can, and the row loop needs every register)
+template <int NE, bool P2P, bool BULK, bool STASH = false>
+__device__ __forceinline__ void hjb_fused_body(const Args &a, unsigned bx, unsigned by, unsigned ngx, unsigned ngy) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     Smem &sm = *reinterpret_cast<Smem *>(smem_raw);
     const int tid = threadIdx.x;
-    const int x0 = blockIdx.x * VX - HX;                            // global column of tile position 0
+    const int x0 = bx * VX - HX;                            // global column of tile position 0
     const int gx = x0 + tid;
     const int c0 = max(x0, 0), c1 = min(x0 + BX, a.Nx);             // columns of the grid this tile covers
     const int gxm = min(max(mirror(gx, a.Nx), c0), c1 - 1);         // column this thread's state comes from
     const int lt = BULK ? gxm - x0 : tid;                           // its position in the staged row
-    const int y0 = a.own0 + blockIdx.y * a.RC;
+    const int y0 = a.own0 + by * a.RC;
     const int y1 = min(y0 + a.RC, a.own1);
     const bool col_out = tid >= HX && tid < BX - HX && gx < a.Nx;  // columns this thread stores
     const int phi_shift = (a.row_base - a.phi_row_base) * a.Nx;    // phi slices may start at another global row
@@ -291,6 +297,7 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
 #pragma unroll
         for (int ee = 0; ee < NE; ee++) sm.cst[6 * (ee + 1) + tid] = a.w[ee][j];
     }
+    if (STASH && tid == 0) { sm.tile[0] = bx; sm.tile[1] = by; sm.tile[2] = ngx; sm.tile[3] = ngy; }
     if (BULK && tid == 0) {
 #pragma unroll
         for (int s = 0; s < NG; s++) mbar_init(&sm.full[s], 1);
@@ -536,6 +543,7 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
                 a.peer_k7[1][gp] = a.k7[g];
             }
     }
+    if (STASH) { bx = sm.tile[0]; by = sm.tile[1]; ngx = sm.tile[2]; ngy = sm.tile[3]; }
     // fixed-order CTA reduction of the error partial sum
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
@@ -545,7 +553,7 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
         double s = 0.0;
 #pragma unroll
         for (int i = 0; i < BX / 32; i++) s += sm.red[i];
-        a.partial[(size_t)blockIdx.y * gridDim.x + blockIdx.x] = s;
+        a.partial[(size_t)by * ngx + bx] = s;
     }
     if (a.ticket == nullptr) return;
     // ---- last CTA: fixed-order final reduction (see Args)
@@ -554,13 +562,13 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
         if (P2P) __threadfence_system();  // this CTA's peer stores are ordered before its ticket
         else __threadfence();
         const unsigned t = atomicAdd(a.ticket, 1u);
-        is_last = (t == gridDim.x * gridDim.y - 1);
+        is_last = (t == ngx * ngy - 1);
     }
     __syncthreads();
     if (!is_last) return;
     __threadfence();
     double *rows = reinterpret_cast<double *>(&sm.ex[0][0][0]);
-    const int ngx = gridDim.x, gy = gridDim.y, lane = tid & 31;
+    const int ntx = ngx, gy = ngy, lane = tid & 31;
     for (int row = tid >> 5; row < gy; row += BX / 32) {
         // the 8 warps of rowgroup_sum_kernel's 256 threads, emulated by this warp: all loads first (independent, in
         // flight together), then the 8 shuffle trees, then the left-to-right sum of the 8 warp totals
@@ -568,7 +576,7 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
 #pragma unroll
         for (int vw = 0; vw < 8; vw++) {
             v[vw] = 0.0;
-            for (int i = vw * 32 + lane; i < ngx; i += 256) v[vw] += __ldcg(a.partial + (size_t)row * ngx + i);
+            for (int i = vw * 32 + lane; i < ntx; i += 256) v[vw] += __ldcg(a.partial + (size_t)row * ntx + i);
         }
         double srow = 0.0;
 #pragma unroll
@@ -627,21 +635,37 @@ __device__ __forceinline__ void hjb_fused_body(const Args &a) {
 
 template <int NE, bool P2P = false, bool BULK = true>
 __global__ void __launch_bounds__(BX, CTAS_PER_SM) hjb_fused_kernel(const __grid_constant__ Args a) {
-    hjb_fused_body<NE, P2P, BULK>(a);
+    hjb_fused_body<NE, P2P, BULK>(a, blockIdx.x, blockIdx.y, gridDim.x, gridDim.y);
 }
 
-// Ensembles (BASELINE configs[4]): the same step for up to BATCH_MAX independent rooms of one grid shape in ONE launch,
-// blockIdx.z = room.  Every room brings its own Args (its own step size, dense-output weights, arrays, ticket and result
-// slot: the rooms' RK45 controllers are independent), all in kernel-parameter space, so the per-room constants are
-// still uniform-register operands.  Rooms are grouped by their number of dense-output samples NE.
-constexpr int BATCH_MAX = 24;  // 24 x sizeof(Args) < the 32764-byte kernel-parameter limit
+// Ensembles (BASELINE configs[4]): the same step for up to BATCH_MAX independent rooms in ONE launch.  The rooms may
+// differ in grid shape: the launch is a flattened 1-D grid holding exactly the sum of the rooms' tile grids, room q owning
+// CTAs [first[q], first[q + 1]) in its own row-major (chunk row, tile column) order -- the chunking and CTA order of its
+// stand-alone launch.  Every room brings its own Args (its own grid, step size, dense-output weights, arrays, ticket and
+// result slot: the rooms' RK45 controllers are independent), all in kernel-parameter space, so the per-room constants are
+// still uniform-register operands.  Rooms are grouped by their number of dense-output samples NE and by the staging
+// variant (BULK needs an even Nx; see bulk_ok).
+// A CTA finds its room with ONE load from a CTA-to-room table indexed by blockIdx.x >> shift: ptxas repeats that load
+// where the row loop needs the room's Args instead of keeping the room index in a register (a scan of the prefix sums
+// cannot be repeated that way, and the index then spilled inside the row loop).  The table has one entry per 2^shift
+// CTAs, so every room's first CTA must be a multiple of 2^shift (set_batch_table).
+constexpr int BATCH_MAX = 24;
+constexpr int BATCH_PARAM_BYTES = 32704;  // the 32764-byte kernel-parameter limit, rounded down to Args' 64-byte alignment
+constexpr int BATCH_TABLE = BATCH_PARAM_BYTES - BATCH_MAX * (int)sizeof(Args) - (3 * BATCH_MAX + 1) * (int)sizeof(int);
 struct BatchArgs {
     Args a[BATCH_MAX];
+    int first[BATCH_MAX];       // first CTA of room q (prefix sum); INT_MAX past the last room of the launch
+    int ngx[BATCH_MAX], ngy[BATCH_MAX];  // tile grid of room q: tile columns, chunk rows
+    int shift;
+    unsigned char room_of[BATCH_TABLE];  // room of CTAs [c << shift, (c + 1) << shift)
 };
-static_assert(sizeof(BatchArgs) <= 32764, "kernel parameter space");
+static_assert(BATCH_TABLE >= 1024 && sizeof(BatchArgs) <= 32764, "kernel parameter space");
 template <int NE, bool BULK>
 __global__ void __launch_bounds__(BX, CTAS_PER_SM) hjb_fused_batch_kernel(const __grid_constant__ BatchArgs ba) {
-    hjb_fused_body<NE, false, BULK>(ba.a[blockIdx.z]);
+    const int cta = blockIdx.x;
+    const int q = ba.room_of[cta >> ba.shift];
+    const int local = cta - ba.first[q], ngx = ba.ngx[q];
+    hjb_fused_body<NE, false, BULK, true>(ba.a[q], local % ngx, local / ngx, ngx, ba.ngy[q]);
 }
 
 // Launch of one step attempt.  BULK staging needs 16-byte aligned rows: an even number of columns and 16-byte aligned
@@ -726,26 +750,44 @@ inline cudaError_t launch(int ne, const Args &a, dim3 grid, cudaStream_t st) {
 #undef OC_FUSED_CASE
 }
 
-// one launch for `nb` rooms (all with `ne` samples); every room must be TMA-capable or none
+// one launch for `nb` rooms (all with `ne` samples), all TMA-capable (bulk) or none; ba.first / ngx / ngy set by
+// set_batch_table
 template <int NE, bool BULK>
-inline cudaError_t launch_batch_one(const BatchArgs &ba, dim3 grid, cudaStream_t st) {
+inline cudaError_t launch_batch_one(const BatchArgs &ba, int ctas, cudaStream_t st) {
     if (sizeof(Smem) > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(hjb_fused_batch_kernel<NE, BULK>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)sizeof(Smem));
         if (e != cudaSuccess) return e;
     }
-    hjb_fused_batch_kernel<NE, BULK><<<grid, BX, sizeof(Smem), st>>>(ba);
+    hjb_fused_batch_kernel<NE, BULK><<<ctas, BX, sizeof(Smem), st>>>(ba);
     return cudaSuccess;
 }
-inline cudaError_t launch_batch(int ne, const BatchArgs &ba, int nb, dim3 grid2d, cudaStream_t st) {
-    bool bulk = true;
-    for (int q = 0; q < nb; q++) bulk = bulk && bulk_ok(ba.a[q]);
-    const dim3 grid(grid2d.x, grid2d.y, nb);
+// the launch table of rooms [0, nb) with tile grids (ngx[q], ngy[q]); returns the number of CTAs of the launch, or 0 when
+// the CTA-to-room table cannot describe these rooms (more than BATCH_TABLE entries at the coarsest shift their first CTAs
+// allow): the caller then launches fewer rooms.  One room always fits.
+inline int set_batch_table(BatchArgs &ba, int nb, const int *ngx, const int *ngy) {
+    int ctas = 0, align = 30;  // align: the largest shift every room's first CTA is a multiple of
+    for (int q = 0; q < BATCH_MAX; q++) {
+        ba.first[q] = q < nb ? ctas : INT_MAX;
+        ba.ngx[q] = q < nb ? ngx[q] : 1;
+        ba.ngy[q] = q < nb ? ngy[q] : 1;
+        if (q > 0 && q < nb) align = std::min(align, __builtin_ctz((unsigned)ctas));
+        if (q < nb) ctas += ngx[q] * ngy[q];
+    }
+    int shift = 0;
+    while (((ctas - 1) >> shift) + 1 > BATCH_TABLE) shift++;
+    if (shift > align) return 0;
+    ba.shift = shift;
+    for (int q = 0; q < nb; q++)
+        for (int c = ba.first[q] >> shift; c <= (ba.first[q] + ngx[q] * ngy[q] - 1) >> shift; c++) ba.room_of[c] = (unsigned char)q;
+    return ctas;
+}
+inline cudaError_t launch_batch(int ne, bool bulk, const BatchArgs &ba, int ctas, cudaStream_t st) {
 #define OC_FUSED_CASE(NE) \
-    case NE: return bulk ? launch_batch_one<NE, true>(ba, grid, st) : launch_batch_one<NE, false>(ba, grid, st);
+    case NE: return bulk ? launch_batch_one<NE, true>(ba, ctas, st) : launch_batch_one<NE, false>(ba, ctas, st);
     switch (ne) {
         OC_FUSED_CASE(0) OC_FUSED_CASE(1) OC_FUSED_CASE(2) OC_FUSED_CASE(3) OC_FUSED_CASE(4) OC_FUSED_CASE(5)
-        default: return bulk ? launch_batch_one<6, true>(ba, grid, st) : launch_batch_one<6, false>(ba, grid, st);
+        default: return bulk ? launch_batch_one<6, true>(ba, ctas, st) : launch_batch_one<6, false>(ba, ctas, st);
     }
 #undef OC_FUSED_CASE
 }

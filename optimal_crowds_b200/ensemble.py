@@ -7,8 +7,9 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
   * every member is an ordinary ``simulations.simulation`` whose randomness comes from its own
     ``np.random.RandomState(seed)`` -- the very stream ``np.random.seed(seed)`` gives the reference, so member i
     reproduces the stand-alone run with that seed bit for bit (tests/test_gpu_ensemble.py);
-  * the HJB fields of all members of a wave are solved by ONE ``oc_hjb_solve_multi`` call: one RK45 controller and
-    one CUDA stream per member, the members' step kernels overlapping on the GPU;
+  * the HJB fields of all members of a wave -- every target set of every member -- are solved by ONE
+    ``oc_hjb_solve_grids`` call: one RK45 controller and one CUDA stream per field, the step kernels of fields of
+    every grid shape sharing batched launches;
   * the GCFM steps of the members advance in lock-step: every member's sweep is launched on its own stream
     (``oc_gcfm_step_launch``) before any is finished (``oc_gcfm_step_finish``), so the host's per-step work (RNG
     draws, exit bookkeeping) of one member overlaps the other members' kernels;
@@ -16,12 +17,15 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     samples), and only the per-member results are kept;
   * ``configs``: every member may bring its own overrides of config.json (model parameters, ``dt``, re-solve
     frequency, ...; one grid step for all).  Its HJB solves then run with its own sigma, mu, g and horizon inside the
-    same batched call (``oc_hjb_solve_multi``), its re-solves happen at its own steps, and it still equals the
-    stand-alone ``simulation(..., config=...)`` run bit for bit (tests/test_gpu_ensemble_params.py).
+    same batched call, its re-solves happen at its own steps, and it still equals the stand-alone
+    ``simulation(..., config=...)`` run bit for bit (tests/test_gpu_ensemble_params.py);
+  * members may have different rooms: different grid shapes and numbers of target sets (one grid step for all).
+    Every member still equals its stand-alone run bit for bit (tests/test_gpu_ensemble_shapes.py).
 """
 from __future__ import annotations
 
 import contextlib
+import copy
 import os
 import io
 
@@ -38,14 +42,15 @@ def shard(n_members: int, rank: int, world: int):
 
 
 def field_bytes_per_member(Ny: int, Nx: int, T: float, dt: float, n_keys: int = 1, field_storage: str = "phi") -> int:
-    """device bytes one member holds: field samples (optimals.py:80-81 sizes them by round(T/dt)) + solver workspace"""
+    """device bytes one member holds: field samples (optimals.py:80-81 sizes them by round(T/dt)) + solver workspace
+    (the fields of all target sets are solved in one call)"""
     nt = round(T / dt)
     n = Ny * Nx
     field = nt * n * 8 if field_storage == "phi" else 2 * max(nt - 1, 0) * (Ny - 2) * (Nx - 2) * 8
-    return n_keys * (field + 2 * n * 8) + 6 * n * 8
+    return n_keys * (field + 2 * n * 8 + 6 * n * 8)
 
 
-_SOLVER_CTX = {}   # (device, room size, grid step) -> Context owning the batched-solve workspace
+_SOLVER_CTX = {}   # device -> Context owning the batched-solve workspace
 _CTX_POOL = {}     # (device, room size, grid step) -> library contexts of finished members, ready for reuse
 
 
@@ -90,19 +95,23 @@ def gather_results(local: dict, group=None) -> dict:
 
 class ensemble:
     """``ensemble(room, T, seeds)``: one member per seed of the same room; ``ensemble([room0, room1, ...], T, seeds)``:
-    one room per member (all rooms must give the same grid shape).  ``run()`` returns {member index: result} with
+    one room per member (rooms of any size and number of target sets).  ``run()`` returns {member index: result} with
     ``evac_time`` (simulation time when the run stopped), ``steps``, ``inside`` (agents left inside: 0 = evacuation
     complete), ``exit_order`` (agent ids in exit order), ``exit_step`` (per agent, -1 = still inside),
     ``times`` (per-agent clocks, as evac_times() returns them), ``final`` (N,4: x, y, vx, vy) and ``hjb`` (solver
     statistics per target set) and ``config`` (the member's effective configuration).
 
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
-    ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``."""
+    ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
+    their rooms may differ in size and number of target sets.
+
+    ``chunk_rows``: 0 (every room chunked as if it were alone: members are bit-identical to stand-alone runs with
+    default settings), n > 0 (fixed) or "wave" (planned per grid shape for the number of members of that shape in the
+    solve; ``results[i]["chunk_rows"]`` is the value member i was solved with, and ``chunk_rows_used`` the value of a
+    single-shape ensemble)."""
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
                  memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None):
-        # chunk_rows: 0 = every room chunked as if it were alone (members are then bit-identical to stand-alone runs with
-        # default settings, whatever the wave size); n > 0 = fixed; "wave" = planned for the wave size (fastest)
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -133,20 +142,41 @@ class ensemble:
         self.batched_steps = bool(batched_steps)
         self.min_sweep_ctas, self.sweep_ctas = 8, 0   # sweep grid per member: automatic share of the GPU, or fixed
         self.chunk_rows_used = self.chunk_rows
+        self.member_chunk_rows = {}   # member index -> chunk_rows of its last solve
+        self._rooms_loaded = {}       # room name -> parsed room file (read once, whatever the number of members)
         self.results = {}
         self.members = {}          # member index -> simulation (kept only when record=True)
         self.stats = dict(hjb_ms=0.0, gcfm_ms=0.0, build_ms=0.0, agent_steps=0, cell_updates=0, waves=0, launch_ms=0.0,
                           finish_ms=0.0)
 
     # ---------------------------------------------------------------------------------------------
+    def _room(self, idx):
+        room = self.rooms[idx]
+        if isinstance(room, dict):
+            return room
+        if room not in self._rooms_loaded:
+            self._rooms_loaded[room] = simulations._load_room(room)
+        return self._rooms_loaded[room]
+
+    def member_bytes(self, members=None):
+        """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets); no CUDA"""
+        out = []
+        for i in (self.mine if members is None else members):
+            room, cfg = self._room(i), self.configs[i]
+            Ny, Nx = _lib.grid_shape(room["room_length"], room["room_height"], cfg["grid_step"])
+            n_keys = len({' or '.join(b[5:]) for b in room["initial_boxes"].values()})
+            out.append(field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage))
+        return out
+
     def _build(self, idx):
         # a finished member's library context (device workspace, page-locked buffers, streams) serves the next member
         # of the same room size: a wave of 128 members otherwise pays 128 x (cudaMalloc + cudaMallocHost + frees) per pass
-        room = simulations._load_room(self.rooms[idx])
+        room = self._room(idx)
         step = self.configs[idx]["grid_step"]
         free = _CTX_POOL.get(_ctx_key(room["room_length"], room["room_height"], step))
         ctx = free.pop() if free else None
-        return simulations.simulation(self.rooms[idx], self.T, recompute=self.recompute, record=self.record,
+        # (the parsed room, not its name: one file read per room, whatever the number of members; a copy per member)
+        return simulations.simulation(copy.deepcopy(room), self.T, recompute=self.recompute, record=self.record,
                                       field_storage=self.field_storage, fused=1, lookahead=False,
                                       rng=np.random.RandomState(self.seeds[idx]), chunk_rows=self.chunk_rows,
                                       config=self.overrides[idx], _ctx=ctx)
@@ -171,55 +201,69 @@ class ensemble:
                 return list(ex.map(build, wave))
 
     def _solver_ctx(self, first):
-        """the context whose batch workspace (5 arrays per room, 32 streams, one event and one result slot per room) the
-        batched solves of this process use: kept across waves and ensembles of the same grid, so that a wave does not
-        pay ~50 ms of allocations in front of a ~40 ms solve"""
+        """the context whose batch workspace (5 arrays per field, 32 streams, one event and one result slot per field)
+        the batched solves of this process use, one per device: kept across waves and ensembles, so that a wave does not
+        pay ~50 ms of allocations in front of a ~40 ms solve.  Its own grid plays no part: every field is solved on the
+        grid of its member's context."""
         import torch
-        key = (torch.cuda.current_device(), first.room_length, first.room_height, first._ctx.dx)
+        key = torch.cuda.current_device()
         ctx = _SOLVER_CTX.get(key)
         if ctx is None or not getattr(ctx, "h", None):
             ctx = _SOLVER_CTX[key] = _lib.Context(first.room_length, first.room_height, first._ctx.dx)
         return ctx
 
-    def _solve_wave(self, sims):
-        """simulation._solve_all for the given members in one batched call per target set, each member with its own
-        sigma, mu, g, horizon and density"""
+    def _solve_wave(self, sims, idx):
+        """simulation._solve_all for the given members (wave indices idx) in one batched call over the fields of all
+        their target sets, each member with its own grid, sigma, mu, g, horizon and density"""
         import torch
-        first = sims[0]
-        sctx = self._solver_ctx(first)
+        sctx = self._solver_ctx(sims[0])
         # simulations.py:424-425: density * (simu_step > 0), per member
         d_ms = [s._density_device(s.sigma_convolution) if s.simu_step > 0 else None for s in sims]
-        if all(m is None for m in d_ms):
-            d_ms = None
         nts = [round((self.T - s.time) / s.dt) for s in sims]                  # optimals.py:140
         if min(nts) < 1:
             raise ValueError("Values in `t_eval` are not within `t_span`.")
-        cells = 0
-        for k, key in enumerate(first.targets):
-            opts = [list(s.targets.values())[k] for s in sims]
-            for o, nt in zip(opts, nts):
+        chunk = [self.chunk_rows] * len(sims)
+        if self.chunk_plan_for_wave:
+            # chunk height planned per grid shape for the members of that shape in this call (a 512^2 room alone would
+            # be cut into 16-row chunks to fill the GPU; 64 rooms side by side fill it with 64-row chunks and recompute
+            # far fewer halo rows).  The chunking fixes the error-norm summation order: a stand-alone run reproduces a
+            # member bit for bit when it is given the same chunk_rows (results[i]["chunk_rows"]).
+            count = {}
+            for s in sims:
+                count[(s.Ny, s.Nx)] = count.get((s.Ny, s.Nx), 0) + 1
+            plan = {sh: next(s for s in sims if (s.Ny, s.Nx) == sh)._ctx.plan_chunk_rows(c) for sh, c in count.items()}
+            chunk = [plan[(s.Ny, s.Nx)] for s in sims]
+            if len(plan) == 1:
+                self.chunk_rows_used = chunk[0]
+        for i, c in zip(idx, chunk):
+            self.member_chunk_rows[i] = c
+        # one room per (member, target set)
+        opts, grids, Vs, ms, rooms = [], [], [], [], []
+        for s, d_m, nt, c in zip(sims, d_ms, nts, chunk):
+            for o in s.targets.values():
                 if nt - 1 > o._n_slices:
                     raise IndexError("re-solve asks for more slices than the field was allocated for")
-            rooms = [dict(sigma=o.sigma, mu=o.mu, g=o.g, T=self.T, nt=nt) for o, nt in zip(opts, nts)]
-            prm = opts[0]._prm   # (rtol, atol, lim, chunk_rows: the same for every member)
-            if self.chunk_plan_for_wave:
-                # chunk height planned for the whole wave (a 512^2 room alone would be cut into 16-row chunks to fill the
-                # GPU; 64 rooms side by side fill it with 64-row chunks and recompute far fewer halo rows).  The chunking
-                # fixes the error-norm summation order: a stand-alone run reproduces a member bit for bit when it is
-                # given the same chunk_rows (ensemble.chunk_rows_used).
-                self.chunk_rows_used = sctx.plan_chunk_rows(len(sims))
-                prm.chunk_rows = self.chunk_rows_used
-            vel = self.field_storage == "velocity"
-            import time as _t
-            _t0 = _t.perf_counter()
-            res = sctx.hjb_solve_multi([o.d_V for o in opts], d_ms, rooms, prm,
-                                       out_phi=None if vel else [o.d_phi for o in opts],
-                                       out_vx=[o.d_vx for o in opts] if vel else None,
-                                       out_vy=[o.d_vy for o in opts] if vel else None)
-            self.stats["hjb_call_ms"] = self.stats.get("hjb_call_ms", 0.0) + (_t.perf_counter() - _t0) * 1e3
-            self.stats["hjb_calls"] = self.stats.get("hjb_calls", 0) + 1
-            self.stats["hjb_call_rooms"] = self.stats.get("hjb_call_rooms", 0) + len(opts)
-            for o, r, s, nt in zip(opts, res, sims, nts):
+                opts.append(o); grids.append(s._ctx); Vs.append(o.d_V); ms.append(d_m)
+                rooms.append(dict(sigma=o.sigma, mu=o.mu, g=o.g, T=self.T, nt=nt, chunk_rows=c))
+        if all(m is None for m in ms):
+            ms = None
+        prm = opts[0]._prm   # (rtol, atol, lim: the same for every member; chunk_rows per room above)
+        vel = self.field_storage == "velocity"
+        import time as _t
+        _t0 = _t.perf_counter()
+        res = sctx.hjb_solve_grids(grids, Vs, ms, rooms, prm,
+                                   out_phi=None if vel else [o.d_phi for o in opts],
+                                   out_vx=[o.d_vx for o in opts] if vel else None,
+                                   out_vy=[o.d_vy for o in opts] if vel else None)
+        self.stats["hjb_call_ms"] = self.stats.get("hjb_call_ms", 0.0) + (_t.perf_counter() - _t0) * 1e3
+        self.stats["hjb_calls"] = self.stats.get("hjb_calls", 0) + 1
+        self.stats["hjb_call_rooms"] = self.stats.get("hjb_call_rooms", 0) + len(sims)   # (members per call)
+        cells = 0
+        k = 0
+        for s, nt in zip(sims, nts):
+            for o in s.targets.values():
+                r = res[k]
+                k += 1
                 o.t, o.nt_opt, o.last_stats = s.time, nt, r["stats"]
                 o._h_vx = o._h_vy = None
                 if r["stats"]["status"] == -1:
@@ -233,9 +277,6 @@ class ensemble:
         import torch
         t0 = time.perf_counter()
         sims = self._build_wave(wave)
-        shape = {(s.Ny, s.Nx, tuple(s.targets)) for s in sims}
-        if len({sh[:2] for sh in shape}) != 1 or len({len(sh[2]) for sh in shape}) != 1:
-            raise ValueError("ensemble members must share the grid shape and the number of target sets")
         streams = [torch.cuda.Stream() for _ in range(min(len(sims), 128))]
         # the members' sweeps run concurrently: each gets its share of the GPU's resident-CTA slots
         n_sm = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
@@ -245,7 +286,7 @@ class ensemble:
             s._cuda_stream = streams[q % len(streams)].cuda_stream   # the member's steps run on its own stream
         torch.cuda.synchronize()
         t1 = time.perf_counter()
-        self.stats["cell_updates"] += self._solve_wave(sims)
+        self.stats["cell_updates"] += self._solve_wave(sims, wave)
         t2 = time.perf_counter()
         live = list(range(len(sims)))
         batch = None
@@ -267,7 +308,7 @@ class ensemble:
                    and sims[q].simu_step > 0]
             rebind = bool(due)
             if due:
-                self.stats["cell_updates"] += self._solve_wave([sims[q] for q in due])
+                self.stats["cell_updates"] += self._solve_wave([sims[q] for q in due], [wave[q] for q in due])
             tl0 = time.perf_counter()
             if batch is not None:
                 if rebind:
@@ -306,7 +347,8 @@ class ensemble:
             self.results[i] = dict(seed=self.seeds[i], evac_time=s.time, steps=s.simu_step, inside=int(s.inside), N=s.N,
                                    exit_order=np.array(s._exit_order, dtype=np.int64), exit_step=s._exit_step.copy(),
                                    times=np.array(s._h_timev, dtype=float), final=np.array(s._h_now, dtype=float),
-                                   hjb={k: o.last_stats for k, o in s.targets.items()}, config=self.configs[i])
+                                   hjb={k: o.last_stats for k, o in s.targets.items()}, config=self.configs[i],
+                                   chunk_rows=self.member_chunk_rows[i])
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3
@@ -337,12 +379,7 @@ class ensemble:
         import torch
         if not self.mine:
             return gather_results({}) if gather else {}
-        probe = simulations._load_room(self.rooms[self.mine[0]])
-        cfgs = [self.configs[i] for i in self.mine]
-        Ny, Nx = _lib.grid_shape(probe["room_length"], probe["room_height"], cfgs[0]["grid_step"])
-        n_keys = len({' or '.join(b[5:]) for b in probe["initial_boxes"].values()})
-        # (a member's field samples: round(T/dt) slices of its own dt)
-        per = [field_bytes_per_member(Ny, Nx, self.T, c["dt"], n_keys, self.field_storage) for c in cfgs]
+        per = self.member_bytes()
         budget = self.memory_budget
         if budget is None:
             free, _total = torch.cuda.mem_get_info()
