@@ -397,6 +397,39 @@ int oc_pair_force(oc_ctx *ctx, const oc_gcfm_params *prm, int N, const double *d
 int oc_density(oc_ctx *ctx, int N, const double *d_x, const double *d_y, const uint8_t *d_status, double sigma,
                double C, const double *d_Vglobal, double *d_out, void *stream);
 
+/* Density statistics of a run (the frames simulation.write_history stores, simulations.py:579-589, accumulated on the
+ * device instead of kept).  One frame d is oc_density(ctx, N, x, y, status, sigma, C, d_Vglobal) bit for bit; adding it
+ * does, per node, d_sum += d, d_max = np.maximum(d_max, d) (a NaN propagates) and, when d_above is given,
+ * d_above += (d > threshold).  All arrays (Ny,Nx) of the member's grid, caller-owned and initialised by the caller
+ * (zeros).  `every`: oc_gcfm_run_acc adds a frame before the steps whose simu_step is a multiple of it. */
+typedef struct {
+    double *d_sum, *d_max;        /* float64 */
+    int *d_above;                 /* int32 count of frames above threshold, or NULL */
+    const double *d_Vglobal;      /* simulation.V: nodes where it is < 0 are walls (density 0) */
+    double threshold;             /* finite when d_above is given */
+    double sigma, C;              /* sigma_convolution and sqrt(4*pi**2*sigma**2) from the host; finite, > 0 */
+    int every;                    /* >= 1 */
+    int pad_;
+} oc_density_acc;
+/* Adds one frame of the crowd (d_x, d_y, d_status: N agents, NULL allowed when N = 0) to acc.  Asynchronous on stream.
+ * OC_ERR_ARG for a NULL required pointer, every < 1, a sigma or C that is not finite and positive, or a non-finite
+ * threshold with d_above. */
+int oc_density_accum(oc_ctx *ctx, const oc_density_acc *acc, int N, const double *d_x, const double *d_y,
+                     const uint8_t *d_status, void *stream);
+/* One frame for each of n members in ONE launch: member m's crowd (Ns[m] agents at x[m], y[m], status[m]) on the grid
+ * of ctxs[m] into accs[m].  Members may differ in grid shape, sigma, C, crowd size (0 included) and Vglobal; each result
+ * is bit-identical to oc_density_accum of that member alone.  ctxs[0] owns the member table.  OC_ERR_ARG as
+ * oc_density_accum, and for a member context on another device than ctxs[0]. */
+int oc_density_accum_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs, const int *Ns,
+                           const double *const *x, const double *const *y, const uint8_t *const *status, void *stream);
+/* oc_gcfm_run plus density statistics: before step k it adds a frame to acc when (simu_step0 + k) % acc->every == 0, on
+ * `stream`, ahead of the step's randomness and sweep (nothing else changes).  acc = NULL is oc_gcfm_run. */
+int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
+                    double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,
+                    int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss, int n_steps,
+                    int simu_step0, int n_active0, double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
+                    int *steps_done, double *device_ms, long long *pairs, const oc_density_acc *acc, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

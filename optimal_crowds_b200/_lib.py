@@ -82,13 +82,20 @@ class Key(C.Structure):
                 ("n_doors", C.c_int), ("phi_row0", C.c_int), ("phi_rows", C.c_int)]
 
 
+class DensityAcc(C.Structure):
+    _fields_ = [("d_sum", C.c_void_p), ("d_max", C.c_void_p), ("d_above", C.c_void_p), ("d_Vglobal", C.c_void_p),
+                ("threshold", C.c_double), ("sigma", C.c_double), ("C", C.c_double), ("every", C.c_int),
+                ("pad_", C.c_int)]
+
+
 _lib = None
 
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
            "oc_hjb_solve", "oc_hjb_rhs", "oc_hjb_vels", "oc_wall_tiles_bytes", "oc_wall_tiles", "oc_gcfm_step",
            "oc_wall_force", "oc_pair_force", "oc_density", "oc_gcfm_last_ms", "oc_dist_unique_id", "oc_dist_init",
            "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_hjb_solve_grids", "oc_gcfm_step_launch",
-           "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run"]
+           "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run",
+           "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi"]
 
 
 def load():
@@ -118,6 +125,9 @@ def load():
     lib.oc_gcfm_run.argtypes = [C.c_void_p, C.POINTER(GcfmParams), C.c_int] + [C.c_void_p] * 8 + [C.c_void_p, C.c_int,
                                 C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, C.c_int, vpp_, ip, ip, ip, ip, dp,
                                 C.POINTER(C.c_longlong), C.c_void_p]
+    lib.oc_gcfm_run_acc.argtypes = lib.oc_gcfm_run.argtypes[:-1] + [C.POINTER(DensityAcc), C.c_void_p]
+    lib.oc_density_accum.argtypes = [C.c_void_p, C.POINTER(DensityAcc), C.c_int] + [C.c_void_p] * 4
+    lib.oc_density_accum_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, C.c_void_p]
     lib.oc_rng_step_draw.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp]
     lib.oc_rng_step_draw_ckpt.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp, C.c_int,
                                           C.POINTER(C.c_uint32), ip, ip, dp]
@@ -522,11 +532,12 @@ class Context:
         return exit_log[: n_exit.value].copy(), rc
 
     def gcfm_run(self, prm: GcfmParams, state, vdes, key_id, keys, rng_state, n_steps, simu_step0, n_active, rows=None,
-                 stream=None):
-        """up to n_steps steps of the run loop in one call (oc_gcfm_run): randomness drawn in C from the legacy MT19937
+                 stream=None, density=None):
+        """up to n_steps steps of the run loop in one call (oc_gcfm_run_acc): randomness drawn in C from the legacy MT19937
         state tuple `rng_state` (np.random.get_state()), next step's draws overlapped with the GPU.  rows: optional list of
-        n_steps (N,4) CUDA tensors receiving the packed state after each step.  Returns dict(steps, exits (agent ids in
-        exit order), exit_step (0-based step within the call), rc, rng_state (to be set_state()d), device_ms, pairs)."""
+        n_steps (N,4) CUDA tensors receiving the packed state after each step.  density: optional DensityStats that
+        receives the frame of every due step.  Returns dict(steps, exits (agent ids in exit order), exit_step (0-based step
+        within the call), rc, rng_state (to be set_state()d), device_ms, pairs)."""
         N = state["x"].numel()
         karr, keep = keys if isinstance(keys, tuple) else self.make_keys(keys)
         key = np.ascontiguousarray(rng_state[1], dtype=np.uint32).copy()
@@ -539,13 +550,16 @@ class Context:
                 rows_arr[q] = r.data_ptr()
         ex_a, ex_s = np.empty(max(N, 1), dtype=np.int32), np.empty(max(N, 1), dtype=np.int32)
         n_ex, done, ms, pairs = C.c_int(), C.c_int(), C.c_double(), C.c_longlong()
-        rc = load().oc_gcfm_run(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
-                                _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id), karr,
-                                len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
-                                C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
-                                ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done), C.byref(ms),
-                                C.byref(pairs), _stream() if stream is None else C.c_void_p(stream))
+        rc = load().oc_gcfm_run_acc(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
+                                    _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
+                                    karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
+                                    C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
+                                    ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
+                                    C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc),
+                                    _stream() if stream is None else C.c_void_p(stream))
         check(rc, allow=(OC_ERR_SAMPLER_RANGE,))
+        if density is not None:
+            density.frames += density.count(simu_step0, done.value)
         return dict(steps=done.value, exits=ex_a[: n_ex.value].copy(), exit_step=ex_s[: n_ex.value].copy(), rc=rc,
                     rng_state=("MT19937", key, pos.value, has.value, cached.value), device_ms=ms.value, pairs=pairs.value)
 
@@ -597,6 +611,73 @@ class Context:
         check(load().oc_density(self.h, N, _dev(x), _dev(y), _dev(status), float(sigma), Cn, _dev(Vglobal), _dev(d),
                                 _stream()))
         return d
+
+    def density_accum(self, stats, x, y, status, stream=None):
+        """add the density frame of the crowd (x, y, status; None for no agents) to `stats` (oc_density_accum)"""
+        N = 0 if x is None else x.numel()
+        check(load().oc_density_accum(self.h, C.byref(stats.acc), N, _dev(x), _dev(y), _dev(status),
+                                      _stream() if stream is None else C.c_void_p(stream)))
+        stats.frames += 1
+
+
+def density_accum_multi(ctxs, stats, states, stream=None):
+    """one density frame per member in one launch (oc_density_accum_multi): member q's crowd `states[q]` (dict with x, y,
+    status) on the grid of ctxs[q], added to stats[q]"""
+    n = len(ctxs)
+    if not (len(stats) == len(states) == n and n):
+        raise ValueError("one context, statistics and state per member expected")
+    vp = lambda: (C.c_void_p * n)()
+    hs, accs, xs, ys, sts = vp(), vp(), vp(), vp(), vp()
+    Ns = np.empty(n, dtype=np.int32)
+    for q, (c, s, st) in enumerate(zip(ctxs, stats, states)):
+        hs[q] = c.h.value
+        accs[q] = C.addressof(s.acc)
+        Ns[q] = st["x"].numel()
+        xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
+    check(load().oc_density_accum_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, sts,
+                                        _stream() if stream is None else C.c_void_p(stream)))
+    for s in stats:
+        s.frames += 1
+
+
+class DensityStats:
+    """Device accumulators of a run's density frames (oc_density_acc): per node of the (Ny, Nx) grid the sum and the
+    maximum of the frames (float64) and, with a threshold, the number of frames above it (int32); zero at creation.
+    sigma: the run's sigma_convolution; Vglobal: its simulation.V on the device; every: frames are taken at the steps
+    whose simu_step is a multiple of it."""
+
+    def __init__(self, ctx, Vglobal, sigma, every=1, threshold=None):
+        import torch
+        shape = (ctx.Ny, ctx.Nx)
+        self.sum = torch.zeros(shape, dtype=torch.float64, device=ctx.torch_device)
+        self.max = torch.zeros(shape, dtype=torch.float64, device=ctx.torch_device)
+        self.above = None if threshold is None else torch.zeros(shape, dtype=torch.int32, device=ctx.torch_device)
+        self.Vglobal = Vglobal
+        self.every, self.threshold, self.frames = int(every), threshold, 0
+        Cn = float(np.sqrt(4 * np.pi ** 2 * sigma ** 2))  # simulations.py:482, as Context.density
+        self.acc = DensityAcc(self.sum.data_ptr(), self.max.data_ptr(),
+                              None if self.above is None else self.above.data_ptr(), Vglobal.data_ptr(),
+                              0.0 if threshold is None else float(threshold), float(sigma), Cn, self.every, 0)
+
+    def due(self, simu_step):
+        return simu_step % self.every == 0
+
+    def count(self, simu_step0, steps):
+        """frames taken by `steps` consecutive steps from simu_step0"""
+        return sum(1 for k in range(simu_step0, simu_step0 + steps) if k % self.every == 0)
+
+    def result(self):
+        """dict(frames, sum, max, above (None without a threshold), mean = sum / frames (None without frames)), read back
+        from the device (the caller has synchronised the streams that added frames)"""
+        s = self.sum.cpu().numpy()
+        return dict(frames=self.frames, sum=s, max=self.max.cpu().numpy(),
+                    above=None if self.above is None else self.above.cpu().numpy(),
+                    mean=s / self.frames if self.frames else None)
+
+    @staticmethod
+    def nbytes(Ny, Nx, threshold=None):
+        """device bytes of the accumulators of an (Ny, Nx) grid"""
+        return Ny * Nx * (16 + (4 if threshold is not None else 0))
 
 
 class GcfmBatch:

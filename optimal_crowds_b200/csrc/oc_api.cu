@@ -115,6 +115,10 @@ extern "C" void oc_ctx_destroy(oc_ctx *c) {
     oc_gcfm_free_launch_state(c);
     if (c->multi_pinned) cudaFreeHost(c->multi_pinned);
     cudaFree(c->multi_dev);
+    if (c->dens_ev) cudaEventSynchronize(c->dens_ev);
+    if (c->dens_pinned) cudaFreeHost(c->dens_pinned);
+    cudaFree(c->dens_dev);
+    if (c->dens_ev) cudaEventDestroy(c->dens_ev);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->gcfm_pinned) cudaFreeHost(c->gcfm_pinned);
     cudaFree(c->fr_ticket);

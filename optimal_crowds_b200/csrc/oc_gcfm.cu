@@ -1282,18 +1282,38 @@ __global__ void pair_probe_kernel(oc_gcfm_params p, int N, const double *__restr
 
 // K7 density (simulations.py:469-487): per node, sum over active agents in agent order.  exp underflows to
 // exactly 0 beyond r_zero, so agents farther than that from the whole tile are culled without changing a bit.
+// density_tile is the only copy of the arithmetic: tile (bx, by) of DN_TX x DN_TY nodes, every node's value handed to
+// the epilogue `epi(g, value)` (g = flat node index).  DensityStore writes the frame (oc_density); DensityAccum adds it
+// to the run's statistics (oc_density_accum*), so an accumulated frame is the stored frame bit for bit.
 constexpr int DN_TX = 32, DN_TY = 8, DN_CHUNK = 256;
-__global__ void __launch_bounds__(256)
-density_kernel(int N, const double *__restrict__ ax, const double *__restrict__ ay, const uint8_t *__restrict__ status,
-               const double *__restrict__ X, const double *__restrict__ Y, const double *__restrict__ Vg, int Ny,
-               int Nx, double two_s2, double C, double r_zero, double *__restrict__ out) {
+// ocm_exp(x) == 0 exactly for x < -745.14: r^2/two_s2 > 745.2  =>  contribution is exactly 0.0
+inline double density_r_zero(double two_s2) { return std::sqrt(745.2 * two_s2) * (1.0 + 1e-9) + 1e-9; }
+struct DensityStore {
+    double *out;
+    __device__ __forceinline__ void operator()(size_t g, double v) const { out[g] = v; }
+};
+struct DensityAccum {
+    double *sum, *max;
+    int *above;   // nullable
+    double thr;
+    __device__ __forceinline__ void operator()(size_t g, double v) const {
+        sum[g] = sum[g] + v;
+        const double m = max[g];
+        max[g] = (m != m) ? m : ((v != v || v > m) ? v : m);   // np.maximum(m, v): the first NaN wins
+        if (above && v > thr) above[g] += 1;
+    }
+};
+template <class Epi>
+__device__ __forceinline__ void density_tile(int N, const double *__restrict__ ax, const double *__restrict__ ay,
+                                             const uint8_t *__restrict__ status, const double *__restrict__ X,
+                                             const double *__restrict__ Y, const double *__restrict__ Vg, int Ny, int Nx,
+                                             double two_s2, double C, double r_zero, int bx, int by, const Epi &epi) {
     __shared__ double lx[DN_CHUNK], ly[DN_CHUNK];
     __shared__ int wcnt[8];
-    const int ix = blockIdx.x * DN_TX + (threadIdx.x & 31), iy = blockIdx.y * DN_TY + (threadIdx.x >> 5);
+    const int ix = bx * DN_TX + (threadIdx.x & 31), iy = by * DN_TY + (threadIdx.x >> 5);
     const bool in = ix < Nx && iy < Ny;
     const double x = in ? X[ix] : 0.0, y = in ? Y[iy] : 0.0;
-    const int jx0 = blockIdx.x * DN_TX, jx1 = min(jx0 + DN_TX, Nx) - 1, jy0 = blockIdx.y * DN_TY,
-              jy1 = min(jy0 + DN_TY, Ny) - 1;
+    const int jx0 = bx * DN_TX, jx1 = min(jx0 + DN_TX, Nx) - 1, jy0 = by * DN_TY, jy1 = min(jy0 + DN_TY, Ny) - 1;
     const double bx0 = X[jx0] - r_zero, bx1 = X[jx1] + r_zero, by0 = Y[jy0] - r_zero, by1 = Y[jy1] + r_zero;
     double d = 0.0;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -1324,8 +1344,61 @@ density_kernel(int N, const double *__restrict__ ax, const double *__restrict__ 
     }
     if (in) {
         size_t g = (size_t)iy * Nx + ix;
-        out[g] = (Vg[g] < 0) ? 0.0 : d;  // :485
+        epi(g, (Vg[g] < 0) ? 0.0 : d);  // :485
     }
+}
+
+__global__ void __launch_bounds__(256)
+density_kernel(int N, const double *__restrict__ ax, const double *__restrict__ ay, const uint8_t *__restrict__ status,
+               const double *__restrict__ X, const double *__restrict__ Y, const double *__restrict__ Vg, int Ny,
+               int Nx, double two_s2, double C, double r_zero, double *__restrict__ out) {
+    density_tile(N, ax, ay, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y, DensityStore{out});
+}
+
+__global__ void __launch_bounds__(256)
+density_accum_kernel(int N, const double *__restrict__ ax, const double *__restrict__ ay,
+                     const uint8_t *__restrict__ status, const double *__restrict__ X, const double *__restrict__ Y,
+                     const double *__restrict__ Vg, int Ny, int Nx, double two_s2, double C, double r_zero,
+                     DensityAccum acc) {
+    density_tile(N, ax, ay, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y, acc);
+}
+
+// Batched accumulation: one flattened 1-D grid of exactly the members' tiles.  Member m owns blocks [tile0, tile0 +
+// ntx * nty) in row-major tile order; a block finds its member by a (block-uniform) binary search over tile0.
+struct DensityMember {
+    const double *x, *y;
+    const uint8_t *status;
+    const double *X, *Y, *Vg;
+    DensityAccum acc;
+    double two_s2, C, r_zero;
+    int N, Ny, Nx, ntx, tile0, pad_;
+};
+__global__ void __launch_bounds__(256)
+density_accum_multi_kernel(const DensityMember *__restrict__ ms, int n) {
+    const int b = blockIdx.x;
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ms[mid].tile0 <= b) lo = mid;
+        else hi = mid - 1;
+    }
+    const DensityMember &m = ms[lo];
+    const int t = b - m.tile0;
+    density_tile(m.N, m.x, m.y, m.status, m.X, m.Y, m.Vg, m.Ny, m.Nx, m.two_s2, m.C, m.r_zero, t % m.ntx, t / m.ntx,
+                 m.acc);
+}
+
+int density_acc_check(const oc_density_acc *a) {
+    OC_ARG(a && a->d_sum && a->d_max && a->d_Vglobal, "NULL argument");
+    OC_ARG(a->every >= 1, "density statistics: every must be >= 1");
+    OC_ARG(std::isfinite(a->sigma) && a->sigma > 0 && std::isfinite(a->C) && a->C > 0,
+           "density statistics: sigma and C must be finite and positive");
+    OC_ARG(!a->d_above || std::isfinite(a->threshold), "density statistics: the threshold must be finite");
+    return OC_OK;
+}
+
+DensityAccum density_epilogue(const oc_density_acc *a) {
+    return DensityAccum{a->d_sum, a->d_max, a->d_above, a->threshold};
 }
 
 template <class T>
@@ -2074,16 +2147,19 @@ extern "C" int oc_gcfm_step_multi_finish(int n, oc_ctx *const *ctxs, int *const 
 // Stops early when nobody is inside (the reference's loop condition) or on an error; *steps_done steps were executed
 // (on OC_ERR_SAMPLER_RANGE including the offending one, as oc_gcfm_step).  exit_agent / exit_step (capacity N): agents in
 // exit order and the index (0-based within this call) of the step they left in.  *device_ms: sum of the steps' CUDA-event
-// times; *pairs: interacting pairs evaluated.
-extern "C" int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
-                           double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
-                           const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
-                           double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
-                           int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
-                           long long *pairs, void *stream) {
+// times; *pairs: interacting pairs evaluated.  acc (nullable): density statistics, one frame added before every step
+// whose simu_step is a multiple of acc->every (the history frame of that iteration), ahead of the step's randomness.
+extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                               long long *pairs, const oc_density_acc *acc, void *stream) {
     OC_ARG(ctx && prm && mt_key && mt_pos && has_gauss && cached_gauss && exit_agent && exit_step && n_exits && steps_done,
            "NULL argument");
     OC_ARG(N >= 1 && n_steps >= 0 && n_active0 >= 0 && n_active0 <= N && *mt_pos >= 0 && *mt_pos <= 624, "bad sizes");
+    if (acc)
+        if (int rc = density_acc_check(acc)) return rc;
     constexpr int N_CKPT = 64;
     *n_exits = 0;
     *steps_done = 0;
@@ -2099,6 +2175,11 @@ extern "C" int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double
     int n_active = n_active0;
     int rc = OC_OK;
     for (int k = 0; k < n_steps && n_active > 0; k++) {
+        // ---- this iteration's history frame (simulations.py:428), folded into the statistics
+        if (acc && (simu_step0 + k) % acc->every == 0) {
+            rc = oc_density_accum(ctx, acc, N, d_x, d_y, d_status, stream);
+            if (rc) return rc;
+        }
         // ---- this step's randomness (simulations.py:271,303)
         const int q = n_spec - n_active;
         if (spec && q >= 0 && q < n_ckpt) {
@@ -2147,6 +2228,17 @@ extern "C" int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double
     return OC_OK;
 }
 
+extern "C" int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                           double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                           const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                           double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                           int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                           long long *pairs, void *stream) {
+    return oc_gcfm_run_acc(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key, mt_pos,
+                           has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent, exit_step, n_exits,
+                           steps_done, device_ms, pairs, nullptr, stream);
+}
+
 extern "C" double oc_gcfm_last_ms(oc_ctx *ctx) { return ctx ? ctx->gcfm_last_ms : 0.0; }
 extern "C" long long oc_gcfm_last_pairs(oc_ctx *ctx) { return ctx ? ctx->gcfm_last_pairs : 0; }
 extern "C" int oc_gcfm_last_redos(oc_ctx *ctx) { return ctx ? ctx->gcfm_redos : 0; }
@@ -2192,12 +2284,64 @@ extern "C" int oc_density(oc_ctx *ctx, int N, const double *d_x, const double *d
     OC_ARG(ctx && d_Vglobal && d_out && (N == 0 || (d_x && d_y && d_status)), "NULL argument");
     OC_CUDA(cudaSetDevice(ctx->device));
     const double two_s2 = 2 * (sigma * sigma);
-    // ocm_exp(x) == 0 exactly for x < -745.14: r^2/two_s2 > 745.2  =>  contribution is exactly 0.0
-    const double r_zero = std::sqrt(745.2 * two_s2) * (1.0 + 1e-9) + 1e-9;
     dim3 grid((ctx->Nx + DN_TX - 1) / DN_TX, (ctx->Ny + DN_TY - 1) / DN_TY);
     density_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(N, d_x, d_y, d_status, ctx->d_X, ctx->d_Y, d_Vglobal,
-                                                           ctx->Ny, ctx->Nx, two_s2, C, r_zero, d_out);
+                                                           ctx->Ny, ctx->Nx, two_s2, C, density_r_zero(two_s2), d_out);
     oc::count_launch();
     OC_CUDA(cudaGetLastError());
+    return OC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ density statistics
+extern "C" int oc_density_accum(oc_ctx *ctx, const oc_density_acc *acc, int N, const double *d_x, const double *d_y,
+                                const uint8_t *d_status, void *stream) {
+    OC_ARG(ctx && N >= 0 && (N == 0 || (d_x && d_y && d_status)), "NULL argument");
+    if (int rc = density_acc_check(acc)) return rc;
+    OC_CUDA(cudaSetDevice(ctx->device));
+    const double two_s2 = 2 * (acc->sigma * acc->sigma);
+    dim3 grid((ctx->Nx + DN_TX - 1) / DN_TX, (ctx->Ny + DN_TY - 1) / DN_TY);
+    density_accum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(N, d_x, d_y, d_status, ctx->d_X, ctx->d_Y,
+                                                                 acc->d_Vglobal, ctx->Ny, ctx->Nx, two_s2, acc->C,
+                                                                 density_r_zero(two_s2), density_epilogue(acc));
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    return OC_OK;
+}
+
+extern "C" int oc_density_accum_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs, const int *Ns,
+                                      const double *const *x, const double *const *y, const uint8_t *const *status,
+                                      void *stream) {
+    OC_ARG(n >= 1 && ctxs && accs && Ns && x && y && status && ctxs[0], "NULL argument");
+    oc_ctx *c0 = ctxs[0];
+    for (int m = 0; m < n; m++) {
+        OC_ARG(ctxs[m] && Ns[m] >= 0 && (Ns[m] == 0 || (x[m] && y[m] && status[m])), "NULL argument");
+        OC_ARG(ctxs[m]->device == c0->device, "density statistics: member context on another device");
+        if (int rc = density_acc_check(accs[m])) return rc;
+    }
+    OC_CUDA(cudaSetDevice(c0->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t bytes = sizeof(DensityMember) * (size_t)n;
+    // the table (staging and device copy) is reused once the previous call's kernel has read it, whatever its stream
+    if (!c0->dens_ev) OC_CUDA(cudaEventCreateWithFlags(&c0->dens_ev, cudaEventDisableTiming));
+    OC_CUDA(cudaEventSynchronize(c0->dens_ev));
+    if (int rc = oc_ensure_buffer(c0->dens_pinned, c0->dens_pinned_bytes, bytes, true, "density member table")) return rc;
+    if (int rc = oc_ensure_buffer(c0->dens_dev, c0->dens_dev_bytes, bytes, false, "density member table")) return rc;
+    DensityMember *recs = static_cast<DensityMember *>(c0->dens_pinned);
+    long long tiles = 0;
+    for (int m = 0; m < n; m++) {
+        const oc_ctx *c = ctxs[m];
+        const oc_density_acc *a = accs[m];
+        const int ntx = (c->Nx + DN_TX - 1) / DN_TX, nty = (c->Ny + DN_TY - 1) / DN_TY;
+        const double two_s2 = 2 * (a->sigma * a->sigma);
+        recs[m] = DensityMember{x[m], y[m], status[m], c->d_X, c->d_Y, a->d_Vglobal, density_epilogue(a), two_s2, a->C,
+                                density_r_zero(two_s2), Ns[m], c->Ny, c->Nx, ntx, (int)tiles, 0};
+        tiles += (long long)ntx * nty;
+    }
+    OC_ARG(tiles < 0x7fffffff, "density statistics: too many tiles for one launch");
+    OC_CUDA(cudaMemcpyAsync(c0->dens_dev, recs, bytes, cudaMemcpyHostToDevice, st));
+    density_accum_multi_kernel<<<(unsigned)tiles, 256, 0, st>>>(static_cast<const DensityMember *>(c0->dens_dev), n);
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    OC_CUDA(cudaEventRecord(c0->dens_ev, st));
     return OC_OK;
 }

@@ -20,7 +20,10 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     same batched call, its re-solves happen at its own steps, and it still equals the stand-alone
     ``simulation(..., config=...)`` run bit for bit (tests/test_gpu_ensemble_params.py);
   * members may have different rooms: different grid shapes and numbers of target sets (one grid step for all).
-    Every member still equals its stand-alone run bit for bit (tests/test_gpu_ensemble_shapes.py).
+    Every member still equals its stand-alone run bit for bit (tests/test_gpu_ensemble_shapes.py);
+  * ``density_stats``: every member accumulates the sum, maximum and above-threshold count of its density frames on the
+    device (one batched ``oc_density_accum_multi`` launch per step for the due members of a wave) and hands them back
+    in ``results[i]["density"]`` -- no frames, trajectories or members are kept (tests/test_gpu_density_stats.py).
 """
 from __future__ import annotations
 
@@ -101,6 +104,10 @@ class ensemble:
     ``times`` (per-agent clocks, as evac_times() returns them), ``final`` (N,4: x, y, vx, vy) and ``hjb`` (solver
     statistics per target set) and ``config`` (the member's effective configuration).
 
+    ``density_stats``: None, True or dict(every=1, threshold=None) for every member, as ``simulation(...,
+    density_stats=...)`` takes it (each member with its own ``sigma_convolution``); ``results[i]["density"]`` is then the
+    member's ``density_stats()`` dict.
+
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
     ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
     their rooms may differ in size and number of target sets.
@@ -111,7 +118,8 @@ class ensemble:
     single-shape ensemble)."""
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
-                 memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None):
+                 memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None,
+                 density_stats=None):
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -133,6 +141,7 @@ class ensemble:
         self.configs = [optimals._merge_config(base, o) if o is not None else base for o in self.overrides]
         if len({c["grid_step"] for c in self.configs}) > 1:
             raise ValueError("ensemble members must share grid_step (one grid for the batched solves)")
+        self.density_stats = simulations.density_stats_spec(density_stats)   # (every, threshold) or None
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -159,13 +168,17 @@ class ensemble:
         return self._rooms_loaded[room]
 
     def member_bytes(self, members=None):
-        """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets); no CUDA"""
+        """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets, plus the
+        density accumulators when density_stats is on); no CUDA"""
         out = []
         for i in (self.mine if members is None else members):
             room, cfg = self._room(i), self.configs[i]
             Ny, Nx = _lib.grid_shape(room["room_length"], room["room_height"], cfg["grid_step"])
             n_keys = len({' or '.join(b[5:]) for b in room["initial_boxes"].values()})
-            out.append(field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage))
+            b = field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage)
+            if self.density_stats is not None:
+                b += _lib.DensityStats.nbytes(Ny, Nx, self.density_stats[1])
+            out.append(b)
         return out
 
     def _build(self, idx):
@@ -179,7 +192,9 @@ class ensemble:
         return simulations.simulation(copy.deepcopy(room), self.T, recompute=self.recompute, record=self.record,
                                       field_storage=self.field_storage, fused=1, lookahead=False,
                                       rng=np.random.RandomState(self.seeds[idx]), chunk_rows=self.chunk_rows,
-                                      config=self.overrides[idx], _ctx=ctx)
+                                      config=self.overrides[idx], _ctx=ctx,
+                                      density_stats=None if self.density_stats is None else
+                                      dict(every=self.density_stats[0], threshold=self.density_stats[1]))
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -319,6 +334,12 @@ class ensemble:
                     if self.record:
                         s.write_history(s.time)
                     self.stats["agent_steps"] += s.inside
+                if self.density_stats is not None:
+                    # this iteration's frames of the members due at their own step, one launch for all of them
+                    dd = [q for q in live if sims[q]._dstats.due(sims[q].simu_step)]
+                    if dd:
+                        _lib.density_accum_multi([sims[q]._ctx for q in dd], [sims[q]._dstats for q in dd],
+                                                 [sims[q]._state for q in dd], stream=main)
                 batch.launch(live, [sims[q].inside for q in live], [sims[q].simu_step for q in live], stream=main,
                              rebind=rebind)
                 tl1 = time.perf_counter()
@@ -331,6 +352,7 @@ class ensemble:
                     if self.record:
                         s.write_history(s.time)
                     self.stats["agent_steps"] += s.inside
+                    s._density_frame()
                     launched.append(s._step_launch(s.dt))
                 tl1 = time.perf_counter()
                 for q, l in zip(live, launched):
@@ -349,6 +371,8 @@ class ensemble:
                                    times=np.array(s._h_timev, dtype=float), final=np.array(s._h_now, dtype=float),
                                    hjb={k: o.last_stats for k, o in s.targets.items()}, config=self.configs[i],
                                    chunk_rows=self.member_chunk_rows[i])
+            if self.density_stats is not None:
+                self.results[i]["density"] = s._dstats.result()
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3

@@ -26,6 +26,49 @@ from .optimals import _load_config, _load_room, _merge_config
 warnings.filterwarnings("ignore")  # simulations.py:15
 
 
+def density_stats_spec(value):
+    """(every, threshold) of a ``density_stats`` argument, or None when the statistics are off: None / False (off), True
+    (every frame, no threshold) or dict(every=1, threshold=None); checked without touching a GPU"""
+    if value is None or value is False:
+        return None
+    if value is True:
+        return 1, None
+    if not isinstance(value, dict):
+        raise ValueError("density_stats: expected None, True or dict(every=..., threshold=...)")
+    unknown = set(value) - {"every", "threshold"}
+    if unknown:
+        raise ValueError(f"density_stats: unknown keys {sorted(unknown)}")
+    every, thr = value.get("every", 1), value.get("threshold")
+    if isinstance(every, bool) or not isinstance(every, (int, np.integer)) or every < 1:
+        raise ValueError("density_stats: every must be an integer >= 1")
+    if thr is not None:
+        if isinstance(thr, bool) or not isinstance(thr, (int, float, np.integer, np.floating)) or not np.isfinite(thr):
+            raise ValueError("density_stats: threshold must be None or a finite number")
+        thr = float(thr)
+    return int(every), thr
+
+
+def density_frame_steps(T, dt, every, recompute_step=None):
+    """The simu_steps whose frames run() adds to the density statistics when nobody leaves before T: run()'s loop
+    (simulations.py:427-441) as it is cut into blocks here -- one advance() per stretch up to the next re-solve (every
+    ``recompute_step`` steps, None = no re-solves) -- each block taking the frames of its steps that are multiples of
+    ``every``.  The frames do not depend on the cut: this is the plain loop's selection."""
+    out, time, step = [], 0., 0
+    while time < T:
+        n, t = 0, time
+        while t < T:
+            t += dt
+            n += 1
+            if recompute_step and (step + n) % recompute_step == 0:
+                break
+        for _ in range(n):
+            if step % every == 0:
+                out.append(step)
+            time += dt
+            step += 1
+    return out
+
+
 class _Agents:
     """``simulation.agents``: the reference's array of ``ped`` objects (simulations.py:142-151), built on first access.
     A ``ped`` here is a view of row i of the device-resident crowd state, so nothing but the object itself is created;
@@ -127,7 +170,7 @@ class simulation:
     TRACK_CHUNK = 64  # steps per block of the device-resident trajectory record
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
-                 rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, _ctx=None):
+                 rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -141,8 +184,16 @@ class simulation:
         ranks of torch.distributed: a rank solves and stores only its keys' fields and evaluates the field samples / wall
         forces of the agents heading for them; merge and sweep as for ``band``), ``config`` (a dict of overrides of
         config.json, e.g. ``{"dt": 0.01, "hjb_params": {"g": -0.01}}``: nested ``hjb_params`` are merged key by key, a
-        key config.json does not have raises KeyError; ``_config`` is the effective configuration)."""
+        key config.json does not have raises KeyError; ``_config`` is the effective configuration), ``density_stats`` (True
+        or dict(every=1, threshold=None): accumulate on the device, per grid node, the sum and the maximum of the density
+        frames the reference stores in ``history`` (simulations.py:579-589) at the steps of run()'s loop whose simu_step
+        is a multiple of ``every``, and with a threshold the number of frames above it; read them with
+        ``density_stats()``.  Not available with ``band`` or ``shard_keys``)."""
         import torch
+        dstats = density_stats_spec(density_stats)
+        if dstats is not None and (band or shard_keys):
+            raise ValueError("density_stats is not available for row-decomposed (band=True) or key-sharded "
+                             "(shard_keys=True) runs")
         self._np_random = rng if rng is not None else np.random
         self.recompute = recompute
         var_config = _load_config()       # simulations.py:42
@@ -270,6 +321,8 @@ class simulation:
         self._d_vdes = ctx.to_device(self._h_vdes)
         self._d_key = ctx.to_device(self._h_key)
         self._d_Vglobal = ctx.to_device(self.V)
+        # density statistics of the run's frames (device accumulators, written by oc_density_accum / oc_gcfm_run_acc)
+        self._dstats = None if dstats is None else _lib.DensityStats(ctx, self._d_Vglobal, self.sigma_convolution, *dstats)
         # per-step record of (x, y, vx, vy); row k = state after k steps (ped.traj / ped.vels / history views).  It
         # lives on the DEVICE in blocks of TRACK_CHUNK steps, written by one small kernel per step (oc_state_pack), and
         # is read back -- once per row -- only when somebody looks at it
@@ -422,6 +475,7 @@ class simulation:
             done = 0
             while done < n_steps and self.inside > 0:
                 self.write_history(self.time)
+                self._density_frame()
                 self.step(self.dt, verbose=verbose)
                 done += 1
             return done
@@ -437,7 +491,7 @@ class simulation:
             rows.append(self._d_track[blk][off])
         n_active = int(self._h_status.sum())
         res = self._ctx.gcfm_run(self._gcfm_prm, self._state, self._d_vdes, self._d_key, self._keys(), st, n_steps,
-                                 self.simu_step, n_active, rows=rows, stream=self._cuda_stream)
+                                 self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats)
         self._rng.rng.set_state(res["rng_state"])
         self.last_run_stats = dict(steps=res["steps"], device_ms=res["device_ms"], pairs=res["pairs"])
         ex, exs = res["exits"], res["exit_step"]
@@ -459,6 +513,23 @@ class simulation:
             raise IndexError("agent position outside the velocity field's index range "
                              "(numpy raises IndexError in the reference's sampler too: optimals.py:247)")
         return res["steps"]
+
+    def _density_frame(self):
+        """add this iteration's frame to the density statistics when they are on and it is due (before the step)"""
+        if self._dstats is not None and self._dstats.due(self.simu_step):
+            st = self._state
+            self._ctx.density_accum(self._dstats, st["x"], st["y"], st["status"], stream=self._cuda_stream)
+
+    def density_stats(self):
+        """the density statistics of the frames taken so far (``density_stats=`` of the constructor): dict(frames, sum,
+        max, above, mean) -- (Ny, Nx) numpy arrays; ``above`` (int32 counts of frames with density > threshold) is None
+        without a threshold, ``mean`` = sum / frames is None before the first frame"""
+        if self._dstats is None:
+            raise RuntimeError("this simulation was created without density_stats")
+        if self._cuda_stream is not None:
+            import torch
+            torch.cuda.synchronize(self._ctx.torch_device)
+        return self._dstats.result()
 
     def _step_finish(self, launched, verbose=False):
         dt, pending = launched
