@@ -430,6 +430,63 @@ int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, 
                     int simu_step0, int n_active0, double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
                     int *steps_done, double *device_ms, long long *pairs, const oc_density_acc *acc, void *stream);
 
+/* Velocity maps of the density frames (density_stats=dict(velocity=True)).  One frame adds, per node, over the agents of
+ * the density frame (same order, culling and wall rule) with w the value the density frame adds for agent i
+ * (ocm_exp(-r*r / (2*sigma*sigma)) / C): d_vx_sum += sum w*vx_i, d_vy_sum += sum w*vy_i, d_speed_sum += sum w*s_i,
+ * s_i = sqrt(vx_i*vx_i + vy_i*vy_i); 0 on walls.  float64 (Ny,Nx) arrays, caller-owned and zero-initialised. */
+typedef struct {
+    double *d_vx_sum, *d_vy_sum, *d_speed_sum;
+} oc_velocity_acc;
+/* oc_density_accum plus, when vel is not NULL, the frame's velocity maps (vx, vy: the agents' velocities in the state
+ * the frame describes).  The density sum is computed with the same operations in the same order, so acc receives exactly
+ * what oc_density_accum adds.  OC_ERR_ARG as oc_density_accum, and for a NULL vel array or NULL d_vx / d_vy with vel. */
+int oc_density_accum_vel(oc_ctx *ctx, const oc_density_acc *acc, const oc_velocity_acc *vel, int N, const double *d_x,
+                         const double *d_y, const double *d_vx, const double *d_vy, const uint8_t *d_status,
+                         void *stream);
+/* oc_density_accum_multi with velocity maps: vels (NULL, or per member NULL / the member's maps), vx / vy (read for the
+ * members with maps).  Members with and without maps run as one launch each; every result equals the member's
+ * oc_density_accum_vel alone.  oc_density_accum / oc_density_accum_multi forward here with no maps. */
+int oc_density_accum_vel_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs,
+                               const oc_velocity_acc *const *vels, const int *Ns, const double *const *x,
+                               const double *const *y, const double *const *vx, const double *const *vy,
+                               const uint8_t *const *status, void *stream);
+
+/* Pedestrian counts through measurement lines.  With o(u,v,w) = (v.x-u.x)*(w.y-u.y) - (v.y-u.y)*(w.x-u.x) (FP64, no
+ * contraction) and a line's endpoints a, b, an agent inside at the start of a step that moves from p (kept in d_px /
+ * d_py) to q (its position after the step, the step it leaves in included) crosses the line when
+ * (o(a,b,p) > 0) != (o(a,b,q) > 0) and (o(p,q,a) > 0) != (o(p,q,b) > 0): to the left when o(a,b,q) > 0, else to the
+ * right.  Points on the line count as the right side; NaN positions never cross.  d_counts[(step*n_lines + l)*2 + 0] /
+ * [... + 1] count the step's crossings of line l to the left / right.  d_px, d_py, d_inside (17 bytes per agent):
+ * initialised by the caller with the crowd's x, y and status before its first counted step; each update compares them
+ * with the current state and then overwrites them. */
+typedef struct {
+    const double *lines;       /* HOST: n_lines x (x0, y0, x1, y1) in metres; finite, non-zero length */
+    int *d_counts;             /* int32 (capacity, n_lines, 2), caller-owned, zero-initialised */
+    double *d_px, *d_py;       /* (N) previous positions */
+    uint8_t *d_inside;         /* (N) inside at the start of the step */
+    int n_lines;               /* 1..64 */
+    int capacity;              /* steps d_counts has rows for */
+} oc_lines_acc;
+/* Counts the crossings of the step with simu_step `step` (the crowd's state after it, once final: after
+ * oc_gcfm_step_finish).  Asynchronous on stream.  OC_ERR_ARG for a NULL required pointer, n_lines outside 1..64, a
+ * non-finite or zero-length line and step outside [0, capacity). */
+int oc_lines_count(oc_ctx *ctx, const oc_lines_acc *acc, int N, const double *d_x, const double *d_y,
+                   const uint8_t *d_status, int step, void *stream);
+/* oc_lines_count for each of n members (step steps[m]) in ONE launch; ctxs[0] owns the member table.  OC_ERR_ARG as
+ * oc_lines_count, and for a member context on another device than ctxs[0]. */
+int oc_lines_count_multi(int n, oc_ctx *const *ctxs, const oc_lines_acc *const *accs, const int *Ns,
+                         const double *const *x, const double *const *y, const uint8_t *const *status, const int *steps,
+                         void *stream);
+/* The run loop's only implementation: oc_gcfm_run_acc plus the velocity maps of its frames (vel, needs acc) and the
+ * line counts of its steps (lines: every step simu_step0 + k is counted once final; simu_step0 + n_steps must not exceed
+ * lines->capacity, checked before any step).  oc_gcfm_run and oc_gcfm_run_acc forward here. */
+int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
+                     double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,
+                     int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss, int n_steps,
+                     int simu_step0, int n_active0, double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
+                     int *steps_done, double *device_ms, long long *pairs, const oc_density_acc *acc,
+                     const oc_velocity_acc *vel, const oc_lines_acc *lines, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

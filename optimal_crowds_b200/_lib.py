@@ -88,6 +88,15 @@ class DensityAcc(C.Structure):
                 ("pad_", C.c_int)]
 
 
+class VelocityAcc(C.Structure):
+    _fields_ = [("d_vx_sum", C.c_void_p), ("d_vy_sum", C.c_void_p), ("d_speed_sum", C.c_void_p)]
+
+
+class LinesAcc(C.Structure):
+    _fields_ = [("lines", dp), ("d_counts", C.c_void_p), ("d_px", C.c_void_p), ("d_py", C.c_void_p),
+                ("d_inside", C.c_void_p), ("n_lines", C.c_int), ("capacity", C.c_int)]
+
+
 _lib = None
 
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
@@ -95,7 +104,8 @@ EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create"
            "oc_wall_force", "oc_pair_force", "oc_density", "oc_gcfm_last_ms", "oc_dist_unique_id", "oc_dist_init",
            "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_hjb_solve_grids", "oc_gcfm_step_launch",
            "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run",
-           "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi"]
+           "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi", "oc_density_accum_vel",
+           "oc_density_accum_vel_multi", "oc_lines_count", "oc_lines_count_multi", "oc_gcfm_run_flow"]
 
 
 def load():
@@ -128,6 +138,13 @@ def load():
     lib.oc_gcfm_run_acc.argtypes = lib.oc_gcfm_run.argtypes[:-1] + [C.POINTER(DensityAcc), C.c_void_p]
     lib.oc_density_accum.argtypes = [C.c_void_p, C.POINTER(DensityAcc), C.c_int] + [C.c_void_p] * 4
     lib.oc_density_accum_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, C.c_void_p]
+    lib.oc_gcfm_run_flow.argtypes = lib.oc_gcfm_run_acc.argtypes[:-1] + [C.POINTER(VelocityAcc), C.POINTER(LinesAcc),
+                                                                         C.c_void_p]
+    lib.oc_density_accum_vel.argtypes = [C.c_void_p, C.POINTER(DensityAcc), C.POINTER(VelocityAcc), C.c_int] + \
+                                        [C.c_void_p] * 6
+    lib.oc_density_accum_vel_multi.argtypes = [C.c_int, vpp_, vpp_, vpp_, ip, vpp_, vpp_, vpp_, vpp_, vpp_, C.c_void_p]
+    lib.oc_lines_count.argtypes = [C.c_void_p, C.POINTER(LinesAcc), C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
+    lib.oc_lines_count_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, ip, C.c_void_p]
     lib.oc_rng_step_draw.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp]
     lib.oc_rng_step_draw_ckpt.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp, C.c_int,
                                           C.POINTER(C.c_uint32), ip, ip, dp]
@@ -532,11 +549,12 @@ class Context:
         return exit_log[: n_exit.value].copy(), rc
 
     def gcfm_run(self, prm: GcfmParams, state, vdes, key_id, keys, rng_state, n_steps, simu_step0, n_active, rows=None,
-                 stream=None, density=None):
-        """up to n_steps steps of the run loop in one call (oc_gcfm_run_acc): randomness drawn in C from the legacy MT19937
+                 stream=None, density=None, lines=None):
+        """up to n_steps steps of the run loop in one call (oc_gcfm_run_flow): randomness drawn in C from the legacy MT19937
         state tuple `rng_state` (np.random.get_state()), next step's draws overlapped with the GPU.  rows: optional list of
         n_steps (N,4) CUDA tensors receiving the packed state after each step.  density: optional DensityStats that
-        receives the frame of every due step.  Returns dict(steps, exits (agent ids in exit order), exit_step (0-based step
+        receives the frame of every due step (with its velocity maps when it has them).  lines: optional LineCounts that
+        receives the crossings of every step (its capacity must cover simu_step0 + n_steps).  Returns dict(steps, exits (agent ids in exit order), exit_step (0-based step
         within the call), rc, rng_state (to be set_state()d), device_ms, pairs)."""
         N = state["x"].numel()
         karr, keep = keys if isinstance(keys, tuple) else self.make_keys(keys)
@@ -550,13 +568,15 @@ class Context:
                 rows_arr[q] = r.data_ptr()
         ex_a, ex_s = np.empty(max(N, 1), dtype=np.int32), np.empty(max(N, 1), dtype=np.int32)
         n_ex, done, ms, pairs = C.c_int(), C.c_int(), C.c_double(), C.c_longlong()
-        rc = load().oc_gcfm_run_acc(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
-                                    _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
-                                    karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
-                                    C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
-                                    ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
-                                    C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc),
-                                    _stream() if stream is None else C.c_void_p(stream))
+        vel = None if density is None or density.vel is None else C.byref(density.vel)
+        rc = load().oc_gcfm_run_flow(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
+                                     _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
+                                     karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
+                                     C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
+                                     ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
+                                     C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc), vel,
+                                     None if lines is None else C.byref(lines.acc),
+                                     _stream() if stream is None else C.c_void_p(stream))
         check(rc, allow=(OC_ERR_SAMPLER_RANGE,))
         if density is not None:
             density.frames += density.count(simu_step0, done.value)
@@ -612,46 +632,81 @@ class Context:
                                 _stream()))
         return d
 
-    def density_accum(self, stats, x, y, status, stream=None):
-        """add the density frame of the crowd (x, y, status; None for no agents) to `stats` (oc_density_accum)"""
+    def density_accum(self, stats, x, y, status, stream=None, vx=None, vy=None):
+        """add the density frame of the crowd (x, y, status; None for no agents) to `stats` (oc_density_accum_vel; vx, vy:
+        the agents' velocities, read when `stats` has velocity maps)"""
         N = 0 if x is None else x.numel()
-        check(load().oc_density_accum(self.h, C.byref(stats.acc), N, _dev(x), _dev(y), _dev(status),
-                                      _stream() if stream is None else C.c_void_p(stream)))
+        check(load().oc_density_accum_vel(self.h, C.byref(stats.acc), None if stats.vel is None else C.byref(stats.vel),
+                                          N, _dev(x), _dev(y), _dev(vx), _dev(vy), _dev(status),
+                                          _stream() if stream is None else C.c_void_p(stream)))
         stats.frames += 1
+
+    def lines_count(self, lines, state, step, stream=None):
+        """count the crossings of the step with simu_step `step` (state: the crowd after it) in `lines` (oc_lines_count)"""
+        check(load().oc_lines_count(self.h, C.byref(lines.acc), state["x"].numel(), _dev(state["x"]), _dev(state["y"]),
+                                    _dev(state["status"]), int(step), _stream() if stream is None else C.c_void_p(stream)))
 
 
 def density_accum_multi(ctxs, stats, states, stream=None):
-    """one density frame per member in one launch (oc_density_accum_multi): member q's crowd `states[q]` (dict with x, y,
-    status) on the grid of ctxs[q], added to stats[q]"""
+    """one density frame per member in one launch per variant (oc_density_accum_vel_multi): member q's crowd `states[q]`
+    (dict with x, y, status, and vx, vy when stats[q] has velocity maps) on the grid of ctxs[q], added to stats[q]"""
     n = len(ctxs)
     if not (len(stats) == len(states) == n and n):
         raise ValueError("one context, statistics and state per member expected")
     vp = lambda: (C.c_void_p * n)()
-    hs, accs, xs, ys, sts = vp(), vp(), vp(), vp(), vp()
+    hs, accs, vels, xs, ys, vxs, vys, sts = vp(), vp(), vp(), vp(), vp(), vp(), vp(), vp()
     Ns = np.empty(n, dtype=np.int32)
     for q, (c, s, st) in enumerate(zip(ctxs, stats, states)):
         hs[q] = c.h.value
         accs[q] = C.addressof(s.acc)
         Ns[q] = st["x"].numel()
         xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
-    check(load().oc_density_accum_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, sts,
-                                        _stream() if stream is None else C.c_void_p(stream)))
+        if s.vel is not None:
+            vels[q] = C.addressof(s.vel)
+            vxs[q], vys[q] = st["vx"].data_ptr(), st["vy"].data_ptr()
+    check(load().oc_density_accum_vel_multi(n, hs, accs, vels, Ns.ctypes.data_as(ip), xs, ys, vxs, vys, sts,
+                                            _stream() if stream is None else C.c_void_p(stream)))
     for s in stats:
         s.frames += 1
+
+
+def lines_count_multi(ctxs, lines, states, steps, stream=None):
+    """the crossings of one step per member in one launch (oc_lines_count_multi): member q's crowd after its step
+    `steps[q]` (`states[q]`: dict with x, y, status) counted in lines[q]"""
+    n = len(ctxs)
+    if not (len(lines) == len(states) == len(steps) == n and n):
+        raise ValueError("one context, line counter, state and step per member expected")
+    vp = lambda: (C.c_void_p * n)()
+    hs, accs, xs, ys, sts = vp(), vp(), vp(), vp(), vp()
+    Ns = np.empty(n, dtype=np.int32)
+    ss = np.ascontiguousarray(steps, dtype=np.int32)
+    for q, (c, lc, st) in enumerate(zip(ctxs, lines, states)):
+        hs[q] = c.h.value
+        accs[q] = C.addressof(lc.acc)
+        Ns[q] = st["x"].numel()
+        xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
+    check(load().oc_lines_count_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, sts, ss.ctypes.data_as(ip),
+                                      _stream() if stream is None else C.c_void_p(stream)))
 
 
 class DensityStats:
     """Device accumulators of a run's density frames (oc_density_acc): per node of the (Ny, Nx) grid the sum and the
     maximum of the frames (float64) and, with a threshold, the number of frames above it (int32); zero at creation.
     sigma: the run's sigma_convolution; Vglobal: its simulation.V on the device; every: frames are taken at the steps
-    whose simu_step is a multiple of it."""
+    whose simu_step is a multiple of it.  velocity: also the velocity maps of the frames (oc_velocity_acc: per node the
+    density-weighted sums of vx, vy and the speed, float64)."""
 
-    def __init__(self, ctx, Vglobal, sigma, every=1, threshold=None):
+    def __init__(self, ctx, Vglobal, sigma, every=1, threshold=None, velocity=False):
         import torch
         shape = (ctx.Ny, ctx.Nx)
         self.sum = torch.zeros(shape, dtype=torch.float64, device=ctx.torch_device)
         self.max = torch.zeros(shape, dtype=torch.float64, device=ctx.torch_device)
         self.above = None if threshold is None else torch.zeros(shape, dtype=torch.int32, device=ctx.torch_device)
+        self.vx_sum = self.vy_sum = self.speed_sum = self.vel = None
+        if velocity:
+            self.vx_sum, self.vy_sum, self.speed_sum = (torch.zeros(shape, dtype=torch.float64, device=ctx.torch_device)
+                                                        for _ in range(3))
+            self.vel = VelocityAcc(self.vx_sum.data_ptr(), self.vy_sum.data_ptr(), self.speed_sum.data_ptr())
         self.Vglobal = Vglobal
         self.every, self.threshold, self.frames = int(every), threshold, 0
         Cn = float(np.sqrt(4 * np.pi ** 2 * sigma ** 2))  # simulations.py:482, as Context.density
@@ -670,14 +725,68 @@ class DensityStats:
         """dict(frames, sum, max, above (None without a threshold), mean = sum / frames (None without frames)), read back
         from the device (the caller has synchronised the streams that added frames)"""
         s = self.sum.cpu().numpy()
-        return dict(frames=self.frames, sum=s, max=self.max.cpu().numpy(),
-                    above=None if self.above is None else self.above.cpu().numpy(),
-                    mean=s / self.frames if self.frames else None)
+        r = dict(frames=self.frames, sum=s, max=self.max.cpu().numpy(),
+                 above=None if self.above is None else self.above.cpu().numpy(),
+                 mean=s / self.frames if self.frames else None)
+        if self.vel is not None:
+            # + vx_sum, vy_sum, speed_sum and the density-weighted means velocity = (vx_sum, vy_sum) / sum (Ny, Nx, 2) and
+            # speed = speed_sum / sum, NaN where sum == 0
+            vx, vy, sp = self.vx_sum.cpu().numpy(), self.vy_sum.cpu().numpy(), self.speed_sum.cpu().numpy()
+            zero = s == 0
+            with np.errstate(divide="ignore", invalid="ignore"):
+                mean = lambda a: np.where(zero, np.nan, a / np.where(zero, 1.0, s))
+                r.update(vx_sum=vx, vy_sum=vy, speed_sum=sp, velocity=np.stack([mean(vx), mean(vy)], axis=-1),
+                         speed=mean(sp))
+        return r
 
     @staticmethod
-    def nbytes(Ny, Nx, threshold=None):
+    def nbytes(Ny, Nx, threshold=None, velocity=False):
         """device bytes of the accumulators of an (Ny, Nx) grid"""
-        return Ny * Nx * (16 + (4 if threshold is not None else 0))
+        return Ny * Nx * (16 + (4 if threshold is not None else 0) + (24 if velocity else 0))
+
+
+class LineCounts:
+    """Device accumulator of pedestrian counts through measurement lines (oc_lines_acc): per step and line the crossings
+    to the left and to the right (int32 (capacity, n_lines, 2), zero at creation), and per agent the previous position
+    and whether it was inside (initialised from `state`, the crowd before its first step).  names: the lines' names;
+    lines: (n_lines, 4) array of (x0, y0, x1, y1) in metres; capacity: rows (steps) allocated, grown by ensure()."""
+
+    def __init__(self, ctx, names, lines, state, capacity):
+        import torch
+        self.names = list(names)
+        self.lines = np.ascontiguousarray(lines, dtype=np.float64).reshape(-1, 4)
+        self.px, self.py = state["x"].clone(), state["y"].clone()
+        self.inside = state["status"].clone()
+        self.device = ctx.torch_device
+        self.counts = torch.zeros((max(int(capacity), 1), len(self.lines), 2), dtype=torch.int32, device=self.device)
+        self.acc = LinesAcc(self.lines.ctypes.data_as(dp), self.counts.data_ptr(), self.px.data_ptr() or None,
+                            self.py.data_ptr() or None, self.inside.data_ptr() or None, len(self.lines),
+                            self.counts.shape[0])
+
+    def ensure(self, steps):
+        """grow the count rows (on the host: rare) so that steps 0 .. steps-1 fit"""
+        import torch
+        have = self.counts.shape[0]
+        if steps <= have:
+            return
+        torch.cuda.synchronize(self.device)   # (no update of the old rows may be in flight on any stream)
+        grown = torch.zeros((max(steps, 2 * have), len(self.lines), 2), dtype=torch.int32, device=self.device)
+        grown[:have] = self.counts
+        torch.cuda.synchronize(self.device)
+        self.counts = grown
+        self.acc.d_counts, self.acc.capacity = grown.data_ptr(), grown.shape[0]
+
+    def result(self, steps):
+        """dict(names, to_left, to_right): int32 (steps, n_lines) arrays, row k = the step with simu_step k (the caller
+        has synchronised the streams that counted)"""
+        c = self.counts[:steps].cpu().numpy()
+        return dict(names=list(self.names), to_left=np.ascontiguousarray(c[:, :, 0]),
+                    to_right=np.ascontiguousarray(c[:, :, 1]))
+
+    @staticmethod
+    def nbytes(N, n_lines, capacity):
+        """device bytes of the accumulator of N agents: previous positions and inside bytes, and the count rows"""
+        return 17 * N + 8 * n_lines * max(int(capacity), 1)
 
 
 class GcfmBatch:

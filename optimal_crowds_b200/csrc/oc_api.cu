@@ -119,6 +119,10 @@ extern "C" void oc_ctx_destroy(oc_ctx *c) {
     if (c->dens_pinned) cudaFreeHost(c->dens_pinned);
     cudaFree(c->dens_dev);
     if (c->dens_ev) cudaEventDestroy(c->dens_ev);
+    if (c->lines_ev) cudaEventSynchronize(c->lines_ev);
+    if (c->lines_pinned) cudaFreeHost(c->lines_pinned);
+    cudaFree(c->lines_dev);
+    if (c->lines_ev) cudaEventDestroy(c->lines_ev);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->gcfm_pinned) cudaFreeHost(c->gcfm_pinned);
     cudaFree(c->fr_ticket);

@@ -1285,6 +1285,9 @@ __global__ void pair_probe_kernel(oc_gcfm_params p, int N, const double *__restr
 // density_tile is the only copy of the arithmetic: tile (bx, by) of DN_TX x DN_TY nodes, every node's value handed to
 // the epilogue `epi(g, value)` (g = flat node index).  DensityStore writes the frame (oc_density); DensityAccum adds it
 // to the run's statistics (oc_density_accum*), so an accumulated frame is the stored frame bit for bit.
+// VEL (velocity maps): the kept agents' vx, vy and speed s = sqrt(vx*vx + vy*vy) are staged next to lx / ly, and with
+// the frame's weight w of an agent three more sums run, w*vx, w*vy and w*s; the density sum is the same operations in
+// the same order, and the epilogue gets `epi(g, value, vx_sum, vy_sum, speed_sum)` (all 0 on walls).
 constexpr int DN_TX = 32, DN_TY = 8, DN_CHUNK = 256;
 // ocm_exp(x) == 0 exactly for x < -745.14: r^2/two_s2 > 745.2  =>  contribution is exactly 0.0
 inline double density_r_zero(double two_s2) { return std::sqrt(745.2 * two_s2) * (1.0 + 1e-9) + 1e-9; }
@@ -1303,19 +1306,35 @@ struct DensityAccum {
         if (above && v > thr) above[g] += 1;
     }
 };
-template <class Epi>
+struct DensityVelAccum {
+    DensityAccum acc;
+    double *vx, *vy, *speed;
+    __device__ __forceinline__ void operator()(size_t g, double v, double u, double w, double s) const {
+        acc(g, v);
+        vx[g] = vx[g] + u;
+        vy[g] = vy[g] + w;
+        speed[g] = speed[g] + s;
+    }
+};
+template <bool VEL, class Epi>
 __device__ __forceinline__ void density_tile(int N, const double *__restrict__ ax, const double *__restrict__ ay,
+                                             const double *__restrict__ avx, const double *__restrict__ avy,
                                              const uint8_t *__restrict__ status, const double *__restrict__ X,
                                              const double *__restrict__ Y, const double *__restrict__ Vg, int Ny, int Nx,
                                              double two_s2, double C, double r_zero, int bx, int by, const Epi &epi) {
     __shared__ double lx[DN_CHUNK], ly[DN_CHUNK];
     __shared__ int wcnt[8];
+    double *lvx = nullptr, *lvy = nullptr, *lsp = nullptr;
+    if constexpr (VEL) {
+        __shared__ double lv[3][DN_CHUNK];
+        lvx = lv[0]; lvy = lv[1]; lsp = lv[2];
+    }
     const int ix = bx * DN_TX + (threadIdx.x & 31), iy = by * DN_TY + (threadIdx.x >> 5);
     const bool in = ix < Nx && iy < Ny;
     const double x = in ? X[ix] : 0.0, y = in ? Y[iy] : 0.0;
     const int jx0 = bx * DN_TX, jx1 = min(jx0 + DN_TX, Nx) - 1, jy0 = by * DN_TY, jy1 = min(jy0 + DN_TY, Ny) - 1;
     const double bx0 = X[jx0] - r_zero, bx1 = X[jx1] + r_zero, by0 = Y[jy0] - r_zero, by1 = Y[jy1] + r_zero;
-    double d = 0.0;
+    double d = 0.0, su = 0.0, sv = 0.0, ss = 0.0;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     for (int base = 0; base < N; base += DN_CHUNK) {
         int a = base + threadIdx.x;
@@ -1333,18 +1352,33 @@ __device__ __forceinline__ void density_tile(int N, const double *__restrict__ a
         if (keep) {
             int pos = off + __popc(m & ((1u << lane) - 1));  // preserves agent order
             lx[pos] = px; ly[pos] = py;
+            if constexpr (VEL) {
+                const double u = avx[a], v = avy[a];
+                lvx[pos] = u; lvy[pos] = v; lsp[pos] = sqrt(u * u + v * v);
+            }
         }
         __syncthreads();
         if (in)
             for (int q = 0; q < total; q++) {
                 double cx = x - lx[q], cy = y - ly[q];
-                d += ocm_exp(-(cx * cx + cy * cy) / two_s2) / C;  // :480-483
+                if constexpr (VEL) {
+                    const double w = ocm_exp(-(cx * cx + cy * cy) / two_s2) / C;
+                    d += w;
+                    su += w * lvx[q]; sv += w * lvy[q]; ss += w * lsp[q];
+                } else {
+                    d += ocm_exp(-(cx * cx + cy * cy) / two_s2) / C;  // :480-483
+                }
             }
         __syncthreads();
     }
     if (in) {
         size_t g = (size_t)iy * Nx + ix;
-        epi(g, (Vg[g] < 0) ? 0.0 : d);  // :485
+        if constexpr (VEL) {
+            const bool wall = Vg[g] < 0;
+            epi(g, wall ? 0.0 : d, wall ? 0.0 : su, wall ? 0.0 : sv, wall ? 0.0 : ss);
+        } else {
+            epi(g, (Vg[g] < 0) ? 0.0 : d);  // :485
+        }
     }
 }
 
@@ -1352,7 +1386,8 @@ __global__ void __launch_bounds__(256)
 density_kernel(int N, const double *__restrict__ ax, const double *__restrict__ ay, const uint8_t *__restrict__ status,
                const double *__restrict__ X, const double *__restrict__ Y, const double *__restrict__ Vg, int Ny,
                int Nx, double two_s2, double C, double r_zero, double *__restrict__ out) {
-    density_tile(N, ax, ay, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y, DensityStore{out});
+    density_tile<false>(N, ax, ay, nullptr, nullptr, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y,
+                        DensityStore{out});
 }
 
 __global__ void __launch_bounds__(256)
@@ -1360,19 +1395,40 @@ density_accum_kernel(int N, const double *__restrict__ ax, const double *__restr
                      const uint8_t *__restrict__ status, const double *__restrict__ X, const double *__restrict__ Y,
                      const double *__restrict__ Vg, int Ny, int Nx, double two_s2, double C, double r_zero,
                      DensityAccum acc) {
-    density_tile(N, ax, ay, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y, acc);
+    density_tile<false>(N, ax, ay, nullptr, nullptr, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y,
+                        acc);
+}
+
+__global__ void __launch_bounds__(256)
+density_accum_vel_kernel(int N, const double *__restrict__ ax, const double *__restrict__ ay,
+                         const double *__restrict__ avx, const double *__restrict__ avy,
+                         const uint8_t *__restrict__ status, const double *__restrict__ X, const double *__restrict__ Y,
+                         const double *__restrict__ Vg, int Ny, int Nx, double two_s2, double C, double r_zero,
+                         DensityVelAccum acc) {
+    density_tile<true>(N, ax, ay, avx, avy, status, X, Y, Vg, Ny, Nx, two_s2, C, r_zero, blockIdx.x, blockIdx.y, acc);
 }
 
 // Batched accumulation: one flattened 1-D grid of exactly the members' tiles.  Member m owns blocks [tile0, tile0 +
-// ntx * nty) in row-major tile order; a block finds its member by a (block-uniform) binary search over tile0.
+// ntx * nty) in row-major tile order; a block finds its member by a (block-uniform) binary search over tile0.  The
+// velocity variant reads vx / vy and the velocity accumulators (NULL in the members of the other variant).
 struct DensityMember {
-    const double *x, *y;
+    const double *x, *y, *vx, *vy;
     const uint8_t *status;
     const double *X, *Y, *Vg;
     DensityAccum acc;
+    double *vx_sum, *vy_sum, *speed_sum;
     double two_s2, C, r_zero;
     int N, Ny, Nx, ntx, tile0, pad_;
 };
+// (the velocity epilogue reads the member's accumulator pointers from the table when it runs: held in registers through
+// the agent loop they would be spilled around every ocm_exp call)
+struct DensityMemberVelAccum {
+    const DensityMember *m;
+    __device__ __forceinline__ void operator()(size_t g, double v, double u, double w, double s) const {
+        DensityVelAccum{m->acc, m->vx_sum, m->vy_sum, m->speed_sum}(g, v, u, w, s);
+    }
+};
+template <bool VEL>
 __global__ void __launch_bounds__(256)
 density_accum_multi_kernel(const DensityMember *__restrict__ ms, int n) {
     const int b = blockIdx.x;
@@ -1384,8 +1440,12 @@ density_accum_multi_kernel(const DensityMember *__restrict__ ms, int n) {
     }
     const DensityMember &m = ms[lo];
     const int t = b - m.tile0;
-    density_tile(m.N, m.x, m.y, m.status, m.X, m.Y, m.Vg, m.Ny, m.Nx, m.two_s2, m.C, m.r_zero, t % m.ntx, t / m.ntx,
-                 m.acc);
+    if constexpr (VEL)
+        density_tile<true>(m.N, m.x, m.y, m.vx, m.vy, m.status, m.X, m.Y, m.Vg, m.Ny, m.Nx, m.two_s2, m.C, m.r_zero,
+                           t % m.ntx, t / m.ntx, DensityMemberVelAccum{&m});
+    else
+        density_tile<false>(m.N, m.x, m.y, nullptr, nullptr, m.status, m.X, m.Y, m.Vg, m.Ny, m.Nx, m.two_s2, m.C,
+                            m.r_zero, t % m.ntx, t / m.ntx, m.acc);
 }
 
 int density_acc_check(const oc_density_acc *a) {
@@ -1397,8 +1457,95 @@ int density_acc_check(const oc_density_acc *a) {
     return OC_OK;
 }
 
+int velocity_acc_check(const oc_velocity_acc *v) {
+    OC_ARG(!v || (v->d_vx_sum && v->d_vy_sum && v->d_speed_sum), "NULL argument");
+    return OC_OK;
+}
+
 DensityAccum density_epilogue(const oc_density_acc *a) {
     return DensityAccum{a->d_sum, a->d_max, a->d_above, a->threshold};
+}
+
+// Pedestrian counts through measurement lines (lines_count_kernel, lines_count_multi_kernel): one thread per agent.  An
+// agent inside at the start of the step (its "inside" byte) moved from its kept previous position p to its position q
+// after the step.  With o(u, v, w) = (v.x-u.x)*(w.y-u.y) - (v.y-u.y)*(w.x-u.x) (FP64, no contraction: this unit is built
+// with -fmad=false) and the line's endpoints a, b it crosses when (o(a,b,p) > 0) != (o(a,b,q) > 0) and
+// (o(p,q,a) > 0) != (o(p,q,b) > 0); to the left when o(a,b,q) > 0, else to the right.  Points on the line are on the
+// right; NaN compares false, so a NaN position never crosses.  Then p = q and inside = status.
+constexpr int LN_MAX = 64;
+struct LineSet {
+    double c[LN_MAX][4];
+};
+__device__ __forceinline__ double line_orient(double ux, double uy, double vx, double vy, double wx, double wy) {
+    return (vx - ux) * (wy - uy) - (vy - uy) * (wx - ux);
+}
+__device__ __forceinline__ void lines_agent(int i, const double *__restrict__ x, const double *__restrict__ y,
+                                            const uint8_t *__restrict__ status, double *__restrict__ px,
+                                            double *__restrict__ py, uint8_t *__restrict__ inside,
+                                            const double (*L)[4], int nl, int *__restrict__ counts) {
+    const double qx = x[i], qy = y[i];
+    if (inside[i]) {
+        const double ox = px[i], oy = py[i];
+        for (int l = 0; l < nl; l++) {
+            const double ax_ = L[l][0], ay_ = L[l][1], bx_ = L[l][2], by_ = L[l][3];
+            const bool sp = line_orient(ax_, ay_, bx_, by_, ox, oy) > 0, sq = line_orient(ax_, ay_, bx_, by_, qx, qy) > 0;
+            if (sp != sq && (line_orient(ox, oy, qx, qy, ax_, ay_) > 0) != (line_orient(ox, oy, qx, qy, bx_, by_) > 0))
+                atomicAdd(&counts[2 * l + (sq ? 0 : 1)], 1);
+        }
+    }
+    px[i] = qx; py[i] = qy;
+    inside[i] = status[i];
+}
+
+__global__ void __launch_bounds__(256)
+lines_count_kernel(int N, const double *__restrict__ x, const double *__restrict__ y, const uint8_t *__restrict__ status,
+                   double *__restrict__ px, double *__restrict__ py, uint8_t *__restrict__ inside, LineSet ls, int nl,
+                   int *__restrict__ counts) {
+    __shared__ double L[LN_MAX][4];
+    for (int t = threadIdx.x; t < 4 * nl; t += blockDim.x) L[t >> 2][t & 3] = ls.c[t >> 2][t & 3];
+    __syncthreads();
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < N) lines_agent(i, x, y, status, px, py, inside, L, nl, counts);
+}
+
+// Batched counts: member m owns blocks [blk0, blk0 + ceil(N / 256)); its lines follow the member table in the same
+// device buffer; `counts` points at the row of the member's step.
+struct LinesMember {
+    const double *x, *y;
+    const uint8_t *status;
+    double *px, *py;
+    uint8_t *inside;
+    const double *lines;
+    int *counts;
+    int N, nl, blk0, pad_;
+};
+__global__ void __launch_bounds__(256) lines_count_multi_kernel(const LinesMember *__restrict__ ms, int n) {
+    __shared__ double L[LN_MAX][4];
+    const int b = blockIdx.x;
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ms[mid].blk0 <= b) lo = mid;
+        else hi = mid - 1;
+    }
+    const LinesMember &m = ms[lo];
+    for (int t = threadIdx.x; t < 4 * m.nl; t += blockDim.x) L[t >> 2][t & 3] = m.lines[t];
+    __syncthreads();
+    const int i = (b - m.blk0) * blockDim.x + threadIdx.x;
+    if (i < m.N) lines_agent(i, m.x, m.y, m.status, m.px, m.py, m.inside, L, m.nl, m.counts);
+}
+
+int lines_acc_check(const oc_lines_acc *a) {
+    OC_ARG(a && a->lines && a->d_counts, "NULL argument");
+    OC_ARG(a->n_lines >= 1 && a->n_lines <= LN_MAX, "measurement lines: n_lines must be in 1..64");
+    OC_ARG(a->capacity >= 0, "measurement lines: negative capacity");
+    for (int l = 0; l < a->n_lines; l++) {
+        const double *c = a->lines + 4 * l;
+        OC_ARG(std::isfinite(c[0]) && std::isfinite(c[1]) && std::isfinite(c[2]) && std::isfinite(c[3]),
+               "measurement lines: coordinates must be finite");
+        OC_ARG(c[0] != c[2] || c[1] != c[3], "measurement lines: a line must have non-zero length");
+    }
+    return OC_OK;
 }
 
 template <class T>
@@ -2148,18 +2295,29 @@ extern "C" int oc_gcfm_step_multi_finish(int n, oc_ctx *const *ctxs, int *const 
 // (on OC_ERR_SAMPLER_RANGE including the offending one, as oc_gcfm_step).  exit_agent / exit_step (capacity N): agents in
 // exit order and the index (0-based within this call) of the step they left in.  *device_ms: sum of the steps' CUDA-event
 // times; *pairs: interacting pairs evaluated.  acc (nullable): density statistics, one frame added before every step
-// whose simu_step is a multiple of acc->every (the history frame of that iteration), ahead of the step's randomness.
-extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
-                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
-                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
-                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
-                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
-                               long long *pairs, const oc_density_acc *acc, void *stream) {
+// whose simu_step is a multiple of acc->every (the history frame of that iteration), ahead of the step's randomness;
+// vel (nullable, needs acc): that frame's velocity maps too.  lines (nullable): after every step, once the step is final
+// (oc_gcfm_step_finish), its crossings of the measurement lines are counted in row simu_step of lines->d_counts.
+extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                                double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                                const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                                double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                                int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                                long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
+                                const oc_lines_acc *lines, void *stream) {
     OC_ARG(ctx && prm && mt_key && mt_pos && has_gauss && cached_gauss && exit_agent && exit_step && n_exits && steps_done,
            "NULL argument");
     OC_ARG(N >= 1 && n_steps >= 0 && n_active0 >= 0 && n_active0 <= N && *mt_pos >= 0 && *mt_pos <= 624, "bad sizes");
     if (acc)
         if (int rc = density_acc_check(acc)) return rc;
+    OC_ARG(!vel || acc, "velocity maps without density statistics");
+    if (int rc = velocity_acc_check(vel)) return rc;
+    if (lines) {
+        if (int rc = lines_acc_check(lines)) return rc;
+        OC_ARG(lines->d_px && lines->d_py && lines->d_inside, "NULL argument");
+        OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= lines->capacity,
+               "measurement lines: step beyond the count capacity");
+    }
     constexpr int N_CKPT = 64;
     *n_exits = 0;
     *steps_done = 0;
@@ -2177,7 +2335,7 @@ extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
     for (int k = 0; k < n_steps && n_active > 0; k++) {
         // ---- this iteration's history frame (simulations.py:428), folded into the statistics
         if (acc && (simu_step0 + k) % acc->every == 0) {
-            rc = oc_density_accum(ctx, acc, N, d_x, d_y, d_status, stream);
+            rc = oc_density_accum_vel(ctx, acc, vel, N, d_x, d_y, d_vx, d_vy, d_status, stream);
             if (rc) return rc;
         }
         // ---- this step's randomness (simulations.py:271,303)
@@ -2216,6 +2374,10 @@ extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
             (*n_exits)++;
         }
         n_active -= ne;
+        if (lines) {
+            int r2 = oc_lines_count(ctx, lines, N, d_x, d_y, d_status, simu_step0 + k, stream);
+            if (r2) return r2;
+        }
         if (device_ms) *device_ms += ctx->gcfm_last_ms;
         if (pairs) *pairs += ctx->gcfm_last_pairs;
         if (d_rows && d_rows[k]) {
@@ -2228,15 +2390,26 @@ extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
     return OC_OK;
 }
 
+extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                               long long *pairs, const oc_density_acc *acc, void *stream) {
+    return oc_gcfm_run_flow(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key,
+                            mt_pos, has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent, exit_step,
+                            n_exits, steps_done, device_ms, pairs, acc, nullptr, nullptr, stream);
+}
+
 extern "C" int oc_gcfm_run(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
                            double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
                            const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
                            double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
                            int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
                            long long *pairs, void *stream) {
-    return oc_gcfm_run_acc(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key, mt_pos,
-                           has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent, exit_step, n_exits,
-                           steps_done, device_ms, pairs, nullptr, stream);
+    return oc_gcfm_run_flow(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key,
+                            mt_pos, has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent, exit_step,
+                            n_exits, steps_done, device_ms, pairs, nullptr, nullptr, nullptr, stream);
 }
 
 extern "C" double oc_gcfm_last_ms(oc_ctx *ctx) { return ctx ? ctx->gcfm_last_ms : 0.0; }
@@ -2293,30 +2466,51 @@ extern "C" int oc_density(oc_ctx *ctx, int N, const double *d_x, const double *d
 }
 
 // ------------------------------------------------------------------------------------------------ density statistics
-extern "C" int oc_density_accum(oc_ctx *ctx, const oc_density_acc *acc, int N, const double *d_x, const double *d_y,
-                                const uint8_t *d_status, void *stream) {
-    OC_ARG(ctx && N >= 0 && (N == 0 || (d_x && d_y && d_status)), "NULL argument");
+extern "C" int oc_density_accum_vel(oc_ctx *ctx, const oc_density_acc *acc, const oc_velocity_acc *vel, int N,
+                                    const double *d_x, const double *d_y, const double *d_vx, const double *d_vy,
+                                    const uint8_t *d_status, void *stream) {
+    OC_ARG(ctx && N >= 0 && (N == 0 || (d_x && d_y && d_status && (!vel || (d_vx && d_vy)))), "NULL argument");
     if (int rc = density_acc_check(acc)) return rc;
+    if (int rc = velocity_acc_check(vel)) return rc;
     OC_CUDA(cudaSetDevice(ctx->device));
     const double two_s2 = 2 * (acc->sigma * acc->sigma);
     dim3 grid((ctx->Nx + DN_TX - 1) / DN_TX, (ctx->Ny + DN_TY - 1) / DN_TY);
-    density_accum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(N, d_x, d_y, d_status, ctx->d_X, ctx->d_Y,
-                                                                 acc->d_Vglobal, ctx->Ny, ctx->Nx, two_s2, acc->C,
-                                                                 density_r_zero(two_s2), density_epilogue(acc));
+    if (vel)
+        density_accum_vel_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+            N, d_x, d_y, d_vx, d_vy, d_status, ctx->d_X, ctx->d_Y, acc->d_Vglobal, ctx->Ny, ctx->Nx, two_s2, acc->C,
+            density_r_zero(two_s2), DensityVelAccum{density_epilogue(acc), vel->d_vx_sum, vel->d_vy_sum, vel->d_speed_sum});
+    else
+        density_accum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(N, d_x, d_y, d_status, ctx->d_X, ctx->d_Y,
+                                                                     acc->d_Vglobal, ctx->Ny, ctx->Nx, two_s2, acc->C,
+                                                                     density_r_zero(two_s2), density_epilogue(acc));
     oc::count_launch();
     OC_CUDA(cudaGetLastError());
     return OC_OK;
 }
 
-extern "C" int oc_density_accum_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs, const int *Ns,
-                                      const double *const *x, const double *const *y, const uint8_t *const *status,
-                                      void *stream) {
+extern "C" int oc_density_accum(oc_ctx *ctx, const oc_density_acc *acc, int N, const double *d_x, const double *d_y,
+                                const uint8_t *d_status, void *stream) {
+    return oc_density_accum_vel(ctx, acc, nullptr, N, d_x, d_y, nullptr, nullptr, d_status, stream);
+}
+
+// The members with velocity maps and those without run as two launches (one per kernel variant), each over the flattened
+// tiles of its own members: a plain member then costs what it cost alone, not the velocity variant's registers and
+// shared memory.  Both launches read one member table (velocity members first), copied to the device once per call.
+extern "C" int oc_density_accum_vel_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs,
+                                          const oc_velocity_acc *const *vels, const int *Ns, const double *const *x,
+                                          const double *const *y, const double *const *vx, const double *const *vy,
+                                          const uint8_t *const *status, void *stream) {
     OC_ARG(n >= 1 && ctxs && accs && Ns && x && y && status && ctxs[0], "NULL argument");
     oc_ctx *c0 = ctxs[0];
+    int nv = 0;
     for (int m = 0; m < n; m++) {
+        const oc_velocity_acc *v = vels ? vels[m] : nullptr;
         OC_ARG(ctxs[m] && Ns[m] >= 0 && (Ns[m] == 0 || (x[m] && y[m] && status[m])), "NULL argument");
+        OC_ARG(!v || Ns[m] == 0 || (vx && vy && vx[m] && vy[m]), "NULL argument");
         OC_ARG(ctxs[m]->device == c0->device, "density statistics: member context on another device");
         if (int rc = density_acc_check(accs[m])) return rc;
+        if (int rc = velocity_acc_check(v)) return rc;
+        nv += v != nullptr;
     }
     OC_CUDA(cudaSetDevice(c0->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -2327,21 +2521,105 @@ extern "C" int oc_density_accum_multi(int n, oc_ctx *const *ctxs, const oc_densi
     if (int rc = oc_ensure_buffer(c0->dens_pinned, c0->dens_pinned_bytes, bytes, true, "density member table")) return rc;
     if (int rc = oc_ensure_buffer(c0->dens_dev, c0->dens_dev_bytes, bytes, false, "density member table")) return rc;
     DensityMember *recs = static_cast<DensityMember *>(c0->dens_pinned);
-    long long tiles = 0;
+    long long tiles[2] = {0, 0};   // [velocity members, plain members]
+    int slot[2] = {0, nv};
     for (int m = 0; m < n; m++) {
         const oc_ctx *c = ctxs[m];
         const oc_density_acc *a = accs[m];
+        const oc_velocity_acc *v = vels ? vels[m] : nullptr;
+        const int k = v ? 0 : 1;
         const int ntx = (c->Nx + DN_TX - 1) / DN_TX, nty = (c->Ny + DN_TY - 1) / DN_TY;
         const double two_s2 = 2 * (a->sigma * a->sigma);
-        recs[m] = DensityMember{x[m], y[m], status[m], c->d_X, c->d_Y, a->d_Vglobal, density_epilogue(a), two_s2, a->C,
-                                density_r_zero(two_s2), Ns[m], c->Ny, c->Nx, ntx, (int)tiles, 0};
-        tiles += (long long)ntx * nty;
+        recs[slot[k]++] = DensityMember{x[m], y[m], v ? vx[m] : nullptr, v ? vy[m] : nullptr, status[m], c->d_X, c->d_Y,
+                                        a->d_Vglobal, density_epilogue(a), v ? v->d_vx_sum : nullptr,
+                                        v ? v->d_vy_sum : nullptr, v ? v->d_speed_sum : nullptr, two_s2, a->C,
+                                        density_r_zero(two_s2), Ns[m], c->Ny, c->Nx, ntx, (int)tiles[k], 0};
+        tiles[k] += (long long)ntx * nty;
     }
-    OC_ARG(tiles < 0x7fffffff, "density statistics: too many tiles for one launch");
+    OC_ARG(tiles[0] < 0x7fffffff && tiles[1] < 0x7fffffff, "density statistics: too many tiles for one launch");
     OC_CUDA(cudaMemcpyAsync(c0->dens_dev, recs, bytes, cudaMemcpyHostToDevice, st));
-    density_accum_multi_kernel<<<(unsigned)tiles, 256, 0, st>>>(static_cast<const DensityMember *>(c0->dens_dev), n);
-    oc::count_launch();
+    const DensityMember *dev = static_cast<const DensityMember *>(c0->dens_dev);
+    if (nv) {
+        density_accum_multi_kernel<true><<<(unsigned)tiles[0], 256, 0, st>>>(dev, nv);
+        oc::count_launch();
+    }
+    if (nv < n) {
+        density_accum_multi_kernel<false><<<(unsigned)tiles[1], 256, 0, st>>>(dev + nv, n - nv);
+        oc::count_launch();
+    }
     OC_CUDA(cudaGetLastError());
     OC_CUDA(cudaEventRecord(c0->dens_ev, st));
+    return OC_OK;
+}
+
+extern "C" int oc_density_accum_multi(int n, oc_ctx *const *ctxs, const oc_density_acc *const *accs, const int *Ns,
+                                      const double *const *x, const double *const *y, const uint8_t *const *status,
+                                      void *stream) {
+    return oc_density_accum_vel_multi(n, ctxs, accs, nullptr, Ns, x, y, nullptr, nullptr, status, stream);
+}
+
+// ------------------------------------------------------------------------------------------------ measurement lines
+extern "C" int oc_lines_count(oc_ctx *ctx, const oc_lines_acc *acc, int N, const double *d_x, const double *d_y,
+                              const uint8_t *d_status, int step, void *stream) {
+    OC_ARG(ctx && N >= 0, "NULL argument");
+    if (int rc = lines_acc_check(acc)) return rc;
+    OC_ARG(N == 0 || (d_x && d_y && d_status && acc->d_px && acc->d_py && acc->d_inside), "NULL argument");
+    OC_ARG(step >= 0 && step < acc->capacity, "measurement lines: step beyond the count capacity");
+    if (N == 0) return OC_OK;
+    OC_CUDA(cudaSetDevice(ctx->device));
+    LineSet ls;
+    memcpy(ls.c, acc->lines, sizeof(double) * 4 * acc->n_lines);
+    lines_count_kernel<<<(N + 255) / 256, 256, 0, (cudaStream_t)stream>>>(
+        N, d_x, d_y, d_status, acc->d_px, acc->d_py, acc->d_inside, ls, acc->n_lines,
+        acc->d_counts + (size_t)step * acc->n_lines * 2);
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    return OC_OK;
+}
+
+extern "C" int oc_lines_count_multi(int n, oc_ctx *const *ctxs, const oc_lines_acc *const *accs, const int *Ns,
+                                    const double *const *x, const double *const *y, const uint8_t *const *status,
+                                    const int *steps, void *stream) {
+    OC_ARG(n >= 1 && ctxs && accs && Ns && x && y && status && steps && ctxs[0], "NULL argument");
+    oc_ctx *c0 = ctxs[0];
+    size_t n_line_vals = 0;
+    for (int m = 0; m < n; m++) {
+        OC_ARG(ctxs[m] && Ns[m] >= 0, "NULL argument");
+        OC_ARG(ctxs[m]->device == c0->device, "measurement lines: member context on another device");
+        if (int rc = lines_acc_check(accs[m])) return rc;
+        const oc_lines_acc *a = accs[m];
+        OC_ARG(Ns[m] == 0 || (x[m] && y[m] && status[m] && a->d_px && a->d_py && a->d_inside), "NULL argument");
+        OC_ARG(steps[m] >= 0 && steps[m] < a->capacity, "measurement lines: step beyond the count capacity");
+        n_line_vals += 4 * (size_t)a->n_lines;
+    }
+    OC_CUDA(cudaSetDevice(c0->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t rec_bytes = ((sizeof(LinesMember) * (size_t)n + 15) / 16) * 16;
+    const size_t bytes = rec_bytes + sizeof(double) * n_line_vals;
+    // the table (staging and device copy) is reused once the previous call's kernel has read it, whatever its stream
+    if (!c0->lines_ev) OC_CUDA(cudaEventCreateWithFlags(&c0->lines_ev, cudaEventDisableTiming));
+    OC_CUDA(cudaEventSynchronize(c0->lines_ev));
+    if (int rc = oc_ensure_buffer(c0->lines_pinned, c0->lines_pinned_bytes, bytes, true, "line member table")) return rc;
+    if (int rc = oc_ensure_buffer(c0->lines_dev, c0->lines_dev_bytes, bytes, false, "line member table")) return rc;
+    LinesMember *recs = static_cast<LinesMember *>(c0->lines_pinned);
+    double *hl = reinterpret_cast<double *>(static_cast<char *>(c0->lines_pinned) + rec_bytes);
+    const double *dl = reinterpret_cast<const double *>(static_cast<char *>(c0->lines_dev) + rec_bytes);
+    long long blocks = 0;
+    size_t off = 0;
+    for (int m = 0; m < n; m++) {
+        const oc_lines_acc *a = accs[m];
+        memcpy(hl + off, a->lines, sizeof(double) * 4 * a->n_lines);
+        recs[m] = LinesMember{x[m], y[m], status[m], a->d_px, a->d_py, a->d_inside, dl + off,
+                              a->d_counts + (size_t)steps[m] * a->n_lines * 2, Ns[m], a->n_lines, (int)blocks, 0};
+        off += 4 * (size_t)a->n_lines;
+        blocks += (Ns[m] + 255) / 256;
+    }
+    OC_ARG(blocks < 0x7fffffff, "measurement lines: too many agents for one launch");
+    if (blocks == 0) return OC_OK;
+    OC_CUDA(cudaMemcpyAsync(c0->lines_dev, recs, bytes, cudaMemcpyHostToDevice, st));
+    lines_count_multi_kernel<<<(unsigned)blocks, 256, 0, st>>>(static_cast<const LinesMember *>(c0->lines_dev), n);
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    OC_CUDA(cudaEventRecord(c0->lines_ev, st));
     return OC_OK;
 }

@@ -23,7 +23,11 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     Every member still equals its stand-alone run bit for bit (tests/test_gpu_ensemble_shapes.py);
   * ``density_stats``: every member accumulates the sum, maximum and above-threshold count of its density frames on the
     device (one batched ``oc_density_accum_multi`` launch per step for the due members of a wave) and hands them back
-    in ``results[i]["density"]`` -- no frames, trajectories or members are kept (tests/test_gpu_density_stats.py).
+    in ``results[i]["density"]`` -- no frames, trajectories or members are kept (tests/test_gpu_density_stats.py);
+    with ``velocity=True`` also the frames' density-weighted velocity and speed maps;
+  * ``lines``: every member counts, per step, the agents crossing each measurement line in each direction on the device
+    (one batched ``oc_lines_count_multi`` launch per step for a wave) and hands them back in ``results[i]["lines"]``
+    (tests/test_gpu_flow_stats.py).
 """
 from __future__ import annotations
 
@@ -104,9 +108,12 @@ class ensemble:
     ``times`` (per-agent clocks, as evac_times() returns them), ``final`` (N,4: x, y, vx, vy) and ``hjb`` (solver
     statistics per target set) and ``config`` (the member's effective configuration).
 
-    ``density_stats``: None, True or dict(every=1, threshold=None) for every member, as ``simulation(...,
+    ``density_stats``: None, True or dict(every=1, threshold=None, velocity=False) for every member, as ``simulation(...,
     density_stats=...)`` takes it (each member with its own ``sigma_convolution``); ``results[i]["density"]`` is then the
     member's ``density_stats()`` dict.
+
+    ``lines``: None or {name: (x0, y0, x1, y1)} in metres (at most 64), the same measurement lines for every member, as
+    ``simulation(..., lines=...)`` takes them; ``results[i]["lines"]`` is then the member's ``line_counts()`` dict.
 
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
     ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
@@ -119,7 +126,7 @@ class ensemble:
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
                  memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None,
-                 density_stats=None):
+                 density_stats=None, lines=None):
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -141,7 +148,9 @@ class ensemble:
         self.configs = [optimals._merge_config(base, o) if o is not None else base for o in self.overrides]
         if len({c["grid_step"] for c in self.configs}) > 1:
             raise ValueError("ensemble members must share grid_step (one grid for the batched solves)")
-        self.density_stats = simulations.density_stats_spec(density_stats)   # (every, threshold) or None
+        self.density_stats = simulations.density_stats_spec(density_stats, with_velocity=True)  # (every, thr, vel) / None
+        self.lines = simulations.lines_spec(lines)                            # (names, (n, 4) array) or None
+        self._lines_arg = None if self.lines is None else dict(zip(self.lines[0], map(tuple, self.lines[1])))
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -169,7 +178,7 @@ class ensemble:
 
     def member_bytes(self, members=None):
         """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets, plus the
-        density accumulators when density_stats is on); no CUDA"""
+        density accumulators when density_stats is on and the line accumulator with lines); no CUDA"""
         out = []
         for i in (self.mine if members is None else members):
             room, cfg = self._room(i), self.configs[i]
@@ -177,7 +186,10 @@ class ensemble:
             n_keys = len({' or '.join(b[5:]) for b in room["initial_boxes"].values()})
             b = field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage)
             if self.density_stats is not None:
-                b += _lib.DensityStats.nbytes(Ny, Nx, self.density_stats[1])
+                b += _lib.DensityStats.nbytes(Ny, Nx, self.density_stats[1], self.density_stats[2])
+            if self.lines is not None:
+                N = sum(int(box[4] * box[2] * box[3]) for box in room["initial_boxes"].values())   # simulations.py:122
+                b += _lib.LineCounts.nbytes(N, len(self.lines[0]), len(simulations.density_frame_steps(self.T, cfg["dt"], 1)))
             out.append(b)
         return out
 
@@ -194,7 +206,8 @@ class ensemble:
                                       rng=np.random.RandomState(self.seeds[idx]), chunk_rows=self.chunk_rows,
                                       config=self.overrides[idx], _ctx=ctx,
                                       density_stats=None if self.density_stats is None else
-                                      dict(every=self.density_stats[0], threshold=self.density_stats[1]))
+                                      dict(every=self.density_stats[0], threshold=self.density_stats[1],
+                                           velocity=self.density_stats[2]), lines=self._lines_arg)
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -343,7 +356,16 @@ class ensemble:
                 batch.launch(live, [sims[q].inside for q in live], [sims[q].simu_step for q in live], stream=main,
                              rebind=rebind)
                 tl1 = time.perf_counter()
-                for q, (exits, rc) in zip(live, batch.finish()):
+                finished = batch.finish()
+                if self.lines is not None:
+                    # the crossings of this step (final once finish() returns), one launch for the wave
+                    lc = [q for q in live if sims[q].N > 0]
+                    for q in lc:
+                        sims[q]._lines.ensure(sims[q].simu_step + 1)
+                    if lc:
+                        _lib.lines_count_multi([sims[q]._ctx for q in lc], [sims[q]._lines for q in lc],
+                                               [sims[q]._state for q in lc], [sims[q].simu_step for q in lc], stream=main)
+                for q, (exits, rc) in zip(live, finished):
                     sims[q]._step_finish((sims[q].dt, ("batched", exits, rc)))
             else:
                 launched = []
@@ -373,6 +395,8 @@ class ensemble:
                                    chunk_rows=self.member_chunk_rows[i])
             if self.density_stats is not None:
                 self.results[i]["density"] = s._dstats.result()
+            if self.lines is not None:
+                self.results[i]["lines"] = s._lines.result(s.simu_step)
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3

@@ -26,26 +26,58 @@ from .optimals import _load_config, _load_room, _merge_config
 warnings.filterwarnings("ignore")  # simulations.py:15
 
 
-def density_stats_spec(value):
-    """(every, threshold) of a ``density_stats`` argument, or None when the statistics are off: None / False (off), True
-    (every frame, no threshold) or dict(every=1, threshold=None); checked without touching a GPU"""
+def density_stats_spec(value, with_velocity=False):
+    """(every, threshold) of a ``density_stats`` argument -- (every, threshold, velocity) with ``with_velocity`` -- or None
+    when the statistics are off: None / False (off), True (every frame, no threshold, no velocity maps) or
+    dict(every=1, threshold=None, velocity=False); checked without touching a GPU"""
     if value is None or value is False:
         return None
     if value is True:
-        return 1, None
+        return (1, None, False) if with_velocity else (1, None)
     if not isinstance(value, dict):
-        raise ValueError("density_stats: expected None, True or dict(every=..., threshold=...)")
-    unknown = set(value) - {"every", "threshold"}
+        raise ValueError("density_stats: expected None, True or dict(every=..., threshold=..., velocity=...)")
+    unknown = set(value) - {"every", "threshold", "velocity"}
     if unknown:
         raise ValueError(f"density_stats: unknown keys {sorted(unknown)}")
-    every, thr = value.get("every", 1), value.get("threshold")
+    every, thr, vel = value.get("every", 1), value.get("threshold"), value.get("velocity", False)
     if isinstance(every, bool) or not isinstance(every, (int, np.integer)) or every < 1:
         raise ValueError("density_stats: every must be an integer >= 1")
     if thr is not None:
         if isinstance(thr, bool) or not isinstance(thr, (int, float, np.integer, np.floating)) or not np.isfinite(thr):
             raise ValueError("density_stats: threshold must be None or a finite number")
         thr = float(thr)
-    return int(every), thr
+    if not isinstance(vel, (bool, np.bool_)):
+        raise ValueError("density_stats: velocity must be True or False")
+    return (int(every), thr, bool(vel)) if with_velocity else (int(every), thr)
+
+
+MAX_LINES = 64
+
+
+def lines_spec(value):
+    """(names, (n, 4) float64 array) of a ``lines`` argument -- {name: (x0, y0, x1, y1)} in metres, 1 to 64 lines, finite
+    coordinates, non-zero length -- or None for None; checked without touching a GPU"""
+    if value is None:
+        return None
+    if not isinstance(value, dict) or not value:
+        raise ValueError("lines: expected a non-empty dict {name: (x0, y0, x1, y1)}")
+    if len(value) > MAX_LINES:
+        raise ValueError(f"lines: at most {MAX_LINES} measurement lines")
+    names, rows = [], []
+    for name, seg in value.items():
+        try:
+            c = np.asarray(seg, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise ValueError(f"lines: {name!r} is not (x0, y0, x1, y1)") from None
+        if c.shape != (4,) or isinstance(seg, (str, bytes)) or any(isinstance(v, (bool, np.bool_)) for v in seg):
+            raise ValueError(f"lines: {name!r} is not (x0, y0, x1, y1)")
+        if not np.isfinite(c).all():
+            raise ValueError(f"lines: the coordinates of {name!r} must be finite")
+        if c[0] == c[2] and c[1] == c[3]:
+            raise ValueError(f"lines: {name!r} has zero length")
+        names.append(name)
+        rows.append(c)
+    return names, np.array(rows, dtype=np.float64)
 
 
 def density_frame_steps(T, dt, every, recompute_step=None):
@@ -170,7 +202,8 @@ class simulation:
     TRACK_CHUNK = 64  # steps per block of the device-resident trajectory record
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
-                 rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, _ctx=None):
+                 rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, lines=None,
+                 _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -188,11 +221,18 @@ class simulation:
         or dict(every=1, threshold=None): accumulate on the device, per grid node, the sum and the maximum of the density
         frames the reference stores in ``history`` (simulations.py:579-589) at the steps of run()'s loop whose simu_step
         is a multiple of ``every``, and with a threshold the number of frames above it; read them with
-        ``density_stats()``.  Not available with ``band`` or ``shard_keys``)."""
+        ``density_stats()``; with ``velocity=True`` also the density-weighted sums of the agents' vx, vy and speed, and
+        their means ``velocity`` and ``speed``.  Not available with ``band`` or ``shard_keys``), ``lines`` ({name: (x0, y0,
+        x1, y1)} in metres, at most 64: count on the device, per step, the agents crossing each line to its left and to
+        its right; read them with ``line_counts()``.  Not available with ``band`` or ``shard_keys``)."""
         import torch
-        dstats = density_stats_spec(density_stats)
+        dstats = density_stats_spec(density_stats, with_velocity=True)
+        lspec = lines_spec(lines)
         if dstats is not None and (band or shard_keys):
             raise ValueError("density_stats is not available for row-decomposed (band=True) or key-sharded "
+                             "(shard_keys=True) runs")
+        if lspec is not None and (band or shard_keys):
+            raise ValueError("lines are not available for row-decomposed (band=True) or key-sharded "
                              "(shard_keys=True) runs")
         self._np_random = rng if rng is not None else np.random
         self.recompute = recompute
@@ -323,6 +363,10 @@ class simulation:
         self._d_Vglobal = ctx.to_device(self.V)
         # density statistics of the run's frames (device accumulators, written by oc_density_accum / oc_gcfm_run_acc)
         self._dstats = None if dstats is None else _lib.DensityStats(ctx, self._d_Vglobal, self.sigma_convolution, *dstats)
+        # counts through measurement lines (written after every step by oc_lines_count* / oc_gcfm_run_flow), one row per
+        # step of a run that lasts until T, grown on the host when the steps go past that
+        self._lines = None if lspec is None else _lib.LineCounts(ctx, *lspec, self._state,
+                                                                 len(density_frame_steps(T, self.dt, 1)))
         # per-step record of (x, y, vx, vy); row k = state after k steps (ped.traj / ped.vels / history views).  It
         # lives on the DEVICE in blocks of TRACK_CHUNK steps, written by one small kernel per step (oc_state_pack), and
         # is read back -- once per row -- only when somebody looks at it
@@ -490,8 +534,11 @@ class simulation:
                                                  device=self._ctx.torch_device))
             rows.append(self._d_track[blk][off])
         n_active = int(self._h_status.sum())
+        if self._lines is not None:
+            self._lines.ensure(self.simu_step + n_steps)
         res = self._ctx.gcfm_run(self._gcfm_prm, self._state, self._d_vdes, self._d_key, self._keys(), st, n_steps,
-                                 self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats)
+                                 self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats,
+                                 lines=self._lines)
         self._rng.rng.set_state(res["rng_state"])
         self.last_run_stats = dict(steps=res["steps"], device_ms=res["device_ms"], pairs=res["pairs"])
         ex, exs = res["exits"], res["exit_step"]
@@ -518,7 +565,8 @@ class simulation:
         """add this iteration's frame to the density statistics when they are on and it is due (before the step)"""
         if self._dstats is not None and self._dstats.due(self.simu_step):
             st = self._state
-            self._ctx.density_accum(self._dstats, st["x"], st["y"], st["status"], stream=self._cuda_stream)
+            self._ctx.density_accum(self._dstats, st["x"], st["y"], st["status"], stream=self._cuda_stream, vx=st["vx"],
+                                    vy=st["vy"])
 
     def density_stats(self):
         """the density statistics of the frames taken so far (``density_stats=`` of the constructor): dict(frames, sum,
@@ -531,11 +579,30 @@ class simulation:
             torch.cuda.synchronize(self._ctx.torch_device)
         return self._dstats.result()
 
+    def _count_lines(self):
+        """count this step's crossings of the measurement lines (after the step is final, before simu_step advances)"""
+        if self._lines is not None:
+            self._lines.ensure(self.simu_step + 1)
+            self._ctx.lines_count(self._lines, self._state, self.simu_step, stream=self._cuda_stream)
+
+    def line_counts(self):
+        """the crossings of the measurement lines (``lines=`` of the constructor) by the steps taken so far:
+        dict(names, to_left, to_right) -- int32 (simu_step, n_lines) arrays, row k = the step with simu_step k"""
+        if self._lines is None:
+            raise RuntimeError("this simulation was created without lines")
+        import torch
+        torch.cuda.synchronize(self._ctx.torch_device)
+        return self._lines.result(self.simu_step)
+
     def _step_finish(self, launched, verbose=False):
         dt, pending = launched
         if pending is not None:
             # ("batched", exits, rc): the step ran inside a batched launch of an ensemble wave and has finished already
-            exits, rc = pending[1:] if pending[0] == "batched" else self._ctx.gcfm_step_finish(pending)
+            if pending[0] == "batched":
+                exits, rc = pending[1:]
+            else:
+                exits, rc = self._ctx.gcfm_step_finish(pending)
+                self._count_lines()
             if rc == _lib.OC_ERR_SAMPLER_RANGE:
                 raise IndexError("agent position outside the velocity field's index range "
                                  "(numpy raises IndexError in the reference's sampler too: optimals.py:247)")
