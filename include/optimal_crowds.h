@@ -477,15 +477,60 @@ int oc_lines_count(oc_ctx *ctx, const oc_lines_acc *acc, int N, const double *d_
 int oc_lines_count_multi(int n, oc_ctx *const *ctxs, const oc_lines_acc *const *accs, const int *Ns,
                          const double *const *x, const double *const *y, const uint8_t *const *status, const int *steps,
                          void *stream);
-/* The run loop's only implementation: oc_gcfm_run_acc plus the velocity maps of its frames (vel, needs acc) and the
- * line counts of its steps (lines: every step simu_step0 + k is counted once final; simu_step0 + n_steps must not exceed
- * lines->capacity, checked before any step).  oc_gcfm_run and oc_gcfm_run_acc forward here. */
+/* oc_gcfm_run_acc plus the velocity maps of its frames (vel, needs acc) and the line counts of its steps (lines: every
+ * step simu_step0 + k is counted once final; simu_step0 + n_steps must not exceed lines->capacity, checked before any
+ * step).  oc_gcfm_run and oc_gcfm_run_acc forward here; this forwards to oc_gcfm_run_obs. */
 int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
                      double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,
                      int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss, int n_steps,
                      int simu_step0, int n_active0, double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
                      int *steps_done, double *device_ms, long long *pairs, const oc_density_acc *acc,
                      const oc_velocity_acc *vel, const oc_lines_acc *lines, void *stream);
+
+/* Measurement areas: per step and polygon, the pedestrians inside and the sums of their speeds and velocities.
+ * Membership (even-odd rule, FP64, no contraction, o as for the measurement lines): for every edge (a, b) of the polygon
+ * (vertex k to vertex k+1, the last to the first), when (a.y <= p.y) != (b.y <= p.y), `inside` toggles if
+ * (b.y > a.y) ? o(a,b,p) > 0 : o(a,b,p) < 0.  Points on an edge fall where this puts them; a NaN position is outside.
+ * Only agents with status 1 count.  Row `step`, area a: d_count = agents inside, d_speed_sum = sum of
+ * sqrt(vx*vx + vy*vy), d_vx_sum / d_vy_sum = sums of vx / vy.  The float sums have one order, whatever the launch:
+ * agents in blocks of 256; in a block each warp of 32 sums by an xor butterfly (16, 8, 4, 2, 1; agents outside, left or
+ * beyond N add +0.0), the 8 warp sums are added in warp order from 0.0, and the block sums in block order from 0.0.
+ * A measurement writes its row (no accumulation), so rows need no initialisation. */
+typedef struct {
+    const double *verts;         /* HOST: (x, y) vertices in metres, area after area; finite */
+    const double *d_verts;       /* the same vertices on the device (owned by the caller, uploaded once) */
+    const int *offsets;          /* HOST: n_areas + 1; area a is vertices offsets[a] .. offsets[a+1]-1: 3..64 of them,
+                                    1024 in all, non-zero area */
+    int *d_count;                /* int32 (capacity, n_areas) */
+    double *d_speed_sum, *d_vx_sum, *d_vy_sum;   /* float64 (capacity, n_areas) */
+    double *d_partials;          /* scratch: float64 (partial_blocks, n_areas, 4), the per-block sums */
+    int n_areas;                 /* 1..64 */
+    int capacity;                /* rows (steps) of the arrays above */
+    int partial_blocks;          /* blocks of 256 agents d_partials has room for: >= ceil(N / 256) */
+    int pad_;
+} oc_areas_acc;
+/* Measures the crowd's state (N agents; the state a step starts from) into row `step`.  Asynchronous on stream: two
+ * launches (per-block sums, then the block-order reduction).  OC_ERR_ARG for a NULL required pointer, n_areas outside
+ * 1..64, an area with fewer than 3 or more than 64 vertices, more than 1024 vertices, a non-finite vertex, a zero area,
+ * step outside [0, capacity) and too few partial blocks for N. */
+int oc_areas_measure(oc_ctx *ctx, const oc_areas_acc *acc, int N, const double *d_x, const double *d_y,
+                     const double *d_vx, const double *d_vy, const uint8_t *d_status, int step, void *stream);
+/* oc_areas_measure for each of n members (row steps[m]) in two launches; ctxs[0] owns the member table.  Every row
+ * equals the member's oc_areas_measure alone.  OC_ERR_ARG as oc_areas_measure, and for a member context on another
+ * device than ctxs[0]. */
+int oc_areas_measure_multi(int n, oc_ctx *const *ctxs, const oc_areas_acc *const *accs, const int *Ns,
+                           const double *const *x, const double *const *y, const double *const *vx,
+                           const double *const *vy, const uint8_t *const *status, const int *steps, void *stream);
+/* The run loop's only implementation: oc_gcfm_run_flow plus the measurement areas (areas, nullable): before step k, next
+ * to the density frame and ahead of the step's randomness, the state the step starts from is measured into row
+ * simu_step0 + k.  simu_step0 + n_steps must not exceed areas->capacity, checked before any step.  oc_gcfm_run_flow
+ * forwards here with areas = NULL. */
+int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
+                    double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,
+                    int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss, int n_steps,
+                    int simu_step0, int n_active0, double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
+                    int *steps_done, double *device_ms, long long *pairs, const oc_density_acc *acc,
+                    const oc_velocity_acc *vel, const oc_lines_acc *lines, const oc_areas_acc *areas, void *stream);
 
 #ifdef __cplusplus
 }

@@ -97,6 +97,13 @@ class LinesAcc(C.Structure):
                 ("d_inside", C.c_void_p), ("n_lines", C.c_int), ("capacity", C.c_int)]
 
 
+class AreasAcc(C.Structure):
+    _fields_ = [("verts", dp), ("d_verts", C.c_void_p), ("offsets", ip), ("d_count", C.c_void_p),
+                ("d_speed_sum", C.c_void_p), ("d_vx_sum", C.c_void_p), ("d_vy_sum", C.c_void_p),
+                ("d_partials", C.c_void_p), ("n_areas", C.c_int), ("capacity", C.c_int), ("partial_blocks", C.c_int),
+                ("pad_", C.c_int)]
+
+
 _lib = None
 
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
@@ -105,7 +112,8 @@ EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create"
            "oc_dist_finalize", "oc_dist_p2p_export", "oc_dist_p2p_import", "oc_dist_p2p_enabled", "oc_dist_p2p_disable", "oc_hjb_solve_band", "oc_rasterise_band", "oc_upload", "oc_hjb_solve_batch", "oc_hjb_solve_multi", "oc_hjb_solve_grids", "oc_gcfm_step_launch",
            "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run",
            "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi", "oc_density_accum_vel",
-           "oc_density_accum_vel_multi", "oc_lines_count", "oc_lines_count_multi", "oc_gcfm_run_flow"]
+           "oc_density_accum_vel_multi", "oc_lines_count", "oc_lines_count_multi", "oc_gcfm_run_flow",
+           "oc_areas_measure", "oc_areas_measure_multi", "oc_gcfm_run_obs"]
 
 
 def load():
@@ -145,6 +153,9 @@ def load():
     lib.oc_density_accum_vel_multi.argtypes = [C.c_int, vpp_, vpp_, vpp_, ip, vpp_, vpp_, vpp_, vpp_, vpp_, C.c_void_p]
     lib.oc_lines_count.argtypes = [C.c_void_p, C.POINTER(LinesAcc), C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     lib.oc_lines_count_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, ip, C.c_void_p]
+    lib.oc_gcfm_run_obs.argtypes = lib.oc_gcfm_run_flow.argtypes[:-1] + [C.POINTER(AreasAcc), C.c_void_p]
+    lib.oc_areas_measure.argtypes = [C.c_void_p, C.POINTER(AreasAcc), C.c_int] + [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
+    lib.oc_areas_measure_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, vpp_, vpp_, ip, C.c_void_p]
     lib.oc_rng_step_draw.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp]
     lib.oc_rng_step_draw_ckpt.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp, C.c_int,
                                           C.POINTER(C.c_uint32), ip, ip, dp]
@@ -549,13 +560,15 @@ class Context:
         return exit_log[: n_exit.value].copy(), rc
 
     def gcfm_run(self, prm: GcfmParams, state, vdes, key_id, keys, rng_state, n_steps, simu_step0, n_active, rows=None,
-                 stream=None, density=None, lines=None):
-        """up to n_steps steps of the run loop in one call (oc_gcfm_run_flow): randomness drawn in C from the legacy MT19937
+                 stream=None, density=None, lines=None, areas=None):
+        """up to n_steps steps of the run loop in one call (oc_gcfm_run_obs): randomness drawn in C from the legacy MT19937
         state tuple `rng_state` (np.random.get_state()), next step's draws overlapped with the GPU.  rows: optional list of
         n_steps (N,4) CUDA tensors receiving the packed state after each step.  density: optional DensityStats that
         receives the frame of every due step (with its velocity maps when it has them).  lines: optional LineCounts that
-        receives the crossings of every step (its capacity must cover simu_step0 + n_steps).  Returns dict(steps, exits (agent ids in exit order), exit_step (0-based step
-        within the call), rc, rng_state (to be set_state()d), device_ms, pairs)."""
+        receives the crossings of every step (its capacity must cover simu_step0 + n_steps).  areas: optional AreaStats
+        that receives the measurement of the state every step starts from (the same capacity rule).  Returns dict(steps,
+        exits (agent ids in exit order), exit_step (0-based step within the call), rc, rng_state (to be set_state()d),
+        device_ms, pairs)."""
         N = state["x"].numel()
         karr, keep = keys if isinstance(keys, tuple) else self.make_keys(keys)
         key = np.ascontiguousarray(rng_state[1], dtype=np.uint32).copy()
@@ -569,14 +582,15 @@ class Context:
         ex_a, ex_s = np.empty(max(N, 1), dtype=np.int32), np.empty(max(N, 1), dtype=np.int32)
         n_ex, done, ms, pairs = C.c_int(), C.c_int(), C.c_double(), C.c_longlong()
         vel = None if density is None or density.vel is None else C.byref(density.vel)
-        rc = load().oc_gcfm_run_flow(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
-                                     _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
-                                     karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
-                                     C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
-                                     ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
-                                     C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc), vel,
-                                     None if lines is None else C.byref(lines.acc),
-                                     _stream() if stream is None else C.c_void_p(stream))
+        rc = load().oc_gcfm_run_obs(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
+                                    _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
+                                    karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
+                                    C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
+                                    ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
+                                    C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc), vel,
+                                    None if lines is None else C.byref(lines.acc),
+                                    None if areas is None else C.byref(areas.acc),
+                                    _stream() if stream is None else C.c_void_p(stream))
         check(rc, allow=(OC_ERR_SAMPLER_RANGE,))
         if density is not None:
             density.frames += density.count(simu_step0, done.value)
@@ -646,6 +660,14 @@ class Context:
         check(load().oc_lines_count(self.h, C.byref(lines.acc), state["x"].numel(), _dev(state["x"]), _dev(state["y"]),
                                     _dev(state["status"]), int(step), _stream() if stream is None else C.c_void_p(stream)))
 
+    def areas_measure(self, areas, state, step, stream=None):
+        """measure the crowd `state` (the state the step with simu_step `step` starts from) into row `step` of `areas`
+        (oc_areas_measure)"""
+        N = state["x"].numel()
+        P = (lambda k: None) if N == 0 else (lambda k: _dev(state[k]))
+        check(load().oc_areas_measure(self.h, C.byref(areas.acc), N, P("x"), P("y"), P("vx"), P("vy"), P("status"),
+                                      int(step), _stream() if stream is None else C.c_void_p(stream)))
+
 
 def density_accum_multi(ctxs, stats, states, stream=None):
     """one density frame per member in one launch per variant (oc_density_accum_vel_multi): member q's crowd `states[q]`
@@ -687,6 +709,27 @@ def lines_count_multi(ctxs, lines, states, steps, stream=None):
         xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
     check(load().oc_lines_count_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, sts, ss.ctypes.data_as(ip),
                                       _stream() if stream is None else C.c_void_p(stream)))
+
+
+def areas_measure_multi(ctxs, areas, states, steps, stream=None):
+    """one measurement per member in two launches (oc_areas_measure_multi): member q's crowd `states[q]` (dict with x, y,
+    vx, vy, status) measured into row steps[q] of areas[q]"""
+    n = len(ctxs)
+    if not (len(areas) == len(states) == len(steps) == n and n):
+        raise ValueError("one context, area accumulator, state and step per member expected")
+    vp = lambda: (C.c_void_p * n)()
+    hs, accs, xs, ys, vxs, vys, sts = vp(), vp(), vp(), vp(), vp(), vp(), vp()
+    Ns = np.empty(n, dtype=np.int32)
+    ss = np.ascontiguousarray(steps, dtype=np.int32)
+    for q, (c, a, st) in enumerate(zip(ctxs, areas, states)):
+        hs[q] = c.h.value
+        accs[q] = C.addressof(a.acc)
+        Ns[q] = st["x"].numel()
+        if Ns[q]:
+            xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
+            vxs[q], vys[q] = st["vx"].data_ptr(), st["vy"].data_ptr()
+    check(load().oc_areas_measure_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, vxs, vys, sts, ss.ctypes.data_as(ip),
+                                        _stream() if stream is None else C.c_void_p(stream)))
 
 
 class DensityStats:
@@ -787,6 +830,79 @@ class LineCounts:
     def nbytes(N, n_lines, capacity):
         """device bytes of the accumulator of N agents: previous positions and inside bytes, and the count rows"""
         return 17 * N + 8 * n_lines * max(int(capacity), 1)
+
+
+AREA_BLOCK = 256   # agents per block of the fixed summation order (oc_areas_acc)
+
+
+def polygon_area(v):
+    """|shoelace area| of a polygon given as an (n, 2) array of vertices"""
+    x, y = v[:, 0], v[:, 1]
+    return abs(float(np.sum(x * np.roll(y, -1) - np.roll(x, -1) * y))) / 2
+
+
+class AreaStats:
+    """Device accumulator of measurement areas (oc_areas_acc): per step and area the pedestrians inside (int32) and the
+    sums of their speeds, vx and vy (float64), rows (capacity, n_areas), grown by ensure(); the vertices on the device
+    (uploaded once) and the per-block scratch of a crowd of N agents.  names: the areas' names; verts: (V, 2) array of
+    all vertices in metres, area after area; offsets: (n_areas + 1) int array (simulations.areas_spec)."""
+
+    def __init__(self, ctx, names, verts, offsets, N, capacity):
+        import torch
+        self.names = list(names)
+        self.verts = np.ascontiguousarray(verts, dtype=np.float64).reshape(-1, 2)
+        self.offsets = np.ascontiguousarray(offsets, dtype=np.int32)
+        self.device = ctx.torch_device
+        na = len(self.names)
+        self.d_verts = torch.from_numpy(self.verts).to(self.device)
+        self.partials = torch.empty((max(-(-int(N) // AREA_BLOCK), 1), na, 4), dtype=torch.float64, device=self.device)
+        self._rows(max(int(capacity), 1))
+        self.acc = AreasAcc(self.verts.ctypes.data_as(dp), self.d_verts.data_ptr(), self.offsets.ctypes.data_as(ip),
+                            self.count.data_ptr(), self.speed_sum.data_ptr(), self.vx_sum.data_ptr(),
+                            self.vy_sum.data_ptr(), self.partials.data_ptr(), na, self.count.shape[0],
+                            self.partials.shape[0], 0)
+
+    def _rows(self, cap, old=None):
+        import torch
+        na = len(self.names)
+        self.count = torch.zeros((cap, na), dtype=torch.int32, device=self.device)
+        self.speed_sum, self.vx_sum, self.vy_sum = (torch.zeros((cap, na), dtype=torch.float64, device=self.device)
+                                                    for _ in range(3))
+        if old is not None:
+            for new, o in zip((self.count, self.speed_sum, self.vx_sum, self.vy_sum), old):
+                new[:o.shape[0]] = o
+
+    def ensure(self, steps):
+        """grow the rows (on the host: rare) so that steps 0 .. steps-1 fit"""
+        import torch
+        have = self.count.shape[0]
+        if steps <= have:
+            return
+        torch.cuda.synchronize(self.device)   # (no measurement of the old rows may be in flight on any stream)
+        self._rows(max(steps, 2 * have), (self.count, self.speed_sum, self.vx_sum, self.vy_sum))
+        torch.cuda.synchronize(self.device)
+        self.acc.d_count, self.acc.d_speed_sum = self.count.data_ptr(), self.speed_sum.data_ptr()
+        self.acc.d_vx_sum, self.acc.d_vy_sum = self.vx_sum.data_ptr(), self.vy_sum.data_ptr()
+        self.acc.capacity = self.count.shape[0]
+
+    def result(self, steps):
+        """dict(names, area (n_areas,) in m^2, count (steps, n_areas) int32, speed_sum, vx_sum, vy_sum (float64),
+        density = count / area in ped/m^2, speed = speed_sum / count and velocity (steps, n_areas, 2) = (vx_sum, vy_sum)
+        / count, NaN where count is 0); row k = the state the step with simu_step k started from (the caller has
+        synchronised the streams that measured)"""
+        area = np.array([polygon_area(self.verts[a:b]) for a, b in zip(self.offsets[:-1], self.offsets[1:])])
+        c = self.count[:steps].cpu().numpy()
+        sp, vx, vy = (t[:steps].cpu().numpy() for t in (self.speed_sum, self.vx_sum, self.vy_sum))
+        zero = c == 0
+        with np.errstate(divide="ignore", invalid="ignore"):
+            mean = lambda a: np.where(zero, np.nan, a / np.where(zero, 1, c))
+            return dict(names=list(self.names), area=area, count=c, speed_sum=sp, vx_sum=vx, vy_sum=vy,
+                        density=c / area, speed=mean(sp), velocity=np.stack([mean(vx), mean(vy)], axis=-1))
+
+    @staticmethod
+    def nbytes(N, n_areas, n_verts, capacity):
+        """device bytes of the accumulator of N agents: vertices, per-block scratch and the rows"""
+        return 16 * n_verts + 32 * n_areas * max(-(-int(N) // AREA_BLOCK), 1) + 28 * n_areas * max(int(capacity), 1)
 
 
 class GcfmBatch:

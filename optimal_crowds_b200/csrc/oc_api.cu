@@ -123,6 +123,10 @@ extern "C" void oc_ctx_destroy(oc_ctx *c) {
     if (c->lines_pinned) cudaFreeHost(c->lines_pinned);
     cudaFree(c->lines_dev);
     if (c->lines_ev) cudaEventDestroy(c->lines_ev);
+    if (c->areas_ev) cudaEventSynchronize(c->areas_ev);
+    if (c->areas_pinned) cudaFreeHost(c->areas_pinned);
+    cudaFree(c->areas_dev);
+    if (c->areas_ev) cudaEventDestroy(c->areas_ev);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->gcfm_pinned) cudaFreeHost(c->gcfm_pinned);
     cudaFree(c->fr_ticket);

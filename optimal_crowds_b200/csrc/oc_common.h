@@ -58,6 +58,9 @@ struct oc_ctx {
     void *lines_pinned = nullptr, *lines_dev = nullptr;  // batched line counts: member table and lines (staging, device)
     size_t lines_pinned_bytes = 0, lines_dev_bytes = 0;
     cudaEvent_t lines_ev = nullptr;                      //   recorded after the kernel; the staging is reused after it
+    void *areas_pinned = nullptr, *areas_dev = nullptr;  // batched area measurements: member table and offsets
+    size_t areas_pinned_bytes = 0, areas_dev_bytes = 0;
+    cudaEvent_t areas_ev = nullptr;                      //   recorded after the kernels; the staging is reused after it
     int gcfm_poll_ns = 100;    // oc_ctx_set_int("gcfm_poll_ns"): back-off between polls of a neighbour's done-flag
     int gcfm_sweep_ctas = 0;  // oc_ctx_set_int("gcfm_sweep_ctas"): cap of the sweep grid (0 = fill the GPU)
     int gcfm_margin_mm = 250;  // oc_ctx_set_int("gcfm_margin_mm"): displacement margin (2 x per-axis bound) of the fast attempt

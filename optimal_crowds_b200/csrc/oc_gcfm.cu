@@ -1548,6 +1548,190 @@ int lines_acc_check(const oc_lines_acc *a) {
     return OC_OK;
 }
 
+// Measurement areas (areas_measure_kernel / areas_measure_multi_kernel, then areas_reduce_kernel /
+// areas_reduce_multi_kernel): one thread per agent, the areas' vertices and offsets in shared memory.  The even-odd rule
+// and the summation order are stated at oc_areas_acc (include/optimal_crowds.h).  AR_BLOCK, the 256 agents of a block,
+// is part of that order, not a tuning parameter.  A block writes its sums (count, speed, vx, vy per area) to the
+// partials; the reduction adds them in block order and writes the step's row.
+constexpr int AR_MAX = 64, AR_MAX_POLY = 64, AR_MAX_VERTS = 1024, AR_BLOCK = 256, AR_WARPS = AR_BLOCK / 32;
+struct AreaOffsets {
+    int o[AR_MAX + 1];
+};
+__device__ __forceinline__ bool area_contains(const double2 *v, int n, double px, double py) {
+    bool in = false;
+    double ax = v[n - 1].x, ay = v[n - 1].y;   // edge (v[k-1], v[k]); the closing edge first
+    for (int k = 0; k < n; k++) {
+        const double bx = v[k].x, by = v[k].y;
+        if ((ay <= py) != (by <= py)) {
+            const double o = line_orient(ax, ay, bx, by, px, py);
+            if ((by > ay) ? o > 0 : o < 0) in = !in;
+        }
+        ax = bx; ay = by;
+    }
+    return in;
+}
+// (lane l adds lane l ^ off's value to its own: every lane ends with the same sum, by commutativity)
+__device__ __forceinline__ double warp_butterfly(double v) {
+    for (int off = 16; off >= 1; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
+    return v;
+}
+// Block `blk` of a crowd of N agents against the na areas of V / O (shared memory, loaded by the caller).
+__device__ __forceinline__ void areas_block(int blk, int N, const double *__restrict__ x, const double *__restrict__ y,
+                                            const double *__restrict__ vx, const double *__restrict__ vy,
+                                            const uint8_t *__restrict__ status, const double2 *V, const int *O, int na,
+                                            double *__restrict__ partials) {
+    __shared__ double W[AR_WARPS][AR_MAX][4];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int i = blk * AR_BLOCK + threadIdx.x;
+    const bool act = i < N && status[i] == 1;
+    double px = 0.0, py = 0.0, u = 0.0, w = 0.0, s = 0.0;
+    if (act) {
+        px = x[i]; py = y[i]; u = vx[i]; w = vy[i];
+        s = sqrt(u * u + w * w);
+    }
+    for (int a = 0; a < na; a++) {
+        const bool in = act && area_contains(V + O[a], O[a + 1] - O[a], px, py);
+        const unsigned m = __ballot_sync(0xffffffffu, in);
+        double cs = 0.0, cu = 0.0, cw = 0.0;
+        if (m) {   // (warp-uniform: a warp with nobody inside would add +0.0 to +0.0, which is 0.0)
+            cs = warp_butterfly(in ? s : 0.0);
+            cu = warp_butterfly(in ? u : 0.0);
+            cw = warp_butterfly(in ? w : 0.0);
+        }
+        if (lane == 0) {
+            W[wid][a][0] = __popc(m); W[wid][a][1] = cs; W[wid][a][2] = cu; W[wid][a][3] = cw;
+        }
+    }
+    __syncthreads();
+    for (int t = threadIdx.x; t < 4 * na; t += AR_BLOCK) {
+        const int a = t >> 2, q = t & 3;
+        double sum = 0.0;
+        for (int k = 0; k < AR_WARPS; k++) sum += W[k][a][q];
+        partials[((size_t)blk * na + a) * 4 + q] = sum;
+    }
+}
+// The row of a crowd whose nb block sums are in `partials`: the counts as integers, the float sums in block order.
+__device__ __forceinline__ void areas_reduce(const double *__restrict__ partials, int nb, int na, int *__restrict__ count,
+                                             double *__restrict__ speed_sum, double *__restrict__ vx_sum,
+                                             double *__restrict__ vy_sum) {
+    for (int t = threadIdx.x; t < 4 * na; t += blockDim.x) {
+        const int a = t >> 2, q = t & 3;
+        if (q == 0) {
+            int c = 0;
+            for (int b = 0; b < nb; b++) c += (int)partials[((size_t)b * na + a) * 4];
+            count[a] = c;
+        } else {
+            double s = 0.0;
+            for (int b = 0; b < nb; b++) s += partials[((size_t)b * na + a) * 4 + q];
+            (q == 1 ? speed_sum : q == 2 ? vx_sum : vy_sum)[a] = s;
+        }
+    }
+}
+
+__global__ void __launch_bounds__(AR_BLOCK)
+areas_measure_kernel(int N, const double *__restrict__ x, const double *__restrict__ y, const double *__restrict__ vx,
+                     const double *__restrict__ vy, const uint8_t *__restrict__ status,
+                     const double2 *__restrict__ verts, AreaOffsets ao, int na, double *__restrict__ partials) {
+    __shared__ double2 V[AR_MAX_VERTS];
+    __shared__ int O[AR_MAX + 1];
+    for (int t = threadIdx.x; t <= na; t += AR_BLOCK) O[t] = ao.o[t];
+    for (int t = threadIdx.x, nv = ao.o[na]; t < nv; t += AR_BLOCK) V[t] = verts[t];
+    __syncthreads();
+    areas_block(blockIdx.x, N, x, y, vx, vy, status, V, O, na, partials);
+}
+
+__global__ void __launch_bounds__(256)
+areas_reduce_kernel(const double *__restrict__ partials, int nb, int na, int *__restrict__ count,
+                    double *__restrict__ speed_sum, double *__restrict__ vx_sum, double *__restrict__ vy_sum) {
+    areas_reduce(partials, nb, na, count, speed_sum, vx_sum, vy_sum);
+}
+
+// Batched measurements: member m owns blocks [blk0, blk0 + ceil(N / 256)) of the first launch and block m of the
+// reduction; its offsets follow the member table in the same device buffer, its vertices stay in its own buffer; the
+// row pointers point at the row of the member's step.
+struct AreasMember {
+    const double *x, *y, *vx, *vy;
+    const uint8_t *status;
+    const double2 *verts;
+    const int *offsets;
+    double *partials;
+    int *count;
+    double *speed_sum, *vx_sum, *vy_sum;
+    int N, na, blk0, pad_;
+};
+__global__ void __launch_bounds__(AR_BLOCK) areas_measure_multi_kernel(const AreasMember *__restrict__ ms, int n) {
+    __shared__ double2 V[AR_MAX_VERTS];
+    __shared__ int O[AR_MAX + 1];
+    const int b = blockIdx.x;
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (ms[mid].blk0 <= b) lo = mid;
+        else hi = mid - 1;
+    }
+    const AreasMember &m = ms[lo];
+    for (int t = threadIdx.x; t <= m.na; t += AR_BLOCK) O[t] = m.offsets[t];
+    for (int t = threadIdx.x, nv = m.offsets[m.na]; t < nv; t += AR_BLOCK) V[t] = m.verts[t];
+    __syncthreads();
+    areas_block(b - m.blk0, m.N, m.x, m.y, m.vx, m.vy, m.status, V, O, m.na, m.partials);
+}
+__global__ void __launch_bounds__(256) areas_reduce_multi_kernel(const AreasMember *__restrict__ ms) {
+    const AreasMember &m = ms[blockIdx.x];
+    areas_reduce(m.partials, (m.N + AR_BLOCK - 1) / AR_BLOCK, m.na, m.count, m.speed_sum, m.vx_sum, m.vy_sum);
+}
+
+int areas_acc_check(const oc_areas_acc *a) {
+    OC_ARG(a && a->verts && a->d_verts && a->offsets && a->d_count && a->d_speed_sum && a->d_vx_sum && a->d_vy_sum &&
+           a->d_partials, "NULL argument");
+    OC_ARG(((uintptr_t)a->d_verts & 15) == 0, "measurement areas: d_verts must be 16-byte aligned");
+    OC_ARG(a->n_areas >= 1 && a->n_areas <= AR_MAX, "measurement areas: n_areas must be in 1..64");
+    OC_ARG(a->capacity >= 0 && a->partial_blocks >= 0, "measurement areas: negative capacity");
+    OC_ARG(a->offsets[0] == 0, "measurement areas: offsets must start at 0");
+    for (int k = 0; k < a->n_areas; k++) {
+        const int v0 = a->offsets[k], n = a->offsets[k + 1] - v0;
+        OC_ARG(n >= 3 && n <= AR_MAX_POLY, "measurement areas: an area must have 3..64 vertices");
+        OC_ARG(a->offsets[k + 1] <= AR_MAX_VERTS, "measurement areas: at most 1024 vertices in all");
+        const double *v = a->verts + 2 * (size_t)v0;
+        double s = 0.0;
+        for (int j = 0; j < n; j++) {
+            const int j1 = (j + 1) % n;
+            OC_ARG(std::isfinite(v[2 * j]) && std::isfinite(v[2 * j + 1]), "measurement areas: vertices must be finite");
+            s += v[2 * j] * v[2 * j1 + 1] - v[2 * j1] * v[2 * j + 1];
+        }
+        OC_ARG(s != 0.0, "measurement areas: an area must be non-zero");
+    }
+    return OC_OK;
+}
+
+int areas_args_check(const oc_areas_acc *a, int N, bool ptrs, int step) {
+    if (int rc = areas_acc_check(a)) return rc;
+    OC_ARG(N >= 0 && (N == 0 || ptrs), "NULL argument");
+    OC_ARG(step >= 0 && step < a->capacity, "measurement areas: step beyond the row capacity");
+    OC_ARG((N + AR_BLOCK - 1) / AR_BLOCK <= a->partial_blocks, "measurement areas: too few partial blocks for N");
+    return OC_OK;
+}
+
+// the two launches of one measurement (arguments checked by the caller)
+int areas_enqueue(oc_ctx *ctx, const oc_areas_acc *acc, int N, const double *d_x, const double *d_y, const double *d_vx,
+                  const double *d_vy, const uint8_t *d_status, int step, cudaStream_t st) {
+    OC_CUDA(cudaSetDevice(ctx->device));
+    const int nb = (N + AR_BLOCK - 1) / AR_BLOCK, na = acc->n_areas;
+    const size_t row = (size_t)step * na;
+    if (nb) {
+        AreaOffsets ao;
+        memcpy(ao.o, acc->offsets, sizeof(int) * (na + 1));
+        areas_measure_kernel<<<nb, AR_BLOCK, 0, st>>>(N, d_x, d_y, d_vx, d_vy, d_status,
+                                                      reinterpret_cast<const double2 *>(acc->d_verts), ao, na,
+                                                      acc->d_partials);
+        oc::count_launch();
+    }
+    areas_reduce_kernel<<<1, 256, 0, st>>>(acc->d_partials, nb, na, acc->d_count + row, acc->d_speed_sum + row,
+                                           acc->d_vx_sum + row, acc->d_vy_sum + row);
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    return OC_OK;
+}
+
 template <class T>
 T *carve(char *&p, size_t n) {
     T *r = reinterpret_cast<T *>(p);
@@ -2298,13 +2482,14 @@ extern "C" int oc_gcfm_step_multi_finish(int n, oc_ctx *const *ctxs, int *const 
 // whose simu_step is a multiple of acc->every (the history frame of that iteration), ahead of the step's randomness;
 // vel (nullable, needs acc): that frame's velocity maps too.  lines (nullable): after every step, once the step is final
 // (oc_gcfm_step_finish), its crossings of the measurement lines are counted in row simu_step of lines->d_counts.
-extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
-                                double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
-                                const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
-                                double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
-                                int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
-                                long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
-                                const oc_lines_acc *lines, void *stream) {
+// areas (nullable): next to the frame, the state the step starts from is measured into row simu_step of its arrays.
+extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                               long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
+                               const oc_lines_acc *lines, const oc_areas_acc *areas, void *stream) {
     OC_ARG(ctx && prm && mt_key && mt_pos && has_gauss && cached_gauss && exit_agent && exit_step && n_exits && steps_done,
            "NULL argument");
     OC_ARG(N >= 1 && n_steps >= 0 && n_active0 >= 0 && n_active0 <= N && *mt_pos >= 0 && *mt_pos <= 624, "bad sizes");
@@ -2317,6 +2502,13 @@ extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, d
         OC_ARG(lines->d_px && lines->d_py && lines->d_inside, "NULL argument");
         OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= lines->capacity,
                "measurement lines: step beyond the count capacity");
+    }
+    if (areas) {
+        if (int rc = areas_acc_check(areas)) return rc;
+        OC_ARG(d_vx && d_vy, "NULL argument");
+        OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= areas->capacity,
+               "measurement areas: step beyond the row capacity");
+        OC_ARG((N + AR_BLOCK - 1) / AR_BLOCK <= areas->partial_blocks, "measurement areas: too few partial blocks for N");
     }
     constexpr int N_CKPT = 64;
     *n_exits = 0;
@@ -2336,6 +2528,10 @@ extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, d
         // ---- this iteration's history frame (simulations.py:428), folded into the statistics
         if (acc && (simu_step0 + k) % acc->every == 0) {
             rc = oc_density_accum_vel(ctx, acc, vel, N, d_x, d_y, d_vx, d_vy, d_status, stream);
+            if (rc) return rc;
+        }
+        if (areas) {
+            rc = areas_enqueue(ctx, areas, N, d_x, d_y, d_vx, d_vy, d_status, simu_step0 + k, (cudaStream_t)stream);
             if (rc) return rc;
         }
         // ---- this step's randomness (simulations.py:271,303)
@@ -2388,6 +2584,18 @@ extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, d
         if (rc == OC_ERR_SAMPLER_RANGE) return rc;
     }
     return OC_OK;
+}
+
+extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                                double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                                const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                                double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                                int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                                long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
+                                const oc_lines_acc *lines, void *stream) {
+    return oc_gcfm_run_obs(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key,
+                           mt_pos, has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent, exit_step,
+                           n_exits, steps_done, device_ms, pairs, acc, vel, lines, nullptr, stream);
 }
 
 extern "C" int oc_gcfm_run_acc(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
@@ -2621,5 +2829,65 @@ extern "C" int oc_lines_count_multi(int n, oc_ctx *const *ctxs, const oc_lines_a
     oc::count_launch();
     OC_CUDA(cudaGetLastError());
     OC_CUDA(cudaEventRecord(c0->lines_ev, st));
+    return OC_OK;
+}
+
+// ------------------------------------------------------------------------------------------------ measurement areas
+extern "C" int oc_areas_measure(oc_ctx *ctx, const oc_areas_acc *acc, int N, const double *d_x, const double *d_y,
+                                const double *d_vx, const double *d_vy, const uint8_t *d_status, int step,
+                                void *stream) {
+    OC_ARG(ctx, "NULL argument");
+    if (int rc = areas_args_check(acc, N, d_x && d_y && d_vx && d_vy && d_status, step)) return rc;
+    return areas_enqueue(ctx, acc, N, d_x, d_y, d_vx, d_vy, d_status, step, (cudaStream_t)stream);
+}
+
+extern "C" int oc_areas_measure_multi(int n, oc_ctx *const *ctxs, const oc_areas_acc *const *accs, const int *Ns,
+                                      const double *const *x, const double *const *y, const double *const *vx,
+                                      const double *const *vy, const uint8_t *const *status, const int *steps,
+                                      void *stream) {
+    OC_ARG(n >= 1 && ctxs && accs && Ns && x && y && vx && vy && status && steps && ctxs[0], "NULL argument");
+    oc_ctx *c0 = ctxs[0];
+    size_t n_offsets = 0;
+    for (int m = 0; m < n; m++) {
+        OC_ARG(ctxs[m], "NULL argument");
+        OC_ARG(ctxs[m]->device == c0->device, "measurement areas: member context on another device");
+        if (int rc = areas_args_check(accs[m], Ns[m], x[m] && y[m] && vx[m] && vy[m] && status[m], steps[m])) return rc;
+        n_offsets += (size_t)accs[m]->n_areas + 1;
+    }
+    OC_CUDA(cudaSetDevice(c0->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t rec_bytes = ((sizeof(AreasMember) * (size_t)n + 15) / 16) * 16;
+    const size_t bytes = rec_bytes + sizeof(int) * n_offsets;
+    // the table (staging and device copy) is reused once the previous call's kernels have read it, whatever its stream
+    if (!c0->areas_ev) OC_CUDA(cudaEventCreateWithFlags(&c0->areas_ev, cudaEventDisableTiming));
+    OC_CUDA(cudaEventSynchronize(c0->areas_ev));
+    if (int rc = oc_ensure_buffer(c0->areas_pinned, c0->areas_pinned_bytes, bytes, true, "area member table")) return rc;
+    if (int rc = oc_ensure_buffer(c0->areas_dev, c0->areas_dev_bytes, bytes, false, "area member table")) return rc;
+    AreasMember *recs = static_cast<AreasMember *>(c0->areas_pinned);
+    int *ho = reinterpret_cast<int *>(static_cast<char *>(c0->areas_pinned) + rec_bytes);
+    const int *dof = reinterpret_cast<const int *>(static_cast<char *>(c0->areas_dev) + rec_bytes);
+    long long blocks = 0;
+    size_t off = 0;
+    for (int m = 0; m < n; m++) {
+        const oc_areas_acc *a = accs[m];
+        const size_t row = (size_t)steps[m] * a->n_areas;
+        memcpy(ho + off, a->offsets, sizeof(int) * (a->n_areas + 1));
+        recs[m] = AreasMember{x[m], y[m], vx[m], vy[m], status[m], reinterpret_cast<const double2 *>(a->d_verts),
+                              dof + off, a->d_partials, a->d_count + row, a->d_speed_sum + row, a->d_vx_sum + row,
+                              a->d_vy_sum + row, Ns[m], a->n_areas, (int)blocks, 0};
+        off += (size_t)a->n_areas + 1;
+        blocks += (Ns[m] + AR_BLOCK - 1) / AR_BLOCK;
+    }
+    OC_ARG(blocks < 0x7fffffff && n < 0x7fffffff, "measurement areas: too many agents for one launch");
+    OC_CUDA(cudaMemcpyAsync(c0->areas_dev, recs, bytes, cudaMemcpyHostToDevice, st));
+    const AreasMember *dev = static_cast<const AreasMember *>(c0->areas_dev);
+    if (blocks) {
+        areas_measure_multi_kernel<<<(unsigned)blocks, AR_BLOCK, 0, st>>>(dev, n);
+        oc::count_launch();
+    }
+    areas_reduce_multi_kernel<<<n, 256, 0, st>>>(dev);
+    oc::count_launch();
+    OC_CUDA(cudaGetLastError());
+    OC_CUDA(cudaEventRecord(c0->areas_ev, st));
     return OC_OK;
 }

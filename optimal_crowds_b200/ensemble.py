@@ -27,7 +27,10 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     with ``velocity=True`` also the frames' density-weighted velocity and speed maps;
   * ``lines``: every member counts, per step, the agents crossing each measurement line in each direction on the device
     (one batched ``oc_lines_count_multi`` launch per step for a wave) and hands them back in ``results[i]["lines"]``
-    (tests/test_gpu_flow_stats.py).
+    (tests/test_gpu_flow_stats.py);
+  * ``areas``: every member measures, at the start of every step, the pedestrians inside each measurement area and the
+    sums of their speeds and velocities on the device (one batched ``oc_areas_measure_multi`` call per step for a wave)
+    and hands them back in ``results[i]["areas"]`` (tests/test_gpu_areas.py).
 """
 from __future__ import annotations
 
@@ -115,6 +118,9 @@ class ensemble:
     ``lines``: None or {name: (x0, y0, x1, y1)} in metres (at most 64), the same measurement lines for every member, as
     ``simulation(..., lines=...)`` takes them; ``results[i]["lines"]`` is then the member's ``line_counts()`` dict.
 
+    ``areas``: None or {name: [(x0, y0), (x1, y1), ...]} in metres, the same measurement areas for every member, as
+    ``simulation(..., areas=...)`` takes them; ``results[i]["areas"]`` is then the member's ``area_stats()`` dict.
+
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
     ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
     their rooms may differ in size and number of target sets.
@@ -126,7 +132,7 @@ class ensemble:
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
                  memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None,
-                 density_stats=None, lines=None):
+                 density_stats=None, lines=None, areas=None):
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -151,6 +157,7 @@ class ensemble:
         self.density_stats = simulations.density_stats_spec(density_stats, with_velocity=True)  # (every, thr, vel) / None
         self.lines = simulations.lines_spec(lines)                            # (names, (n, 4) array) or None
         self._lines_arg = None if self.lines is None else dict(zip(self.lines[0], map(tuple, self.lines[1])))
+        self.areas = simulations.areas_spec(areas)                            # (names, vertices, offsets) or None
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -178,7 +185,8 @@ class ensemble:
 
     def member_bytes(self, members=None):
         """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets, plus the
-        density accumulators when density_stats is on and the line accumulator with lines); no CUDA"""
+        density accumulators when density_stats is on, the line accumulator with lines and the area accumulator with
+        areas); no CUDA"""
         out = []
         for i in (self.mine if members is None else members):
             room, cfg = self._room(i), self.configs[i]
@@ -187,9 +195,12 @@ class ensemble:
             b = field_bytes_per_member(Ny, Nx, self.T, cfg["dt"], n_keys, self.field_storage)
             if self.density_stats is not None:
                 b += _lib.DensityStats.nbytes(Ny, Nx, self.density_stats[1], self.density_stats[2])
+            N = sum(int(box[4] * box[2] * box[3]) for box in room["initial_boxes"].values())   # simulations.py:122
+            steps = len(simulations.density_frame_steps(self.T, cfg["dt"], 1))
             if self.lines is not None:
-                N = sum(int(box[4] * box[2] * box[3]) for box in room["initial_boxes"].values())   # simulations.py:122
-                b += _lib.LineCounts.nbytes(N, len(self.lines[0]), len(simulations.density_frame_steps(self.T, cfg["dt"], 1)))
+                b += _lib.LineCounts.nbytes(N, len(self.lines[0]), steps)
+            if self.areas is not None:
+                b += _lib.AreaStats.nbytes(N, len(self.areas[0]), len(self.areas[1]), steps)
             out.append(b)
         return out
 
@@ -207,7 +218,8 @@ class ensemble:
                                       config=self.overrides[idx], _ctx=ctx,
                                       density_stats=None if self.density_stats is None else
                                       dict(every=self.density_stats[0], threshold=self.density_stats[1],
-                                           velocity=self.density_stats[2]), lines=self._lines_arg)
+                                           velocity=self.density_stats[2]), lines=self._lines_arg,
+                                      areas=self.areas)
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -353,6 +365,15 @@ class ensemble:
                     if dd:
                         _lib.density_accum_multi([sims[q]._ctx for q in dd], [sims[q]._dstats for q in dd],
                                                  [sims[q]._state for q in dd], stream=main)
+                if self.areas is not None:
+                    # the state this step starts from, measured for the whole wave in one call
+                    for q in live:
+                        sims[q]._areas.ensure(sims[q].simu_step + 1)
+                    am = [q for q in live if sims[q].N > 0]
+                    if am:
+                        _lib.areas_measure_multi([sims[q]._ctx for q in am], [sims[q]._areas for q in am],
+                                                 [sims[q]._state for q in am], [sims[q].simu_step for q in am],
+                                                 stream=main)
                 batch.launch(live, [sims[q].inside for q in live], [sims[q].simu_step for q in live], stream=main,
                              rebind=rebind)
                 tl1 = time.perf_counter()
@@ -397,6 +418,8 @@ class ensemble:
                 self.results[i]["density"] = s._dstats.result()
             if self.lines is not None:
                 self.results[i]["lines"] = s._lines.result(s.simu_step)
+            if self.areas is not None:
+                self.results[i]["areas"] = s._areas.result(s.simu_step)
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3

@@ -80,6 +80,86 @@ def lines_spec(value):
     return names, np.array(rows, dtype=np.float64)
 
 
+MAX_AREAS, MAX_AREA_VERTS, MAX_VERTS = 64, 64, 1024
+
+
+def _polygon_simple(v):
+    """True when the closed polygon v ((n, 2) float64, n >= 3) does not touch itself: consecutive edges meet only at
+    their common vertex (no zero-length edge, no fold back along the same line) and other edges have no point in common"""
+    n = len(v)
+    a, b = v, np.roll(v, -1, axis=0)                  # edge k: a[k] -> b[k]
+    d = b - a
+    if (np.all(d == 0, axis=1)).any():
+        return False
+    # consecutive edges k, k+1: a fold back is collinear with opposite directions
+    dn = np.roll(d, -1, axis=0)
+    cross = d[:, 0] * dn[:, 1] - d[:, 1] * dn[:, 0]
+    if ((cross == 0) & (np.sum(d * dn, axis=1) < 0)).any():
+        return False
+    i, j = np.triu_indices(n, 2)
+    keep = ~((i == 0) & (j == n - 1))                 # (edges n-1 and 0 are consecutive)
+    i, j = i[keep], j[keep]
+    if not len(i):
+        return True
+    p1, p2, p3, p4 = a[i], b[i], a[j], b[j]
+    o = lambda u, w, z: (w[:, 0] - u[:, 0]) * (z[:, 1] - u[:, 1]) - (w[:, 1] - u[:, 1]) * (z[:, 0] - u[:, 0])
+    d1, d2, d3, d4 = o(p3, p4, p1), o(p3, p4, p2), o(p1, p2, p3), o(p1, p2, p4)
+    proper = (np.sign(d1) * np.sign(d2) < 0) & (np.sign(d3) * np.sign(d4) < 0)
+
+    def on(u, w, z, dz):                              # z collinear with u-w and inside its bounding box
+        return (dz == 0) & (np.minimum(u[:, 0], w[:, 0]) <= z[:, 0]) & (z[:, 0] <= np.maximum(u[:, 0], w[:, 0])) & \
+            (np.minimum(u[:, 1], w[:, 1]) <= z[:, 1]) & (z[:, 1] <= np.maximum(u[:, 1], w[:, 1]))
+    touch = on(p3, p4, p1, d1) | on(p3, p4, p2, d2) | on(p1, p2, p3, d3) | on(p1, p2, p4, d4)
+    return not (proper | touch).any()
+
+
+class AreasSpec(tuple):
+    """(names, (V, 2) float64 vertices, (A + 1) int32 offsets): a checked ``areas`` argument"""
+
+
+def areas_spec(value):
+    """AreasSpec (names, (V, 2) float64 vertices, (A + 1) int32 offsets) of an ``areas`` argument -- {name: [(x0, y0),
+    (x1, y1), ...]} in metres: 1 to 64 simple polygons of 3 to 64 vertices, 1024 vertices in all, finite coordinates,
+    non-zero area -- or None for None; checked without touching a GPU.  An AreasSpec is returned as it is (ensemble
+    members take the ensemble's checked areas)"""
+    if value is None or isinstance(value, AreasSpec):
+        return value
+    if not isinstance(value, dict) or not value:
+        raise ValueError("areas: expected a non-empty dict {name: [(x0, y0), (x1, y1), ...]}")
+    if len(value) > MAX_AREAS:
+        raise ValueError(f"areas: at most {MAX_AREAS} measurement areas")
+    names, polys, total = [], [], 0
+    for name, poly in value.items():
+        bad = ValueError(f"areas: {name!r} is not a list of (x, y) vertices")
+        if isinstance(poly, (str, bytes, dict)):
+            raise bad
+        try:
+            pts = list(poly)
+            if any(isinstance(p, (str, bytes, dict)) or any(isinstance(c, (bool, np.bool_, str, bytes)) for c in p)
+                   for p in pts):
+                raise bad
+            v = np.asarray(pts, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise bad from None
+        if v.ndim != 2 or v.shape[1] != 2:
+            raise bad
+        if not MAX_AREA_VERTS >= len(v) >= 3:
+            raise ValueError(f"areas: {name!r} must have 3 to {MAX_AREA_VERTS} vertices")
+        if not np.isfinite(v).all():
+            raise ValueError(f"areas: the vertices of {name!r} must be finite")
+        if _lib.polygon_area(v) == 0:
+            raise ValueError(f"areas: {name!r} has zero area")
+        if not _polygon_simple(v):
+            raise ValueError(f"areas: {name!r} is not a simple polygon (its edges touch or cross)")
+        total += len(v)
+        if total > MAX_VERTS:
+            raise ValueError(f"areas: at most {MAX_VERTS} vertices in all")
+        names.append(name)
+        polys.append(v)
+    offsets = np.concatenate([[0], np.cumsum([len(v) for v in polys])]).astype(np.int32)
+    return AreasSpec((names, np.concatenate(polys), offsets))
+
+
 def density_frame_steps(T, dt, every, recompute_step=None):
     """The simu_steps whose frames run() adds to the density statistics when nobody leaves before T: run()'s loop
     (simulations.py:427-441) as it is cut into blocks here -- one advance() per stretch up to the next re-solve (every
@@ -203,7 +283,7 @@ class simulation:
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
                  rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, lines=None,
-                 _ctx=None):
+                 areas=None, _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -224,10 +304,17 @@ class simulation:
         ``density_stats()``; with ``velocity=True`` also the density-weighted sums of the agents' vx, vy and speed, and
         their means ``velocity`` and ``speed``.  Not available with ``band`` or ``shard_keys``), ``lines`` ({name: (x0, y0,
         x1, y1)} in metres, at most 64: count on the device, per step, the agents crossing each line to its left and to
-        its right; read them with ``line_counts()``.  Not available with ``band`` or ``shard_keys``)."""
+        its right; read them with ``line_counts()``.  Not available with ``band`` or ``shard_keys``), ``areas`` ({name:
+        [(x0, y0), (x1, y1), ...]} in metres, at most 64 simple polygons of 3 to 64 vertices, 1024 in all: measure on
+        the device, at the start of every step, the pedestrians inside each polygon and the sums of their speeds and
+        velocities; read them with ``area_stats()``.  Not available with ``band`` or ``shard_keys``)."""
         import torch
         dstats = density_stats_spec(density_stats, with_velocity=True)
         lspec = lines_spec(lines)
+        aspec = areas_spec(areas)
+        if aspec is not None and (band or shard_keys):
+            raise ValueError("areas are not available for row-decomposed (band=True) or key-sharded "
+                             "(shard_keys=True) runs")
         if dstats is not None and (band or shard_keys):
             raise ValueError("density_stats is not available for row-decomposed (band=True) or key-sharded "
                              "(shard_keys=True) runs")
@@ -367,6 +454,8 @@ class simulation:
         # step of a run that lasts until T, grown on the host when the steps go past that
         self._lines = None if lspec is None else _lib.LineCounts(ctx, *lspec, self._state,
                                                                  len(density_frame_steps(T, self.dt, 1)))
+        # measurement areas (written before every step by oc_areas_measure* / oc_gcfm_run_obs), rows sized as the lines'
+        self._areas = None if aspec is None else _lib.AreaStats(ctx, *aspec, N, len(density_frame_steps(T, self.dt, 1)))
         # per-step record of (x, y, vx, vy); row k = state after k steps (ped.traj / ped.vels / history views).  It
         # lives on the DEVICE in blocks of TRACK_CHUNK steps, written by one small kernel per step (oc_state_pack), and
         # is read back -- once per row -- only when somebody looks at it
@@ -495,6 +584,7 @@ class simulation:
         else:
             prm = self._gcfm_prm
         pending = None
+        self._measure_areas()
         if self.N > 0:
             n_active = int(self._h_status.sum())
             # np.random.choice(np.arange(N), N, replace=False) (simulations.py:271) and one normal pair per active
@@ -534,11 +624,12 @@ class simulation:
                                                  device=self._ctx.torch_device))
             rows.append(self._d_track[blk][off])
         n_active = int(self._h_status.sum())
-        if self._lines is not None:
-            self._lines.ensure(self.simu_step + n_steps)
+        for acc in (self._lines, self._areas):
+            if acc is not None:
+                acc.ensure(self.simu_step + n_steps)
         res = self._ctx.gcfm_run(self._gcfm_prm, self._state, self._d_vdes, self._d_key, self._keys(), st, n_steps,
                                  self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats,
-                                 lines=self._lines)
+                                 lines=self._lines, areas=self._areas)
         self._rng.rng.set_state(res["rng_state"])
         self.last_run_stats = dict(steps=res["steps"], device_ms=res["device_ms"], pairs=res["pairs"])
         ex, exs = res["exits"], res["exit_step"]
@@ -593,6 +684,25 @@ class simulation:
         import torch
         torch.cuda.synchronize(self._ctx.torch_device)
         return self._lines.result(self.simu_step)
+
+    def _measure_areas(self):
+        """measure the state this step starts from into row simu_step of the measurement areas (before the step's
+        randomness; a crowd without agents keeps the zero row)"""
+        if self._areas is not None:
+            self._areas.ensure(self.simu_step + 1)
+            if self.N > 0:
+                self._ctx.areas_measure(self._areas, self._state, self.simu_step, stream=self._cuda_stream)
+
+    def area_stats(self):
+        """the measurement areas (``areas=`` of the constructor) of the steps taken so far: dict(names, area, count,
+        speed_sum, vx_sum, vy_sum, density, speed, velocity) -- (simu_step, n_areas) arrays (velocity: (simu_step,
+        n_areas, 2)), row k = the state the step with simu_step k started from; ``speed`` and ``velocity`` are NaN where
+        nobody is inside"""
+        if self._areas is None:
+            raise RuntimeError("this simulation was created without areas")
+        import torch
+        torch.cuda.synchronize(self._ctx.torch_device)
+        return self._areas.result(self.simu_step)
 
     def _step_finish(self, launched, verbose=False):
         dt, pending = launched
