@@ -521,10 +521,93 @@ int oc_areas_measure(oc_ctx *ctx, const oc_areas_acc *acc, int N, const double *
 int oc_areas_measure_multi(int n, oc_ctx *const *ctxs, const oc_areas_acc *const *accs, const int *Ns,
                            const double *const *x, const double *const *y, const double *const *vx,
                            const double *const *vy, const uint8_t *const *status, const int *steps, void *stream);
-/* The run loop's only implementation: oc_gcfm_run_flow plus the measurement areas (areas, nullable): before step k, next
- * to the density frame and ahead of the step's randomness, the state the step starts from is measured into row
- * simu_step0 + k.  simu_step0 + n_steps must not exceed areas->capacity, checked before any step.  oc_gcfm_run_flow
- * forwards here with areas = NULL. */
+/* Voronoi density, speed and velocity in the measurement areas (Steffen & Seyfried 2010, jpsreport's method D), per step
+ * and area.  FP64 without contraction, every formula evaluated exactly as written; o(a,b,p) =
+ * (b.x-a.x)*(p.y-a.y) - (b.y-a.y)*(p.x-a.x); r = cutoff, n = edges.
+ *  1. Generators G: agents with status 1 and finite x and y.  Others neither own a cell nor clip one.
+ *  2. Cut-off polygon: d_ring holds ox[k] = r*cos(2*pi*k/n), oy[k] = r*sin(2*pi*k/n), k = 0..n-1, computed on the host;
+ *     agent i starts from P = [(x_i + ox[k], y_i + oy[k])], counter-clockwise.
+ *  3. Clip(P, s), one Sutherland-Hodgman pass keeping s <= 0: for k = 0..m-1 (m vertices), a = P[k], b = P[(k+1) % m],
+ *     each vertex's s evaluated once: emit a if sa <= 0; if (sa <= 0) != (sb <= 0) emit a + t*(b - a) per component with
+ *     t = sa / (sa - sb).  Fewer than 3 output vertices make the polygon empty (empty stays empty).  A clip whose output
+ *     would exceed 64 vertices overflows: the polygon's area is NaN.
+ *  4. The cell V_i: P clipped by s = -p.x, s = p.x - L, s = -p.y, s = p.y - H (the room [0, L] x [0, H] of the
+ *     context, in this order), then by every j in G, j != i, in ascending agent index, with dx = x_j - x_i,
+ *     dy = y_j - y_i, dx*dx + dy*dy <= (2*r)*(2*r) and not (dx == 0 && dy == 0) (coincident agents do not clip each
+ *     other): s = dx*(p.x - mx) + dy*(p.y - my), mx = 0.5*(x_i + x_j), my = 0.5*(y_i + y_j).
+ *  5. |V| = 0.5 * (sum over k of x_k*y_{k+1} - x_{k+1}*y_k, in k order from 0.0); 0.0 for an empty polygon.
+ *  6. Areas as triangles (d_tris, counter-clockwise, a fixed order per area; simulations.voronoi_triangles): for
+ *     triangle t = (a, b, c), |V_i n t| = +0.0 when the square [x_i - r, x_i + r] x [y_i - r, y_i + r] does not meet t's
+ *     bounding box (closed intervals: x_i - r <= xmax && x_i + r >= xmin, the same in y); else V_i clipped by
+ *     s = -o(a,b,p), -o(b,c,p), -o(c,a,p) in that order, and its |.|.  w_ia = sum over the area's triangles in order
+ *     from 0.0.  An overflowed cell gives w_ia = NaN for the areas with a triangle its square meets.
+ *  7. Per-agent terms of area a, s_i = sqrt(vx*vx + vy*vy): w, w / |V_i|, w*s_i, w*vx_i, w*vy_i; +0.0 (all five) for
+ *     non-generators, for cells with |V_i| <= 0 and wherever w == 0.
+ *  8. The five sums per area in the measurement areas' order (blocks of 256 agents, xor butterfly per warp, warp sums in
+ *     warp order from 0.0, block sums in block order from 0.0), each divided by |A| (d_area_info[a*5 + 4], the area's
+ *     shoelace area): row `step`, area a of d_rows holds density = sum(w/|V|) / |A|, speed = sum(w*s) / |A|,
+ *     vx = sum(w*vx) / |A|, vy = sum(w*vy) / |A|, covered = sum(w) / |A|.  A NaN means a cell touching the area
+ *     overflowed (or a NaN velocity of an agent whose cell covers part of it, in speed and velocity).
+ * Neighbour search: the generators are binned on a bins_x x bins_y grid over the room (bin index clamped in double, so
+ * agents outside the room land in edge bins) with sides of at least 2r*(1 + 1e-6), sorted by index inside each bin,
+ * and the 3x3 bins around a cell's bin are merged in ascending index.  Cells whose square meets no area's bounding box
+ * are not built (their terms are +0.0 by rule 6). */
+typedef struct {
+    const double *d_ring;        /* (edges, 2): ox, oy of rule 2 */
+    const double *d_tris;        /* (n_tris, 10): ax, ay, bx, by, cx, cy, xmin, xmax, ymin, ymax of every triangle */
+    const double *d_area_info;   /* (n_areas, 5): xmin, xmax, ymin, ymax of the area's vertices, |A| (> 0) */
+    const int *tri_offsets;      /* HOST: n_areas + 1; area a is triangles tri_offsets[a] .. tri_offsets[a+1]-1 (>= 1
+                                    each), 992 in all */
+    const int *d_tri_offsets;    /* the same offsets on the device */
+    int *d_bin_count;            /* int32 (bin_capacity): zero before the first measurement, left zero by every one */
+    int *d_bin_start;            /* int32 (bin_capacity) */
+    int *d_slot;                 /* int32 (agent_capacity, 2): each generator's bin and place in it */
+    int *d_order;                /* int32 (2 * agent_capacity): the binned generators, then the same sorted by index */
+    double *d_partials;          /* scratch: float64 (partial_blocks, n_areas, 5), the per-block sums */
+    double *d_rows;              /* float64 (capacity, n_areas, 5): density, speed, vx, vy, covered */
+    double cutoff;               /* r: finite, in (0, 100] metres */
+    int edges;                   /* n: 4..32 */
+    int n_areas;                 /* 1..64 */
+    int bins_x, bins_y;          /* >= 1; bins_x == 1 or L / bins_x >= 2r*(1 + 1e-6) (the same for y) */
+    int bin_capacity;            /* >= bins_x * bins_y + 1 */
+    int agent_capacity;          /* >= N */
+    int partial_blocks;          /* >= ceil(N / 256) */
+    int capacity;                /* rows (steps) of d_rows */
+} oc_voronoi_acc;
+/* Measures the crowd's state (N agents; the state a step starts from) into row `step` of acc->d_rows.  Asynchronous on
+ * stream: six launches (bin, scan, place, sort, cells, block-order reduction).  OC_ERR_ARG for a NULL required pointer,
+ * a cutoff that is not finite or outside (0, 100], edges outside 4..32, n_areas outside 1..64, bad triangle offsets
+ * (an area without triangles, more than 992 in all), bins too small or too many, too small agent or partial capacities
+ * for N and step outside [0, capacity). */
+int oc_voronoi_measure(oc_ctx *ctx, const oc_voronoi_acc *acc, int N, const double *d_x, const double *d_y,
+                       const double *d_vx, const double *d_vy, const uint8_t *d_status, int step, void *stream);
+/* oc_voronoi_measure for each of n members (row steps[m]) in six launches; ctxs[0] owns the member table.  Every row
+ * equals the member's oc_voronoi_measure alone.  OC_ERR_ARG as oc_voronoi_measure, for a member context on another
+ * device than ctxs[0] and for two members sharing d_bin_count, d_bin_start, d_slot, d_order or d_partials. */
+int oc_voronoi_measure_multi(int n, oc_ctx *const *ctxs, const oc_voronoi_acc *const *accs, const int *Ns,
+                             const double *const *x, const double *const *y, const double *const *vx,
+                             const double *const *vy, const uint8_t *const *status, const int *steps, void *stream);
+
+/* The observers of a run loop, each nullable: density frames (acc) and their velocity maps (vel, needs acc), line
+ * counts, measurement areas and their Voronoi measures. */
+typedef struct {
+    const oc_density_acc *density;
+    const oc_velocity_acc *velocity;
+    const oc_lines_acc *lines;
+    const oc_areas_acc *areas;
+    const oc_voronoi_acc *voronoi;
+} oc_observers;
+/* The run loop's only implementation: oc_gcfm_run_flow plus the measurement areas and their Voronoi measures (obs: every
+ * pointer nullable; obs itself nullable): before step k, next to the density frame and ahead of the step's randomness,
+ * the state the step starts from is measured into row simu_step0 + k.  simu_step0 + n_steps must not exceed the
+ * capacity of the areas' and the Voronoi rows, checked before any step.  oc_gcfm_run_obs forwards here. */
+int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                         double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                         const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                         double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                         int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                         long long *pairs, const oc_observers *obs, void *stream);
+/* oc_gcfm_run_flow plus the measurement areas (areas, nullable): forwards to oc_gcfm_run_observed. */
 int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
                     double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,
                     int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss, int n_steps,

@@ -104,6 +104,20 @@ class AreasAcc(C.Structure):
                 ("pad_", C.c_int)]
 
 
+class VoronoiAcc(C.Structure):
+    _fields_ = [("d_ring", C.c_void_p), ("d_tris", C.c_void_p), ("d_area_info", C.c_void_p), ("tri_offsets", ip),
+                ("d_tri_offsets", C.c_void_p), ("d_bin_count", C.c_void_p), ("d_bin_start", C.c_void_p),
+                ("d_slot", C.c_void_p), ("d_order", C.c_void_p), ("d_partials", C.c_void_p), ("d_rows", C.c_void_p),
+                ("cutoff", C.c_double), ("edges", C.c_int), ("n_areas", C.c_int), ("bins_x", C.c_int),
+                ("bins_y", C.c_int), ("bin_capacity", C.c_int), ("agent_capacity", C.c_int),
+                ("partial_blocks", C.c_int), ("capacity", C.c_int)]
+
+
+class Observers(C.Structure):
+    _fields_ = [("density", C.POINTER(DensityAcc)), ("velocity", C.POINTER(VelocityAcc)),
+                ("lines", C.POINTER(LinesAcc)), ("areas", C.POINTER(AreasAcc)), ("voronoi", C.POINTER(VoronoiAcc))]
+
+
 _lib = None
 
 EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create", "oc_ctx_destroy", "oc_ctx_set_int", "oc_rasterise",
@@ -113,7 +127,8 @@ EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create"
            "oc_gcfm_step_finish", "oc_gcfm_last_pairs", "oc_gcfm_last_redos", "oc_state_pack", "oc_fp64_peak", "oc_place_box", "oc_hjb_plan_chunk_rows", "oc_rng_step_draw", "oc_rng_step_draw_ckpt", "oc_gcfm_step_multi_launch", "oc_gcfm_step_multi_finish", "oc_gcfm_run",
            "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi", "oc_density_accum_vel",
            "oc_density_accum_vel_multi", "oc_lines_count", "oc_lines_count_multi", "oc_gcfm_run_flow",
-           "oc_areas_measure", "oc_areas_measure_multi", "oc_gcfm_run_obs"]
+           "oc_areas_measure", "oc_areas_measure_multi", "oc_gcfm_run_obs",
+           "oc_voronoi_measure", "oc_voronoi_measure_multi", "oc_gcfm_run_observed"]
 
 
 def load():
@@ -154,6 +169,10 @@ def load():
     lib.oc_lines_count.argtypes = [C.c_void_p, C.POINTER(LinesAcc), C.c_int] + [C.c_void_p] * 3 + [C.c_int, C.c_void_p]
     lib.oc_lines_count_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, ip, C.c_void_p]
     lib.oc_gcfm_run_obs.argtypes = lib.oc_gcfm_run_flow.argtypes[:-1] + [C.POINTER(AreasAcc), C.c_void_p]
+    lib.oc_gcfm_run_observed.argtypes = lib.oc_gcfm_run_acc.argtypes[:-2] + [C.POINTER(Observers), C.c_void_p]
+    lib.oc_voronoi_measure.argtypes = [C.c_void_p, C.POINTER(VoronoiAcc), C.c_int] + [C.c_void_p] * 5 + [C.c_int,
+                                                                                                       C.c_void_p]
+    lib.oc_voronoi_measure_multi.argtypes = lib.oc_areas_measure_multi.argtypes
     lib.oc_areas_measure.argtypes = [C.c_void_p, C.POINTER(AreasAcc), C.c_int] + [C.c_void_p] * 5 + [C.c_int, C.c_void_p]
     lib.oc_areas_measure_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, vpp_, vpp_, ip, C.c_void_p]
     lib.oc_rng_step_draw.argtypes = [C.POINTER(C.c_uint32), ip, ip, dp, C.c_int, C.c_int, ip, dp]
@@ -560,13 +579,14 @@ class Context:
         return exit_log[: n_exit.value].copy(), rc
 
     def gcfm_run(self, prm: GcfmParams, state, vdes, key_id, keys, rng_state, n_steps, simu_step0, n_active, rows=None,
-                 stream=None, density=None, lines=None, areas=None):
-        """up to n_steps steps of the run loop in one call (oc_gcfm_run_obs): randomness drawn in C from the legacy MT19937
+                 stream=None, density=None, lines=None, areas=None, voronoi=None):
+        """up to n_steps steps of the run loop in one call (oc_gcfm_run_observed): randomness drawn in C from the legacy MT19937
         state tuple `rng_state` (np.random.get_state()), next step's draws overlapped with the GPU.  rows: optional list of
         n_steps (N,4) CUDA tensors receiving the packed state after each step.  density: optional DensityStats that
         receives the frame of every due step (with its velocity maps when it has them).  lines: optional LineCounts that
         receives the crossings of every step (its capacity must cover simu_step0 + n_steps).  areas: optional AreaStats
-        that receives the measurement of the state every step starts from (the same capacity rule).  Returns dict(steps,
+        that receives the measurement of the state every step starts from (the same capacity rule); voronoi: optional
+        VoronoiStats that receives that state's Voronoi measures (the same capacity rule).  Returns dict(steps,
         exits (agent ids in exit order), exit_step (0-based step within the call), rc, rng_state (to be set_state()d),
         device_ms, pairs)."""
         N = state["x"].numel()
@@ -581,16 +601,20 @@ class Context:
                 rows_arr[q] = r.data_ptr()
         ex_a, ex_s = np.empty(max(N, 1), dtype=np.int32), np.empty(max(N, 1), dtype=np.int32)
         n_ex, done, ms, pairs = C.c_int(), C.c_int(), C.c_double(), C.c_longlong()
-        vel = None if density is None or density.vel is None else C.byref(density.vel)
-        rc = load().oc_gcfm_run_obs(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]), _dev(state["vx"]),
-                                    _dev(state["vy"]), _dev(state["time"]), _dev(state["status"]), _dev(vdes), _dev(key_id),
-                                    karr, len(karr), key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
-                                    C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
-                                    ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
-                                    C.byref(ms), C.byref(pairs), None if density is None else C.byref(density.acc), vel,
-                                    None if lines is None else C.byref(lines.acc),
-                                    None if areas is None else C.byref(areas.acc),
-                                    _stream() if stream is None else C.c_void_p(stream))
+        obs = Observers()
+        for field, owner, attr in (("density", density, "acc"), ("velocity", density, "vel"), ("lines", lines, "acc"),
+                                   ("areas", areas, "acc"), ("voronoi", voronoi, "acc")):
+            acc = None if owner is None else getattr(owner, attr)
+            if acc is not None:
+                setattr(obs, field, C.pointer(acc))
+        rc = load().oc_gcfm_run_observed(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]),
+                                         _dev(state["vx"]), _dev(state["vy"]), _dev(state["time"]),
+                                         _dev(state["status"]), _dev(vdes), _dev(key_id), karr, len(karr),
+                                         key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
+                                         C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
+                                         ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
+                                         C.byref(ms), C.byref(pairs), C.byref(obs),
+                                         _stream() if stream is None else C.c_void_p(stream))
         check(rc, allow=(OC_ERR_SAMPLER_RANGE,))
         if density is not None:
             density.frames += density.count(simu_step0, done.value)
@@ -668,6 +692,14 @@ class Context:
         check(load().oc_areas_measure(self.h, C.byref(areas.acc), N, P("x"), P("y"), P("vx"), P("vy"), P("status"),
                                       int(step), _stream() if stream is None else C.c_void_p(stream)))
 
+    def voronoi_measure(self, voronoi, state, step, stream=None):
+        """the Voronoi measures of the crowd `state` (the state the step with simu_step `step` starts from) into row
+        `step` of `voronoi` (oc_voronoi_measure)"""
+        N = state["x"].numel()
+        P = (lambda k: None) if N == 0 else (lambda k: _dev(state[k]))
+        check(load().oc_voronoi_measure(self.h, C.byref(voronoi.acc), N, P("x"), P("y"), P("vx"), P("vy"), P("status"),
+                                        int(step), _stream() if stream is None else C.c_void_p(stream)))
+
 
 def density_accum_multi(ctxs, stats, states, stream=None):
     """one density frame per member in one launch per variant (oc_density_accum_vel_multi): member q's crowd `states[q]`
@@ -711,25 +743,36 @@ def lines_count_multi(ctxs, lines, states, steps, stream=None):
                                       _stream() if stream is None else C.c_void_p(stream)))
 
 
+def voronoi_measure_multi(ctxs, voronoi, states, steps, stream=None):
+    """one Voronoi measurement per member in six launches (oc_voronoi_measure_multi): member q's crowd `states[q]`
+    (dict with x, y, vx, vy, status) measured into row steps[q] of voronoi[q]"""
+    _measure_multi(load().oc_voronoi_measure_multi, ctxs, voronoi, states, steps, stream)
+
+
 def areas_measure_multi(ctxs, areas, states, steps, stream=None):
     """one measurement per member in two launches (oc_areas_measure_multi): member q's crowd `states[q]` (dict with x, y,
     vx, vy, status) measured into row steps[q] of areas[q]"""
+    _measure_multi(load().oc_areas_measure_multi, ctxs, areas, states, steps, stream)
+
+
+def _measure_multi(fn, ctxs, accs_, states, steps, stream):
+    """marshal the members of a batched measurement (oc_areas_measure_multi, oc_voronoi_measure_multi) and call fn"""
     n = len(ctxs)
-    if not (len(areas) == len(states) == len(steps) == n and n):
-        raise ValueError("one context, area accumulator, state and step per member expected")
+    if not (len(accs_) == len(states) == len(steps) == n and n):
+        raise ValueError("one context, accumulator, state and step per member expected")
     vp = lambda: (C.c_void_p * n)()
     hs, accs, xs, ys, vxs, vys, sts = vp(), vp(), vp(), vp(), vp(), vp(), vp()
     Ns = np.empty(n, dtype=np.int32)
     ss = np.ascontiguousarray(steps, dtype=np.int32)
-    for q, (c, a, st) in enumerate(zip(ctxs, areas, states)):
+    for q, (c, a, st) in enumerate(zip(ctxs, accs_, states)):
         hs[q] = c.h.value
         accs[q] = C.addressof(a.acc)
         Ns[q] = st["x"].numel()
         if Ns[q]:
             xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
             vxs[q], vys[q] = st["vx"].data_ptr(), st["vy"].data_ptr()
-    check(load().oc_areas_measure_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, vxs, vys, sts, ss.ctypes.data_as(ip),
-                                        _stream() if stream is None else C.c_void_p(stream)))
+    check(fn(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, vxs, vys, sts, ss.ctypes.data_as(ip),
+             _stream() if stream is None else C.c_void_p(stream)))
 
 
 class DensityStats:
@@ -903,6 +946,94 @@ class AreaStats:
     def nbytes(N, n_areas, n_verts, capacity):
         """device bytes of the accumulator of N agents: vertices, per-block scratch and the rows"""
         return 16 * n_verts + 32 * n_areas * max(-(-int(N) // AREA_BLOCK), 1) + 28 * n_areas * max(int(capacity), 1)
+
+
+VORONOI_MAX_BINS = 256          # bins per axis at most (oc_voronoi_acc)
+VORONOI_BIN_MARGIN = 1.0 + 1e-6  # bin side >= 2 * cutoff * margin
+
+
+def voronoi_bins(length, cutoff):
+    """bins along a room side of `length` metres for the Voronoi neighbour search: as many as fit with a side of at
+    least 2 * cutoff * VORONOI_BIN_MARGIN, between 1 and VORONOI_MAX_BINS"""
+    bound = 2.0 * cutoff * VORONOI_BIN_MARGIN
+    nb = int(min(max(length // bound, 1), VORONOI_MAX_BINS))
+    while nb > 1 and length / nb < bound:
+        nb -= 1
+    return nb
+
+
+class VoronoiStats:
+    """Device accumulator of the Voronoi measures of measurement areas (oc_voronoi_acc): per step and area the Voronoi
+    density, speed, velocity and covered fraction (float64 rows (capacity, n_areas, 5), grown by ensure()); the cut-off
+    polygon, the areas' triangles and bounding boxes on the device (uploaded once); the neighbour bins and per-block
+    scratch of a crowd of N agents.  verts / offsets: the areas (simulations.areas_spec); tris: (T, 3, 2)
+    counter-clockwise triangles and tri_offsets (n_areas + 1) (simulations.voronoi_triangles)."""
+
+    def __init__(self, ctx, verts, offsets, tris, tri_offsets, cutoff, edges, N, capacity):
+        import torch
+        self.cutoff, self.edges = float(cutoff), int(edges)
+        self.device = ctx.torch_device
+        offsets = np.asarray(offsets)
+        na = len(offsets) - 1
+        self.n_areas = na
+        k = np.arange(self.edges)
+        ring = np.stack([self.cutoff * np.cos(2 * np.pi * k / self.edges),
+                         self.cutoff * np.sin(2 * np.pi * k / self.edges)], axis=1)
+        tris = np.asarray(tris, dtype=np.float64).reshape(-1, 3, 2)
+        tri_rows = np.concatenate([tris.reshape(-1, 6), tris[:, :, 0].min(1)[:, None], tris[:, :, 0].max(1)[:, None],
+                                   tris[:, :, 1].min(1)[:, None], tris[:, :, 1].max(1)[:, None]], axis=1)
+        info = np.zeros((na, 5))
+        for a in range(na):
+            v = np.asarray(verts[offsets[a]:offsets[a + 1]], dtype=np.float64)
+            info[a] = (v[:, 0].min(), v[:, 0].max(), v[:, 1].min(), v[:, 1].max(), polygon_area(v))
+        self.area = info[:, 4].copy()
+        self.tri_offsets = np.ascontiguousarray(tri_offsets, dtype=np.int32)
+        dev = lambda a, dt=torch.float64: torch.from_numpy(np.ascontiguousarray(a)).to(self.device, dt)
+        self.d_ring, self.d_tris, self.d_info = dev(ring), dev(tri_rows), dev(info)
+        self.d_toff = dev(self.tri_offsets, torch.int32)
+        bx, by = voronoi_bins(ctx.room_length, self.cutoff), voronoi_bins(ctx.room_height, self.cutoff)
+        n = max(int(N), 1)
+        self.bin_count = torch.zeros(bx * by + 1, dtype=torch.int32, device=self.device)
+        self.bin_start = torch.empty(bx * by + 1, dtype=torch.int32, device=self.device)
+        self.slot = torch.empty((n, 2), dtype=torch.int32, device=self.device)
+        self.order = torch.empty(2 * n, dtype=torch.int32, device=self.device)
+        self.partials = torch.empty((max(-(-int(N) // AREA_BLOCK), 1), na, 5), dtype=torch.float64,
+                                    device=self.device)
+        self.rows = torch.zeros((max(int(capacity), 1), na, 5), dtype=torch.float64, device=self.device)
+        self.acc = VoronoiAcc(self.d_ring.data_ptr(), self.d_tris.data_ptr(), self.d_info.data_ptr(),
+                              self.tri_offsets.ctypes.data_as(ip), self.d_toff.data_ptr(), self.bin_count.data_ptr(),
+                              self.bin_start.data_ptr(), self.slot.data_ptr(), self.order.data_ptr(),
+                              self.partials.data_ptr(), self.rows.data_ptr(), self.cutoff, self.edges, na, bx, by,
+                              bx * by + 1, n, self.partials.shape[0], self.rows.shape[0])
+
+    def ensure(self, steps):
+        """grow the rows (on the host: rare) so that steps 0 .. steps-1 fit"""
+        import torch
+        have = self.rows.shape[0]
+        if steps <= have:
+            return
+        torch.cuda.synchronize(self.device)   # (no measurement of the old rows may be in flight on any stream)
+        rows = torch.zeros((max(steps, 2 * have),) + tuple(self.rows.shape[1:]), dtype=torch.float64,
+                           device=self.device)
+        rows[:have] = self.rows
+        torch.cuda.synchronize(self.device)
+        self.rows = rows
+        self.acc.d_rows, self.acc.capacity = rows.data_ptr(), rows.shape[0]
+
+    def result(self, steps):
+        """dict(cutoff, edges, density, speed, covered (steps, n_areas) and velocity (steps, n_areas, 2)), float64; row k
+        = the state the step with simu_step k started from (the caller has synchronised the streams that measured)"""
+        r = self.rows[:steps].cpu().numpy()
+        return dict(cutoff=self.cutoff, edges=self.edges, density=r[:, :, 0].copy(), speed=r[:, :, 1].copy(),
+                    velocity=r[:, :, 2:4].copy(), covered=r[:, :, 4].copy())
+
+    @staticmethod
+    def nbytes(N, n_areas, n_tris, edges, bins, capacity):
+        """device bytes of the accumulator of N agents: cut-off polygon, triangles, area boxes, bins, per-agent and
+        per-block scratch and the rows"""
+        n = max(int(N), 1)
+        return (16 * edges + 80 * n_tris + 44 * n_areas + 4 + 8 * (bins + 1) + 16 * n
+                + 40 * n_areas * max(-(-int(N) // AREA_BLOCK), 1) + 40 * n_areas * max(int(capacity), 1))
 
 
 class GcfmBatch:

@@ -20,6 +20,7 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcompiler",
 UNITS = {  # source -> extra flags
     "oc_api.cu": ["-fmad=false"],
     "oc_gcfm.cu": ["-fmad=false"],
+    "oc_voronoi.cu": ["-fmad=false"],
     "oc_hjb.cu": [],
     "oc_hjb_dist.cu": [],
 }

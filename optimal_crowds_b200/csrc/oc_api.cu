@@ -127,6 +127,10 @@ extern "C" void oc_ctx_destroy(oc_ctx *c) {
     if (c->areas_pinned) cudaFreeHost(c->areas_pinned);
     cudaFree(c->areas_dev);
     if (c->areas_ev) cudaEventDestroy(c->areas_ev);
+    if (c->vor_ev) cudaEventSynchronize(c->vor_ev);
+    if (c->vor_pinned) cudaFreeHost(c->vor_pinned);
+    cudaFree(c->vor_dev);
+    if (c->vor_ev) cudaEventDestroy(c->vor_ev);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->gcfm_pinned) cudaFreeHost(c->gcfm_pinned);
     cudaFree(c->fr_ticket);

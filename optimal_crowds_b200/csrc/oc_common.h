@@ -61,6 +61,9 @@ struct oc_ctx {
     void *areas_pinned = nullptr, *areas_dev = nullptr;  // batched area measurements: member table and offsets
     size_t areas_pinned_bytes = 0, areas_dev_bytes = 0;
     cudaEvent_t areas_ev = nullptr;                      //   recorded after the kernels; the staging is reused after it
+    void *vor_pinned = nullptr, *vor_dev = nullptr;      // batched Voronoi measures: member table
+    size_t vor_pinned_bytes = 0, vor_dev_bytes = 0;
+    cudaEvent_t vor_ev = nullptr;                        //   recorded after the kernels; the staging is reused after it
     int gcfm_poll_ns = 100;    // oc_ctx_set_int("gcfm_poll_ns"): back-off between polls of a neighbour's done-flag
     int gcfm_sweep_ctas = 0;  // oc_ctx_set_int("gcfm_sweep_ctas"): cap of the sweep grid (0 = fill the GPU)
     int gcfm_margin_mm = 250;  // oc_ctx_set_int("gcfm_margin_mm"): displacement margin (2 x per-axis bound) of the fast attempt
@@ -102,6 +105,10 @@ struct oc_ctx {
 
 int oc_dist_allreduce_max_u64(oc_ctx *ctx, void *d_buf, size_t count, cudaStream_t st);  // oc_hjb_dist.cu
 void oc_gcfm_free_launch_state(oc_ctx *ctx);                                               // oc_gcfm.cu
+// oc_voronoi.cu: the accumulator and size checks of a Voronoi measurement (everything but the step), and its launches
+int oc_voronoi_check(const oc_ctx *ctx, const oc_voronoi_acc *a, int N);
+int oc_voronoi_enqueue(oc_ctx *ctx, const oc_voronoi_acc *a, int N, const double *d_x, const double *d_y,
+                       const double *d_vx, const double *d_vy, const uint8_t *d_status, int step, cudaStream_t st);
 
 namespace oc {
 void set_error(const char *fmt, ...);

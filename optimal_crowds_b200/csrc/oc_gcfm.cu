@@ -2482,14 +2482,22 @@ extern "C" int oc_gcfm_step_multi_finish(int n, oc_ctx *const *ctxs, int *const 
 // whose simu_step is a multiple of acc->every (the history frame of that iteration), ahead of the step's randomness;
 // vel (nullable, needs acc): that frame's velocity maps too.  lines (nullable): after every step, once the step is final
 // (oc_gcfm_step_finish), its crossings of the measurement lines are counted in row simu_step of lines->d_counts.
-// areas (nullable): next to the frame, the state the step starts from is measured into row simu_step of its arrays.
-extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
-                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
-                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
-                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
-                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
-                               long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
-                               const oc_lines_acc *lines, const oc_areas_acc *areas, void *stream) {
+// areas (nullable): next to the frame, the state the step starts from is measured into row simu_step of its arrays;
+// voronoi (nullable): the same state's Voronoi measures, right after the areas.  All of them come from obs (nullable).
+extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y,
+                                    double *d_vx, double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes,
+                                    const int *d_key, const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos,
+                                    int *has_gauss, double *cached_gauss, int n_steps, int simu_step0, int n_active0,
+                                    double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
+                                    int *steps_done, double *device_ms, long long *pairs, const oc_observers *obs,
+                                    void *stream) {
+    const oc_observers none{};
+    if (!obs) obs = &none;
+    const oc_density_acc *acc = obs->density;
+    const oc_velocity_acc *vel = obs->velocity;
+    const oc_lines_acc *lines = obs->lines;
+    const oc_areas_acc *areas = obs->areas;
+    const oc_voronoi_acc *voronoi = obs->voronoi;
     OC_ARG(ctx && prm && mt_key && mt_pos && has_gauss && cached_gauss && exit_agent && exit_step && n_exits && steps_done,
            "NULL argument");
     OC_ARG(N >= 1 && n_steps >= 0 && n_active0 >= 0 && n_active0 <= N && *mt_pos >= 0 && *mt_pos <= 624, "bad sizes");
@@ -2509,6 +2517,12 @@ extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
         OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= areas->capacity,
                "measurement areas: step beyond the row capacity");
         OC_ARG((N + AR_BLOCK - 1) / AR_BLOCK <= areas->partial_blocks, "measurement areas: too few partial blocks for N");
+    }
+    if (voronoi) {
+        if (int rc = oc_voronoi_check(ctx, voronoi, N)) return rc;
+        OC_ARG(d_vx && d_vy, "NULL argument");
+        OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= voronoi->capacity,
+               "Voronoi measures: step beyond the row capacity");
     }
     constexpr int N_CKPT = 64;
     *n_exits = 0;
@@ -2532,6 +2546,11 @@ extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
         }
         if (areas) {
             rc = areas_enqueue(ctx, areas, N, d_x, d_y, d_vx, d_vy, d_status, simu_step0 + k, (cudaStream_t)stream);
+            if (rc) return rc;
+        }
+        if (voronoi) {
+            rc = oc_voronoi_enqueue(ctx, voronoi, N, d_x, d_y, d_vx, d_vy, d_status, simu_step0 + k,
+                                    (cudaStream_t)stream);
             if (rc) return rc;
         }
         // ---- this step's randomness (simulations.py:271,303)
@@ -2584,6 +2603,19 @@ extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, do
         if (rc == OC_ERR_SAMPLER_RANGE) return rc;
     }
     return OC_OK;
+}
+
+extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                               double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                               const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                               double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                               int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                               long long *pairs, const oc_density_acc *acc, const oc_velocity_acc *vel,
+                               const oc_lines_acc *lines, const oc_areas_acc *areas, void *stream) {
+    const oc_observers obs{acc, vel, lines, areas, nullptr};
+    return oc_gcfm_run_observed(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys, mt_key,
+                                mt_pos, has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows, exit_agent,
+                                exit_step, n_exits, steps_done, device_ms, pairs, &obs, stream);
 }
 
 extern "C" int oc_gcfm_run_flow(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,

@@ -30,7 +30,10 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     (tests/test_gpu_flow_stats.py);
   * ``areas``: every member measures, at the start of every step, the pedestrians inside each measurement area and the
     sums of their speeds and velocities on the device (one batched ``oc_areas_measure_multi`` call per step for a wave)
-    and hands them back in ``results[i]["areas"]`` (tests/test_gpu_areas.py).
+    and hands them back in ``results[i]["areas"]`` (tests/test_gpu_areas.py);
+  * ``voronoi``: with ``areas``, every member also measures each area's Voronoi density, speed, velocity and covered
+    fraction (one batched ``oc_voronoi_measure_multi`` call per step for a wave, next to the areas' call), handed back in
+    ``results[i]["areas"]["voronoi"]`` (tests/test_gpu_voronoi.py).
 """
 from __future__ import annotations
 
@@ -121,6 +124,9 @@ class ensemble:
     ``areas``: None or {name: [(x0, y0), (x1, y1), ...]} in metres, the same measurement areas for every member, as
     ``simulation(..., areas=...)`` takes them; ``results[i]["areas"]`` is then the member's ``area_stats()`` dict.
 
+    ``voronoi``: None, True or dict(cutoff=1.0, edges=12), as ``simulation(..., voronoi=...)`` takes it (needs ``areas``);
+    ``results[i]["areas"]["voronoi"]`` then holds the member's Voronoi measures.
+
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
     ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
     their rooms may differ in size and number of target sets.
@@ -132,7 +138,7 @@ class ensemble:
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
                  memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None,
-                 density_stats=None, lines=None, areas=None):
+                 density_stats=None, lines=None, areas=None, voronoi=None):
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -158,6 +164,9 @@ class ensemble:
         self.lines = simulations.lines_spec(lines)                            # (names, (n, 4) array) or None
         self._lines_arg = None if self.lines is None else dict(zip(self.lines[0], map(tuple, self.lines[1])))
         self.areas = simulations.areas_spec(areas)                            # (names, vertices, offsets) or None
+        self.voronoi = simulations.voronoi_spec(voronoi)                      # (cutoff, edges) or None
+        if self.voronoi is not None and self.areas is None:
+            raise ValueError("voronoi needs measurement areas (areas=...)")
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -185,8 +194,8 @@ class ensemble:
 
     def member_bytes(self, members=None):
         """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets, plus the
-        density accumulators when density_stats is on, the line accumulator with lines and the area accumulator with
-        areas); no CUDA"""
+        density accumulators when density_stats is on, the line accumulator with lines, the area accumulator with
+        areas and the Voronoi accumulator with voronoi); no CUDA"""
         out = []
         for i in (self.mine if members is None else members):
             room, cfg = self._room(i), self.configs[i]
@@ -201,6 +210,11 @@ class ensemble:
                 b += _lib.LineCounts.nbytes(N, len(self.lines[0]), steps)
             if self.areas is not None:
                 b += _lib.AreaStats.nbytes(N, len(self.areas[0]), len(self.areas[1]), steps)
+            if self.voronoi is not None:
+                cut, edges = self.voronoi
+                bins = _lib.voronoi_bins(room["room_length"], cut) * _lib.voronoi_bins(room["room_height"], cut)
+                n_tris = len(simulations.voronoi_triangles(self.areas)[0])
+                b += _lib.VoronoiStats.nbytes(N, len(self.areas[0]), n_tris, edges, bins, steps)
             out.append(b)
         return out
 
@@ -219,7 +233,7 @@ class ensemble:
                                       density_stats=None if self.density_stats is None else
                                       dict(every=self.density_stats[0], threshold=self.density_stats[1],
                                            velocity=self.density_stats[2]), lines=self._lines_arg,
-                                      areas=self.areas)
+                                      areas=self.areas, voronoi=self.voronoi)
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -374,6 +388,13 @@ class ensemble:
                         _lib.areas_measure_multi([sims[q]._ctx for q in am], [sims[q]._areas for q in am],
                                                  [sims[q]._state for q in am], [sims[q].simu_step for q in am],
                                                  stream=main)
+                    if self.voronoi is not None:
+                        for q in live:
+                            sims[q]._voronoi.ensure(sims[q].simu_step + 1)
+                        if am:
+                            _lib.voronoi_measure_multi([sims[q]._ctx for q in am], [sims[q]._voronoi for q in am],
+                                                       [sims[q]._state for q in am],
+                                                       [sims[q].simu_step for q in am], stream=main)
                 batch.launch(live, [sims[q].inside for q in live], [sims[q].simu_step for q in live], stream=main,
                              rebind=rebind)
                 tl1 = time.perf_counter()
@@ -420,6 +441,8 @@ class ensemble:
                 self.results[i]["lines"] = s._lines.result(s.simu_step)
             if self.areas is not None:
                 self.results[i]["areas"] = s._areas.result(s.simu_step)
+                if self.voronoi is not None:
+                    self.results[i]["areas"]["voronoi"] = s._voronoi.result(s.simu_step)
             if self.record:
                 self.members[i] = s
         self.stats["build_ms"] += (t1 - t0) * 1e3

@@ -160,6 +160,97 @@ def areas_spec(value):
     return AreasSpec((names, np.concatenate(polys), offsets))
 
 
+class VoronoiSpec(tuple):
+    """(cutoff, edges): a checked ``voronoi`` argument"""
+
+
+def voronoi_spec(value):
+    """VoronoiSpec (cutoff in metres, edges of the cut-off polygon) of a ``voronoi`` argument -- True (cutoff=1.0,
+    edges=12) or dict(cutoff=..., edges=...): cutoff finite in (0, 100], edges an integer in 4..32 -- or None for None
+    and False; checked without touching a GPU.  A VoronoiSpec is returned as it is"""
+    if value is None or value is False or isinstance(value, VoronoiSpec):
+        return value if value is not False else None
+    if value is True:
+        value = {}
+    if not isinstance(value, dict):
+        raise ValueError("voronoi: expected True or dict(cutoff=1.0, edges=12)")
+    unknown = set(value) - {"cutoff", "edges"}
+    if unknown:
+        raise ValueError(f"voronoi: unknown keys {sorted(map(str, unknown))}")
+    cutoff, edges = value.get("cutoff", 1.0), value.get("edges", 12)
+    if isinstance(cutoff, (bool, np.bool_)) or not isinstance(cutoff, (int, float, np.integer, np.floating)) or \
+            not (np.isfinite(cutoff) and 0 < cutoff <= 100):
+        raise ValueError("voronoi: cutoff must be a finite number of metres in (0, 100]")
+    if isinstance(edges, (bool, np.bool_)) or not isinstance(edges, (int, np.integer)) or not 4 <= edges <= 32:
+        raise ValueError("voronoi: edges must be an integer in 4..32")
+    return VoronoiSpec((float(cutoff), int(edges)))
+
+
+def _turn(a, b, c):
+    """orientation of the corner a -> b -> c: > 0 for a left (counter-clockwise) turn, 0 when collinear"""
+    return (b[0] - a[0]) * (c[1] - b[1]) - (b[1] - a[1]) * (c[0] - b[0])
+
+
+def _drop_straight(pts):
+    """drop vertices whose turn is exactly zero, one at a time from the front, until none is left"""
+    k = 0
+    while len(pts) > 3 and k < len(pts):
+        if _turn(pts[k - 1], pts[k], pts[(k + 1) % len(pts)]) == 0:
+            del pts[k]
+            k = 0
+        else:
+            k += 1
+    return pts
+
+
+def _triangulate(v):
+    """counter-clockwise triangles covering the simple polygon v ((n, 2)), by ear clipping: the polygon turned
+    counter-clockwise, vertices with a zero turn dropped (again after every ear); the ear is the first vertex, in the
+    current order, with a left turn whose triangle holds no other vertex (closed triangle; if no vertex qualifies, open)"""
+    pts = [(float(x), float(y)) for x, y in v]
+    if sum(a[0] * b[1] - b[0] * a[1] for a, b in zip(pts, pts[1:] + pts[:1])) < 0:
+        pts.reverse()
+    pts = _drop_straight(pts)
+    tris = []
+
+    def holds(a, b, c, p, closed):
+        o = (_turn(a, b, p), _turn(b, c, p), _turn(c, a, p))   # (sign of o(a,b,p) etc. for a counter-clockwise a, b, c)
+        return all(t >= 0 for t in o) if closed else all(t > 0 for t in o)
+
+    while len(pts) > 3:
+        n, ear = len(pts), None
+        for closed in (True, False):
+            for k in range(n):
+                a, b, c = pts[k - 1], pts[k], pts[(k + 1) % n]
+                if _turn(a, b, c) <= 0:
+                    continue
+                if not any(holds(a, b, c, pts[j], closed) for j in range(n) if j not in ((k - 1) % n, k, (k + 1) % n)):
+                    ear = k
+                    break
+            if ear is not None:
+                break
+        if ear is None:
+            raise ValueError("areas: a polygon could not be triangulated")
+        tris.append((pts[ear - 1], pts[ear], pts[(ear + 1) % n]))
+        del pts[ear]
+        pts = _drop_straight(pts)
+    tris.append(tuple(pts))
+    return tris
+
+
+def voronoi_triangles(aspec):
+    """(T, 3, 2) float64 counter-clockwise triangles of the areas of an AreasSpec, area after area in a fixed order,
+    and (n_areas + 1) int32 offsets into them; computed once per AreasSpec"""
+    cached = getattr(aspec, "_triangles", None)
+    if cached is None:
+        names, verts, offsets = aspec
+        per = [_triangulate(verts[a:b]) for a, b in zip(offsets[:-1], offsets[1:])]
+        tris = np.array([t for p in per for t in p], dtype=np.float64).reshape(-1, 3, 2)
+        toff = np.concatenate([[0], np.cumsum([len(p) for p in per])]).astype(np.int32)
+        cached = aspec._triangles = (tris, toff)
+    return cached
+
+
 def density_frame_steps(T, dt, every, recompute_step=None):
     """The simu_steps whose frames run() adds to the density statistics when nobody leaves before T: run()'s loop
     (simulations.py:427-441) as it is cut into blocks here -- one advance() per stretch up to the next re-solve (every
@@ -283,7 +374,7 @@ class simulation:
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
                  rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, lines=None,
-                 areas=None, _ctx=None):
+                 areas=None, voronoi=None, _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -307,11 +398,21 @@ class simulation:
         its right; read them with ``line_counts()``.  Not available with ``band`` or ``shard_keys``), ``areas`` ({name:
         [(x0, y0), (x1, y1), ...]} in metres, at most 64 simple polygons of 3 to 64 vertices, 1024 in all: measure on
         the device, at the start of every step, the pedestrians inside each polygon and the sums of their speeds and
-        velocities; read them with ``area_stats()``.  Not available with ``band`` or ``shard_keys``)."""
+        velocities; read them with ``area_stats()``.  Not available with ``band`` or ``shard_keys``), ``voronoi`` (True
+        = dict(cutoff=1.0, edges=12), needs ``areas``: measure also, at the start of every step, each area's Voronoi
+        density, speed and velocity and the fraction of it the cells cover (Steffen & Seyfried's method D; cells are
+        bounded by the room rectangle and a polygon of ``edges`` vertices at ``cutoff`` metres from the agent, not by
+        internal walls); ``area_stats()["voronoi"]`` returns them.  Not available with ``band`` or ``shard_keys``)."""
         import torch
         dstats = density_stats_spec(density_stats, with_velocity=True)
         lspec = lines_spec(lines)
         aspec = areas_spec(areas)
+        vspec = voronoi_spec(voronoi)
+        if vspec is not None and (band or shard_keys):
+            raise ValueError("voronoi is not available for row-decomposed (band=True) or key-sharded "
+                             "(shard_keys=True) runs")
+        if vspec is not None and aspec is None:
+            raise ValueError("voronoi needs measurement areas (areas=...)")
         if aspec is not None and (band or shard_keys):
             raise ValueError("areas are not available for row-decomposed (band=True) or key-sharded "
                              "(shard_keys=True) runs")
@@ -456,6 +557,9 @@ class simulation:
                                                                  len(density_frame_steps(T, self.dt, 1)))
         # measurement areas (written before every step by oc_areas_measure* / oc_gcfm_run_obs), rows sized as the lines'
         self._areas = None if aspec is None else _lib.AreaStats(ctx, *aspec, N, len(density_frame_steps(T, self.dt, 1)))
+        # their Voronoi measures (oc_voronoi_measure* / oc_gcfm_run_observed, right after the areas), rows sized alike
+        self._voronoi = None if vspec is None else _lib.VoronoiStats(ctx, aspec[1], aspec[2], *voronoi_triangles(aspec),
+                                                                     *vspec, N, self._areas.count.shape[0])
         # per-step record of (x, y, vx, vy); row k = state after k steps (ped.traj / ped.vels / history views).  It
         # lives on the DEVICE in blocks of TRACK_CHUNK steps, written by one small kernel per step (oc_state_pack), and
         # is read back -- once per row -- only when somebody looks at it
@@ -624,12 +728,12 @@ class simulation:
                                                  device=self._ctx.torch_device))
             rows.append(self._d_track[blk][off])
         n_active = int(self._h_status.sum())
-        for acc in (self._lines, self._areas):
+        for acc in (self._lines, self._areas, self._voronoi):
             if acc is not None:
                 acc.ensure(self.simu_step + n_steps)
         res = self._ctx.gcfm_run(self._gcfm_prm, self._state, self._d_vdes, self._d_key, self._keys(), st, n_steps,
                                  self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats,
-                                 lines=self._lines, areas=self._areas)
+                                 lines=self._lines, areas=self._areas, voronoi=self._voronoi)
         self._rng.rng.set_state(res["rng_state"])
         self.last_run_stats = dict(steps=res["steps"], device_ms=res["device_ms"], pairs=res["pairs"])
         ex, exs = res["exits"], res["exit_step"]
@@ -687,22 +791,32 @@ class simulation:
 
     def _measure_areas(self):
         """measure the state this step starts from into row simu_step of the measurement areas (before the step's
-        randomness; a crowd without agents keeps the zero row)"""
+        randomness; a crowd without agents keeps the zero row), and its Voronoi measures when they are on"""
         if self._areas is not None:
             self._areas.ensure(self.simu_step + 1)
             if self.N > 0:
                 self._ctx.areas_measure(self._areas, self._state, self.simu_step, stream=self._cuda_stream)
+        if self._voronoi is not None:
+            self._voronoi.ensure(self.simu_step + 1)
+            if self.N > 0:
+                self._ctx.voronoi_measure(self._voronoi, self._state, self.simu_step, stream=self._cuda_stream)
 
     def area_stats(self):
         """the measurement areas (``areas=`` of the constructor) of the steps taken so far: dict(names, area, count,
         speed_sum, vx_sum, vy_sum, density, speed, velocity) -- (simu_step, n_areas) arrays (velocity: (simu_step,
         n_areas, 2)), row k = the state the step with simu_step k started from; ``speed`` and ``velocity`` are NaN where
-        nobody is inside"""
+        nobody is inside.  With ``voronoi`` also "voronoi": dict(cutoff, edges, density, speed, covered (simu_step,
+        n_areas) and velocity (simu_step, n_areas, 2)): per area sum(w/|V|) / area, sum(w*speed) / area, sum(w*(vx, vy))
+        / area and sum(w) / area over the agents' Voronoi cells V, w the part of V inside the area
+        (include/optimal_crowds.h, oc_voronoi_acc)"""
         if self._areas is None:
             raise RuntimeError("this simulation was created without areas")
         import torch
         torch.cuda.synchronize(self._ctx.torch_device)
-        return self._areas.result(self.simu_step)
+        out = self._areas.result(self.simu_step)
+        if self._voronoi is not None:
+            out["voronoi"] = self._voronoi.result(self.simu_step)
+        return out
 
     def _step_finish(self, launched, verbose=False):
         dt, pending = launched
