@@ -588,6 +588,58 @@ int oc_voronoi_measure_multi(int n, oc_ctx *const *ctxs, const oc_voronoi_acc *c
                              const double *const *x, const double *const *y, const double *const *vx,
                              const double *const *vy, const uint8_t *const *status, const int *steps, void *stream);
 
+/* Voronoi maps: per grid node, statistics of the Voronoi density 1/|V_i| and velocity of the pedestrian whose cell
+ * holds the node (Steffen & Seyfried's method D as a field; jpsreport's profiles), accumulated over frames like the
+ * density statistics.  FP64 without contraction, o and the symbols as for oc_voronoi_acc; r = cutoff.
+ *  1. Generators, ring and the cell V_i are rules 1-5 of oc_voronoi_acc, unchanged; every generator gets its cell.
+ *  2. A node is p = (X[ix], Y[iy]), the context's node coordinates the density uses.  Nodes where d_Vglobal < 0 are
+ *     walls: never covered, all their terms 0.
+ *  3. Owner: for each generator j, d2_j = (X-x_j)*(X-x_j) + (Y-y_j)*(Y-y_j); among those with d2_j <= r*r the one with
+ *     the smallest d2_j, the lowest index on ties.  With none, p is uncovered.
+ *  4. p must lie in the owner's cut-off polygon: o(a_k, a_{k+1}, p) >= 0 for every ring edge, a_k = (x_i + ox[k],
+ *     y_i + oy[k]), a_n = a_0.  Otherwise p is uncovered.
+ *  5. A covered node takes rho = 1/|V_i|, s_i = sqrt(vx*vx + vy*vy), vx_i and vy_i.  |V_i| <= 0 makes it uncovered;
+ *     |V_i| NaN (an overflowed cell) leaves it covered with all four terms NaN.
+ *  6. Per frame and node, in this order: d_density_sum += rho; d_density_max = np.maximum(d_density_max, rho) with
+ *     rho = 0 when uncovered (the first NaN wins); d_covered += 1; d_speed_sum += s, d_vx_sum += vx, d_vy_sum += vy.
+ *     Nothing but d_density_max changes at an uncovered node.
+ * Consequences: of coincident generators the lower index owns the nodes (in the area measures both cells count); and
+ * ownership is decided by distances while |V_i| is decided by the clip, which agree up to rounding on cell boundaries.
+ * Cells are not clipped by internal walls, holes or cylinders.  Neighbour search as oc_voronoi_acc: the bins hold every
+ * generator within r of a node in the 3x3 bins around the node's bin.  A frame is six launches: bin, scan, place,
+ * sort, the cells' areas into d_vol (one thread per generator), and the nodes (tiles of 32 x 8). */
+typedef struct {
+    double *d_density_sum, *d_density_max;   /* float64 (Ny, Nx) of the context's grid */
+    int *d_covered;                           /* int32 (Ny, Nx): frames in which the node lay in a cell */
+    double *d_speed_sum, *d_vx_sum, *d_vy_sum;   /* float64 (Ny, Nx), sums over the covered frames */
+    const double *d_Vglobal;     /* simulation.V: nodes where it is < 0 are walls */
+    const double *d_ring;        /* (edges, 2): ox, oy of oc_voronoi_acc's rule 2 */
+    int *d_bin_count;            /* int32 (bin_capacity): zero before the first frame, left zero by every one */
+    int *d_bin_start;            /* int32 (bin_capacity) */
+    int *d_slot;                 /* int32 (agent_capacity, 2) */
+    int *d_order;                /* int32 (2 * agent_capacity) */
+    double *d_vol;               /* float64 (agent_capacity): |V_i| of the frame */
+    double cutoff;               /* r: finite, in (0, 100] metres */
+    int edges;                   /* 4..32 */
+    int every;                   /* >= 1: run loops take a frame before the steps whose simu_step is a multiple of it */
+    int bins_x, bins_y;          /* as oc_voronoi_acc */
+    int bin_capacity;            /* >= bins_x * bins_y + 1 */
+    int agent_capacity;          /* >= N */
+} oc_vormap_acc;
+/* Adds one frame of the crowd (N agents; NULL arrays allowed when N = 0) to acc.  Asynchronous on stream.  The
+ * accumulators are caller-owned and initialised by the caller (zeros).  OC_ERR_ARG, before any launch, for a NULL
+ * required pointer, a cutoff that is not finite or outside (0, 100], edges outside 4..32, every < 1, bins too small or
+ * too many and too small an agent capacity for N. */
+int oc_vormap_accum(oc_ctx *ctx, const oc_vormap_acc *acc, int N, const double *d_x, const double *d_y,
+                    const double *d_vx, const double *d_vy, const uint8_t *d_status, void *stream);
+/* oc_vormap_accum for each of n members in six launches; ctxs[0] owns the member tables.  Members may differ in grid
+ * shape, crowd size (0 included), cutoff, edges and bins; each result equals the member's oc_vormap_accum alone.
+ * OC_ERR_ARG as oc_vormap_accum, for a member context on another device than ctxs[0] and for two members sharing a
+ * bin, scratch or accumulator buffer. */
+int oc_vormap_accum_multi(int n, oc_ctx *const *ctxs, const oc_vormap_acc *const *accs, const int *Ns,
+                          const double *const *x, const double *const *y, const double *const *vx,
+                          const double *const *vy, const uint8_t *const *status, void *stream);
+
 /* The observers of a run loop, each nullable: density frames (acc) and their velocity maps (vel, needs acc), line
  * counts, measurement areas and their Voronoi measures. */
 typedef struct {
@@ -597,16 +649,25 @@ typedef struct {
     const oc_areas_acc *areas;
     const oc_voronoi_acc *voronoi;
 } oc_observers;
-/* The run loop's only implementation: oc_gcfm_run_flow plus the measurement areas and their Voronoi measures (obs: every
- * pointer nullable; obs itself nullable): before step k, next to the density frame and ahead of the step's randomness,
- * the state the step starts from is measured into row simu_step0 + k.  simu_step0 + n_steps must not exceed the
- * capacity of the areas' and the Voronoi rows, checked before any step.  oc_gcfm_run_obs forwards here. */
+/* oc_gcfm_run_flow plus the measurement areas and their Voronoi measures (obs: every pointer nullable; obs itself
+ * nullable): before step k, next to the density frame and ahead of the step's randomness, the state the step starts
+ * from is measured into row simu_step0 + k.  simu_step0 + n_steps must not exceed the capacity of the areas' and the
+ * Voronoi rows, checked before any step.  oc_gcfm_run_obs forwards here; this forwards to oc_gcfm_run_observed_maps. */
 int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
                          double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
                          const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
                          double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
                          int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
                          long long *pairs, const oc_observers *obs, void *stream);
+/* The run loop's only implementation: oc_gcfm_run_observed plus Voronoi maps (maps, nullable): before the steps whose
+ * simu_step is a multiple of maps->every, next to the density frame and ahead of the step's randomness, a frame of the
+ * state the step starts from is added to maps.  maps is checked before any step.  oc_gcfm_run_observed forwards here. */
+int oc_gcfm_run_observed_maps(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,
+                              double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key,
+                              const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos, int *has_gauss,
+                              double *cached_gauss, int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                              int *exit_agent, int *exit_step, int *n_exits, int *steps_done, double *device_ms,
+                              long long *pairs, const oc_observers *obs, const oc_vormap_acc *maps, void *stream);
 /* oc_gcfm_run_flow plus the measurement areas (areas, nullable): forwards to oc_gcfm_run_observed. */
 int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx, double *d_vy,
                     double *d_time, uint8_t *d_status, const double *d_vdes, const int *d_key, const oc_key *keys,

@@ -113,6 +113,15 @@ class VoronoiAcc(C.Structure):
                 ("partial_blocks", C.c_int), ("capacity", C.c_int)]
 
 
+class VormapAcc(C.Structure):
+    _fields_ = [("d_density_sum", C.c_void_p), ("d_density_max", C.c_void_p), ("d_covered", C.c_void_p),
+                ("d_speed_sum", C.c_void_p), ("d_vx_sum", C.c_void_p), ("d_vy_sum", C.c_void_p),
+                ("d_Vglobal", C.c_void_p), ("d_ring", C.c_void_p), ("d_bin_count", C.c_void_p),
+                ("d_bin_start", C.c_void_p), ("d_slot", C.c_void_p), ("d_order", C.c_void_p), ("d_vol", C.c_void_p),
+                ("cutoff", C.c_double), ("edges", C.c_int), ("every", C.c_int), ("bins_x", C.c_int),
+                ("bins_y", C.c_int), ("bin_capacity", C.c_int), ("agent_capacity", C.c_int)]
+
+
 class Observers(C.Structure):
     _fields_ = [("density", C.POINTER(DensityAcc)), ("velocity", C.POINTER(VelocityAcc)),
                 ("lines", C.POINTER(LinesAcc)), ("areas", C.POINTER(AreasAcc)), ("voronoi", C.POINTER(VoronoiAcc))]
@@ -128,7 +137,8 @@ EXPORTS = ["oc_abi_version", "oc_last_error", "oc_launch_count", "oc_ctx_create"
            "oc_gcfm_run_acc", "oc_density_accum", "oc_density_accum_multi", "oc_density_accum_vel",
            "oc_density_accum_vel_multi", "oc_lines_count", "oc_lines_count_multi", "oc_gcfm_run_flow",
            "oc_areas_measure", "oc_areas_measure_multi", "oc_gcfm_run_obs",
-           "oc_voronoi_measure", "oc_voronoi_measure_multi", "oc_gcfm_run_observed"]
+           "oc_voronoi_measure", "oc_voronoi_measure_multi", "oc_gcfm_run_observed",
+           "oc_vormap_accum", "oc_vormap_accum_multi", "oc_gcfm_run_observed_maps"]
 
 
 def load():
@@ -170,6 +180,10 @@ def load():
     lib.oc_lines_count_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, ip, C.c_void_p]
     lib.oc_gcfm_run_obs.argtypes = lib.oc_gcfm_run_flow.argtypes[:-1] + [C.POINTER(AreasAcc), C.c_void_p]
     lib.oc_gcfm_run_observed.argtypes = lib.oc_gcfm_run_acc.argtypes[:-2] + [C.POINTER(Observers), C.c_void_p]
+    lib.oc_gcfm_run_observed_maps.argtypes = lib.oc_gcfm_run_observed.argtypes[:-1] + [C.POINTER(VormapAcc),
+                                                                                     C.c_void_p]
+    lib.oc_vormap_accum.argtypes = [C.c_void_p, C.POINTER(VormapAcc), C.c_int] + [C.c_void_p] * 6
+    lib.oc_vormap_accum_multi.argtypes = [C.c_int, vpp_, vpp_, ip, vpp_, vpp_, vpp_, vpp_, vpp_, C.c_void_p]
     lib.oc_voronoi_measure.argtypes = [C.c_void_p, C.POINTER(VoronoiAcc), C.c_int] + [C.c_void_p] * 5 + [C.c_int,
                                                                                                        C.c_void_p]
     lib.oc_voronoi_measure_multi.argtypes = lib.oc_areas_measure_multi.argtypes
@@ -579,14 +593,15 @@ class Context:
         return exit_log[: n_exit.value].copy(), rc
 
     def gcfm_run(self, prm: GcfmParams, state, vdes, key_id, keys, rng_state, n_steps, simu_step0, n_active, rows=None,
-                 stream=None, density=None, lines=None, areas=None, voronoi=None):
+                 stream=None, density=None, lines=None, areas=None, voronoi=None, maps=None):
         """up to n_steps steps of the run loop in one call (oc_gcfm_run_observed): randomness drawn in C from the legacy MT19937
         state tuple `rng_state` (np.random.get_state()), next step's draws overlapped with the GPU.  rows: optional list of
         n_steps (N,4) CUDA tensors receiving the packed state after each step.  density: optional DensityStats that
         receives the frame of every due step (with its velocity maps when it has them).  lines: optional LineCounts that
         receives the crossings of every step (its capacity must cover simu_step0 + n_steps).  areas: optional AreaStats
         that receives the measurement of the state every step starts from (the same capacity rule); voronoi: optional
-        VoronoiStats that receives that state's Voronoi measures (the same capacity rule).  Returns dict(steps,
+        VoronoiStats that receives that state's Voronoi measures (the same capacity rule); maps: optional VoronoiMaps
+        that receives a frame before every due step.  Returns dict(steps,
         exits (agent ids in exit order), exit_step (0-based step within the call), rc, rng_state (to be set_state()d),
         device_ms, pairs)."""
         N = state["x"].numel()
@@ -607,17 +622,19 @@ class Context:
             acc = None if owner is None else getattr(owner, attr)
             if acc is not None:
                 setattr(obs, field, C.pointer(acc))
-        rc = load().oc_gcfm_run_observed(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]),
+        rc = load().oc_gcfm_run_observed_maps(self.h, C.byref(prm), N, _dev(state["x"]), _dev(state["y"]),
                                          _dev(state["vx"]), _dev(state["vy"]), _dev(state["time"]),
                                          _dev(state["status"]), _dev(vdes), _dev(key_id), karr, len(karr),
                                          key.ctypes.data_as(C.POINTER(C.c_uint32)), C.byref(pos), C.byref(has),
                                          C.byref(cached), int(n_steps), int(simu_step0), int(n_active), rows_arr,
                                          ex_a.ctypes.data_as(ip), ex_s.ctypes.data_as(ip), C.byref(n_ex), C.byref(done),
                                          C.byref(ms), C.byref(pairs), C.byref(obs),
+                                         None if maps is None else C.byref(maps.acc),
                                          _stream() if stream is None else C.c_void_p(stream))
         check(rc, allow=(OC_ERR_SAMPLER_RANGE,))
-        if density is not None:
-            density.frames += density.count(simu_step0, done.value)
+        for acc in (density, maps):
+            if acc is not None:
+                acc.frames += acc.count(simu_step0, done.value)
         return dict(steps=done.value, exits=ex_a[: n_ex.value].copy(), exit_step=ex_s[: n_ex.value].copy(), rc=rc,
                     rng_state=("MT19937", key, pos.value, has.value, cached.value), device_ms=ms.value, pairs=pairs.value)
 
@@ -699,6 +716,37 @@ class Context:
         P = (lambda k: None) if N == 0 else (lambda k: _dev(state[k]))
         check(load().oc_voronoi_measure(self.h, C.byref(voronoi.acc), N, P("x"), P("y"), P("vx"), P("vy"), P("status"),
                                         int(step), _stream() if stream is None else C.c_void_p(stream)))
+
+
+    def vormap_accum(self, maps, state, stream=None):
+        """add the Voronoi map frame of the crowd `state` (dict with x, y, vx, vy, status) to `maps` (oc_vormap_accum)"""
+        N = state["x"].numel()
+        P = (lambda k: None) if N == 0 else (lambda k: _dev(state[k]))
+        check(load().oc_vormap_accum(self.h, C.byref(maps.acc), N, P("x"), P("y"), P("vx"), P("vy"), P("status"),
+                                     _stream() if stream is None else C.c_void_p(stream)))
+        maps.frames += 1
+
+
+def vormap_accum_multi(ctxs, maps, states, stream=None):
+    """one Voronoi map frame per member in six launches (oc_vormap_accum_multi): member q's crowd `states[q]` (dict with
+    x, y, vx, vy, status) on the grid of ctxs[q], added to maps[q]"""
+    n = len(ctxs)
+    if not (len(maps) == len(states) == n and n):
+        raise ValueError("one context, map accumulator and state per member expected")
+    vp = lambda: (C.c_void_p * n)()
+    hs, accs, xs, ys, vxs, vys, sts = vp(), vp(), vp(), vp(), vp(), vp(), vp()
+    Ns = np.empty(n, dtype=np.int32)
+    for q, (c, a, st) in enumerate(zip(ctxs, maps, states)):
+        hs[q] = c.h.value
+        accs[q] = C.addressof(a.acc)
+        Ns[q] = st["x"].numel()
+        if Ns[q]:
+            xs[q], ys[q], sts[q] = st["x"].data_ptr(), st["y"].data_ptr(), st["status"].data_ptr()
+            vxs[q], vys[q] = st["vx"].data_ptr(), st["vy"].data_ptr()
+    check(load().oc_vormap_accum_multi(n, hs, accs, Ns.ctypes.data_as(ip), xs, ys, vxs, vys, sts,
+                                       _stream() if stream is None else C.c_void_p(stream)))
+    for a in maps:
+        a.frames += 1
 
 
 def density_accum_multi(ctxs, stats, states, stream=None):
@@ -1034,6 +1082,68 @@ class VoronoiStats:
         n = max(int(N), 1)
         return (16 * edges + 80 * n_tris + 44 * n_areas + 4 + 8 * (bins + 1) + 16 * n
                 + 40 * n_areas * max(-(-int(N) // AREA_BLOCK), 1) + 40 * n_areas * max(int(capacity), 1))
+
+
+class VoronoiMaps:
+    """Device accumulators of a run's Voronoi maps (oc_vormap_acc): per node of the (Ny, Nx) grid the sum and the maximum
+    of the Voronoi density 1/|V|, the number of frames in which the node lay in a cell (int32), and the sums of the
+    owner's speed, vx and vy over those frames (float64); zero at creation.  Vglobal: the run's simulation.V on the
+    device; every: frames are taken at the steps whose simu_step is a multiple of it; N: the crowd size (per-agent
+    scratch: bins, order, cell areas)."""
+
+    def __init__(self, ctx, Vglobal, cutoff=1.0, edges=12, every=1, N=0):
+        import torch
+        self.cutoff, self.edges, self.every, self.frames = float(cutoff), int(edges), int(every), 0
+        dev = ctx.torch_device
+        shape = (ctx.Ny, ctx.Nx)
+        self.density_sum, self.density_max, self.speed_sum, self.vx_sum, self.vy_sum = (
+            torch.zeros(shape, dtype=torch.float64, device=dev) for _ in range(5))
+        self.covered = torch.zeros(shape, dtype=torch.int32, device=dev)
+        self.Vglobal = Vglobal
+        k = np.arange(self.edges)
+        ring = np.stack([self.cutoff * np.cos(2 * np.pi * k / self.edges),
+                         self.cutoff * np.sin(2 * np.pi * k / self.edges)], axis=1)   # as VoronoiStats
+        self.d_ring = torch.from_numpy(np.ascontiguousarray(ring)).to(dev)
+        bx, by = voronoi_bins(ctx.room_length, self.cutoff), voronoi_bins(ctx.room_height, self.cutoff)
+        n = max(int(N), 1)
+        self.bin_count = torch.zeros(bx * by + 1, dtype=torch.int32, device=dev)
+        self.bin_start = torch.empty(bx * by + 1, dtype=torch.int32, device=dev)
+        self.slot = torch.empty((n, 2), dtype=torch.int32, device=dev)
+        self.order = torch.empty(2 * n, dtype=torch.int32, device=dev)
+        self.vol = torch.empty(n, dtype=torch.float64, device=dev)
+        self.acc = VormapAcc(self.density_sum.data_ptr(), self.density_max.data_ptr(), self.covered.data_ptr(),
+                             self.speed_sum.data_ptr(), self.vx_sum.data_ptr(), self.vy_sum.data_ptr(),
+                             Vglobal.data_ptr(), self.d_ring.data_ptr(), self.bin_count.data_ptr(),
+                             self.bin_start.data_ptr(), self.slot.data_ptr(), self.order.data_ptr(),
+                             self.vol.data_ptr(), self.cutoff, self.edges, self.every, bx, by, bx * by + 1, n)
+
+    def due(self, simu_step):
+        return simu_step % self.every == 0
+
+    def count(self, simu_step0, steps):
+        """frames taken by `steps` consecutive steps from simu_step0"""
+        return sum(1 for k in range(simu_step0, simu_step0 + steps) if k % self.every == 0)
+
+    def result(self):
+        """dict(cutoff, edges, frames, density_sum, density_max, covered, speed_sum, vx_sum, vy_sum and the means
+        density = density_sum / frames (None without frames), speed = speed_sum / covered and velocity = (vx_sum,
+        vy_sum) / covered (Ny, Nx, 2), NaN where covered == 0), read back from the device (the caller has synchronised
+        the streams that added frames)"""
+        ds, cov = self.density_sum.cpu().numpy(), self.covered.cpu().numpy()
+        sp, vx, vy = self.speed_sum.cpu().numpy(), self.vx_sum.cpu().numpy(), self.vy_sum.cpu().numpy()
+        zero = cov == 0
+        with np.errstate(divide="ignore", invalid="ignore"):
+            mean = lambda a: np.where(zero, np.nan, a / np.where(zero, 1, cov))
+            return dict(cutoff=self.cutoff, edges=self.edges, frames=self.frames, density_sum=ds,
+                        density_max=self.density_max.cpu().numpy(), covered=cov, speed_sum=sp, vx_sum=vx, vy_sum=vy,
+                        density=ds / self.frames if self.frames else None, speed=mean(sp),
+                        velocity=np.stack([mean(vx), mean(vy)], axis=-1))
+
+    @staticmethod
+    def nbytes(Ny, Nx, N, edges, bins):
+        """device bytes of the accumulator of an (Ny, Nx) grid and N agents: 5 float64 and 1 int32 per node, the
+        cut-off polygon, the bins and 24 bytes of per-agent scratch (slot, order, cell area)"""
+        return 44 * Ny * Nx + 16 * edges + 8 * (bins + 1) + 24 * max(int(N), 1)
 
 
 class GcfmBatch:

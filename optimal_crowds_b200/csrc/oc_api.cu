@@ -131,6 +131,10 @@ extern "C" void oc_ctx_destroy(oc_ctx *c) {
     if (c->vor_pinned) cudaFreeHost(c->vor_pinned);
     cudaFree(c->vor_dev);
     if (c->vor_ev) cudaEventDestroy(c->vor_ev);
+    if (c->vmap_ev) cudaEventSynchronize(c->vmap_ev);
+    if (c->vmap_pinned) cudaFreeHost(c->vmap_pinned);
+    cudaFree(c->vmap_dev);
+    if (c->vmap_ev) cudaEventDestroy(c->vmap_ev);
     if (c->h_pinned) cudaFreeHost(c->h_pinned);
     if (c->gcfm_pinned) cudaFreeHost(c->gcfm_pinned);
     cudaFree(c->fr_ticket);

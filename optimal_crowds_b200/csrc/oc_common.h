@@ -64,6 +64,9 @@ struct oc_ctx {
     void *vor_pinned = nullptr, *vor_dev = nullptr;      // batched Voronoi measures: member table
     size_t vor_pinned_bytes = 0, vor_dev_bytes = 0;
     cudaEvent_t vor_ev = nullptr;                        //   recorded after the kernels; the staging is reused after it
+    void *vmap_pinned = nullptr, *vmap_dev = nullptr;    // batched Voronoi maps: member tables
+    size_t vmap_pinned_bytes = 0, vmap_dev_bytes = 0;
+    cudaEvent_t vmap_ev = nullptr;                       //   recorded after the kernels; the staging is reused after it
     int gcfm_poll_ns = 100;    // oc_ctx_set_int("gcfm_poll_ns"): back-off between polls of a neighbour's done-flag
     int gcfm_sweep_ctas = 0;  // oc_ctx_set_int("gcfm_sweep_ctas"): cap of the sweep grid (0 = fill the GPU)
     int gcfm_margin_mm = 250;  // oc_ctx_set_int("gcfm_margin_mm"): displacement margin (2 x per-axis bound) of the fast attempt
@@ -109,6 +112,10 @@ void oc_gcfm_free_launch_state(oc_ctx *ctx);                                    
 int oc_voronoi_check(const oc_ctx *ctx, const oc_voronoi_acc *a, int N);
 int oc_voronoi_enqueue(oc_ctx *ctx, const oc_voronoi_acc *a, int N, const double *d_x, const double *d_y,
                        const double *d_vx, const double *d_vy, const uint8_t *d_status, int step, cudaStream_t st);
+// oc_voronoi.cu: the accumulator and size checks of a Voronoi map frame, and its launches
+int oc_vormap_check(const oc_ctx *ctx, const oc_vormap_acc *a, int N);
+int oc_vormap_enqueue(oc_ctx *ctx, const oc_vormap_acc *a, int N, const double *d_x, const double *d_y,
+                      const double *d_vx, const double *d_vy, const uint8_t *d_status, cudaStream_t st);
 
 namespace oc {
 void set_error(const char *fmt, ...);

@@ -2484,13 +2484,16 @@ extern "C" int oc_gcfm_step_multi_finish(int n, oc_ctx *const *ctxs, int *const 
 // (oc_gcfm_step_finish), its crossings of the measurement lines are counted in row simu_step of lines->d_counts.
 // areas (nullable): next to the frame, the state the step starts from is measured into row simu_step of its arrays;
 // voronoi (nullable): the same state's Voronoi measures, right after the areas.  All of them come from obs (nullable).
-extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y,
-                                    double *d_vx, double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes,
-                                    const int *d_key, const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos,
-                                    int *has_gauss, double *cached_gauss, int n_steps, int simu_step0, int n_active0,
-                                    double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
-                                    int *steps_done, double *device_ms, long long *pairs, const oc_observers *obs,
-                                    void *stream) {
+// maps (nullable): Voronoi maps, a frame added right after the density frame before every step whose simu_step is a
+// multiple of maps->every.
+extern "C" int oc_gcfm_run_observed_maps(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y,
+                                         double *d_vx, double *d_vy, double *d_time, uint8_t *d_status,
+                                         const double *d_vdes, const int *d_key, const oc_key *keys, int n_keys,
+                                         uint32_t *mt_key, int *mt_pos, int *has_gauss, double *cached_gauss,
+                                         int n_steps, int simu_step0, int n_active0, double *const *d_rows,
+                                         int *exit_agent, int *exit_step, int *n_exits, int *steps_done,
+                                         double *device_ms, long long *pairs, const oc_observers *obs,
+                                         const oc_vormap_acc *maps, void *stream) {
     const oc_observers none{};
     if (!obs) obs = &none;
     const oc_density_acc *acc = obs->density;
@@ -2524,6 +2527,10 @@ extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int 
         OC_ARG(simu_step0 >= 0 && (long long)simu_step0 + n_steps <= voronoi->capacity,
                "Voronoi measures: step beyond the row capacity");
     }
+    if (maps) {
+        if (int rc = oc_vormap_check(ctx, maps, N)) return rc;
+        OC_ARG(d_vx && d_vy, "NULL argument");
+    }
     constexpr int N_CKPT = 64;
     *n_exits = 0;
     *steps_done = 0;
@@ -2542,6 +2549,10 @@ extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int 
         // ---- this iteration's history frame (simulations.py:428), folded into the statistics
         if (acc && (simu_step0 + k) % acc->every == 0) {
             rc = oc_density_accum_vel(ctx, acc, vel, N, d_x, d_y, d_vx, d_vy, d_status, stream);
+            if (rc) return rc;
+        }
+        if (maps && (simu_step0 + k) % maps->every == 0) {
+            rc = oc_vormap_enqueue(ctx, maps, N, d_x, d_y, d_vx, d_vy, d_status, (cudaStream_t)stream);
             if (rc) return rc;
         }
         if (areas) {
@@ -2603,6 +2614,18 @@ extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int 
         if (rc == OC_ERR_SAMPLER_RANGE) return rc;
     }
     return OC_OK;
+}
+
+extern "C" int oc_gcfm_run_observed(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y,
+                                    double *d_vx, double *d_vy, double *d_time, uint8_t *d_status, const double *d_vdes,
+                                    const int *d_key, const oc_key *keys, int n_keys, uint32_t *mt_key, int *mt_pos,
+                                    int *has_gauss, double *cached_gauss, int n_steps, int simu_step0, int n_active0,
+                                    double *const *d_rows, int *exit_agent, int *exit_step, int *n_exits,
+                                    int *steps_done, double *device_ms, long long *pairs, const oc_observers *obs,
+                                    void *stream) {
+    return oc_gcfm_run_observed_maps(ctx, prm, N, d_x, d_y, d_vx, d_vy, d_time, d_status, d_vdes, d_key, keys, n_keys,
+                                     mt_key, mt_pos, has_gauss, cached_gauss, n_steps, simu_step0, n_active0, d_rows,
+                                     exit_agent, exit_step, n_exits, steps_done, device_ms, pairs, obs, nullptr, stream);
 }
 
 extern "C" int oc_gcfm_run_obs(oc_ctx *ctx, const oc_gcfm_params *prm, int N, double *d_x, double *d_y, double *d_vx,

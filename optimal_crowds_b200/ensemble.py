@@ -33,7 +33,10 @@ i % world, no data-path collective) and, inside a batch, run concurrently on one
     and hands them back in ``results[i]["areas"]`` (tests/test_gpu_areas.py);
   * ``voronoi``: with ``areas``, every member also measures each area's Voronoi density, speed, velocity and covered
     fraction (one batched ``oc_voronoi_measure_multi`` call per step for a wave, next to the areas' call), handed back in
-    ``results[i]["areas"]["voronoi"]`` (tests/test_gpu_voronoi.py).
+    ``results[i]["areas"]["voronoi"]`` (tests/test_gpu_voronoi.py);
+  * ``voronoi_maps``: every member accumulates Voronoi density, speed and velocity maps of its density frames on the
+    device (one batched ``oc_vormap_accum_multi`` call per step for the members due), handed back in
+    ``results[i]["voronoi_maps"]`` (tests/test_gpu_voronoi_maps.py).
 """
 from __future__ import annotations
 
@@ -127,6 +130,9 @@ class ensemble:
     ``voronoi``: None, True or dict(cutoff=1.0, edges=12), as ``simulation(..., voronoi=...)`` takes it (needs ``areas``);
     ``results[i]["areas"]["voronoi"]`` then holds the member's Voronoi measures.
 
+    ``voronoi_maps``: None, True or dict(every=1, cutoff=1.0, edges=12), as ``simulation(..., voronoi_maps=...)`` takes
+    it; ``results[i]["voronoi_maps"]`` is then the member's ``voronoi_maps()`` dict.
+
     ``configs``: None (every member runs config.json) or one dict of overrides per member, merged onto config.json as
     ``simulation(..., config=...)`` merges them (unknown keys raise KeyError).  All members must share ``grid_step``;
     their rooms may differ in size and number of target sets.
@@ -138,7 +144,7 @@ class ensemble:
 
     def __init__(self, rooms, T, seeds, recompute=False, field_storage="phi", chunk_rows=0, rank=0, world=1,
                  memory_budget=None, max_wave=256, record=False, verbose=False, batched_steps=True, configs=None,
-                 density_stats=None, lines=None, areas=None, voronoi=None):
+                 density_stats=None, lines=None, areas=None, voronoi=None, voronoi_maps=None):
         self.chunk_plan_for_wave = chunk_rows == "wave"
         self.T, self.recompute, self.field_storage = T, recompute, field_storage
         self.chunk_rows = 0 if self.chunk_plan_for_wave else int(chunk_rows)
@@ -167,6 +173,7 @@ class ensemble:
         self.voronoi = simulations.voronoi_spec(voronoi)                      # (cutoff, edges) or None
         if self.voronoi is not None and self.areas is None:
             raise ValueError("voronoi needs measurement areas (areas=...)")
+        self.voronoi_maps = simulations.voronoi_maps_spec(voronoi_maps)      # (every, cutoff, edges) or None
         self.rank, self.world = rank, world
         self.mine = shard(len(self.seeds), rank, world)
         self.memory_budget, self.max_wave = memory_budget, max_wave
@@ -195,7 +202,7 @@ class ensemble:
     def member_bytes(self, members=None):
         """device bytes of each member (field_bytes_per_member of its own grid, dt and number of target sets, plus the
         density accumulators when density_stats is on, the line accumulator with lines, the area accumulator with
-        areas and the Voronoi accumulator with voronoi); no CUDA"""
+        areas, the Voronoi accumulator with voronoi and the map accumulators with voronoi_maps); no CUDA"""
         out = []
         for i in (self.mine if members is None else members):
             room, cfg = self._room(i), self.configs[i]
@@ -215,6 +222,10 @@ class ensemble:
                 bins = _lib.voronoi_bins(room["room_length"], cut) * _lib.voronoi_bins(room["room_height"], cut)
                 n_tris = len(simulations.voronoi_triangles(self.areas)[0])
                 b += _lib.VoronoiStats.nbytes(N, len(self.areas[0]), n_tris, edges, bins, steps)
+            if self.voronoi_maps is not None:
+                _, cut, edges = self.voronoi_maps
+                bins = _lib.voronoi_bins(room["room_length"], cut) * _lib.voronoi_bins(room["room_height"], cut)
+                b += _lib.VoronoiMaps.nbytes(Ny, Nx, N, edges, bins)
             out.append(b)
         return out
 
@@ -233,7 +244,7 @@ class ensemble:
                                       density_stats=None if self.density_stats is None else
                                       dict(every=self.density_stats[0], threshold=self.density_stats[1],
                                            velocity=self.density_stats[2]), lines=self._lines_arg,
-                                      areas=self.areas, voronoi=self.voronoi)
+                                      areas=self.areas, voronoi=self.voronoi, voronoi_maps=self.voronoi_maps)
 
     def _build_wave(self, wave):
         """the members of a wave, constructed by a few host threads: a member's crowd placement (oc_place_box: sequential
@@ -379,6 +390,12 @@ class ensemble:
                     if dd:
                         _lib.density_accum_multi([sims[q]._ctx for q in dd], [sims[q]._dstats for q in dd],
                                                  [sims[q]._state for q in dd], stream=main)
+                if self.voronoi_maps is not None:
+                    # the Voronoi map frames of the same members, in one call for all of them
+                    dm = [q for q in live if sims[q]._vmaps.due(sims[q].simu_step)]
+                    if dm:
+                        _lib.vormap_accum_multi([sims[q]._ctx for q in dm], [sims[q]._vmaps for q in dm],
+                                                [sims[q]._state for q in dm], stream=main)
                 if self.areas is not None:
                     # the state this step starts from, measured for the whole wave in one call
                     for q in live:
@@ -437,6 +454,8 @@ class ensemble:
                                    chunk_rows=self.member_chunk_rows[i])
             if self.density_stats is not None:
                 self.results[i]["density"] = s._dstats.result()
+            if self.voronoi_maps is not None:
+                self.results[i]["voronoi_maps"] = s._vmaps.result()
             if self.lines is not None:
                 self.results[i]["lines"] = s._lines.result(s.simu_step)
             if self.areas is not None:

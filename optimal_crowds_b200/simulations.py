@@ -177,13 +177,43 @@ def voronoi_spec(value):
     unknown = set(value) - {"cutoff", "edges"}
     if unknown:
         raise ValueError(f"voronoi: unknown keys {sorted(map(str, unknown))}")
+    return VoronoiSpec(_cutoff_edges(value, "voronoi"))
+
+
+def _cutoff_edges(value, name):
+    """(cutoff, edges) of a dict argument: cutoff finite in (0, 100] metres (default 1.0), edges an integer in 4..32
+    (default 12); ValueError naming the option `name` otherwise"""
     cutoff, edges = value.get("cutoff", 1.0), value.get("edges", 12)
     if isinstance(cutoff, (bool, np.bool_)) or not isinstance(cutoff, (int, float, np.integer, np.floating)) or \
             not (np.isfinite(cutoff) and 0 < cutoff <= 100):
-        raise ValueError("voronoi: cutoff must be a finite number of metres in (0, 100]")
+        raise ValueError(f"{name}: cutoff must be a finite number of metres in (0, 100]")
     if isinstance(edges, (bool, np.bool_)) or not isinstance(edges, (int, np.integer)) or not 4 <= edges <= 32:
-        raise ValueError("voronoi: edges must be an integer in 4..32")
-    return VoronoiSpec((float(cutoff), int(edges)))
+        raise ValueError(f"{name}: edges must be an integer in 4..32")
+    return float(cutoff), int(edges)
+
+
+class VoronoiMapsSpec(tuple):
+    """(every, cutoff, edges): a checked ``voronoi_maps`` argument"""
+
+
+def voronoi_maps_spec(value):
+    """VoronoiMapsSpec (every, cutoff in metres, edges of the cut-off polygon) of a ``voronoi_maps`` argument -- True
+    (every=1, cutoff=1.0, edges=12) or dict(every=..., cutoff=..., edges=...): every an integer >= 1, cutoff and edges
+    as for ``voronoi`` -- or None for None and False; checked without touching a GPU.  A VoronoiMapsSpec is returned as
+    it is"""
+    if value is None or value is False or isinstance(value, VoronoiMapsSpec):
+        return value if value is not False else None
+    if value is True:
+        value = {}
+    if not isinstance(value, dict):
+        raise ValueError("voronoi_maps: expected True or dict(every=1, cutoff=1.0, edges=12)")
+    unknown = set(value) - {"every", "cutoff", "edges"}
+    if unknown:
+        raise ValueError(f"voronoi_maps: unknown keys {sorted(map(str, unknown))}")
+    every = value.get("every", 1)
+    if isinstance(every, (bool, np.bool_)) or not isinstance(every, (int, np.integer)) or every < 1:
+        raise ValueError("voronoi_maps: every must be an integer >= 1")
+    return VoronoiMapsSpec((int(every),) + _cutoff_edges(value, "voronoi_maps"))
 
 
 def _turn(a, b, c):
@@ -374,7 +404,7 @@ class simulation:
 
     def __init__(self, room, T, recompute=False, record=True, field_storage="phi", fused=1, lookahead=True,
                  rng=None, chunk_rows=0, band=False, shard_keys=False, config=None, density_stats=None, lines=None,
-                 areas=None, voronoi=None, _ctx=None):
+                 areas=None, voronoi=None, voronoi_maps=None, _ctx=None):
         """``room, T, recompute`` as in the reference (simulations.py:20).  Extras, all defaulting to reference
         behaviour: ``record`` (keep the per-step record behind ped.traj / ped.vels / history; it lives on the device and
         is read back on access), ``field_storage`` ('phi': the value-function samples, from which ``vx_opt`` /
@@ -402,12 +432,21 @@ class simulation:
         = dict(cutoff=1.0, edges=12), needs ``areas``: measure also, at the start of every step, each area's Voronoi
         density, speed and velocity and the fraction of it the cells cover (Steffen & Seyfried's method D; cells are
         bounded by the room rectangle and a polygon of ``edges`` vertices at ``cutoff`` metres from the agent, not by
-        internal walls); ``area_stats()["voronoi"]`` returns them.  Not available with ``band`` or ``shard_keys``)."""
+        internal walls); ``area_stats()["voronoi"]`` returns them.  Not available with ``band`` or ``shard_keys``),
+        ``voronoi_maps`` (True = dict(every=1, cutoff=1.0, edges=12): accumulate on the device, per grid node and over
+        the frames of ``density_stats`` -- the steps of run()'s loop whose simu_step is a multiple of ``every`` -- the
+        Voronoi density 1/|V| and the speed and velocity of the pedestrian whose Voronoi cell holds the node (cells as
+        for ``voronoi``); read them with ``voronoi_maps()``.  Independent of ``density_stats``, ``areas`` and
+        ``voronoi``.  Not available with ``band`` or ``shard_keys``)."""
         import torch
         dstats = density_stats_spec(density_stats, with_velocity=True)
         lspec = lines_spec(lines)
         aspec = areas_spec(areas)
         vspec = voronoi_spec(voronoi)
+        mspec = voronoi_maps_spec(voronoi_maps)
+        if mspec is not None and (band or shard_keys):
+            raise ValueError("voronoi_maps is not available for row-decomposed (band=True) or key-sharded "
+                             "(shard_keys=True) runs")
         if vspec is not None and (band or shard_keys):
             raise ValueError("voronoi is not available for row-decomposed (band=True) or key-sharded "
                              "(shard_keys=True) runs")
@@ -560,6 +599,8 @@ class simulation:
         # their Voronoi measures (oc_voronoi_measure* / oc_gcfm_run_observed, right after the areas), rows sized alike
         self._voronoi = None if vspec is None else _lib.VoronoiStats(ctx, aspec[1], aspec[2], *voronoi_triangles(aspec),
                                                                      *vspec, N, self._areas.count.shape[0])
+        # Voronoi maps of the run's frames (oc_vormap_accum* / oc_gcfm_run_observed_maps, next to the density frame)
+        self._vmaps = None if mspec is None else _lib.VoronoiMaps(ctx, self._d_Vglobal, mspec[1], mspec[2], mspec[0], N)
         # per-step record of (x, y, vx, vy); row k = state after k steps (ped.traj / ped.vels / history views).  It
         # lives on the DEVICE in blocks of TRACK_CHUNK steps, written by one small kernel per step (oc_state_pack), and
         # is read back -- once per row -- only when somebody looks at it
@@ -733,7 +774,7 @@ class simulation:
                 acc.ensure(self.simu_step + n_steps)
         res = self._ctx.gcfm_run(self._gcfm_prm, self._state, self._d_vdes, self._d_key, self._keys(), st, n_steps,
                                  self.simu_step, n_active, rows=rows, stream=self._cuda_stream, density=self._dstats,
-                                 lines=self._lines, areas=self._areas, voronoi=self._voronoi)
+                                 lines=self._lines, areas=self._areas, voronoi=self._voronoi, maps=self._vmaps)
         self._rng.rng.set_state(res["rng_state"])
         self.last_run_stats = dict(steps=res["steps"], device_ms=res["device_ms"], pairs=res["pairs"])
         ex, exs = res["exits"], res["exit_step"]
@@ -757,11 +798,26 @@ class simulation:
         return res["steps"]
 
     def _density_frame(self):
-        """add this iteration's frame to the density statistics when they are on and it is due (before the step)"""
+        """add this iteration's frame to the density statistics and the Voronoi maps when they are on and it is due
+        (before the step)"""
+        st = self._state
         if self._dstats is not None and self._dstats.due(self.simu_step):
-            st = self._state
             self._ctx.density_accum(self._dstats, st["x"], st["y"], st["status"], stream=self._cuda_stream, vx=st["vx"],
                                     vy=st["vy"])
+        if self._vmaps is not None and self._vmaps.due(self.simu_step):
+            self._ctx.vormap_accum(self._vmaps, st, stream=self._cuda_stream)
+
+    def voronoi_maps(self):
+        """the Voronoi maps of the frames taken so far (``voronoi_maps=`` of the constructor): dict(cutoff, edges, frames,
+        density_sum, density_max, covered, speed_sum, vx_sum, vy_sum, density, speed, velocity) -- (Ny, Nx) numpy
+        arrays (velocity (Ny, Nx, 2)); ``density`` = density_sum / frames is None before the first frame, ``speed`` and
+        ``velocity`` are means over the covered frames, NaN where a node was never covered (include/optimal_crowds.h,
+        oc_vormap_acc)"""
+        if self._vmaps is None:
+            raise RuntimeError("this simulation was created without voronoi_maps")
+        import torch
+        torch.cuda.synchronize(self._ctx.torch_device)
+        return self._vmaps.result()
 
     def density_stats(self):
         """the density statistics of the frames taken so far (``density_stats=`` of the constructor): dict(frames, sum,
